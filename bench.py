@@ -38,6 +38,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 CPU_SAMPLE_PLIES = 2   # the one CPU sample both arms use: `cores` games x 2 plies x `sims` simulations per step
+DUMP_SLOTS = 1024      # game slots whose last EpisodeStep --dump-outputs writes (their dense policies are 16 MB)
 
 
 def load_pkg():
@@ -181,7 +182,7 @@ def run_reference(args, rank, world):
 
     cores = os.cpu_count() or 1
     weights = orc.random_weights(seed=42)
-    warm, steps = args.warmup, max(1, args.steps)   # about 7.5 s of host work per step on 16 threads (20 + 5 steps: 3 minutes)
+    warm, steps = args.warmup, args.steps   # about 7.5 s of host work per step on 16 threads (20 + 5 steps: 3 minutes)
     cpu_shared_sample(weights, args.sims, cores, warm, first_step=0)
     r = cpu_shared_sample(weights, args.sims, cores, steps, first_step=warm)
     value = r["simulations"] / r["seconds"] if r["seconds"] > 0 else 0.0
@@ -427,6 +428,35 @@ def single_game_leg(az, local_rank):
     return {"sims_per_sec": 256 / dt, "ms_per_move": dt * 1e3, "config": "1 game x 256 sims/move through az_search (one evaluation in flight: batch 1)"}
 
 
+def dump_selfplay_outputs(az, eng, stats, G, S, out_dir):
+    """--dump-outputs: what the last timed self-play step handed its caller, as float arrays, so that two builds can be compared
+    output for output.  selfplay_stats holds what that az_selfplay_step call returned (running totals since selfplay_begin), in
+    az_selfplay_stats order.  The other arrays hold, for a fixed
+    seeded sample of game slots, the EpisodeStep that step produced (the last record the slot's game has staged): the searched
+    position's 72 bytes, the policy index played, the search depth, the improved policy and the record's ply and game id.  A slot
+    whose game ended in that step has nothing staged (its game went to the sample queue): ply -1 and zeros mark it."""
+    os.makedirs(out_dir, exist_ok=True)
+    slots = np.sort(np.random.default_rng(0).choice(G, min(G, DUMP_SLOTS), replace=False))
+    n = len(slots)
+    out = {"position": np.zeros((n, az.POSITION_DTYPE.itemsize), np.float32), "action": np.zeros(n, np.float32),
+           "search_depth": np.zeros(n, np.float32), "improved_policy": np.zeros((n, az.ACTION_SPACE), np.float32),
+           "ply": np.full(n, -1.0), "game_id": np.zeros(n)}
+    for k, slot in enumerate(slots):
+        staged = eng.selfplay_staged(int(slot))
+        if len(staged) == 0:
+            continue
+        rec = staged[np.argmax(staged["ply"])]
+        out["position"][k] = np.frombuffer(rec["position"].tobytes(), np.uint8)
+        out["action"][k] = rec["action"]
+        out["search_depth"][k] = rec["search_depth"]
+        out["improved_policy"][k] = az.improved_policy(rec, S)
+        out["ply"][k] = rec["ply"]
+        out["game_id"][k] = rec["game_id"]
+    out["selfplay_stats"] = np.array([getattr(stats, f) for f, _ in az.SelfplayStats._fields_], np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------ the GPU arm
 def run_ours(args, rank, world, local_rank):
     import torch
@@ -487,6 +517,8 @@ def run_ours(args, rank, world, local_rank):
     eng.profile_enable(0)
     d = {k: getattr(st1, k) - getattr(st0, k) for k in ("simulations", "positions", "evaluations", "terminal_leaves", "games_finished",
                                                        "sum_leaf_depth", "sum_edges", "cache_hits")}
+    if args.dump_outputs and rank == 0:
+        dump_selfplay_outputs(az, eng, st1, G, S, args.dump_outputs)
     eng.selfplay_drain()
 
     # ---- end to end through the reference-facing call: MCTree::init + monte_carlo_tree_search for G host-resident roots
@@ -703,7 +735,13 @@ def main():
     ap.add_argument("--cache-log2", type=int, default=0, help="log2 slots of the GPU evaluation cache (0 = off)")
     ap.add_argument("--min-replay", type=int, default=20_000, help="generation mode: MIN_REPLAY_SIZE (parameters.rs:11)")
     ap.add_argument("--slots", type=int, default=0, help="generation mode: concurrent games per GPU (0 = all games of the generation at once, like the reference's NUM_EPISODES tasks)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="selfplay mode: after the timed steps write what the last one computed (rank 0's games) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.mode != "selfplay" or args.impl != "ours"):
+        ap.error("--dump-outputs writes the GPU self-play path's outputs: it needs --mode selfplay --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
