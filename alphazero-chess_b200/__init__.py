@@ -51,6 +51,12 @@ class SelfplayStats(ctypes.Structure):
                                                "active_games", "parked_games", "cache_evictions", "sum_search_depth")]
 
 
+class SearchStats(ctypes.Structure):
+    """az_search_stats of az_search_vl."""
+
+    _fields_ = [(n, ctypes.c_uint64) for n in ("waves", "evaluations", "terminal_leaves", "collisions")]
+
+
 class EngineError(RuntimeError):
     pass
 
@@ -293,6 +299,26 @@ class Engine:
         self._check(self._L.az_search(self._h, n, _ptr(p), _ptr(h), _ptr(ho), sims, _ptr(ids), _ptr(pl), _ptr(visits), _ptr(scores),
                                       _ptr(depth)), "az_search")
         return visits, scores, depth
+
+    def search_vl(self, roots, num_simulations, leaves_per_root, virtual_loss=1.0, history=None, hist_offsets=None,
+                  noise_game_ids=None, noise_plies=None, want_scores=False):
+        """Leaf-parallel search with virtual loss (az_search_vl; not in the reference, identical to search() at
+        leaves_per_root = 1): up to leaves_per_root leaves per root share one network round.
+        Returns (visits [n,4096], scores or None, depth [n], SearchStats)."""
+        p = self._positions(roots)
+        n = p.shape[0]
+        visits = np.empty((n, ACTION_SPACE), np.float32)
+        scores = np.empty((n, ACTION_SPACE), np.float32) if want_scores else None
+        depth = np.empty(n, np.int32)
+        h = self._positions(history) if history is not None else None
+        ho = np.ascontiguousarray(hist_offsets, np.uint32) if hist_offsets is not None else None
+        ids = np.ascontiguousarray(noise_game_ids, np.uint64) if noise_game_ids is not None else None
+        pl = np.ascontiguousarray(noise_plies, np.uint32) if noise_plies is not None else None
+        st = SearchStats()
+        self._check(self._L.az_search_vl(self._h, n, _ptr(p), _ptr(h), _ptr(ho), int(num_simulations), int(leaves_per_root),
+                                         ctypes.c_float(virtual_loss), _ptr(ids), _ptr(pl), _ptr(visits), _ptr(scores), _ptr(depth),
+                                         ctypes.byref(st)), "az_search_vl")
+        return visits, scores, depth, st
 
     # ---- training.rs ------------------------------------------------------------------------------------------
     def selfplay_begin(self, n_games, first_game_id=0, total_games=0):

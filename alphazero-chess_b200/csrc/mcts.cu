@@ -14,6 +14,7 @@
 #include <cstdio>
 #include <cstring>
 #include <algorithm>
+#include <cmath>
 
 namespace azb {
 
@@ -144,8 +145,9 @@ __device__ __forceinline__ void lane0_make_child(Ctx& x, const DPos& parent, uin
 
 // chess.rs:52-60: pos_count[child] (this occurrence included) reaches REPETITIONS, or a move counter hits its limit.
 // Candidates are the positions with the same side to move since the last irreversible move: they live on the
-// search path (depth >= 1) or in the game history.  `depth_child` = edges from the root to the child.
-__device__ __forceinline__ bool draw_by_rules(Ctx& x, const DPos& child, int depth_child) {
+// search path (depth >= 1) or in the game history.  `depth_child` = edges from the root to the child, `path` = the
+// descent that reached it (entries as in SearchPtrs::path).
+__device__ __forceinline__ bool draw_by_rules(Ctx& x, const uint2* path, const DPos& child, int depth_child) {
     const int hm = meta_halfmoves(child.meta);
     if (hm >= x.prm.num_halfmoves || meta_fullmoves(child.meta) >= x.prm.num_fullmoves) return true;
     const int root_v = (int)x.c.hist_len - 1;          // virtual index of the root
@@ -158,7 +160,7 @@ __device__ __forceinline__ bool draw_by_rules(Ctx& x, const DPos& child, int dep
         const int j = v - 2 * k;
         if (k <= n_cand && j >= 0) {
             const DPos* q;
-            if (j > root_v) q = &x.ptr.node_pos[x.nbase + (x.ptr.path[(size_t)x.g * x.prm.node_cap + (j - root_v)].x & 0xFFFF)];
+            if (j > root_v) q = &x.ptr.node_pos[x.nbase + (path[j - root_v].x & 0xFFFF)];
             else q = &x.ptr.hist[(size_t)x.g * HIST_CAP + j];
             eq = same_position_key(*q, child);
         }
@@ -595,7 +597,7 @@ __device__ void move_step(Ctx& x) {
     const int child_node = child_link == EDGE_NO_CHILD ? -1 : (int)(child_link & 0xFFFF);
     lane0_make_child(x, root, (uint16_t)(amv & 0xFFFF));
     int term = x.sh->term;
-    if (term == 0 && draw_by_rules(x, x.sh->child, 1)) term = 1;
+    if (term == 0 && draw_by_rules(x, x.ptr.path + (size_t)x.g * x.prm.node_cap, x.sh->child, 1)) term = 1;
     if (term == 0) {
         // traverse_new (tree.rs:239-256): keep the child's priors, drop everything else, fresh noise
         float keepP[7];
@@ -728,7 +730,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB * 4 / WARPS) k_advance(const 
         lane0_make_child(x, parent, (uint16_t)(leaf_mv & 0xFFFF));
         int term = x.sh->term;
         ADV_T(2);
-        if (term == 0 && draw_by_rules(x, x.sh->child, depth + 1)) term = 1;
+        if (term == 0 && draw_by_rules(x, ptr.path + (size_t)g * prm.node_cap, x.sh->child, depth + 1)) term = 1;
         ADV_T(3);
         if (x.lane == 0) x.st_depth += depth + 1;
         if (term != 0) {
@@ -917,6 +919,208 @@ __global__ void k_count_active(SearchParams prm, SearchPtrs ptr, int* out) {
     }
 }
 
+// ------------------------------------------------------------------------------------------- leaf-parallel search (az_search_vl)
+// Not in the reference: each root gathers up to K leaves per network round, steering later descents away from the paths
+// already taken with a virtual loss (semantics in DESIGN.md section 5).  A wave is k_vl_gather (one warp per root: back up the
+// previous batch in leaf order, then descend K times), k_vl_expand (one warp per leaf) and the network.  With K = 1 every
+// in-flight count is 0 at every selection and the results are those of az_search.
+struct VLPtrs {
+    uint32_t* V;          // [G * edge_cap] descents of the current batch through each edge (0 between batches)
+    uint2* path;          // [max_batch][node_cap] the descent of leaf g * K + k, entries as in SearchPtrs::path
+    int* len;             // [max_batch] edges on that descent
+    int* slot;            // [max_batch] request slot of the leaf's evaluation, or -1: terminal, its value is in `value`
+    float* value;         // [max_batch]
+    int* count;           // [G] leaves of the root's current batch
+    unsigned long long* stats;  // [4] leaves gathered, terminal leaves, collisions
+    int K;
+    float lambda;
+};
+
+// One descent of the gather: PUCT on N' = N + V and W' = W - lambda * V.  `total` is the root's N' (sims done + leaves
+// gathered so far + 1).  Writes path[0..depth] and returns the depth of the leaf edge, or -1 when the chosen edge has no child
+// but another descent of this batch already ends there (a collision).
+__device__ __forceinline__ int vl_descend(Ctx& x, const VLPtrs& vl, uint2* path, float total) {
+    int node = 0, depth = 0;
+    uint32_t eoff = 0;
+    int L = (int)((x.c.flags >> 8) & 0xFF);
+    for (;;) {
+        const size_t off = x.ebase + eoff;
+        const float sq = __fsqrt_rn(total);
+        float best = -INFINITY;
+        int best_e = 0x7FFFFFFF;
+        u64 my_k = EDGE_NO_CHILD;
+        float my_n = 0.0f;
+        uint32_t my_v = 0;
+        for (int e = x.lane; e < L; e += 32) {
+            const float P = x.ptr.edge_P[off + e], N = x.ptr.edge_N[off + e], W = x.ptr.edge_W[off + e];
+            const u64 K = x.ptr.edge_link[off + e];
+            const uint32_t V = vl.V[off + e];
+            const float fv = __uint2float_rn(V);
+            const float n = __fadd_rn(N, fv);
+            const float w = __fsub_rn(W, __fmul_rn(vl.lambda, fv));
+            const float u = __fdiv_rn(__fmul_rn(__fmul_rn(x.prm.c_puct, P), sq), __fadd_rn(1.0f, n));
+            const float q = n > 0.0f ? __fdiv_rn(w, n) : 0.0f;
+            const float v = __fadd_rn(q, u);
+            if (v > best) { best = v; best_e = e; my_k = K; my_n = n; my_v = V; }
+            else if (e == x.lane) { my_k = K; my_n = n; my_v = V; }   // lane 0 holds edge 0 for the NaN fallback
+        }
+        for (int d = 16; d; d >>= 1) {
+            const float ov = __shfl_xor_sync(0xffffffffu, best, d);
+            const int oe = __shfl_xor_sync(0xffffffffu, best_e, d);
+            if (ov > best || (ov == best && oe < best_e)) { best = ov; best_e = oe; }
+        }
+        if (best_e == 0x7FFFFFFF) best_e = 0;
+        const int owner = best_e & 31;
+        const u64 best_k = shfl_u64(my_k, owner);
+        const float best_n = __shfl_sync(0xffffffffu, my_n, owner);
+        const uint32_t best_v = __shfl_sync(0xffffffffu, my_v, owner);
+        if (x.lane == 0) path[depth] = make_uint2((uint32_t)node | ((uint32_t)best_e << 16), eoff + (uint32_t)best_e);
+        if (best_k == EDGE_NO_CHILD) {
+            __syncwarp();
+            return best_v > 0 ? -1 : depth;
+        }
+        node = (int)(best_k & 0xFFFF);
+        L = (int)((best_k >> 16) & 0xFF);
+        eoff = (uint32_t)(best_k >> 24);
+        total = best_n;
+        depth++;
+    }
+}
+
+// one warp per root: consume the previous batch (the root's own evaluation on the first wave), then gather the next one
+__global__ void __launch_bounds__(WARPS * 32) k_vl_gather(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
+                                                          const __grid_constant__ VLPtrs vl) {
+    __shared__ WarpShared shared[WARPS];
+    const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (g == 0 && (threadIdx.x & 31) == 0) *ptr.batch_count = 0;   // requests of this wave are counted by k_vl_expand, which runs next
+    if (g >= prm.n_games) return;
+    Ctx x{prm, ptr, &shared[threadIdx.x >> 5], g, (int)(threadIdx.x & 31), (size_t)g * prm.node_cap, (size_t)g * prm.edge_cap,
+          ptr.ctl[g], 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    if (x.c.status != 0) return;
+    // ---- 1. the evaluations of the previous wave have arrived
+    if (x.c.pending_node == 0) {   // MCTree::init: root priors, optional noise
+        const int L = ptr.node_nedges[x.nbase];
+        if (!prm.priors_scattered) {
+            const float* pol = ptr.res_policy + (size_t)x.c.pending_slot * AZ_ACTION_SPACE;
+            for (int e = x.lane; e < L; e += 32) ptr.edge_P[x.ebase + e] = pol[ptr.edge_mv[x.ebase + e] >> 16];
+        }
+        for (int e = x.lane; e < L; e += 32) vl.V[x.ebase + e] = 0;
+        __syncwarp();
+        if (x.c.flags & 1) apply_noise(x, 0, x.c.game_id, x.c.noise_ply);
+        x.c.pending_node = -1;
+    } else {
+        // backups in leaf order: the f32 additions on a shared edge happen in a fixed order
+        const int nl = vl.count[g];
+        for (int k = 0; k < nl; k++) {
+            const int leaf = g * vl.K + k;
+            const int s = vl.slot[leaf];
+            float value;
+            if (s >= 0) {
+                if (!prm.priors_scattered) {
+                    const size_t off = ptr.req_edge_off[s];
+                    const int L = ptr.req_nedges[s];
+                    const float* pol = ptr.res_policy + (size_t)s * AZ_ACTION_SPACE;
+                    for (int e = x.lane; e < L; e += 32) ptr.edge_P[off + e] = pol[ptr.edge_mv[off + e] >> 16];
+                }
+                value = ptr.res_value[s];
+            } else {
+                value = vl.value[leaf];
+            }
+            const int len = vl.len[leaf];
+            const uint2* path = vl.path + (size_t)leaf * prm.node_cap;
+            for (int i = x.lane; i < len; i += 32) {
+                const size_t e = x.ebase + path[i].y;
+                const float v = ((len - 1 - i) & 1) ? value : -value;
+                ptr.edge_W[e] = __fadd_rn(ptr.edge_W[e], v);
+                ptr.edge_N[e] = __fadd_rn(ptr.edge_N[e], 1.0f);
+                vl.V[e] -= 1;
+            }
+            __syncwarp();
+        }
+        x.c.sims_done += nl;
+    }
+    // ---- 2. gather the next batch
+    int n_leaf = 0, collided = 0;
+    if ((int)x.c.sims_done >= prm.S) {
+        x.c.status = 1;
+    } else {
+        const int kb = min(vl.K, prm.S - (int)x.c.sims_done);
+        for (int k = 0; k < kb; k++) {
+            const int leaf = g * vl.K + k;
+            uint2* path = vl.path + (size_t)leaf * prm.node_cap;
+            const int depth = vl_descend(x, vl, path, __fadd_rn((float)(x.c.sims_done + k), 1.0f));
+            if (depth < 0) { collided = 1; break; }
+            for (int i = x.lane; i <= depth; i += 32) vl.V[x.ebase + path[i].y] += 1;
+            if (x.lane == 0) vl.len[leaf] = depth + 1;
+            __syncwarp();
+            n_leaf++;
+        }
+    }
+    if (x.lane == 0) {
+        vl.count[g] = n_leaf;
+        if (n_leaf) atomicAdd(&vl.stats[0], (unsigned long long)n_leaf);
+        if (collided) atomicAdd(&vl.stats[2], 1ULL);
+        ptr.ctl[g] = x.c;
+    }
+}
+
+// one warp per gathered leaf (g * K + k): tree.rs expand; the new node is linked to the leaf edge and queued for evaluation
+__global__ void __launch_bounds__(WARPS * 32) k_vl_expand(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
+                                                          const __grid_constant__ VLPtrs vl) {
+    __shared__ WarpShared shared[WARPS];
+    const int leaf = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int g = leaf / vl.K;
+    if (g >= prm.n_games || leaf - g * vl.K >= vl.count[g] || ptr.ctl[g].status != 0) return;
+    GameCtl c;
+    memset(&c, 0, sizeof c);
+    c.hist_len = ptr.ctl[g].hist_len;
+    Ctx x{prm, ptr, &shared[threadIdx.x >> 5], g, (int)(threadIdx.x & 31), (size_t)g * prm.node_cap, (size_t)g * prm.edge_cap, c,
+          0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    const uint2* path = vl.path + (size_t)leaf * prm.node_cap;
+    const int len = vl.len[leaf];
+    const uint2 last = path[len - 1];
+    const size_t pe = x.ebase + last.y;
+    const DPos parent = ptr.node_pos[x.nbase + (last.x & 0xFFFF)];
+    lane0_make_child(x, parent, (uint16_t)(ptr.edge_mv[pe] & 0xFFFF));
+    int term = x.sh->term;
+    if (term == 0 && draw_by_rules(x, path, x.sh->child, len)) term = 1;
+    if (term != 0) {   // draw -> 0, decisive -> -1 from the child's side (tree.rs:233-234); nothing is stored
+        if (x.lane == 0) {
+            vl.slot[leaf] = -1;
+            vl.value[leaf] = term == 1 ? 0.0f : -1.0f;
+            atomicAdd(&vl.stats[1], 1ULL);
+        }
+        return;
+    }
+    // the node id and the edge range come from the game's counters, shared by the expansions of this wave
+    const int n = x.sh->n_moves;
+    int L = 0;
+    for (int i0 = 0; i0 < n; i0 += 32) {
+        const int i = i0 + x.lane;
+        bool keep = false;
+        if (i < n) { const int pr = (x.sh->moves[i] >> 12) & 7; keep = pr == 0 || pr == 4; }
+        L += __popc(__ballot_sync(0xffffffffu, keep));
+    }
+    uint32_t node = 0, eoff = 0;
+    if (x.lane == 0) { node = atomicAdd(&ptr.ctl[g].n_nodes, 1u); eoff = atomicAdd(&ptr.ctl[g].n_edges, (uint32_t)L); }
+    node = __shfl_sync(0xffffffffu, node, 0);
+    eoff = __shfl_sync(0xffffffffu, eoff, 0);
+    x.c.n_nodes = node;
+    x.c.n_edges = eoff;
+    const int child = create_node(x, len);
+    if (child < 0) {
+        if (x.lane == 0) { ptr.ctl[g].status = 2; atomicAdd(&ptr.counters->errors, 1ULL); }
+        return;
+    }
+    for (int e = x.lane; e < L; e += 32) vl.V[x.ebase + eoff + e] = 0;
+    if (x.lane == 0) {
+        ptr.edge_link[pe] = x.new_link;
+        atomicMax(&ptr.ctl[g].max_depth, (uint32_t)len);
+    }
+    const int slot = submit_request(x, child);
+    if (x.lane == 0) vl.slot[leaf] = slot;
+}
+
 // ------------------------------------------------------------------------------------------- host side
 template <class T>
 static int salloc(az_engine* e, SearchState* st, T** p, size_t n) {
@@ -1035,6 +1239,15 @@ int search_clear_pending(az_engine* e) {
     return 0;
 }
 
+// az_profile: when the coming forward will be sampled, the search kernels launched from here on are timed up to its start
+static void prof_mark_search(az_engine* e) {
+    if (e->prof_every > 0 && e->stub_kind == 0 && e->cfg.precision != 1 && (e->prof_counter % (uint64_t)e->prof_every) == 0 &&
+        !e->prof_adv_event) {
+        cudaEventCreate(&e->prof_adv_event);
+        cudaEventRecord(e->prof_adv_event, e->stream);
+    }
+}
+
 static int run_wave(az_engine* e, SearchState* st) {
     const int blocks = (st->prm.n_games + WARPS - 1) / WARPS;
     st->prm.priors_scattered = (e->stub_kind == 0 && e->cfg.precision != 1) ? 1 : 0;
@@ -1044,11 +1257,7 @@ static int run_wave(az_engine* e, SearchState* st) {
     st->batch_parity ^= 1;
     st->ptr.batch_count = st->batch_base + st->batch_parity;
     st->ptr.batch_zero = st->batch_base + (st->batch_parity ^ 1);
-    if (e->prof_every > 0 && e->stub_kind == 0 && e->cfg.precision != 1 && (e->prof_counter % (uint64_t)e->prof_every) == 0 &&
-        !e->prof_adv_event) {
-        cudaEventCreate(&e->prof_adv_event);
-        cudaEventRecord(e->prof_adv_event, e->stream);
-    }
+    prof_mark_search(e);
     // AZ_ADV_PASSES > 1 (experiment, default 1): extra k_advance passes per wave in which only the games that completed their
     // max_iters network-free simulations without needing the network go on.  Measured at 14 % / 45 % / 63 % cache hits
     // (profiles/r2_passes_raw.jsonl): always slower -- the fuller batch costs tower time in proportion, and more simulations
@@ -1074,26 +1283,15 @@ static int run_wave(az_engine* e, SearchState* st) {
     return evaluate_batch(e, st);
 }
 
-}  // namespace azb
-
-using namespace azb;
-
-extern "C" {
-
-int az_set_evaluator_stub(az_engine* e, int kind, uint64_t seed) {
-    if (!e || kind < 0 || kind > 1) return AZ_ERR_INVALID_ARGUMENT;
-    e->stub_kind = kind;
-    e->stub_seed = seed;
-    return AZ_OK;
-}
-
-int az_search(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
-              int num_simulations, const uint64_t* noise_game_ids, const uint32_t* noise_plies, float* visits_out, float* scores_out,
-              int32_t* depth_out) {
-    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+// Input staging of az_search and az_search_vl (MCTree::init for n roots): validates the arguments, copies roots, history and
+// noise keys to the device, creates every root (k_init_search) and evaluates the roots.  `run` becomes the call's copy of the
+// search state.  Returns AZ_OK, an error, or 1 when there is nothing to do (n == 0).
+static int search_begin(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
+                        int num_simulations, const uint64_t* noise_game_ids, const uint32_t* noise_plies, const float* visits_out,
+                        SearchState& run) {
     SearchState* st = e->search;
     if (n < 0 || n > st->G) return set_err(e, AZ_ERR_CAPACITY, "more roots than az_config.max_games");
-    if (n == 0) return AZ_OK;
+    if (n == 0) return 1;
     if (!roots || !visits_out) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "null buffer");
     if (num_simulations <= 0 || num_simulations + 2 > st->prm.node_cap)
         return set_err(e, AZ_ERR_CAPACITY, "num_simulations exceeds az_config.num_simulations (pool size)");
@@ -1102,7 +1300,7 @@ int az_search(az_engine* e, int n, const az_position* roots, const az_position* 
     st->selfplay_active = false;
     SearchParams prm = st->prm;
     prm.n_games = n; prm.S = num_simulations; prm.mode = 0;
-    SearchState run = *st;
+    run = *st;
     run.prm = prm;
     // stage inputs
     AZ_CUDA(e, cudaMemcpyAsync(e->d_wire, roots, (size_t)n * sizeof(az_position), cudaMemcpyHostToDevice, e->stream));
@@ -1145,38 +1343,138 @@ int az_search(az_engine* e, int n, const az_position* roots, const az_position* 
     e->n_launches++;
     k_init_search<<<blocks, WARPS * 32, 0, e->stream>>>(run.prm, run.ptr, e->d_wire, d_hist, e->d_hist_off, d_ids, d_plies);
     AZ_CUDA(e, cudaGetLastError());
-    int r = evaluate_batch(e, &run);
-    if (r) return r;
-    // every wave completes at least one simulation per active game
+    return evaluate_batch(e, &run);
+}
+
+// dense export of the roots' statistics (Box<[f32; 4096]> visits / scores, max_subtree_depth) to the caller's buffers
+static int search_export(az_engine* e, const SearchState& run, int n, float* visits_out, float* scores_out, int32_t* depth_out) {
+    float* d_vis = e->d_policy;  // reuse the result buffers for the dense export
+    float* d_sc = nullptr;
+    if (scores_out) {
+        if (!e->d_scores) AZ_CUDA(e, cudaMalloc(&e->d_scores, (size_t)e->max_batch * AZ_ACTION_SPACE * 4));
+        d_sc = e->d_scores;
+    }
+    k_export_root<<<n, 256, 0, e->stream>>>(run.prm, run.ptr, d_vis, d_sc, e->d_count);
+    AZ_CUDA(e, cudaGetLastError());
+    AZ_CUDA(e, cudaMemcpyAsync(visits_out, d_vis, (size_t)n * AZ_ACTION_SPACE * 4, cudaMemcpyDeviceToHost, e->stream));
+    if (scores_out) AZ_CUDA(e, cudaMemcpyAsync(scores_out, d_sc, (size_t)n * AZ_ACTION_SPACE * 4, cudaMemcpyDeviceToHost, e->stream));
+    if (depth_out) AZ_CUDA(e, cudaMemcpyAsync(depth_out, e->d_count, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+    AZ_CUDA(e, cudaStreamSynchronize(e->stream));
+    return AZ_OK;
+}
+
+// k_count_active over the call's roots: flags[0] active, flags[1] failed (pool overflow or illegal state)
+static int search_poll(az_engine* e, const SearchState& run, int n, int flags[4]) {
     int* d_flags = run.batch_base + 4;
+    AZ_CUDA(e, cudaMemsetAsync(d_flags, 0, 16, e->stream));
+    k_count_active<<<(n + 127) / 128, 128, 0, e->stream>>>(run.prm, run.ptr, d_flags);
+    AZ_CUDA(e, cudaMemcpyAsync(flags, d_flags, 16, cudaMemcpyDeviceToHost, e->stream));
+    AZ_CUDA(e, cudaStreamSynchronize(e->stream));
+    return AZ_OK;
+}
+
+}  // namespace azb
+
+using namespace azb;
+
+extern "C" {
+
+int az_set_evaluator_stub(az_engine* e, int kind, uint64_t seed) {
+    if (!e || kind < 0 || kind > 1) return AZ_ERR_INVALID_ARGUMENT;
+    e->stub_kind = kind;
+    e->stub_seed = seed;
+    return AZ_OK;
+}
+
+int az_search(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
+              int num_simulations, const uint64_t* noise_game_ids, const uint32_t* noise_plies, float* visits_out, float* scores_out,
+              int32_t* depth_out) {
+    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+    SearchState run;
+    int r = search_begin(e, n, roots, history, hist_offsets, num_simulations, noise_game_ids, noise_plies, visits_out, run);
+    if (r) return r == 1 ? AZ_OK : r;
+    // every wave completes at least one simulation per active game
     int rc = AZ_OK;
     for (int wave = 0;; wave++) {
         r = run_wave(e, &run);
         if (r) { rc = r; break; }
         if (wave + 1 >= num_simulations && (wave + 1 - num_simulations) % 4 == 0) {
             int flags[4] = {0, 0, 0, 0};
-            AZ_CUDA(e, cudaMemsetAsync(d_flags, 0, 16, e->stream));
-            k_count_active<<<(n + 127) / 128, 128, 0, e->stream>>>(run.prm, run.ptr, d_flags);
-            AZ_CUDA(e, cudaMemcpyAsync(flags, d_flags, 16, cudaMemcpyDeviceToHost, e->stream));
-            AZ_CUDA(e, cudaStreamSynchronize(e->stream));
+            r = search_poll(e, run, n, flags);
+            if (r) return r;
             if (flags[1]) { rc = set_err(e, AZ_ERR_CAPACITY, "a per-game node/edge pool overflowed (raise edge_capacity_per_node)"); break; }
             if (flags[0] == 0) break;
             if (wave > 4 * num_simulations + 16) { rc = set_err(e, AZ_ERR_STATE, "search did not converge"); break; }
         }
     }
-    if (rc == AZ_OK) {
-        float* d_vis = e->d_policy;  // reuse the result buffers for the dense export
-        float* d_sc = nullptr;
-        if (scores_out) {
-            if (!e->d_scores) AZ_CUDA(e, cudaMalloc(&e->d_scores, (size_t)e->max_batch * AZ_ACTION_SPACE * 4));
-            d_sc = e->d_scores;
-        }
-        k_export_root<<<n, 256, 0, e->stream>>>(run.prm, run.ptr, d_vis, d_sc, e->d_count);
+    if (rc == AZ_OK) rc = search_export(e, run, n, visits_out, scores_out, depth_out);
+    return rc;
+}
+
+int az_search_vl(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
+                 int num_simulations, int leaves_per_root, float virtual_loss, const uint64_t* noise_game_ids, const uint32_t* noise_plies,
+                 float* visits_out, float* scores_out, int32_t* depth_out, az_search_stats* stats_out) {
+    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+    if (stats_out) std::memset(stats_out, 0, sizeof *stats_out);
+    if (leaves_per_root < 1) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "leaves_per_root must be >= 1");
+    if (!(virtual_loss >= 0.0f) || !std::isfinite(virtual_loss))
+        return set_err(e, AZ_ERR_INVALID_ARGUMENT, "virtual_loss must be finite and >= 0");
+    if (n > 0 && (long long)n * leaves_per_root > (long long)e->max_batch)
+        return set_err(e, AZ_ERR_CAPACITY, "roots x leaves_per_root exceeds az_config.max_batch");
+    SearchState* st = e->search;
+    if (n >= 0 && n <= st->G && !st->vl_V) {   // first call: the in-flight counts and the per-leaf records
+        cudaSetDevice(e->cfg.device);
+        const size_t NE = (size_t)st->G * st->prm.edge_cap, B = (size_t)e->max_batch;
+        int a = salloc(e, st, &st->vl_V, NE);
+        a |= salloc(e, st, &st->vl_path, B * st->prm.node_cap);
+        a |= salloc(e, st, &st->vl_len, B); a |= salloc(e, st, &st->vl_slot, B); a |= salloc(e, st, &st->vl_value, B);
+        a |= salloc(e, st, &st->vl_count, (size_t)st->G); a |= salloc(e, st, &st->vl_stats, 4);
+        if (a) return AZ_ERR_OUT_OF_MEMORY;
+    }
+    SearchState run;
+    int r = search_begin(e, n, roots, history, hist_offsets, num_simulations, noise_game_ids, noise_plies, visits_out, run);
+    if (r) return r == 1 ? AZ_OK : r;
+    const int K = leaves_per_root;
+    VLPtrs vl{st->vl_V, st->vl_path, st->vl_len, st->vl_slot, st->vl_value, st->vl_count, st->vl_stats, K, virtual_loss};
+    AZ_CUDA(e, cudaMemsetAsync(vl.count, 0, (size_t)n * sizeof(int), e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(vl.stats, 0, 4 * sizeof(unsigned long long), e->stream));
+    run.prm.priors_scattered = (e->stub_kind == 0 && e->cfg.precision != 1) ? 1 : 0;
+    uint64_t waves = 1;   // the roots' evaluation
+    // a batch adds at least one leaf per active root, so every root is done after at most S batches; the first poll comes
+    // after the earliest wave at which the last batch can have been consumed
+    const int first_poll = (num_simulations + K - 1) / K;
+    int rc = AZ_OK;
+    for (int wave = 0;; wave++) {
+        prof_mark_search(e);
+        e->n_launches += 2;
+        k_vl_gather<<<(n + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(run.prm, run.ptr, vl);
         AZ_CUDA(e, cudaGetLastError());
-        AZ_CUDA(e, cudaMemcpyAsync(visits_out, d_vis, (size_t)n * AZ_ACTION_SPACE * 4, cudaMemcpyDeviceToHost, e->stream));
-        if (scores_out) AZ_CUDA(e, cudaMemcpyAsync(scores_out, d_sc, (size_t)n * AZ_ACTION_SPACE * 4, cudaMemcpyDeviceToHost, e->stream));
-        if (depth_out) AZ_CUDA(e, cudaMemcpyAsync(depth_out, e->d_count, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-        AZ_CUDA(e, cudaStreamSynchronize(e->stream));
+        if (wave >= first_poll) {
+            int flags[4] = {0, 0, 0, 0};
+            r = search_poll(e, run, n, flags);
+            if (r) return r;
+            if (flags[1]) { rc = set_err(e, AZ_ERR_CAPACITY, "a per-game node/edge pool overflowed (raise edge_capacity_per_node)"); break; }
+            if (flags[0] == 0) break;
+            if (wave > num_simulations + 16) { rc = set_err(e, AZ_ERR_STATE, "search did not converge"); break; }
+        }
+        k_vl_expand<<<(n * K + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(run.prm, run.ptr, vl);
+        AZ_CUDA(e, cudaGetLastError());
+        r = evaluate_batch(e, &run);
+        if (r) return r;
+        waves++;
+    }
+    if (e->prof_adv_event) {   // the last gather is followed by no forward: its mark must not time the next call's kernels
+        cudaEventDestroy(e->prof_adv_event);
+        e->prof_adv_event = nullptr;
+    }
+    if (rc == AZ_OK) rc = search_export(e, run, n, visits_out, scores_out, depth_out);
+    if (rc == AZ_OK && stats_out) {
+        unsigned long long s[4];
+        AZ_CUDA(e, cudaMemcpy(s, vl.stats, sizeof s, cudaMemcpyDeviceToHost));
+        stats_out->waves = waves;
+        stats_out->evaluations = (uint64_t)n + s[0] - s[1];   // the roots, then every leaf that was not terminal
+        stats_out->terminal_leaves = s[1];
+        stats_out->collisions = s[2];
     }
     return rc;
 }

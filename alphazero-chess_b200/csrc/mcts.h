@@ -128,6 +128,14 @@ struct SearchState {
     unsigned long long wave_counter = 0;   // self-play waves since az_selfplay_begin (cache epoch = wave_counter / S)
     unsigned long long* d_noise_ids = nullptr;  // [max_games] az_search staging (no allocation per call)
     uint32_t* d_noise_plies = nullptr;
+    // az_search_vl, allocated on its first call (az_engine_create's footprint does not include them)
+    uint32_t* vl_V = nullptr;              // [G * edge_cap] descents of the current batch through each edge
+    uint2* vl_path = nullptr;              // [max_batch][node_cap] one descent per leaf
+    int* vl_len = nullptr;                 // [max_batch]
+    int* vl_slot = nullptr;                // [max_batch]
+    float* vl_value = nullptr;             // [max_batch]
+    int* vl_count = nullptr;               // [G]
+    unsigned long long* vl_stats = nullptr; // [4]
     std::vector<void*> allocs;
 };
 

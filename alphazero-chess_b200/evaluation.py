@@ -42,16 +42,24 @@ def _weighted_index(weights, u):
 
 
 class MctsPlayer:
-    """Player::MctsModel: MCTree::init(model, state, false) + search, then argmax or sampling (validation.rs:293-308)."""
+    """Player::MctsModel: MCTree::init(model, state, false) + search, then argmax or sampling (validation.rs:293-308).
+    leaves_per_root > 1 searches with virtual loss (Engine.search_vl, not in the reference): up to that many leaves per
+    root share one network round, which cuts the latency of searches over few roots."""
 
-    def __init__(self, engine, num_simulations=None):
+    def __init__(self, engine, num_simulations=None, leaves_per_root=1, virtual_loss=1.0):
         self.engine, self.sims = engine, num_simulations
+        self.leaves_per_root, self.virtual_loss = int(leaves_per_root), float(virtual_loss)
 
     def choose(self, positions, histories, fullmoves, stochastic, seed, game_ids, plies):
         hist = np.concatenate(histories)
         offs = np.zeros(len(histories) + 1, np.uint32)
         offs[1:] = np.cumsum([len(h) for h in histories])
-        visits, _, _ = self.engine.search(positions, num_simulations=self.sims, history=hist, hist_offsets=offs)
+        if self.leaves_per_root > 1:
+            sims = int(self.sims or self.engine.config.num_simulations)
+            visits, _, _, _ = self.engine.search_vl(positions, sims, self.leaves_per_root, self.virtual_loss, history=hist,
+                                                    hist_offsets=offs)
+        else:
+            visits, _, _ = self.engine.search(positions, num_simulations=self.sims, history=hist, hist_offsets=offs)
         out = []
         for k in range(len(positions)):
             w = visits[k] / visits[k].sum()

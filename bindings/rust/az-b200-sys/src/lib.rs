@@ -22,6 +22,8 @@ pub struct az_config { pub device: i32, pub max_games: i32, pub max_batch: i32, 
     pub cache_hits: u64, pub terminal_leaves: u64, pub games_finished: u64, pub sum_leaf_depth: u64, pub sum_edges: u64,
     pub waves: u64, pub pending_samples: u64, pub active_games: u64, pub parked_games: u64, pub cache_evictions: u64,
     pub sum_search_depth: u64 }
+#[repr(C)] #[derive(Default)] pub struct az_search_stats { pub waves: u64, pub evaluations: u64, pub terminal_leaves: u64,
+    pub collisions: u64 }                                                                       // not in the reference
 pub enum az_engine {}
 
 extern "C" {
@@ -43,6 +45,10 @@ extern "C" {
     pub fn az_search(eng: *mut az_engine, n: c_int, roots: *const az_position, history: *const az_position,
                      hist_offsets: *const u32, num_simulations: c_int, noise_game_ids: *const u64, noise_plies: *const u32,
                      visits: *mut f32, scores: *mut f32, depth: *mut i32) -> c_int;
+    pub fn az_search_vl(eng: *mut az_engine, n: c_int, roots: *const az_position, history: *const az_position,
+                        hist_offsets: *const u32, num_simulations: c_int, leaves_per_root: c_int, virtual_loss: f32,
+                        noise_game_ids: *const u64, noise_plies: *const u32, visits: *mut f32, scores: *mut f32, depth: *mut i32,
+                        stats: *mut az_search_stats) -> c_int;
     pub fn az_selfplay_begin(eng: *mut az_engine, n_games: c_int, first_game_id: u64) -> c_int;
     pub fn az_selfplay_begin_n(eng: *mut az_engine, n_concurrent: c_int, first_game_id: u64, total_games: u64) -> c_int;
     pub fn az_selfplay_step(eng: *mut az_engine, waves: c_int, stats: *mut az_selfplay_stats) -> c_int;

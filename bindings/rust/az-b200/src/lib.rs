@@ -80,6 +80,24 @@ impl Engine {
         Ok((visits, depth))
     }
 
+    /// Not in the reference: `search` with up to `leaves_per_root` leaves per root in each network round, steered apart by
+    /// `virtual_loss` (az_search_vl); `leaves_per_root = 1` gives `search`'s results.  Returns visits, depths and the stats.
+    pub fn search_vl(&mut self, roots: &[sys::az_position], history: &[Vec<sys::az_position>], sims: i32, leaves_per_root: i32,
+                     virtual_loss: f32, noise: Option<(&[u64], &[u32])>) -> Result<(Vec<f32>, Vec<i32>, sys::az_search_stats)> {
+        let n = roots.len();
+        let mut flat = Vec::new();
+        let mut offs = vec![0u32; n + 1];
+        for (i, h) in history.iter().enumerate() { flat.extend_from_slice(h); offs[i + 1] = flat.len() as u32; }
+        let (ids, plies) = match noise { Some((g, p)) => (g.as_ptr(), p.as_ptr()), None => (ptr::null(), ptr::null()) };
+        let mut visits = vec![0f32; n * ACTION_SPACE];
+        let mut depth = vec![0i32; n];
+        let mut stats = sys::az_search_stats::default();
+        self.check(unsafe { sys::az_search_vl(self.raw, n as i32, roots.as_ptr(), flat.as_ptr(), offs.as_ptr(), sims, leaves_per_root,
+                                              virtual_loss, ids, plies, visits.as_mut_ptr(), ptr::null_mut(), depth.as_mut_ptr(),
+                                              &mut stats) })?;
+        Ok((visits, depth, stats))
+    }
+
     /// run_all_episodes (training.rs:340-378): EXACTLY `n_games` self-play games (ids first_game_id ..), each played to
     /// completion; the callback receives the finished games' steps (values already back-filled) as they become available.
     /// Returns the average batch size (= evaluations per wave).

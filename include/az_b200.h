@@ -132,6 +132,26 @@ int az_search(az_engine* eng, int n, const az_position* roots, const az_position
               int num_simulations, const uint64_t* noise_game_ids, const uint32_t* noise_plies, float* visits_out,
               float* scores_out, int32_t* depth_out);
 
+/* NOT IN THE REFERENCE: leaf-parallel search with virtual loss for callers with few roots (a non-parity mode, except at
+ * leaves_per_root = 1, where results are bit-identical to az_search).  Each root runs its simulations in batches of up to
+ * leaves_per_root (K) leaves that share one network round: descents score every edge with N' = N + V and W' = W -
+ * virtual_loss * V, V being the descents of the current batch through the edge; a descent ending on an edge another descent of
+ * the batch already took (a collision) ends the root's batch.  Leaves are expanded as in tree.rs and backed up in gather
+ * order, so results are deterministic.  Exactly num_simulations visits per non-terminal root.  n * K <= az_config.max_batch
+ * (else AZ_ERR_CAPACITY); K >= 1 and a finite virtual_loss >= 0 (else AZ_ERR_INVALID_ARGUMENT).  The other arguments are
+ * those of az_search.  The in-flight counts (4 bytes per edge of the pool) and per-leaf paths (8 bytes x (num_simulations + 2)
+ * per max_batch slot) are allocated by the first call. */
+typedef struct az_search_stats {
+    uint64_t waves;           /* network rounds */
+    uint64_t evaluations;     /* boards sent to the network */
+    uint64_t terminal_leaves;
+    uint64_t collisions;      /* descents discarded because their leaf edge was already taken in the batch */
+} az_search_stats;
+int az_search_vl(az_engine* eng, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
+                 int num_simulations, int leaves_per_root, float virtual_loss, const uint64_t* noise_game_ids,
+                 const uint32_t* noise_plies, float* visits_out, float* scores_out, int32_t* depth_out,
+                 az_search_stats* stats_out /* nullable */);
+
 /* test hook: replace the network by the deterministic synthetic evaluator shared with the oracle (kind 1) or
  * restore the network (kind 0) */
 int az_set_evaluator_stub(az_engine* eng, int kind, uint64_t seed);

@@ -167,6 +167,23 @@ public:
         if (sum > 0.0f) for (float& v : visits) v = v / sum;
         return visits;
     }
+    // NOT IN THE REFERENCE: the same search with up to leaves_per_root leaves per network round and virtual loss
+    // (az_search_vl); leaves_per_root = 1 is the overload above bit for bit
+    Policy monte_carlo_tree_search(int num_simulations, int leaves_per_root, float virtual_loss) {
+        Engine& e = model_->engine();
+        const int sims = num_simulations > 0 ? num_simulations : e.config().num_simulations;
+        const uint32_t offs[2] = {0, (uint32_t)state.pos_count.size()};
+        Policy visits;
+        int32_t depth = 0;
+        e.check(az_search_vl(e.handle(), 1, &state.position, state.pos_count.data(), offs, sims, leaves_per_root, virtual_loss,
+                             noise_ ? &noise_game_ : nullptr, noise_ ? &noise_ply_ : nullptr, visits.data(), nullptr, &depth, nullptr),
+                "az_search_vl");
+        depth_ = (std::size_t)depth;
+        float sum = 0.0f;
+        for (float v : visits) sum += v;
+        if (sum > 0.0f) for (float& v : visits) v = v / sum;
+        return visits;
+    }
     std::size_t max_subtree_depth() const { return depth_; }   // of the last search (tree.rs:258-269)
     // traverse_new(action, apply_noise): the played move must be legal and the game ongoing (the reference panics otherwise)
     MCTree traverse_new(std::size_t action, bool apply_noise) && {
