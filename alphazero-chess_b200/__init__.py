@@ -184,14 +184,18 @@ class Engine:
         return a
 
     # ---- agent.rs ---------------------------------------------------------------------------------------------
-    def load_weights(self, arrays):
-        """load_model (main.rs:109-116): 144 f32 arrays in az_weight_name order."""
+    def load_weights(self, arrays, network=0):
+        """load_model (main.rs:109-116): 144 f32 arrays in az_weight_name order, into network slot `network`
+        (0 = what every single-network call uses; 1 = the second network of forward_networks / search_networks)."""
         arrs = [np.ascontiguousarray(a, np.float32).ravel() for a in arrays]
         sizes = weight_sizes()
         if len(arrs) != NUM_WEIGHT_ARRAYS or any(a.size != s for a, s in zip(arrs, sizes)):
             raise ValueError("expected 144 arrays with the sizes of az_weight_size")
         ptrs = (ctypes.c_void_p * NUM_WEIGHT_ARRAYS)(*[a.ctypes.data for a in arrs])
-        self._check(self._L.az_load_weights(self._h, ptrs, NUM_WEIGHT_ARRAYS), "az_load_weights")
+        if network == 0:
+            self._check(self._L.az_load_weights(self._h, ptrs, NUM_WEIGHT_ARRAYS), "az_load_weights")
+        else:
+            self._check(self._L.az_load_network(self._h, int(network), ptrs, NUM_WEIGHT_ARRAYS), "az_load_network")
 
     def load_mpk(self, path):
         """load_model (main.rs:109-116) from a burn `.mpk` checkpoint (see mpk.py)."""
@@ -217,6 +221,23 @@ class Engine:
         policy = np.empty((n, ACTION_SPACE), np.float32)
         value = np.empty(n, np.float32)
         self._check(self._L.az_forward(self._h, n, _ptr(p), _ptr(policy), _ptr(value)), "az_forward")
+        return policy, value
+
+    @staticmethod
+    def _networks(network, n):
+        net = np.ascontiguousarray(np.broadcast_to(np.asarray(network), (n,)), np.uint8)
+        if np.any(np.asarray(network) < 0):
+            raise ValueError("network ids must be >= 0")
+        return net
+
+    def forward_networks(self, pos, network):
+        """forward() with a network slot per board (an int or [n] ids): both networks run in the same launches."""
+        p = self._positions(pos)
+        n = p.shape[0]
+        net = self._networks(network, n)
+        policy = np.empty((n, ACTION_SPACE), np.float32)
+        value = np.empty(n, np.float32)
+        self._check(self._L.az_forward_networks(self._h, n, _ptr(p), _ptr(net), _ptr(policy), _ptr(value)), "az_forward_networks")
         return policy, value
 
     # ---- chess.rs ---------------------------------------------------------------------------------------------
@@ -318,6 +339,26 @@ class Engine:
         self._check(self._L.az_search_vl(self._h, n, _ptr(p), _ptr(h), _ptr(ho), int(num_simulations), int(leaves_per_root),
                                          ctypes.c_float(virtual_loss), _ptr(ids), _ptr(pl), _ptr(visits), _ptr(scores), _ptr(depth),
                                          ctypes.byref(st)), "az_search_vl")
+        return visits, scores, depth, st
+
+    def search_networks(self, roots, network, num_simulations, leaves_per_root=1, virtual_loss=1.0, history=None, hist_offsets=None,
+                        noise_game_ids=None, noise_plies=None, want_scores=False):
+        """search_vl() with a network slot per root (an int or [n] ids): the roots of both networks share every network round.
+        Returns (visits [n,4096], scores or None, depth [n], SearchStats)."""
+        p = self._positions(roots)
+        n = p.shape[0]
+        net = self._networks(network, n)
+        visits = np.empty((n, ACTION_SPACE), np.float32)
+        scores = np.empty((n, ACTION_SPACE), np.float32) if want_scores else None
+        depth = np.empty(n, np.int32)
+        h = self._positions(history) if history is not None else None
+        ho = np.ascontiguousarray(hist_offsets, np.uint32) if hist_offsets is not None else None
+        ids = np.ascontiguousarray(noise_game_ids, np.uint64) if noise_game_ids is not None else None
+        pl = np.ascontiguousarray(noise_plies, np.uint32) if noise_plies is not None else None
+        st = SearchStats()
+        self._check(self._L.az_search_networks(self._h, n, _ptr(p), _ptr(h), _ptr(ho), int(num_simulations), int(leaves_per_root),
+                                               ctypes.c_float(virtual_loss), _ptr(net), _ptr(ids), _ptr(pl), _ptr(visits), _ptr(scores),
+                                               _ptr(depth), ctypes.byref(st)), "az_search_networks")
         return visits, scores, depth, st
 
     # ---- training.rs ------------------------------------------------------------------------------------------

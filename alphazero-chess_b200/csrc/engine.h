@@ -83,6 +83,11 @@ struct az_engine {
     } knobs;
 
     azb::NetWeights* net = nullptr;
+    azb::NetWeights* net1 = nullptr;   // network slot 1 (az_load_network): weights only, allocated by its first load
+    // az_forward_networks (allocated on its first call): boards per network, the slot of each board, its gathered value
+    int* d_net_counts = nullptr;       // [AZ_MAX_NETWORKS]
+    int* d_net_slot = nullptr;         // [max_batch]
+    float* d_net_value = nullptr;      // [max_batch]
     azb::SearchState* search = nullptr;
     int stub_kind = 0;
     uint64_t stub_seed = 0;

@@ -249,11 +249,27 @@ __device__ __forceinline__ int create_node(Ctx& x, int depth) {
     return node;
 }
 
+// Request routing of az_search_networks: game g's requests go to the range of network net[g] (network 0 from slot 0, network 1
+// from slot base1), each range with its own counter
+struct NetRoute {
+    const uint8_t* net;   // [G]
+    int* counts;          // [AZ_MAX_NETWORKS]
+    int base1;
+};
+
 // Queues the position in sh->child (the node create_node made last: its edge range is in x.new_link) for evaluation;
-// returns the batch slot.
-__device__ __forceinline__ int submit_request(Ctx& x, int node) {
+// returns the batch slot.  ROUTE: the slot is taken in the range of the game's network (rt).
+template <bool ROUTE = false>
+__device__ __forceinline__ int submit_request(Ctx& x, int node, const NetRoute* rt = nullptr) {
     int slot = 0;
-    if (x.lane == 0) slot = atomicAdd(x.ptr.batch_count, 1);
+    if (x.lane == 0) {
+        if constexpr (ROUTE) {
+            const int s = rt->net[x.g];
+            slot = (s ? rt->base1 : 0) + atomicAdd(rt->counts + s, 1);
+        } else {
+            slot = atomicAdd(x.ptr.batch_count, 1);
+        }
+    }
     slot = __shfl_sync(0xffffffffu, slot, 0);
     const DPos child = x.sh->child;
     if (x.lane == 0) {
@@ -794,10 +810,11 @@ __global__ void __launch_bounds__(WARPS * 32, MINB * 4 / WARPS) k_advance(const 
 }
 
 // Root set-up for az_search (MCTree::init): node 0 from the given position, evaluation pending.
-__global__ void __launch_bounds__(WARPS * 32) k_init_search(SearchParams prm, SearchPtrs ptr, const az_position* __restrict__ roots,
-                                                            const az_position* __restrict__ hist, const uint32_t* __restrict__ hist_off,
-                                                            const unsigned long long* __restrict__ noise_ids,
-                                                            const uint32_t* __restrict__ noise_plies) {
+template <bool ROUTE>
+__device__ __forceinline__ void init_search_body(const SearchParams& prm, const SearchPtrs& ptr, const az_position* __restrict__ roots,
+                                                 const az_position* __restrict__ hist, const uint32_t* __restrict__ hist_off,
+                                                 const unsigned long long* __restrict__ noise_ids, const uint32_t* __restrict__ noise_plies,
+                                                 const NetRoute& rt) {
     __shared__ WarpShared shared[WARPS];
     const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (g >= prm.n_games) return;
@@ -837,9 +854,22 @@ __global__ void __launch_bounds__(WARPS * 32) k_init_search(SearchParams prm, Se
     x.c.hist_len = hl;
     setup_root_from_shared(x);
     x.c.pending_node = 0;
-    x.c.pending_slot = submit_request(x, 0);
+    x.c.pending_slot = submit_request<ROUTE>(x, 0, &rt);
     if (x.sh->n_moves == 0) x.c.status = 1;  // nothing to search in a terminal position
     if (x.lane == 0) ptr.ctl[g] = x.c;
+}
+__global__ void __launch_bounds__(WARPS * 32) k_init_search(SearchParams prm, SearchPtrs ptr, const az_position* __restrict__ roots,
+                                                            const az_position* __restrict__ hist, const uint32_t* __restrict__ hist_off,
+                                                            const unsigned long long* __restrict__ noise_ids,
+                                                            const uint32_t* __restrict__ noise_plies) {
+    init_search_body<false>(prm, ptr, roots, hist, hist_off, noise_ids, noise_plies, NetRoute{nullptr, nullptr, 0});
+}
+// the same with the root's request in the range of its network (az_search_networks)
+__global__ void __launch_bounds__(WARPS * 32) k_init_search_nets(SearchParams prm, SearchPtrs ptr, const az_position* __restrict__ roots,
+                                                                 const az_position* __restrict__ hist, const uint32_t* __restrict__ hist_off,
+                                                                 const unsigned long long* __restrict__ noise_ids,
+                                                                 const uint32_t* __restrict__ noise_plies, const NetRoute rt) {
+    init_search_body<true>(prm, ptr, roots, hist, hist_off, noise_ids, noise_plies, rt);
 }
 
 // Game set-up for self-play (training.rs:352-361): start position, shared priors, Dirichlet noise.
@@ -1065,8 +1095,8 @@ __global__ void __launch_bounds__(WARPS * 32) k_vl_gather(const __grid_constant_
 }
 
 // one warp per gathered leaf (g * K + k): tree.rs expand; the new node is linked to the leaf edge and queued for evaluation
-__global__ void __launch_bounds__(WARPS * 32) k_vl_expand(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
-                                                          const __grid_constant__ VLPtrs vl) {
+template <bool ROUTE>
+__device__ __forceinline__ void vl_expand_body(const SearchParams& prm, const SearchPtrs& ptr, const VLPtrs& vl, const NetRoute& rt) {
     __shared__ WarpShared shared[WARPS];
     const int leaf = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int g = leaf / vl.K;
@@ -1117,8 +1147,17 @@ __global__ void __launch_bounds__(WARPS * 32) k_vl_expand(const __grid_constant_
         ptr.edge_link[pe] = x.new_link;
         atomicMax(&ptr.ctl[g].max_depth, (uint32_t)len);
     }
-    const int slot = submit_request(x, child);
+    const int slot = submit_request<ROUTE>(x, child, &rt);
     if (x.lane == 0) vl.slot[leaf] = slot;
+}
+__global__ void __launch_bounds__(WARPS * 32) k_vl_expand(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
+                                                          const __grid_constant__ VLPtrs vl) {
+    vl_expand_body<false>(prm, ptr, vl, NetRoute{nullptr, nullptr, 0});
+}
+// the same with the leaf's request in the range of its root's network (az_search_networks)
+__global__ void __launch_bounds__(WARPS * 32) k_vl_expand_nets(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
+                                                               const __grid_constant__ VLPtrs vl, const __grid_constant__ NetRoute rt) {
+    vl_expand_body<true>(prm, ptr, vl, rt);
 }
 
 // ------------------------------------------------------------------------------------------- host side
@@ -1209,9 +1248,26 @@ void search_destroy(az_engine* e) {
     e->search = nullptr;
 }
 
-// evaluates the queued requests: the network (bf16 or fp32) or the synthetic evaluator
-static int evaluate_batch(az_engine* e, SearchState* st) {
+// evaluates the queued requests: the network (bf16 or fp32) or the synthetic evaluator.  nb: a multi-network batch (requests
+// routed by NetRoute); under the synthetic evaluator network s evaluates with seed stub_seed + s
+static int evaluate_batch(az_engine* e, SearchState* st, const NetBatch* nb = nullptr) {
     const SearchPtrs& q = st->ptr;
+    if (nb) {
+        if (e->stub_kind == 1) {
+            const int warps = e->max_batch;
+            for (int s = 0; s < AZ_MAX_NETWORKS; s++) {
+                const size_t base = s ? (size_t)nb->base1 : 0;
+                e->n_launches++;
+                k_stub_eval<<<(warps + 3) / 4, 128, 0, e->stream>>>(q.req_pos + base, nb->counts_dev + s, 0, e->stub_seed + (uint64_t)s,
+                                                                    e->d_policy + base * AZ_ACTION_SPACE, e->d_value + base);
+                AZ_CUDA(e, cudaGetLastError());
+            }
+            return AZ_OK;
+        }
+        if (e->cfg.precision == 1) return net_forward_networks(e, *nb, q.req_f32, e->d_policy, e->d_value);
+        HeadScatter sc{q.req_edge_off, q.req_nedges, q.edge_mv, q.edge_P};
+        return net_forward_networks(e, *nb, nullptr, nullptr, e->d_value, &sc);
+    }
     if (e->stub_kind == 1) {
         const int warps = e->max_batch;
         e->n_launches++;
@@ -1288,14 +1344,14 @@ static int run_wave(az_engine* e, SearchState* st) {
 // search state.  Returns AZ_OK, an error, or 1 when there is nothing to do (n == 0).
 static int search_begin(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
                         int num_simulations, const uint64_t* noise_game_ids, const uint32_t* noise_plies, const float* visits_out,
-                        SearchState& run) {
+                        SearchState& run, const NetRoute* route = nullptr, const NetBatch* nb = nullptr) {
     SearchState* st = e->search;
     if (n < 0 || n > st->G) return set_err(e, AZ_ERR_CAPACITY, "more roots than az_config.max_games");
     if (n == 0) return 1;
     if (!roots || !visits_out) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "null buffer");
     if (num_simulations <= 0 || num_simulations + 2 > st->prm.node_cap)
         return set_err(e, AZ_ERR_CAPACITY, "num_simulations exceeds az_config.num_simulations (pool size)");
-    if (e->stub_kind == 0 && !e->net->loaded) return set_err(e, AZ_ERR_NO_WEIGHTS, "az_load_weights has not been called");
+    if (e->stub_kind == 0 && !route && !e->net->loaded) return set_err(e, AZ_ERR_NO_WEIGHTS, "az_load_weights has not been called");
     cudaSetDevice(e->cfg.device);
     st->selfplay_active = false;
     SearchParams prm = st->prm;
@@ -1341,9 +1397,10 @@ static int search_begin(az_engine* e, int n, const az_position* roots, const az_
     run.ptr.batch_zero = nullptr;
     AZ_CUDA(e, cudaMemsetAsync(run.batch_base, 0, 16, e->stream));
     e->n_launches++;
-    k_init_search<<<blocks, WARPS * 32, 0, e->stream>>>(run.prm, run.ptr, e->d_wire, d_hist, e->d_hist_off, d_ids, d_plies);
+    if (route) k_init_search_nets<<<blocks, WARPS * 32, 0, e->stream>>>(run.prm, run.ptr, e->d_wire, d_hist, e->d_hist_off, d_ids, d_plies, *route);
+    else k_init_search<<<blocks, WARPS * 32, 0, e->stream>>>(run.prm, run.ptr, e->d_wire, d_hist, e->d_hist_off, d_ids, d_plies);
     AZ_CUDA(e, cudaGetLastError());
-    return evaluate_batch(e, &run);
+    return evaluate_batch(e, &run, nb);
 }
 
 // dense export of the roots' statistics (Box<[f32; 4096]> visits / scores, max_subtree_depth) to the caller's buffers
@@ -1411,9 +1468,16 @@ int az_search(az_engine* e, int n, const az_position* roots, const az_position* 
     return rc;
 }
 
-int az_search_vl(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
-                 int num_simulations, int leaves_per_root, float virtual_loss, const uint64_t* noise_game_ids, const uint32_t* noise_plies,
-                 float* visits_out, float* scores_out, int32_t* depth_out, az_search_stats* stats_out) {
+}  // extern "C"
+
+namespace azb {
+
+// az_search_vl, and az_search_networks when `network` (one id per root) is given: the requests of each root then go to the
+// range of its network (k_init_search_nets, k_vl_expand_nets) and every wave evaluates both ranges in one multi-network forward
+static int search_vl_run(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
+                         int num_simulations, int leaves_per_root, float virtual_loss, const uint8_t* network,
+                         const uint64_t* noise_game_ids, const uint32_t* noise_plies, float* visits_out, float* scores_out,
+                         int32_t* depth_out, az_search_stats* stats_out) {
     if (!e) return AZ_ERR_INVALID_ARGUMENT;
     if (stats_out) std::memset(stats_out, 0, sizeof *stats_out);
     if (leaves_per_root < 1) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "leaves_per_root must be >= 1");
@@ -1422,6 +1486,23 @@ int az_search_vl(az_engine* e, int n, const az_position* roots, const az_positio
     if (n > 0 && (long long)n * leaves_per_root > (long long)e->max_batch)
         return set_err(e, AZ_ERR_CAPACITY, "roots x leaves_per_root exceeds az_config.max_batch");
     SearchState* st = e->search;
+    // network ranges: network 0 from slot 0, network 1 from the next multiple of 4 after network 0's n_0 * K slots
+    int count[AZ_MAX_NETWORKS] = {0, 0};
+    int base1 = 0;
+    if (network && n > 0 && n <= st->G) {
+        for (int g = 0; g < n; g++) {
+            if (network[g] >= AZ_MAX_NETWORKS) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "network id must be < AZ_MAX_NETWORKS");
+            count[network[g]]++;
+        }
+        for (int s = 0; s < AZ_MAX_NETWORKS; s++) {
+            const NetWeights* w = net_slot(e, s);
+            if (count[s] && e->stub_kind == 0 && (!w || !w->loaded))
+                return set_err(e, AZ_ERR_NO_WEIGHTS, "a root names a network that has not been loaded");
+        }
+        const long long r0 = ((long long)count[0] * leaves_per_root + 3) & ~3LL, r1 = ((long long)count[1] * leaves_per_root + 3) & ~3LL;
+        if (r0 + r1 > e->max_batch) return set_err(e, AZ_ERR_CAPACITY, "network ranges (roots x leaves_per_root each) exceed az_config.max_batch");
+        base1 = (int)r0;
+    }
     if (n >= 0 && n <= st->G && !st->vl_V) {   // first call: the in-flight counts and the per-leaf records
         cudaSetDevice(e->cfg.device);
         const size_t NE = (size_t)st->G * st->prm.edge_cap, B = (size_t)e->max_batch;
@@ -1431,8 +1512,20 @@ int az_search_vl(az_engine* e, int n, const az_position* roots, const az_positio
         a |= salloc(e, st, &st->vl_count, (size_t)st->G); a |= salloc(e, st, &st->vl_stats, 4);
         if (a) return AZ_ERR_OUT_OF_MEMORY;
     }
+    NetRoute route{nullptr, st->batch_base, base1};
+    NetBatch nb{st->batch_base, base1, base1 + count[1] * leaves_per_root};
+    if (network && n > 0 && n <= st->G) {
+        if (!st->d_net) {
+            cudaSetDevice(e->cfg.device);
+            if (salloc(e, st, &st->d_net, (size_t)st->G)) return AZ_ERR_OUT_OF_MEMORY;
+        }
+        AZ_CUDA(e, cudaMemcpyAsync(st->d_net, network, (size_t)n, cudaMemcpyHostToDevice, e->stream));
+        route.net = st->d_net;
+    }
+    const NetRoute* rt = route.net ? &route : nullptr;
+    const NetBatch* nbp = route.net ? &nb : nullptr;
     SearchState run;
-    int r = search_begin(e, n, roots, history, hist_offsets, num_simulations, noise_game_ids, noise_plies, visits_out, run);
+    int r = search_begin(e, n, roots, history, hist_offsets, num_simulations, noise_game_ids, noise_plies, visits_out, run, rt, nbp);
     if (r) return r == 1 ? AZ_OK : r;
     const int K = leaves_per_root;
     VLPtrs vl{st->vl_V, st->vl_path, st->vl_len, st->vl_slot, st->vl_value, st->vl_count, st->vl_stats, K, virtual_loss};
@@ -1457,9 +1550,14 @@ int az_search_vl(az_engine* e, int n, const az_position* roots, const az_positio
             if (flags[0] == 0) break;
             if (wave > num_simulations + 16) { rc = set_err(e, AZ_ERR_STATE, "search did not converge"); break; }
         }
-        k_vl_expand<<<(n * K + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(run.prm, run.ptr, vl);
+        if (rt) {   // both request counters start the wave at 0 (k_vl_gather clears only the first)
+            AZ_CUDA(e, cudaMemsetAsync(run.batch_base, 0, AZ_MAX_NETWORKS * sizeof(int), e->stream));
+            k_vl_expand_nets<<<(n * K + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(run.prm, run.ptr, vl, *rt);
+        } else {
+            k_vl_expand<<<(n * K + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(run.prm, run.ptr, vl);
+        }
         AZ_CUDA(e, cudaGetLastError());
-        r = evaluate_batch(e, &run);
+        r = evaluate_batch(e, &run, nbp);
         if (r) return r;
         waves++;
     }
@@ -1477,6 +1575,29 @@ int az_search_vl(az_engine* e, int n, const az_position* roots, const az_positio
         stats_out->collisions = s[2];
     }
     return rc;
+}
+
+}  // namespace azb
+
+extern "C" {
+
+int az_search_vl(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
+                 int num_simulations, int leaves_per_root, float virtual_loss, const uint64_t* noise_game_ids, const uint32_t* noise_plies,
+                 float* visits_out, float* scores_out, int32_t* depth_out, az_search_stats* stats_out) {
+    return search_vl_run(e, n, roots, history, hist_offsets, num_simulations, leaves_per_root, virtual_loss, nullptr, noise_game_ids,
+                         noise_plies, visits_out, scores_out, depth_out, stats_out);
+}
+
+int az_search_networks(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
+                       int num_simulations, int leaves_per_root, float virtual_loss, const uint8_t* network, const uint64_t* noise_game_ids,
+                       const uint32_t* noise_plies, float* visits_out, float* scores_out, int32_t* depth_out, az_search_stats* stats_out) {
+    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+    if (n > 0 && !network) {
+        if (stats_out) std::memset(stats_out, 0, sizeof *stats_out);
+        return set_err(e, AZ_ERR_INVALID_ARGUMENT, "null network buffer");
+    }
+    return search_vl_run(e, n, roots, history, hist_offsets, num_simulations, leaves_per_root, virtual_loss, network, noise_game_ids,
+                         noise_plies, visits_out, scores_out, depth_out, stats_out);
 }
 
 int az_selfplay_begin(az_engine* e, int n_games, uint64_t first_game_id) { return az_selfplay_begin_n(e, n_games, first_game_id, 0); }

@@ -136,6 +136,7 @@ struct SearchState {
     float* vl_value = nullptr;             // [max_batch]
     int* vl_count = nullptr;               // [G]
     unsigned long long* vl_stats = nullptr; // [4]
+    uint8_t* d_net = nullptr;              // [G] az_search_networks: network of each root (allocated on its first call)
     std::vector<void*> allocs;
 };
 

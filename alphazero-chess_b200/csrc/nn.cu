@@ -52,11 +52,8 @@ static int dmalloc(az_engine* e, T** p, size_t n) {
     return check_cuda(e, cudaMalloc(p, n * sizeof(T)), "cudaMalloc(net)");
 }
 
-int net_create(az_engine* e) {
-    NetWeights* w = new NetWeights;
-    e->net = w;
-    w->max_boards = e->max_batch;
-    const size_t nb = (size_t)e->max_batch;
+// the weights of one network (fp32 parameters, bf16 operands) and their tensor maps
+static int alloc_weights(az_engine* e, NetWeights* w) {
     int r = 0;
     r |= dmalloc(e, &w->f_w_in, 128 * 19 * 9); r |= dmalloc(e, &w->f_b_in, 128);
     r |= dmalloc(e, &w->f_w_tower, (size_t)20 * 128 * 128 * 9); r |= dmalloc(e, &w->f_b_tower, 21 * 128);  // row 20: copy of f_b_in for the fused launch
@@ -64,10 +61,26 @@ int net_create(az_engine* e) {
     r |= dmalloc(e, &w->f_wp2t, 32 * 64); r |= dmalloc(e, &w->f_bp2, 64);
     r |= dmalloc(e, &w->f_wl1, 512 * 64); r |= dmalloc(e, &w->f_bl1, 64);
     r |= dmalloc(e, &w->f_wl2, 64); r |= dmalloc(e, &w->f_bl2, 1);
-    w->in_ch = e->knobs.input_k32 ? 32 : 64;
     const int ic = w->in_ch;
     r |= dmalloc(e, &w->h_w_in, (size_t)9 * 128 * ic); r |= dmalloc(e, &w->h_w_tower, (size_t)20 * 9 * 128 * 128);
     r |= dmalloc(e, &w->h_w40, 40 * 128); r |= dmalloc(e, &w->h_wp2, 64 * 32); r |= dmalloc(e, &w->h_wl1t, 64 * 512);
+    if (r) return AZ_ERR_OUT_OF_MEMORY;
+    if (tc_make_weight_map(&w->map_w_in, w->h_w_in, ic)) return set_err(e, AZ_ERR_CUDA, "cuTensorMapEncodeTiled(w_in)");
+    for (int l = 0; l < 20; l++)
+        if (tc_make_weight_map(&w->map_w_tower[l], w->h_w_tower + (size_t)l * 9 * 128 * 128, 128))
+            return set_err(e, AZ_ERR_CUDA, "cuTensorMapEncodeTiled(w_tower)");
+    return 0;
+}
+
+int net_create(az_engine* e) {
+    NetWeights* w = new NetWeights;
+    e->net = w;
+    w->max_boards = e->max_batch;
+    const size_t nb = (size_t)e->max_batch;
+    w->in_ch = e->knobs.input_k32 ? 32 : 64;
+    const int ic = w->in_ch;
+    int r = alloc_weights(e, w);
+    if (r) return r;
     r |= dmalloc(e, &w->a_in, nb * 64 * ic);
     for (int i = 0; i < 3; i++) r |= dmalloc(e, &w->a_buf[i], nb * 64 * 128);
     if (r) return AZ_ERR_OUT_OF_MEMORY;
@@ -77,10 +90,6 @@ int net_create(az_engine* e) {
         if (tc_make_act_map(&w->map_a[i], w->a_buf[i], 128, e->max_batch)) return set_err(e, AZ_ERR_CUDA, "cuTensorMapEncodeTiled(act)");
     for (int i = 0; i < 3; i++)
         if (tc_make_rows_map(&w->map_rows[i], w->a_buf[i], e->max_batch)) return set_err(e, AZ_ERR_CUDA, "cuTensorMapEncodeTiled(rows)");
-    if (tc_make_weight_map(&w->map_w_in, w->h_w_in, ic)) return set_err(e, AZ_ERR_CUDA, "cuTensorMapEncodeTiled(w_in)");
-    for (int l = 0; l < 20; l++)
-        if (tc_make_weight_map(&w->map_w_tower[l], w->h_w_tower + (size_t)l * 9 * 128 * 128, 128))
-            return set_err(e, AZ_ERR_CUDA, "cuTensorMapEncodeTiled(w_tower)");
     CUtensorMap host_maps[31];
     for (int i = 0; i < 3; i++) host_maps[i] = w->map_a[i];
     for (int l = 0; l < 20; l++) host_maps[3 + l] = w->map_w_tower[l];
@@ -95,16 +104,41 @@ int net_create(az_engine* e) {
     return 0;
 }
 
+// Network slot 1: its own weights, tensor maps and device map array (the activation maps of slot 0, its weight maps); the
+// activations and every other buffer stay slot 0's
+static int create_slot1(az_engine* e) {
+    NetWeights* w0 = e->net;
+    NetWeights* w = new NetWeights;
+    e->net1 = w;
+    w->max_boards = w0->max_boards;
+    w->in_ch = w0->in_ch;
+    int r = alloc_weights(e, w);
+    if (r) return r;
+    CUtensorMap host_maps[31];
+    AZ_CUDA(e, cudaMemcpy(host_maps, w0->d_maps, sizeof host_maps, cudaMemcpyDeviceToHost));
+    for (int l = 0; l < 20; l++) host_maps[3 + l] = w->map_w_tower[l];
+    host_maps[24] = w->map_w_in;
+    if (dmalloc(e, &w->d_maps, 31)) return AZ_ERR_OUT_OF_MEMORY;
+    AZ_CUDA(e, cudaMemcpy(w->d_maps, host_maps, sizeof host_maps, cudaMemcpyHostToDevice));
+    return 0;
+}
+
+NetWeights* net_slot(az_engine* e, int s) { return s == 0 ? e->net : s == 1 ? e->net1 : nullptr; }
+
 void net_destroy(az_engine* e) {
-    NetWeights* w = e->net;
-    if (!w) return;
-    cudaFree(w->f_w_in); cudaFree(w->f_b_in); cudaFree(w->f_w_tower); cudaFree(w->f_b_tower); cudaFree(w->f_w40t); cudaFree(w->f_b40);
-    cudaFree(w->f_wp2t); cudaFree(w->f_bp2); cudaFree(w->f_wl1); cudaFree(w->f_bl1); cudaFree(w->f_wl2); cudaFree(w->f_bl2);
-    cudaFree(w->d_maps);
-    cudaFree(w->h_w_in); cudaFree(w->h_w_tower); cudaFree(w->a_in); cudaFree(w->h_w40); cudaFree(w->h_wp2); cudaFree(w->h_wl1t);
-    for (int i = 0; i < 3; i++) { cudaFree(w->a_buf[i]); cudaFree(w->g_buf[i]); }
-    delete w;
-    e->net = nullptr;
+    for (NetWeights** slot : {&e->net, &e->net1}) {
+        NetWeights* w = *slot;
+        if (!w) continue;
+        cudaFree(w->f_w_in); cudaFree(w->f_b_in); cudaFree(w->f_w_tower); cudaFree(w->f_b_tower); cudaFree(w->f_w40t); cudaFree(w->f_b40);
+        cudaFree(w->f_wp2t); cudaFree(w->f_bp2); cudaFree(w->f_wl1); cudaFree(w->f_bl1); cudaFree(w->f_wl2); cudaFree(w->f_bl2);
+        cudaFree(w->d_maps);
+        cudaFree(w->h_w_in); cudaFree(w->h_w_tower); cudaFree(w->a_in); cudaFree(w->h_w40); cudaFree(w->h_wp2); cudaFree(w->h_wl1t);
+        for (int i = 0; i < 3; i++) { cudaFree(w->a_buf[i]); cudaFree(w->g_buf[i]); }
+        delete w;
+        *slot = nullptr;
+    }
+    cudaFree(e->d_net_counts); cudaFree(e->d_net_slot); cudaFree(e->d_net_value);
+    e->d_net_counts = nullptr; e->d_net_slot = nullptr; e->d_net_value = nullptr;
 }
 
 // fold BN(gamma, beta, mean, var) into conv (weight [co][k], bias [co])
@@ -121,8 +155,7 @@ static int upload(az_engine* e, void* dst, const void* src, size_t bytes) {
     return check_cuda(e, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, e->stream), "upload weights");
 }
 
-static int load_from_host(az_engine* e, const float* const* a) {
-    NetWeights* w = e->net;
+static int load_from_host(az_engine* e, NetWeights* w, const float* const* a) {
     std::vector<float> fw((size_t)128 * 128 * 9), fb(128);
     std::vector<__nv_bfloat16> hw((size_t)9 * 128 * 128);
     int r = 0;
@@ -200,6 +233,16 @@ __global__ void k_encode_bf16_wire(const az_position* __restrict__ wire, __nv_bf
 }
 void launch_encode_bf16_wire(cudaStream_t s, const az_position* wire, __nv_bfloat16* out, int n, int ch) {
     if (n > 0) k_encode_bf16_wire<<<(n + 3) / 4, 128, 0, s>>>(wire, out, n, ch);
+}
+
+// rows of a multi-network batch back in the caller's order: row i of the outputs is slot[i] of the batch (one block per row)
+__global__ void k_gather_rows(const float* __restrict__ policy, const float* __restrict__ value, const int* __restrict__ slot,
+                              float* __restrict__ policy_out, float* __restrict__ value_out) {
+    const int i = blockIdx.x, s = slot[i];
+    const float4* src = reinterpret_cast<const float4*>(policy + (size_t)s * AZ_ACTION_SPACE);
+    float4* dst = reinterpret_cast<float4*>(policy_out + (size_t)i * AZ_ACTION_SPACE);
+    for (int j = threadIdx.x; j < AZ_ACTION_SPACE / 4; j += blockDim.x) dst[j] = src[j];
+    if (threadIdx.x == 0) value_out[i] = value[s];
 }
 
 // ---------------------------------------------------------------------------------------------- fp32 convolution
@@ -331,8 +374,8 @@ __global__ void __launch_bounds__(256) k_heads_f32(const float* __restrict__ tow
     if (t == 0) value_out[b] = tanhf(red[16] + red[17] + bl2[0]);
 }
 
-static int launch_heads_f32(az_engine* e, const float* tower, const int* n_dev, int n_static, int grid, float* policy_out, float* value_out) {
-    NetWeights* w = e->net;
+static int launch_heads_f32(az_engine* e, const NetWeights* w, const float* tower, const int* n_dev, int n_static, int grid, float* policy_out,
+                            float* value_out) {
     static PerDeviceOnce once;
     if (once.first()) cudaFuncSetAttribute(k_heads_f32, cudaFuncAttributeMaxDynamicSharedMemorySize, HEAD_SMEM);
     if (grid <= 0) return 0;
@@ -341,9 +384,15 @@ static int launch_heads_f32(az_engine* e, const float* tower, const int* n_dev, 
     return check_cuda(e, cudaGetLastError(), "k_heads");
 }
 
-int net_forward_bf16(az_engine* e, const int* n_dev, int n_static, float* policy_out, float* value_out, const HeadScatter* scatter) {
-    NetWeights* w = e->net;
-    if (!w->loaded) return set_err(e, AZ_ERR_NO_WEIGHTS, "az_load_weights has not been called");
+int net_forward_bf16(az_engine* e, const int* n_dev, int n_static, float* policy_out, float* value_out, const HeadScatter* scatter,
+                     const NetBatch* nb) {
+    NetWeights* w = e->net;   // the activations, and network 0
+    // A multi-network batch (nb, the default configuration only: net_forward_networks) runs the *_nets kernels, which split their
+    // CTAs between the two networks.  A network without boards gets no tiles, so when its slot is empty the other network's
+    // weights stand in as kernel arguments.
+    const NetWeights* wn1 = (e->net1 && e->net1->loaded) ? e->net1 : w;
+    const NetWeights* wn0 = w->loaded ? w : wn1;
+    if (!wn0->loaded || (!nb && !w->loaded)) return set_err(e, AZ_ERR_NO_WEIGHTS, "az_load_weights has not been called");
     const int grid = e->sm_count & ~1;
     const int tgrid = e->knobs.tower_grid > 0 ? std::min(grid, e->knobs.tower_grid & ~1) : grid;   // CTAs of the tower launch
     const int rel = e->knobs.tc_release_arrive;
@@ -361,7 +410,12 @@ int net_forward_bf16(az_engine* e, const int* n_dev, int n_static, float* policy
     const int wide = e->knobs.tower_wide;
     const int fused = (e->knobs.tower_fused >= 2 && (w->in_ch != 64 || wide)) ? 1 : e->knobs.tower_fused;
     int r = 0;
-    if (fused < 2) {
+    if (nb) {
+        e->n_launches += 1;
+        r = tc_conv3x3_nets_launch(e->stream, &w->map_a_in, &wn0->map_w_in, &wn1->map_w_in, wn0->f_b_in, wn1->f_b_in, w->a_buf[0],
+                                   nb->counts_dev, nb->base1, grid, (rel ? 32 : 0) | ((e->knobs.tower_l2hint & 8) ? 512 : 0));
+        if (r) return set_err(e, AZ_ERR_CUDA, "tc conv (input, networks) launch failed");
+    } else if (fused < 2) {
         e->n_launches += 1;
         r = tc_conv3x3_launch(e->stream, &w->map_a_in, &w->map_w_in, w->in_ch, w->f_b_in, nullptr, w->a_buf[0], n_dev, n_static, 1, grid,
                               (rel ? 32 : 0) | ((e->knobs.tower_l2hint & 8) ? 512 : 0) | (e->knobs.input_epi2 ? 1024 : 0));
@@ -373,7 +427,14 @@ int net_forward_bf16(az_engine* e, const int* n_dev, int n_static, float* policy
         cudaEventRecord(ps.a, e->stream);
     }
     int x = 0;  // buffer holding the block input
-    if (fused) {
+    if (nb) {
+        void* act[3] = {w->a_buf[0], w->a_buf[1], w->a_buf[2]};
+        e->n_launches += 1;
+        if (sample) e->prof_launches += 1;
+        r = tc_tower_nets_launch(e->stream, wn0->d_maps, wn1->d_maps, wn0->f_b_tower, wn1->f_b_tower, act, nb->counts_dev, nb->base1, tgrid,
+                                 rel, e->knobs.tower_l2hint);
+        if (r) return set_err(e, AZ_ERR_CUDA, "tower (networks) launch failed");
+    } else if (fused) {
         void* act[3] = {w->a_buf[0], w->a_buf[1], w->a_buf[2]};
         // The tower runs over consecutive board ranges whose two activation buffers (block input/output in place, conv1
         // output) stay resident in the 126 MB L2: a range of 2048 boards is 2 x 33.5 MB, and 512 tiles on 74 CTA pairs
@@ -398,7 +459,7 @@ int net_forward_bf16(az_engine* e, const int* n_dev, int n_static, float* policy
         }
         x = 0;  // the fused tower works in place: block input and block output share a_buf[0], a_buf[1] holds conv1's output
     }
-    for (int blk = 0; blk < (fused ? 0 : 10); blk++) {
+    for (int blk = 0; blk < (fused || nb ? 0 : 10); blk++) {
         e->n_launches += 2;
         if (sample) e->prof_launches += 2;
         const int y = (x + 1) % 3, z = (x + 2) % 3;
@@ -411,7 +472,8 @@ int net_forward_bf16(az_engine* e, const int* n_dev, int n_static, float* policy
         x = z;
     }
     if (sample) cudaEventRecord(ps.b, e->stream);
-    const int hr = e->knobs.heads_tc ? launch_heads_tc(e, &w->map_rows[x], n_dev, n_static, policy_out, value_out, scatter)
+    const int hr = nb ? launch_heads_tc_nets(e, wn0, wn1, &w->map_rows[x], nb->counts_dev, nb->base1, nb->cap, policy_out, value_out, scatter)
+                 : e->knobs.heads_tc ? launch_heads_tc(e, &w->map_rows[x], n_dev, n_static, policy_out, value_out, scatter)
                                      : launch_heads_mma(e, w->a_buf[x], n_dev, n_static, policy_out, value_out, scatter);
     if (sample) {
         cudaEventCreate(&ps.h1); cudaEventRecord(ps.h1, e->stream);
@@ -423,9 +485,11 @@ int net_forward_bf16(az_engine* e, const int* n_dev, int n_static, float* policy
     return hr;
 }
 
-int net_forward_fp32(az_engine* e, const float* planes, const int* n_dev, int n_static, float* policy_out, float* value_out) {
+int net_forward_fp32(az_engine* e, const float* planes, const int* n_dev, int n_static, float* policy_out, float* value_out,
+                     const NetWeights* wts) {
     NetWeights* w = e->net;
-    if (!w->loaded) return set_err(e, AZ_ERR_NO_WEIGHTS, "az_load_weights has not been called");
+    if (!wts) wts = w;
+    if (!wts->loaded) return set_err(e, AZ_ERR_NO_WEIGHTS, "az_load_weights has not been called");
     for (int i = 0; i < 3; i++)
         if (!w->g_buf[i]) AZ_CUDA(e, cudaMalloc(&w->g_buf[i], (size_t)w->max_boards * 128 * 64 * sizeof(float)));
     static PerDeviceOnce once;
@@ -433,19 +497,39 @@ int net_forward_fp32(az_engine* e, const float* planes, const int* n_dev, int n_
     const int grid = n_dev ? w->max_boards : n_static;
     if (grid <= 0) return 0;
     e->n_launches += 22;
-    k_conv3x3_f32<19><<<grid, 256, 19 * 64 * 4, e->stream>>>(planes, w->f_w_in, w->f_b_in, nullptr, w->g_buf[0], n_dev, n_static, 1);
+    k_conv3x3_f32<19><<<grid, 256, 19 * 64 * 4, e->stream>>>(planes, wts->f_w_in, wts->f_b_in, nullptr, w->g_buf[0], n_dev, n_static, 1);
     int x = 0;
     for (int blk = 0; blk < 10; blk++) {
         const int y = (x + 1) % 3, z = (x + 2) % 3;
-        k_conv3x3_f32<128><<<grid, 256, 128 * 64 * 4, e->stream>>>(w->g_buf[x], w->f_w_tower + (size_t)(2 * blk) * 128 * 128 * 9,
-                                                                  w->f_b_tower + (2 * blk) * 128, nullptr, w->g_buf[y], n_dev, n_static, 1);
-        k_conv3x3_f32<128><<<grid, 256, 128 * 64 * 4, e->stream>>>(w->g_buf[y], w->f_w_tower + (size_t)(2 * blk + 1) * 128 * 128 * 9,
-                                                                  w->f_b_tower + (2 * blk + 1) * 128, w->g_buf[x], w->g_buf[z], n_dev,
+        k_conv3x3_f32<128><<<grid, 256, 128 * 64 * 4, e->stream>>>(w->g_buf[x], wts->f_w_tower + (size_t)(2 * blk) * 128 * 128 * 9,
+                                                                  wts->f_b_tower + (2 * blk) * 128, nullptr, w->g_buf[y], n_dev, n_static, 1);
+        k_conv3x3_f32<128><<<grid, 256, 128 * 64 * 4, e->stream>>>(w->g_buf[y], wts->f_w_tower + (size_t)(2 * blk + 1) * 128 * 128 * 9,
+                                                                  wts->f_b_tower + (2 * blk + 1) * 128, w->g_buf[x], w->g_buf[z], n_dev,
                                                                   n_static, 1);
         x = z;
     }
     AZ_CUDA(e, cudaGetLastError());
-    return launch_heads_f32(e, w->g_buf[x], n_dev, n_static, grid, policy_out, value_out);
+    return launch_heads_f32(e, wts, w->g_buf[x], n_dev, n_static, grid, policy_out, value_out);
+}
+
+int net_forward_networks(az_engine* e, const NetBatch& nb, const float* planes_f32, float* policy_out, float* value_out,
+                         const HeadScatter* scatter) {
+    if (e->cfg.precision == 1) {   // the parity path: one network after the other over its range
+        for (int s = 0; s < AZ_MAX_NETWORKS; s++) {
+            const NetWeights* ws = net_slot(e, s);
+            if (!ws || !ws->loaded) continue;   // callers route no board to a network that was never loaded
+            const int base = s ? nb.base1 : 0;
+            const int r = net_forward_fp32(e, planes_f32 + (size_t)base * AZ_NUM_PLANES * 64, nb.counts_dev + s, 0,
+                                           policy_out ? policy_out + (size_t)base * AZ_ACTION_SPACE : nullptr, value_out + base, ws);
+            if (r) return r;
+        }
+        return 0;
+    }
+    const az_engine::Knobs& k = e->knobs;
+    if (k.tower_fused != 1 || k.tower_wide != 2 || k.tower_inkernel != 1 || k.tower_split != 0 || k.input_k32 != 1 || k.input_epi2 != 0 ||
+        k.heads_tc != 1)
+        return set_err(e, AZ_ERR_STATE, "a multi-network forward needs the default AZ_TOWER_*, AZ_INPUT_* and AZ_HEADS_TC configuration");
+    return net_forward_bf16(e, nullptr, nb.cap, policy_out, value_out, scatter, &nb);
 }
 
 }  // namespace azb
@@ -467,7 +551,22 @@ int az_load_weights(az_engine* e, const float* const* arrays, int n_arrays) {
     if (n_arrays != AZ_NUM_WEIGHT_ARRAYS) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "expected AZ_NUM_WEIGHT_ARRAYS tensors");
     for (int i = 0; i < n_arrays; i++) if (!arrays[i]) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "null weight tensor");
     cudaSetDevice(e->cfg.device);
-    return load_from_host(e, arrays);
+    return load_from_host(e, e->net, arrays);
+}
+
+int az_load_network(az_engine* e, int network, const float* const* arrays, int n_arrays) {
+    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+    if (network < 0 || network >= AZ_MAX_NETWORKS) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "network must be in [0, AZ_MAX_NETWORKS)");
+    if (network == 0) return az_load_weights(e, arrays, n_arrays);
+    if (!arrays) return AZ_ERR_INVALID_ARGUMENT;
+    if (n_arrays != AZ_NUM_WEIGHT_ARRAYS) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "expected AZ_NUM_WEIGHT_ARRAYS tensors");
+    for (int i = 0; i < n_arrays; i++) if (!arrays[i]) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "null weight tensor");
+    cudaSetDevice(e->cfg.device);
+    if (!e->net1) {
+        const int r = create_slot1(e);
+        if (r) return r;
+    }
+    return load_from_host(e, e->net1, arrays);
 }
 
 int az_load_weights_dev(az_engine* e, const float* const* arrays_dev, int n_arrays) {
@@ -481,7 +580,7 @@ int az_load_weights_dev(az_engine* e, const float* const* arrays_dev, int n_arra
         AZ_CUDA(e, cudaMemcpy(host[i].data(), arrays_dev[i], host[i].size() * 4, cudaMemcpyDeviceToHost));
         ptrs[i] = host[i].data();
     }
-    return load_from_host(e, ptrs.data());
+    return load_from_host(e, e->net, ptrs.data());
 }
 
 static int forward_common(az_engine* e, int n, float* policy_out, float* value_out) {
@@ -526,6 +625,52 @@ int az_forward(az_engine* e, int n, const az_position* pos, float* policy_out, f
     }
     if (r) return r;
     return forward_common(e, n, policy_out, value_out);
+}
+
+int az_forward_networks(az_engine* e, int n, const az_position* pos, const uint8_t* network, float* policy_out, float* value_out) {
+    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+    if (n < 0 || n > e->max_batch) return set_err(e, AZ_ERR_CAPACITY, "batch larger than az_config.max_batch");
+    if (n == 0) return AZ_OK;
+    if (!pos || !network || !policy_out || !value_out) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "null buffer");
+    int count[AZ_MAX_NETWORKS] = {0, 0};
+    for (int i = 0; i < n; i++) {
+        if (network[i] >= AZ_MAX_NETWORKS) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "network id must be < AZ_MAX_NETWORKS");
+        count[network[i]]++;
+    }
+    for (int s = 0; s < AZ_MAX_NETWORKS; s++) {
+        const NetWeights* w = net_slot(e, s);
+        if (count[s] && (!w || !w->loaded)) return set_err(e, AZ_ERR_NO_WEIGHTS, "a board names a network that has not been loaded");
+    }
+    // network ranges: network 0 at board 0, network 1 at the next multiple of 4 (a tile of the convolutions never mixes networks)
+    const int base1 = (count[0] + 3) & ~3;
+    if (base1 + ((count[1] + 3) & ~3) > e->max_batch) return set_err(e, AZ_ERR_CAPACITY, "network ranges exceed az_config.max_batch");
+    const int span = base1 + count[1];
+    std::vector<az_position> staged((size_t)span, pos[0]);   // the padding between the ranges is never evaluated
+    std::vector<int> slot(n);
+    int next[AZ_MAX_NETWORKS] = {0, base1};
+    for (int i = 0; i < n; i++) { slot[i] = next[network[i]]++; staged[slot[i]] = pos[i]; }
+    cudaSetDevice(e->cfg.device);
+    if (!e->d_net_counts) {
+        AZ_CUDA(e, cudaMalloc(&e->d_net_counts, AZ_MAX_NETWORKS * sizeof(int)));
+        AZ_CUDA(e, cudaMalloc(&e->d_net_slot, (size_t)e->max_batch * sizeof(int)));
+        AZ_CUDA(e, cudaMalloc(&e->d_net_value, (size_t)e->max_batch * sizeof(float)));
+    }
+    if (!e->d_scores) AZ_CUDA(e, cudaMalloc(&e->d_scores, (size_t)e->max_batch * AZ_ACTION_SPACE * 4));
+    AZ_CUDA(e, cudaMemcpyAsync(e->d_net_counts, count, sizeof count, cudaMemcpyHostToDevice, e->stream));
+    AZ_CUDA(e, cudaMemcpyAsync(e->d_net_slot, slot.data(), (size_t)n * sizeof(int), cudaMemcpyHostToDevice, e->stream));
+    AZ_CUDA(e, cudaMemcpyAsync(e->d_wire, staged.data(), (size_t)span * sizeof(az_position), cudaMemcpyHostToDevice, e->stream));
+    if (e->cfg.precision == 1) launch_encode_f32(e->stream, e->d_wire, e->d_planes, span);
+    else launch_encode_bf16_wire(e->stream, e->d_wire, e->net->a_in, span, e->net->in_ch);
+    const int r = net_forward_networks(e, NetBatch{e->d_net_counts, base1, span}, e->d_planes, e->d_policy, e->d_value);
+    if (r) return r;
+    // back to the caller's order (the scores export buffer holds the gathered policy rows)
+    e->n_launches++;
+    k_gather_rows<<<n, 256, 0, e->stream>>>(e->d_policy, e->d_value, e->d_net_slot, e->d_scores, e->d_net_value);
+    AZ_CUDA(e, cudaGetLastError());
+    AZ_CUDA(e, cudaMemcpyAsync(policy_out, e->d_scores, (size_t)n * AZ_ACTION_SPACE * 4, cudaMemcpyDeviceToHost, e->stream));
+    AZ_CUDA(e, cudaMemcpyAsync(value_out, e->d_net_value, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+    AZ_CUDA(e, cudaStreamSynchronize(e->stream));
+    return AZ_OK;
 }
 
 }  // extern "C"

@@ -15,6 +15,14 @@ struct HeadScatter {
     float* edge_P;
 };
 
+// Multi-network batch (az_forward_networks, az_search_networks): network 0 (e->net) owns boards [0, counts_dev[0]), network 1
+// (e->net1) owns [base1, base1 + counts_dev[1]); base1 is a multiple of 4 and base1 + the capacity of network 1's range <= cap
+struct NetBatch {
+    const int* counts_dev;   // [AZ_MAX_NETWORKS]
+    int base1;
+    int cap;
+};
+
 struct NetWeights {
     bool loaded = false;
     int max_boards = 0;
@@ -55,15 +63,27 @@ void net_destroy(az_engine* e);
 
 // Forward over boards whose bf16 NHWC planes are already in net->a_in (n read from n_dev when non-null).
 // policy_out [n][4096] f32 (nullable), value_out [n] f32.  Returns the buffer index holding the tower output.
-int net_forward_bf16(az_engine* e, const int* n_dev, int n_static, float* policy_out, float* value_out, const HeadScatter* scatter = nullptr);
+int net_forward_bf16(az_engine* e, const int* n_dev, int n_static, float* policy_out, float* value_out, const HeadScatter* scatter = nullptr,
+                     const NetBatch* nb = nullptr);
 // fp32 parity path from NCHW f32 planes [n][19][64]
-int net_forward_fp32(az_engine* e, const float* planes, const int* n_dev, int n_static, float* policy_out, float* value_out);
+int net_forward_fp32(az_engine* e, const float* planes, const int* n_dev, int n_static, float* policy_out, float* value_out,
+                     const NetWeights* wts = nullptr /* the weights of another slot; activations are always e->net's */);
 // fused heads on warp-level tensor-core MMAs (nn_heads.cu); tower = NHWC bf16 [n][64][128]
 int launch_heads_mma(az_engine* e, const __nv_bfloat16* tower, const int* n_dev, int n_static, float* policy_out, float* value_out,
                      const HeadScatter* scatter);
 // the same heads on tcgen05 (nn_heads_tc.cu, AZ_HEADS_TC=1): tiles of two boards, stage 1 and 2 as UMMA, softmax per pixel thread
 int launch_heads_tc(az_engine* e, const CUtensorMap* act_rows_map, const int* n_dev, int n_static, float* policy_out, float* value_out,
                     const HeadScatter* scatter);
+struct NetWeights;
+// the heads of a multi-network batch on tcgen05 (k_heads_tc_nets): the CTAs are split between the networks
+int launch_heads_tc_nets(az_engine* e, const NetWeights* w0, const NetWeights* w1, const CUtensorMap* act_rows_map, const int* counts_dev,
+                         int base1, int n_max, float* policy_out, float* value_out, const HeadScatter* scatter);
+// the forward of a multi-network batch: bf16 with the default configuration in one set of launches shared by the networks
+// (net_forward_bf16 with nb), otherwise and on the fp32 path one network after the other over its range
+int net_forward_networks(az_engine* e, const NetBatch& nb, const float* planes_f32, float* policy_out, float* value_out,
+                         const HeadScatter* scatter = nullptr);
+// network slot s (0: e->net, 1: e->net1, null until its first load)
+NetWeights* net_slot(az_engine* e, int s);
 // f32 NCHW planes -> bf16 NHWC (`ch` = 64 or 32 channels per square) into net->a_in
 void launch_planes_to_bf16(cudaStream_t s, const float* planes, __nv_bfloat16* out, int n, int ch);
 // positions -> bf16 NHWC planes (to_tensor fused with the layout the first convolution wants)

@@ -112,11 +112,42 @@ __device__ __forceinline__ void htc_mma_16816(float* d, uint32_t a0, uint32_t a1
 #define HTC_T(i) do { } while (0)
 #endif
 
-__global__ void __launch_bounds__(htc::kThreads, 1)
-k_heads_tc(const __grid_constant__ CUtensorMap act_map, const __nv_bfloat16* __restrict__ w40, const float* __restrict__ b40,
-           const __nv_bfloat16* __restrict__ wp2, const float* __restrict__ bp2, const __nv_bfloat16* __restrict__ wl1t,
-           const float* __restrict__ bl1, const float* __restrict__ wl2, const float* __restrict__ bl2, float* __restrict__ policy_out,
-           float* __restrict__ value_out, const int* __restrict__ n_dev, int n_static, HeadScatter sc) {
+// Which tiles a CTA computes and with which weights.  HeadsSched<false> is the single-network launch (its expressions are those
+// the kernel has always had, so its code is unchanged); HeadsSched<true> a multi-network batch (net_part in tc_conv.cuh): the
+// CTAs are split between the networks, and a CTA stages and reads only its own network's weights.
+struct HeadNets {
+    const int* counts;   // device [2]: boards of each network
+    int base1;           // first board of network 1
+    const __nv_bfloat16 *w40, *wp2, *wl1t;   // network 1's weights (the parameters of k_heads_tc)
+    const float *b40, *bp2, *bl1, *wl2, *bl2;
+};
+template <bool NETS> struct HeadsSched;
+template <> struct HeadsSched<false> {
+    __device__ __forceinline__ explicit HeadsSched(const HeadNets&) {}
+    template <class T> __device__ __forceinline__ const T* pick(const T* w0, const T*) const { return w0; }
+    __device__ __forceinline__ int n(const int* n_dev, int n_static) const { return n_dev ? *n_dev : n_static; }
+    __device__ __forceinline__ int n_tiles(int n) const { return (n + 1) >> 1; }
+    __device__ __forceinline__ int tile0() const { return 0; }
+    __device__ __forceinline__ int cta() const { return (int)blockIdx.x; }
+    __device__ __forceinline__ int ncta() const { return (int)gridDim.x; }
+};
+template <> struct HeadsSched<true> {
+    NetPart np;
+    __device__ __forceinline__ explicit HeadsSched(const HeadNets& h) : np(net_part(h.counts, h.base1, gridDim.x, blockIdx.x, 2)) {}
+    template <class T> __device__ __forceinline__ const T* pick(const T* w0, const T* w1) const { return np.net ? w1 : w0; }
+    __device__ __forceinline__ int n(const int*, int) const { return np.end_board; }
+    __device__ __forceinline__ int n_tiles(int) const { return np.n_tiles; }
+    __device__ __forceinline__ int tile0() const { return np.first_tile; }
+    __device__ __forceinline__ int cta() const { return np.unit; }
+    __device__ __forceinline__ int ncta() const { return np.units; }
+};
+
+template <bool NETS>
+__device__ __forceinline__ void heads_tc_body(const CUtensorMap& act_map, const __nv_bfloat16* __restrict__ w40, const float* __restrict__ b40,
+                                              const __nv_bfloat16* __restrict__ wp2, const float* __restrict__ bp2, const __nv_bfloat16* __restrict__ wl1t,
+                                              const float* __restrict__ bl1, const float* __restrict__ wl2, const float* __restrict__ bl2,
+                                              float* __restrict__ policy_out, float* __restrict__ value_out, const int* __restrict__ n_dev,
+                                              int n_static, const HeadScatter& sc, const HeadNets& nets) {
     using namespace htc;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -141,6 +172,9 @@ k_heads_tc(const __grid_constant__ CUtensorMap act_map, const __nv_bfloat16* __r
     const long long tbegin = tlast;
 #endif
     const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
+    const HeadsSched<NETS> sched(nets);
+    w40 = sched.pick(w40, nets.w40); b40 = sched.pick(b40, nets.b40); wp2 = sched.pick(wp2, nets.wp2); bp2 = sched.pick(bp2, nets.bp2);
+    wl1t = sched.pick(wl1t, nets.wl1t); bl1 = sched.pick(bl1, nets.bl1); wl2 = sched.pick(wl2, nets.wl2); bl2 = sched.pick(bl2, nets.bl2);
     // The weight tiles are requested first and stored after everything that needs the board count: the count is a dependent
     // global load itself (the search kernel's batch counter), and the two round trips would otherwise add up in every thread
     uint4 wreg[2] = {make_uint4(0, 0, 0, 0), make_uint4(0, 0, 0, 0)}, w2reg = make_uint4(0, 0, 0, 0);
@@ -153,9 +187,9 @@ k_heads_tc(const __grid_constant__ CUtensorMap act_map, const __nv_bfloat16* __r
     float breg = 0.0f;
     if (t < 40) breg = b40[t];
     else if (t >= 64 && t < 128) breg = bp2[t - 64];
-    const int n = n_dev ? *n_dev : n_static;
-    const int n_tiles = (n + 1) >> 1;
-    const int my_tiles = (int)blockIdx.x < n_tiles ? (n_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
+    const int n = sched.n(n_dev, n_static);
+    const int n_tiles = sched.n_tiles(n);
+    const int my_tiles = sched.cta() < n_tiles ? (n_tiles - sched.cta() + sched.ncta() - 1) / sched.ncta() : 0;
 
     // ---- epilogue thread coordinates (warps 2..17); computed here because the scatter metadata of the first two tiles is requested
     // before the set-up below, so that its (TLB-missing, ~3 us) latency overlaps the weight staging and the first TMA / MMA round trip
@@ -178,7 +212,7 @@ k_heads_tc(const __grid_constant__ CUtensorMap act_map, const __nv_bfloat16* __r
     auto meta = [&](int j, unsigned long long& eo, int& L) {
         eo = 0; L = 0;
         if (sc.edge_P && j < nw) {
-            const int b = ((int)blockIdx.x + (2 * j + w) * (int)gridDim.x) * 2 + bi;
+            const int b = (sched.tile0() + sched.cta() + (2 * j + w) * sched.ncta()) * 2 + bi;
             if (b < n) { eo = sc.edge_off[b]; L = sc.n_edges[b]; }
         }
     };
@@ -193,7 +227,7 @@ k_heads_tc(const __grid_constant__ CUtensorMap act_map, const __nv_bfloat16* __r
         fence_barrier_init();
         // the first tiles are requested before the weights are staged and the block synchronises: their latency hides behind the set-up
         for (int k = 0; k < kStages && k < my_tiles; k++) {
-            const int tile = (int)blockIdx.x + k * (int)gridDim.x;
+            const int tile = sched.tile0() + sched.cta() + k * sched.ncta();
             mbar_arrive_expect_tx(&a_full[k], kStageBytes);
             tma1_load_2d(smem + kOffA + k * kStageBytes, &act_map, &a_full[k], 0, tile * 128);
             tma1_load_2d(smem + kOffA + k * kStageBytes + 16384, &act_map, &a_full[k], 64, tile * 128);
@@ -226,7 +260,7 @@ k_heads_tc(const __grid_constant__ CUtensorMap act_map, const __nv_bfloat16* __r
         // ---------------------------------------------------------------- TMA producer
         int stage = 0; uint32_t phase = 1;   // the first kStages tiles were requested during the set-up
         for (int k = kStages; k < my_tiles; k++) {
-            const int tile = (int)blockIdx.x + k * (int)gridDim.x;
+            const int tile = sched.tile0() + sched.cta() + k * sched.ncta();
             mbar_wait(&a_empty[stage], phase ^ 1, 21);
             HTC_T(1);
             if (elect_one()) {
@@ -348,7 +382,7 @@ k_heads_tc(const __grid_constant__ CUtensorMap act_map, const __nv_bfloat16* __r
         // stage 2 of tile j: D2 -> bias -> softmax over the board (a team of four warps) -> priors / dense policy row
         auto epi2 = [&](int j) {
             const int k = 2 * j + w, slot = j & 1;
-            const int b = ((int)blockIdx.x + k * (int)gridDim.x) * 2 + bi;
+            const int b = (sched.tile0() + sched.cta() + k * sched.ncta()) * 2 + bi;
             const bool active = b < n;
             // rotate the prefetched metadata HERE, a whole tile after the loads were issued (rotating at the end of the previous
             // stage 2 made the register moves wait for loads issued a few thousand clocks earlier)
@@ -476,7 +510,7 @@ k_heads_tc(const __grid_constant__ CUtensorMap act_map, const __nv_bfloat16* __r
             named_bar_sync(1, kEpiThreads);
             if (et < 32) {
                 const int k = g0 + (et >> 1);
-                const int b = ((int)blockIdx.x + k * (int)gridDim.x) * 2 + (et & 1);
+                const int b = (sched.tile0() + sched.cta() + k * sched.ncta()) * 2 + (et & 1);
                 if (k < my_tiles && b < n) value_out[b] = tanhf(bl2[0] + s_vsum[et * 2] + s_vsum[et * 2 + 1]);
             }
             HTC_T(14);
@@ -494,6 +528,23 @@ k_heads_tc(const __grid_constant__ CUtensorMap act_map, const __nv_bfloat16* __r
     if (warp == 1) { tc_fence_after(); tmem1_dealloc(tmem_base, kTmemCols); }
 }
 
+__global__ void __launch_bounds__(htc::kThreads, 1)
+k_heads_tc(const __grid_constant__ CUtensorMap act_map, const __nv_bfloat16* __restrict__ w40, const float* __restrict__ b40,
+           const __nv_bfloat16* __restrict__ wp2, const float* __restrict__ bp2, const __nv_bfloat16* __restrict__ wl1t,
+           const float* __restrict__ bl1, const float* __restrict__ wl2, const float* __restrict__ bl2, float* __restrict__ policy_out,
+           float* __restrict__ value_out, const int* __restrict__ n_dev, int n_static, HeadScatter sc) {
+    heads_tc_body<false>(act_map, w40, b40, wp2, bp2, wl1t, bl1, wl2, bl2, policy_out, value_out, n_dev, n_static, sc, HeadNets{});
+}
+
+// the heads of a multi-network batch (the weight parameters are network 0's, `nets` holds network 1's and the board ranges)
+__global__ void __launch_bounds__(htc::kThreads, 1)
+k_heads_tc_nets(const __grid_constant__ CUtensorMap act_map, const __nv_bfloat16* __restrict__ w40, const float* __restrict__ b40,
+                const __nv_bfloat16* __restrict__ wp2, const float* __restrict__ bp2, const __nv_bfloat16* __restrict__ wl1t,
+                const float* __restrict__ bl1, const float* __restrict__ wl2, const float* __restrict__ bl2, float* __restrict__ policy_out,
+                float* __restrict__ value_out, HeadScatter sc, const HeadNets nets) {
+    heads_tc_body<true>(act_map, w40, b40, wp2, bp2, wl1t, bl1, wl2, bl2, policy_out, value_out, nullptr, 0, sc, nets);
+}
+
 int launch_heads_tc(az_engine* e, const CUtensorMap* act_map, const int* n_dev, int n_static, float* policy_out, float* value_out,
                     const HeadScatter* scatter) {
     NetWeights* w = e->net;
@@ -507,6 +558,20 @@ int launch_heads_tc(az_engine* e, const CUtensorMap* act_map, const int* n_dev, 
     k_heads_tc<<<grid, htc::kThreads, htc::kTotal, e->stream>>>(*act_map, w->h_w40, w->f_b40, w->h_wp2, w->f_bp2, w->h_wl1t, w->f_bl1, w->f_wl2,
                                                                w->f_bl2, policy_out, value_out, n_dev, n_static, sc);
     return check_cuda(e, cudaGetLastError(), "k_heads_tc");
+}
+
+int launch_heads_tc_nets(az_engine* e, const NetWeights* w, const NetWeights* w1, const CUtensorMap* act_map, const int* counts_dev, int base1,
+                         int n_max, float* policy_out, float* value_out, const HeadScatter* scatter) {
+    if (n_max <= 0) return 0;
+    const int grid = std::max(2, std::min((n_max + 1) / 2, e->sm_count));   // one CTA per network at least
+    static PerDeviceOnce once;
+    if (once.first()) cudaFuncSetAttribute(k_heads_tc_nets, cudaFuncAttributeMaxDynamicSharedMemorySize, htc::kTotal);
+    HeadScatter sc{nullptr, nullptr, nullptr, nullptr};
+    if (scatter) sc = *scatter;
+    const HeadNets hn{counts_dev, base1, w1->h_w40, w1->h_wp2, w1->h_wl1t, w1->f_b40, w1->f_bp2, w1->f_bl1, w1->f_wl2, w1->f_bl2};
+    k_heads_tc_nets<<<grid, htc::kThreads, htc::kTotal, e->stream>>>(*act_map, w->h_w40, w->f_b40, w->h_wp2, w->f_bp2, w->h_wl1t, w->f_bl1,
+                                                                    w->f_wl2, w->f_bl2, policy_out, value_out, sc, hn);
+    return check_cuda(e, cudaGetLastError(), "k_heads_tc_nets");
 }
 
 }  // namespace azb

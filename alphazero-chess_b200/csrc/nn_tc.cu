@@ -28,6 +28,9 @@
 
 namespace azb {
 
+// defined before anything that prints, so that the module lists it where it has always been (first)
+__device__ const char kTowerTimeoutMsg[] = "azb: tower epilogue wait timeout\n";
+
 constexpr int kWTileBytes = 64 * 128;    // 64 output channels x 64 input channels bf16
 
 // KROW = bytes per operand row in shared memory = input channels per K block x 2: 128 (64 channels, 128-byte swizzle) for the
@@ -71,11 +74,41 @@ static_assert(kEpiWarps == 8 || kEpiWarps == 16, "epilogue warps: 8 or 16");
 // GROUPS = 2 (the input convolution): two sets of epilogue warps take alternate tiles (set g always drains TMEM buffer g), so the
 // epilogues of consecutive tiles overlap in time.  The layer is bound by the latency of one tile's epilogue (wait, tcgen05.ld,
 // bias / ReLU / pack, stores), not by its width, which is why splitting one tile over 16 warps did not help (profiles/r2_ab.md 4).
-template <int HALVES, int KROW, int WIDE = 0, int GROUPS = 1>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(64 + GROUPS * kEpiThreads, 1)
-conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_constant__ CUtensorMap w_map,
-                   const float* __restrict__ bias, const __nv_bfloat16* __restrict__ residual,
-                   __nv_bfloat16* __restrict__ out, const int* __restrict__ n_boards_ptr, int n_boards_static, int relu, int dbg) {
+// Which tiles a CTA pair computes, and with which weights.  ConvSched<false> is the single-network launch (its expressions are
+// those the kernel has always had, so its code is unchanged); ConvSched<true> a multi-network batch (net_part in tc_conv.cuh).
+struct ConvNets {
+    const int* counts;   // device [2]: boards of each network
+    int base1;           // first board of network 1
+    const CUtensorMap* w_map1;
+    const float* bias1;
+};
+template <bool NETS> struct ConvSched;
+template <> struct ConvSched<false> {
+    __device__ __forceinline__ explicit ConvSched(const ConvNets&) {}
+    __device__ __forceinline__ int n_boards(const int* n_boards_ptr, int n_boards_static) const { return n_boards_ptr ? *n_boards_ptr : n_boards_static; }
+    __device__ __forceinline__ int n_tiles(int n_boards) const { return (n_boards + 3) >> 2; }
+    __device__ __forceinline__ int first_tile() const { return blockIdx.x >> 1; }
+    __device__ __forceinline__ int tile_step() const { return gridDim.x >> 1; }
+    __device__ __forceinline__ const CUtensorMap* w_map(const CUtensorMap* w0) const { return w0; }
+    __device__ __forceinline__ const float* bias(const float* b0) const { return b0; }
+};
+template <> struct ConvSched<true> {
+    NetPart np;
+    const ConvNets& nets;
+    __device__ __forceinline__ explicit ConvSched(const ConvNets& n) : np(net_part(n.counts, n.base1, gridDim.x >> 1, blockIdx.x >> 1, 4)), nets(n) {}
+    __device__ __forceinline__ int n_boards(const int*, int) const { return np.end_board; }
+    __device__ __forceinline__ int n_tiles(int) const { return np.first_tile + np.n_tiles; }
+    __device__ __forceinline__ int first_tile() const { return np.first_tile + np.unit; }
+    __device__ __forceinline__ int tile_step() const { return np.units; }
+    __device__ __forceinline__ const CUtensorMap* w_map(const CUtensorMap* w0) const { return np.net ? nets.w_map1 : w0; }
+    __device__ __forceinline__ const float* bias(const float* b0) const { return np.net ? nets.bias1 : b0; }
+};
+
+template <int HALVES, int KROW, int WIDE, int GROUPS, bool NETS>
+__device__ __forceinline__ void conv3x3_tc2_body(const CUtensorMap& in_map, const CUtensorMap* w_map_p, const float* __restrict__ bias,
+                                                 const __nv_bfloat16* __restrict__ residual, __nv_bfloat16* __restrict__ out,
+                                                 const int* __restrict__ n_boards_ptr, int n_boards_static, int relu, int dbg,
+                                                 const ConvNets& nets) {
     using S = ConvSmem<HALVES, KROW, WIDE>;
     constexpr int kStageBytes = S::kStageB, kWTileBytes = S::kWTileB;   // shadow the 128-byte-row constants of the tower
     constexpr int KSTEPS = KROW / 32;                                   // K = 16 elements = 32 bytes per MMA
@@ -95,9 +128,12 @@ conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t rank = cluster_ctarank();
-    const int n_boards = n_boards_ptr ? *n_boards_ptr : n_boards_static;
-    const int n_tiles = (n_boards + 3) >> 2;
-    const int first_tile = blockIdx.x >> 1, tile_step = gridDim.x >> 1;
+    const ConvSched<NETS> sched(nets);
+    const int n_boards = sched.n_boards(n_boards_ptr, n_boards_static);
+    const int n_tiles = sched.n_tiles(n_boards);
+    const int first_tile = sched.first_tile(), tile_step = sched.tile_step();
+    const CUtensorMap& w_map = *sched.w_map(w_map_p);
+    bias = sched.bias(bias);
 
     if (threadIdx.x == 0) {
         tma_prefetch_desc(&in_map);
@@ -307,6 +343,24 @@ conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
     if (warp == 1) { tc_fence_after(); tmem2_dealloc(tmem_base, kTmemCols2); }
 }
 
+template <int HALVES, int KROW, int WIDE = 0, int GROUPS = 1>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(64 + GROUPS * kEpiThreads, 1)
+conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_constant__ CUtensorMap w_map,
+                   const float* __restrict__ bias, const __nv_bfloat16* __restrict__ residual,
+                   __nv_bfloat16* __restrict__ out, const int* __restrict__ n_boards_ptr, int n_boards_static, int relu, int dbg) {
+    conv3x3_tc2_body<HALVES, KROW, WIDE, GROUPS, false>(in_map, &w_map, bias, residual, out, n_boards_ptr, n_boards_static, relu, dbg,
+                                                        ConvNets{nullptr, 0, nullptr, nullptr});
+}
+
+// the input convolution of a multi-network batch: the CTA pairs are split between the two networks' weights (ConvSched<true>)
+template <int HALVES, int KROW>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads2, 1)
+conv3x3_tc2_nets_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_constant__ CUtensorMap w_map,
+                        const __grid_constant__ CUtensorMap w_map1, const float* __restrict__ bias, const float* __restrict__ bias1,
+                        __nv_bfloat16* __restrict__ out, const int* __restrict__ counts, int base1, int dbg) {
+    conv3x3_tc2_body<HALVES, KROW, 0, 1, true>(in_map, &w_map, bias, nullptr, out, nullptr, 0, 1, dbg, ConvNets{counts, base1, &w_map1, bias1});
+}
+
 // ================================================================================================================
 // Fused residual tower: all 20 3x3 convolutions (agent.rs:118-120) in ONE persistent launch.
 // A convolution is local to a board, and a CTA pair keeps the same boards in every layer, so no grid-wide
@@ -334,9 +388,50 @@ struct TowerParams {
 
 // WIDE = 1 (AZ_TOWER_WIDE): one TMA box per channel half serves the three horizontal taps (see ConvSmem): a third of the L2 -> shared
 // memory traffic and of the TMA instructions; the activation maps are then maps[25..27] (16-file boxes) and there is no stem.
-template <int WIDE>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads2, 1)
-conv_tower_kernel(const TowerParams prm) {
+// Which tiles a CTA pair computes, in which ranges, with which weights (as ConvSched): TowerSched<false> is the single-network
+// launch, TowerSched<true> a multi-network batch.  There a network's pairs walk its tiles in ranges of at most 7 rounds (>= 6 tiles
+// per pair when it has them), the sizing of the single-network launch (net_forward_bf16), so that the ranges the two networks
+// work on at the same time hold about as many boards as one range of the single-network launch and stay in the L2 together.
+struct TowerNets {
+    const int* counts;   // device [2]: boards of each network
+    int base1;           // first board of network 1
+    const CUtensorMap* maps1;   // network 1's device maps: the activation maps of TowerParams::maps and its own weights
+    const float* bias1;
+};
+template <bool NETS> struct TowerSched;
+template <> struct TowerSched<false> {
+    __device__ __forceinline__ TowerSched(const TowerParams&, const TowerNets&) {}
+    __device__ __forceinline__ int n_boards(const TowerParams& prm) const { return prm.n_boards_ptr ? *prm.n_boards_ptr : prm.n_boards_static; }
+    __device__ __forceinline__ int n_tiles(const TowerParams& prm, int n_boards) const { return min((n_boards + 3) >> 2, prm.tile_hi); }
+    __device__ __forceinline__ int tile_step() const { return gridDim.x >> 1; }
+    __device__ __forceinline__ int tile_lo(const TowerParams& prm) const { return prm.tile_lo; }
+    __device__ __forceinline__ int range_tiles(const TowerParams& prm) const { return prm.range_tiles; }
+    __device__ __forceinline__ int pair() const { return blockIdx.x >> 1; }
+    __device__ __forceinline__ const CUtensorMap* maps(const TowerParams& prm) const { return prm.maps; }
+    __device__ __forceinline__ const float* bias(const TowerParams& prm) const { return prm.bias; }
+};
+template <> struct TowerSched<true> {
+    NetPart np;
+    int per;
+    const TowerNets& nets;
+    __device__ __forceinline__ TowerSched(const TowerParams&, const TowerNets& n)
+        : np(net_part(n.counts, n.base1, gridDim.x >> 1, blockIdx.x >> 1, 4)), nets(n) {
+        int nr = max(1, (np.n_tiles + 7 * np.units - 1) / (7 * np.units));
+        if (np.n_tiles < 6 * np.units * nr) nr = max(1, np.n_tiles / (6 * np.units));
+        per = max(1, (np.n_tiles + nr - 1) / nr);
+    }
+    __device__ __forceinline__ int n_boards(const TowerParams&) const { return np.end_board; }
+    __device__ __forceinline__ int n_tiles(const TowerParams&, int) const { return np.first_tile + np.n_tiles; }
+    __device__ __forceinline__ int tile_step() const { return np.units; }
+    __device__ __forceinline__ int tile_lo(const TowerParams&) const { return np.first_tile; }
+    __device__ __forceinline__ int range_tiles(const TowerParams&) const { return per; }
+    __device__ __forceinline__ int pair() const { return np.unit; }
+    __device__ __forceinline__ const CUtensorMap* maps(const TowerParams& prm) const { return np.net ? nets.maps1 : prm.maps; }
+    __device__ __forceinline__ const float* bias(const TowerParams& prm) const { return np.net ? nets.bias1 : prm.bias; }
+};
+
+template <int WIDE, bool NETS>
+__device__ __forceinline__ void conv_tower_body(const TowerParams& prm, const TowerNets& nets) {
     using S = ConvSmem<2, 128, WIDE>;
     constexpr int kStageBytes = S::kStageB;
     constexpr int NS = S::kStages;
@@ -357,17 +452,18 @@ conv_tower_kernel(const TowerParams prm) {
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t rank = cluster_ctarank();
-    const int n_boards = prm.n_boards_ptr ? *prm.n_boards_ptr : prm.n_boards_static;
-    const int n_tiles = min((n_boards + 3) >> 2, prm.tile_hi);
-    const int tile_step = gridDim.x >> 1;
-    const int n_ranges = n_tiles > prm.tile_lo ? (n_tiles - prm.tile_lo + prm.range_tiles - 1) / prm.range_tiles : 0;
+    const TowerSched<NETS> sched(prm, nets);
+    const int n_boards = sched.n_boards(prm);
+    const int n_tiles = sched.n_tiles(prm, n_boards);
+    const int tile_step = sched.tile_step();
+    const int n_ranges = n_tiles > sched.tile_lo(prm) ? (n_tiles - sched.tile_lo(prm) + sched.range_tiles(prm) - 1) / sched.range_tiles(prm) : 0;
     // Per range r every role derives the same numbers: the pair's first tile, its tile count T (ranges without tiles for
     // this pair are skipped by all roles alike), and three running counters -- u0 / u1 = how often the weight groups of
     // channel half 0 / 1 have been loaded so far (barrier parities), cum = tiles this pair finished in earlier ranges.
 #define TOWER_RANGE_BEGIN()                                                                                      \
-    const int range_lo = prm.tile_lo + rg * prm.range_tiles;                                                      \
-    const int range_hi = min(n_tiles, range_lo + prm.range_tiles);                                               \
-    const int first_tile = range_lo + (blockIdx.x >> 1);                                                         \
+    const int range_lo = sched.tile_lo(prm) + rg * sched.range_tiles(prm);                                        \
+    const int range_hi = min(n_tiles, range_lo + sched.range_tiles(prm));                                        \
+    const int first_tile = range_lo + sched.pair();                                                              \
     const int T = first_tile < range_hi ? (range_hi - first_tile + tile_step - 1) / tile_step : 0;               \
     if (T == 0) continue;
     const int stem = prm.stem;
@@ -399,8 +495,8 @@ conv_tower_kernel(const TowerParams prm) {
             const int layer = L - stem;
             const int blk_second = layer >= 0 ? (layer & 1) : 0;
             const int in_buf = blk_second ? 1 : 0;   // block input in act[0], conv1 output in act[1], conv2 back into act[0]
-            const CUtensorMap* in_map = layer >= 0 ? &prm.maps[(WIDE == 2 ? 28 : WIDE ? 25 : 0) + in_buf] : &prm.maps[23];
-            const CUtensorMap* w_map = layer >= 0 ? &prm.maps[3 + layer] : &prm.maps[24];
+            const CUtensorMap* in_map = layer >= 0 ? &sched.maps(prm)[(WIDE == 2 ? 28 : WIDE ? 25 : 0) + in_buf] : &sched.maps(prm)[23];
+            const CUtensorMap* w_map = layer >= 0 ? &sched.maps(prm)[3 + layer] : &sched.maps(prm)[24];
             const int halves = layer >= 0 ? 2 : 1;
             for (int i = 0; i < T; i++) {
                 const int t = first_tile + i * tile_step;
@@ -410,7 +506,7 @@ conv_tower_kernel(const TowerParams prm) {
                     for (;;) {
                         bool ok = lane >= kEpiWarps || epi_done[lane & (kEpiWarps - 1)] >= need;
                         if (__all_sync(0xffffffffu, ok)) break;
-                        if (clock64() - t0 > 4000000000LL) { if (lane == 0) printf("azb: tower epilogue wait timeout\n"); __trap(); }
+                        if (clock64() - t0 > 4000000000LL) { if (lane == 0) printf(kTowerTimeoutMsg); __trap(); }
                     }
                     fence_proxy_async();
                 }
@@ -523,7 +619,7 @@ conv_tower_kernel(const TowerParams prm) {
             const __nv_bfloat16* residual = blk_second ? prm.act[0] : nullptr;
             // the epilogue warps switch layers together: whoever arrives refills the buffer last used two layers ago
             if (threadIdx.x - 64 < 128)
-                bias_s[(g & 1) * 128 + threadIdx.x - 64] = prm.bias[(layer >= 0 ? layer : prm.n_layers) * 128 + threadIdx.x - 64];
+                bias_s[(g & 1) * 128 + threadIdx.x - 64] = sched.bias(prm)[(layer >= 0 ? layer : prm.n_layers) * 128 + threadIdx.x - 64];
             asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory");
             const float* bias = bias_s + (g & 1) * 128 + cg * kEpiCols;
             for (int i = 0; i < T; i++, lt++) {
@@ -603,6 +699,20 @@ conv_tower_kernel(const TowerParams prm) {
     if (warp == 1) { tc_fence_after(); tmem2_dealloc(tmem_base, kTmemCols2); }
 }
 
+template <int WIDE>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads2, 1)
+conv_tower_kernel(const TowerParams prm) {
+    conv_tower_body<WIDE, false>(prm, TowerNets{nullptr, 0, nullptr, nullptr});
+}
+
+// the tower of a multi-network batch: the CTA pairs are split between the two networks' weights (TowerSched<true>); the per-tile
+// work is that of conv_tower_kernel, so a board's activations do not depend on the pair that computed them
+template <int WIDE>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads2, 1)
+conv_tower_nets_kernel(const TowerParams prm, const TowerNets nets) {
+    conv_tower_body<WIDE, true>(prm, nets);
+}
+
 int tc_tower_launch(cudaStream_t stream, const CUtensorMap* maps_dev, const float* bias, void* const* act, const int* n_boards_dev,
                     int n_boards_static, int n_layers, int stem, int grid, int tile_lo, int tile_hi, int range_tiles, int release_arrive,
                     int wide, int l2_hint) {
@@ -625,6 +735,38 @@ int tc_tower_launch(cudaStream_t stream, const CUtensorMap* maps_dev, const floa
     if (wide == 2) conv_tower_kernel<2><<<grid, kThreads2, ConvSmem<2, 128, 2>::kTotal, stream>>>(p);
     else if (wide) conv_tower_kernel<1><<<grid, kThreads2, ConvSmem<2, 128, 1>::kTotal, stream>>>(p);
     else conv_tower_kernel<0><<<grid, kThreads2, ConvSmem<2>::kTotal, stream>>>(p);
+    return cudaGetLastError() == cudaSuccess ? 0 : -4;
+}
+
+int tc_tower_nets_launch(cudaStream_t stream, const CUtensorMap* maps0_dev, const CUtensorMap* maps1_dev, const float* bias0,
+                         const float* bias1, void* const* act, const int* counts_dev, int base1, int grid, int release_arrive, int l2_hint) {
+    static PerDeviceOnce once;
+    if (once.first() &&
+        cudaFuncSetAttribute(conv_tower_nets_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, ConvSmem<2, 128, 2>::kTotal) != cudaSuccess)
+        return -2;
+    grid &= ~1;
+    if (grid < 4) return -3;   // at least one pair per network
+    TowerParams p;
+    p.maps = maps0_dev; p.bias = bias0;
+    for (int i = 0; i < 3; i++) p.act[i] = (__nv_bfloat16*)act[i];
+    p.n_boards_ptr = nullptr; p.n_boards_static = 0; p.n_layers = 20; p.stem = 0;
+    p.tile_lo = 0; p.tile_hi = 0x7FFFFFFF; p.range_tiles = 1;   // unused: the ranges follow from the device counts (TowerSched<true>)
+    p.release_arrive = release_arrive;
+    p.l2_hint = l2_hint;
+    conv_tower_nets_kernel<2><<<grid, kThreads2, ConvSmem<2, 128, 2>::kTotal, stream>>>(p, TowerNets{counts_dev, base1, maps1_dev, bias1});
+    return cudaGetLastError() == cudaSuccess ? 0 : -4;
+}
+
+int tc_conv3x3_nets_launch(cudaStream_t stream, const CUtensorMap* in_map, const CUtensorMap* w_map0, const CUtensorMap* w_map1,
+                           const float* bias0, const float* bias1, void* out, const int* counts_dev, int base1, int grid, int dbg) {
+    static PerDeviceOnce once;
+    if (once.first() &&
+        cudaFuncSetAttribute(conv3x3_tc2_nets_kernel<1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, ConvSmem<1, 64>::kTotal) != cudaSuccess)
+        return -2;
+    grid &= ~1;
+    if (grid < 4) return -3;
+    conv3x3_tc2_nets_kernel<1, 64><<<grid, kThreads2, ConvSmem<1, 64>::kTotal, stream>>>(*in_map, *w_map0, *w_map1, bias0, bias1,
+                                                                                         (__nv_bfloat16*)out, counts_dev, base1, dbg);
     return cudaGetLastError() == cudaSuccess ? 0 : -4;
 }
 

@@ -17,4 +17,11 @@ int tc_conv3x3_launch(cudaStream_t stream, const CUtensorMap* in_map, const CUte
 int tc_tower_launch(cudaStream_t stream, const CUtensorMap* maps_dev, const float* bias, void* const* act, const int* n_boards_dev,
                     int n_boards_static, int n_layers, int stem, int grid, int tile_lo = 0, int tile_hi = 0x7FFFFFFF, int range_tiles = 0,
                     int release_arrive = 0, int wide = 0, int l2_hint = 0);   // wide: one 16-file box per channel half (maps_dev[25..27])
+// Multi-network batches (tc_conv.cuh, net_part): network 0 owns boards [0, counts_dev[0]), network 1 [base1, base1 + counts_dev[1]),
+// base1 a multiple of 4.  The 32-channel input convolution (w_map0 / w_map1 and bias0 / bias1 of the two networks, output bias
+// + ReLU) and the 10-file-box tower (maps0_dev / maps1_dev: the maps array of tc_tower_launch of each network).
+int tc_conv3x3_nets_launch(cudaStream_t stream, const CUtensorMap* in_map, const CUtensorMap* w_map0, const CUtensorMap* w_map1,
+                           const float* bias0, const float* bias1, void* out, const int* counts_dev, int base1, int grid, int dbg = 0);
+int tc_tower_nets_launch(cudaStream_t stream, const CUtensorMap* maps0_dev, const CUtensorMap* maps1_dev, const float* bias0,
+                         const float* bias1, void* const* act, const int* counts_dev, int base1, int grid, int release_arrive, int l2_hint);
 }  // namespace azb

@@ -192,4 +192,32 @@ __device__ __forceinline__ void tma2_load_4d_hint(void* smem_dst, const CUtensor
         : "memory");
 }
 
+// ---------------------------------------------------------------- multi-network batches (az_forward_networks, az_search_networks)
+// Network s owns boards [base_s, base_s + count_s): base_0 = 0, base_1 a multiple of 4, the counts in device memory.  The
+// persistent grid's `units` (CTA pairs of the convolutions, CTAs of the heads) are split between the networks in proportion to
+// their tiles of `tile_boards` boards, with at least one unit for each network that has boards.  Every CTA derives the same
+// split, so a unit only ever streams the weights of its own network and walks that network's tiles.
+struct NetPart {
+    int net;          // network of this unit
+    int unit, units;  // this unit's index among the network's units, and their number
+    int first_tile;   // the network's first tile (base_s / tile_boards)
+    int n_tiles;      // the network's tiles
+    int end_board;    // base_s + count_s
+};
+__device__ __forceinline__ NetPart net_part(const int* counts, int base1, int units, int unit, int tile_boards) {
+    const int c0 = counts[0], c1 = counts[1];
+    const int t0 = (c0 + tile_boards - 1) / tile_boards, t1 = (c1 + tile_boards - 1) / tile_boards;
+    int u0 = t1 == 0 ? units : t0 == 0 ? 0 : (int)(((long long)units * t0 + (t0 + t1) / 2) / (t0 + t1));
+    if (t0 > 0 && t1 > 0) u0 = min(max(u0, 1), units - 1);
+    NetPart p;
+    p.net = unit >= u0 ? 1 : 0;
+    p.unit = p.net ? unit - u0 : unit;
+    p.units = p.net ? units - u0 : u0;
+    const int base = p.net ? base1 : 0;
+    p.first_tile = base / tile_boards;
+    p.n_tiles = p.net ? t1 : t0;
+    p.end_board = base + (p.net ? c1 : c0);
+    return p;
+}
+
 }  // namespace azb

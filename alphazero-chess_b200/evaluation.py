@@ -41,48 +41,100 @@ def _weighted_index(weights, u):
     return idx if idx < len(weights) else int(np.flatnonzero(weights > 0).max())
 
 
+def _stack_histories(histories):
+    hist = np.concatenate(histories)
+    offs = np.zeros(len(histories) + 1, np.uint32)
+    offs[1:] = np.cumsum([len(h) for h in histories])
+    return hist, offs
+
+
+def _choose_from_visits(visits, stochastic, seed, game_ids, plies):
+    out = []
+    for k in range(len(visits)):
+        w = visits[k] / visits[k].sum()
+        out.append(_weighted_index(w, _uniform(seed, game_ids[k], plies[k])) if stochastic[k] else _last_argmax(w))
+    return out
+
+
+def _choose_from_policy(policy, index, count, stochastic, seed, game_ids, plies):
+    out = []
+    for k in range(len(policy)):
+        masked = np.zeros(ACTION_SPACE, np.float32)
+        legal = index[k, : count[k]]
+        masked[legal] = policy[k, legal]
+        out.append(_weighted_index(masked, _uniform(seed, game_ids[k], plies[k])) if stochastic[k] else _last_argmax(masked))
+    return out
+
+
 class MctsPlayer:
     """Player::MctsModel: MCTree::init(model, state, false) + search, then argmax or sampling (validation.rs:293-308).
     leaves_per_root > 1 searches with virtual loss (Engine.search_vl, not in the reference): up to that many leaves per
-    root share one network round, which cuts the latency of searches over few roots."""
+    root share one network round, which cuts the latency of searches over few roots.  `network` names the engine's network
+    slot (Engine.load_weights(..., network)); a non-zero slot searches through Engine.search_networks."""
 
-    def __init__(self, engine, num_simulations=None, leaves_per_root=1, virtual_loss=1.0):
+    def __init__(self, engine, num_simulations=None, leaves_per_root=1, virtual_loss=1.0, network=0):
         self.engine, self.sims = engine, num_simulations
         self.leaves_per_root, self.virtual_loss = int(leaves_per_root), float(virtual_loss)
+        self.network = int(network)
+
+    def _num_simulations(self):
+        return int(self.sims or self.engine.config.num_simulations)
 
     def choose(self, positions, histories, fullmoves, stochastic, seed, game_ids, plies):
-        hist = np.concatenate(histories)
-        offs = np.zeros(len(histories) + 1, np.uint32)
-        offs[1:] = np.cumsum([len(h) for h in histories])
-        if self.leaves_per_root > 1:
-            sims = int(self.sims or self.engine.config.num_simulations)
-            visits, _, _, _ = self.engine.search_vl(positions, sims, self.leaves_per_root, self.virtual_loss, history=hist,
-                                                    hist_offsets=offs)
+        hist, offs = _stack_histories(histories)
+        if self.network != 0:
+            visits, _, _, _ = self.engine.search_networks(positions, self.network, self._num_simulations(), self.leaves_per_root,
+                                                          self.virtual_loss, history=hist, hist_offsets=offs)
+        elif self.leaves_per_root > 1:
+            visits, _, _, _ = self.engine.search_vl(positions, self._num_simulations(), self.leaves_per_root, self.virtual_loss,
+                                                    history=hist, hist_offsets=offs)
         else:
             visits, _, _ = self.engine.search(positions, num_simulations=self.sims, history=hist, hist_offsets=offs)
-        out = []
-        for k in range(len(positions)):
-            w = visits[k] / visits[k].sum()
-            out.append(_weighted_index(w, _uniform(seed, game_ids[k], plies[k])) if stochastic[k] else _last_argmax(w))
-        return out
+        return _choose_from_visits(visits, stochastic, seed, game_ids, plies)
 
 
 class BasePlayer:
-    """Player::BaseModel: the raw policy masked to the legal moves, no search (validation.rs:310-350)."""
+    """Player::BaseModel: the raw policy masked to the legal moves, no search (validation.rs:310-350).  `network` names the
+    engine's network slot; a non-zero slot evaluates through Engine.forward_networks."""
 
-    def __init__(self, engine):
-        self.engine = engine
+    def __init__(self, engine, network=0):
+        self.engine, self.network = engine, int(network)
 
     def choose(self, positions, histories, fullmoves, stochastic, seed, game_ids, plies):
-        policy, _ = self.engine.forward(positions)
+        if self.network != 0:
+            policy, _ = self.engine.forward_networks(positions, self.network)
+        else:
+            policy, _ = self.engine.forward(positions)
         _, index, count = self.engine.movegen(positions)
-        out = []
-        for k in range(len(positions)):
-            masked = np.zeros(ACTION_SPACE, np.float32)
-            legal = index[k, : count[k]]
-            masked[legal] = policy[k, legal]
-            out.append(_weighted_index(masked, _uniform(seed, game_ids[k], plies[k])) if stochastic[k] else _last_argmax(masked))
-        return out
+        return _choose_from_policy(policy, index, count, stochastic, seed, game_ids, plies)
+
+
+def _joint_choose(player_1, player_2):
+    """When both players search (or evaluate) on the same engine with the same search settings, one ply of all games is one
+    search_networks (forward_networks) call with a network slot per game, so both players share every network round.
+    Returns choose(positions, histories, movers, stochastic, seed, game_ids, plies) or None; movers[k] is 0 for player 1."""
+    if player_1.engine is not player_2.engine or type(player_1) is not type(player_2):
+        return None
+    eng = player_1.engine
+    if type(player_1) is MctsPlayer:
+        settings = [(p._num_simulations(), p.leaves_per_root, p.virtual_loss) for p in (player_1, player_2)]
+        if settings[0] != settings[1]:
+            return None
+        sims, k, vl = settings[0]
+
+        def choose(positions, histories, movers, stochastic, seed, game_ids, plies):
+            hist, offs = _stack_histories(histories)
+            nets = np.where(movers == 0, player_1.network, player_2.network)
+            visits, _, _, _ = eng.search_networks(positions, nets, sims, k, vl, history=hist, hist_offsets=offs)
+            return _choose_from_visits(visits, stochastic, seed, game_ids, plies)
+        return choose
+    if type(player_1) is BasePlayer:
+        def choose(positions, histories, movers, stochastic, seed, game_ids, plies):
+            policy, _ = eng.forward_networks(positions, np.where(movers == 0, player_1.network, player_2.network))
+            _, index, count = eng.movegen(positions)
+            return _choose_from_policy(policy, index, count, stochastic, seed, game_ids, plies)
+        return choose
+    return None
 
 
 class RandomPlayer:
@@ -124,12 +176,20 @@ def evaluate(player_1, player_2, rules_engine, n_games=EVALUATION_GAMES, num_sto
     result = np.zeros(n_games, np.float32)       # white's point of view: 1, 0, -1
     active = np.ones(n_games, bool)
     players = (player_1, player_2)
+    joint = _joint_choose(player_1, player_2)
     for ply in range(max_plies):
         if not active.any():
             break
         white_to_move = ply % 2 == 0
         chosen = np.zeros(n_games, np.int64)
-        for which in (0, 1):
+        if joint is not None:
+            # every active game has one mover: player 1 in game g when (g even) == (White to move)
+            ids = np.flatnonzero(active)
+            movers = np.array([0 if (g % 2 == 0) == white_to_move else 1 for g in ids])
+            fm = pos["fullmoves"][ids]
+            chosen[ids] = joint(pos[ids], [np.array(hist[g], POSITION_DTYPE) for g in ids], movers, fm <= num_stochastic_moves, seed,
+                                ids, np.full(len(ids), ply))
+        for which in (0, 1) if joint is None else ():
             # game g: player_1 is White when g is even (validation.rs:196-200)
             owns = np.array([active[g] and ((g % 2 == 0) == (which == 0)) == white_to_move for g in range(n_games)])
             ids = np.flatnonzero(owns)

@@ -35,6 +35,9 @@ extern "C" {
     pub fn az_load_weights(eng: *mut az_engine, arrays: *const *const f32, n_arrays: c_int) -> c_int;
     pub fn az_forward_planes(eng: *mut az_engine, n: c_int, planes: *const f32, policy: *mut f32, value: *mut f32) -> c_int;
     pub fn az_forward(eng: *mut az_engine, n: c_int, pos: *const az_position, policy: *mut f32, value: *mut f32) -> c_int;
+    pub fn az_load_network(eng: *mut az_engine, network: c_int, arrays: *const *const f32, n_arrays: c_int) -> c_int;
+    pub fn az_forward_networks(eng: *mut az_engine, n: c_int, pos: *const az_position, network: *const u8, policy: *mut f32,
+                               value: *mut f32) -> c_int;
     pub fn az_movegen(eng: *mut az_engine, n: c_int, pos: *const az_position, moves: *mut u16, index: *mut u16, count: *mut i32) -> c_int;
     pub fn az_perft(eng: *mut az_engine, n: c_int, pos: *const az_position, depth: c_int, nodes: *mut u64) -> c_int;
     pub fn az_play_move(eng: *mut az_engine, n: c_int, pos: *mut az_position, history: *const az_position,
@@ -49,6 +52,10 @@ extern "C" {
                         hist_offsets: *const u32, num_simulations: c_int, leaves_per_root: c_int, virtual_loss: f32,
                         noise_game_ids: *const u64, noise_plies: *const u32, visits: *mut f32, scores: *mut f32, depth: *mut i32,
                         stats: *mut az_search_stats) -> c_int;
+    pub fn az_search_networks(eng: *mut az_engine, n: c_int, roots: *const az_position, history: *const az_position,
+                              hist_offsets: *const u32, num_simulations: c_int, leaves_per_root: c_int, virtual_loss: f32,
+                              network: *const u8, noise_game_ids: *const u64, noise_plies: *const u32, visits: *mut f32,
+                              scores: *mut f32, depth: *mut i32, stats: *mut az_search_stats) -> c_int;
     pub fn az_selfplay_begin(eng: *mut az_engine, n_games: c_int, first_game_id: u64) -> c_int;
     pub fn az_selfplay_begin_n(eng: *mut az_engine, n_concurrent: c_int, first_game_id: u64, total_games: u64) -> c_int;
     pub fn az_selfplay_step(eng: *mut az_engine, waves: c_int, stats: *mut az_selfplay_stats) -> c_int;

@@ -98,6 +98,33 @@ impl Engine {
         Ok((visits, depth, stats))
     }
 
+    /// Loads a network (144 f32 arrays in az_weight_name order) into slot `network` (az_load_network): slot 0 is what every
+    /// single-network call uses, slot 1 the second network of `search_networks`.
+    pub fn load_network(&mut self, network: i32, arrays: &[&[f32]]) -> Result<()> {
+        let ptrs: Vec<*const f32> = arrays.iter().map(|a| a.as_ptr()).collect();
+        self.check(unsafe { sys::az_load_network(self.raw, network, ptrs.as_ptr(), ptrs.len() as i32) })
+    }
+
+    /// `search_vl` with a network slot per root (az_search_networks): the roots of both networks share every network round,
+    /// the two players of a match in one call.  Returns visits, depths and the stats.
+    pub fn search_networks(&mut self, roots: &[sys::az_position], history: &[Vec<sys::az_position>], network: &[u8], sims: i32,
+                           leaves_per_root: i32, virtual_loss: f32, noise: Option<(&[u64], &[u32])>)
+                           -> Result<(Vec<f32>, Vec<i32>, sys::az_search_stats)> {
+        let n = roots.len();
+        assert_eq!(network.len(), n, "one network id per root");
+        let mut flat = Vec::new();
+        let mut offs = vec![0u32; n + 1];
+        for (i, h) in history.iter().enumerate() { flat.extend_from_slice(h); offs[i + 1] = flat.len() as u32; }
+        let (ids, plies) = match noise { Some((g, p)) => (g.as_ptr(), p.as_ptr()), None => (ptr::null(), ptr::null()) };
+        let mut visits = vec![0f32; n * ACTION_SPACE];
+        let mut depth = vec![0i32; n];
+        let mut stats = sys::az_search_stats::default();
+        self.check(unsafe { sys::az_search_networks(self.raw, n as i32, roots.as_ptr(), flat.as_ptr(), offs.as_ptr(), sims,
+                                                    leaves_per_root, virtual_loss, network.as_ptr(), ids, plies, visits.as_mut_ptr(),
+                                                    ptr::null_mut(), depth.as_mut_ptr(), &mut stats) })?;
+        Ok((visits, depth, stats))
+    }
+
     /// run_all_episodes (training.rs:340-378): EXACTLY `n_games` self-play games (ids first_game_id ..), each played to
     /// completion; the callback receives the finished games' steps (values already back-filled) as they become available.
     /// Returns the average batch size (= evaluations per wave).

@@ -20,6 +20,7 @@ extern "C" {
 #define AZ_MAX_MOVES 256     /* shakmaty MoveList capacity */
 #define AZ_NUM_PLANES 19     /* chess.rs:176-189 */
 #define AZ_NUM_WEIGHT_ARRAYS 144
+#define AZ_MAX_NETWORKS 2    /* network slots of an engine (az_load_network) */
 
 typedef enum az_status {
     AZ_OK = 0,
@@ -97,10 +98,21 @@ int64_t az_weight_size(int i);
 int az_load_weights(az_engine* eng, const float* const* arrays, int n_arrays);
 /* same, from device f32 pointers (e.g. the buffer an NCCL broadcast just filled) */
 int az_load_weights_dev(az_engine* eng, const float* const* arrays_dev, int n_arrays);
+/* Network slots: an engine holds up to AZ_MAX_NETWORKS networks, which the batched calls below select per board or root (the
+ * two players of a match, validation.rs:155-282, SURVEY section 8(f) #3).  Slot 0 is what az_load_weights loads; az_load_network
+ * loads host arrays (as az_load_weights, same validation and BatchNorm folding) into slot `network`: az_load_network(e, 0, ...)
+ * is az_load_weights.  The weights of slot 1 are allocated by its first load; activations and every other buffer are shared. */
+int az_load_network(az_engine* eng, int network, const float* const* arrays, int n_arrays);
 /* AlphaZero::forward (agent.rs:112-144) on planes [n][19][8][8] -> policy [n][4096] (softmax over ALL indices), value [n] */
 int az_forward_planes(az_engine* eng, int n, const float* planes, float* policy_out, float* value_out);
 /* to_tensor + forward: what process_batch does per request (training.rs:383-397) */
 int az_forward(az_engine* eng, int n, const az_position* pos, float* policy_out, float* value_out);
+/* az_forward with a network per board (network[i] < AZ_MAX_NETWORKS, any order): both networks run in the same launches,
+ * and every row is bit-identical to az_forward of that board on an engine holding only its network.  AZ_ERR_INVALID_ARGUMENT
+ * for an id >= AZ_MAX_NETWORKS, AZ_ERR_NO_WEIGHTS for a network never loaded, AZ_ERR_CAPACITY when the sum over networks of
+ * their board counts rounded up to a multiple of 4 exceeds az_config.max_batch.  The bf16 path needs the default AZ_TOWER_*,
+ * AZ_INPUT_* and AZ_HEADS_TC configuration (else AZ_ERR_STATE); the fp32 path (precision 1) runs the networks in turn. */
+int az_forward_networks(az_engine* eng, int n, const az_position* pos, const uint8_t* network, float* policy_out, float* value_out);
 
 /* ---- chess.rs ------------------------------------------------------------------------------------------------- */
 /* Chess::legal_moves() (tree.rs:39,86): moves_out [n][256], index_out [n][256] = move_to_index of each (nullable) */
@@ -151,6 +163,17 @@ int az_search_vl(az_engine* eng, int n, const az_position* roots, const az_posit
                  int num_simulations, int leaves_per_root, float virtual_loss, const uint64_t* noise_game_ids,
                  const uint32_t* noise_plies, float* visits_out, float* scores_out, int32_t* depth_out,
                  az_search_stats* stats_out /* nullable */);
+
+/* az_search_vl with a network per root (network[i] < AZ_MAX_NETWORKS): the match ply of evaluate (validation.rs:155-282) with
+ * both players' roots in one call, so that they share every network round.  The same semantics as az_search_vl -- a parity
+ * mode only at leaves_per_root = 1, where each root's results equal az_search of that root on an engine holding its network --
+ * and the same errors, plus: AZ_ERR_INVALID_ARGUMENT for an id >= AZ_MAX_NETWORKS, AZ_ERR_NO_WEIGHTS for a network never loaded
+ * (not under the synthetic evaluator, where network s uses seed + s), AZ_ERR_CAPACITY when the sum over networks of
+ * (roots x leaves_per_root) rounded up to a multiple of 4 exceeds az_config.max_batch. */
+int az_search_networks(az_engine* eng, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
+                       int num_simulations, int leaves_per_root, float virtual_loss, const uint8_t* network,
+                       const uint64_t* noise_game_ids, const uint32_t* noise_plies, float* visits_out, float* scores_out,
+                       int32_t* depth_out, az_search_stats* stats_out /* nullable */);
 
 /* test hook: replace the network by the deterministic synthetic evaluator shared with the oracle (kind 1) or
  * restore the network (kind 0) */

@@ -117,6 +117,10 @@ public:
     explicit AlphaZero(Engine& e) : e_(e) {}
     // load_model (main.rs:109-116): 144 tensors in az_weight_name order
     void load(const std::vector<const float*>& arrays) { e_.check(az_load_weights(e_.handle(), arrays.data(), (int)arrays.size()), "az_load_weights"); }
+    // a second network for matches (az_load_network): slot 1 is searched by MCTree::monte_carlo_tree_search(.., network)
+    void load(const std::vector<const float*>& arrays, int network) {
+        e_.check(az_load_network(e_.handle(), network, arrays.data(), (int)arrays.size()), "az_load_network");
+    }
     // forward(Tensor<B,4>[N,19,8,8]) -> (Tensor<B,2>[N,4096], Tensor<B,1>[N])
     std::pair<std::vector<float>, std::vector<float>> forward(const float* planes, int n) const {
         std::vector<float> policy((std::size_t)n * ACTION_SPACE), value(n);
@@ -178,6 +182,24 @@ public:
         e.check(az_search_vl(e.handle(), 1, &state.position, state.pos_count.data(), offs, sims, leaves_per_root, virtual_loss,
                              noise_ ? &noise_game_ : nullptr, noise_ ? &noise_ply_ : nullptr, visits.data(), nullptr, &depth, nullptr),
                 "az_search_vl");
+        depth_ = (std::size_t)depth;
+        float sum = 0.0f;
+        for (float v : visits) sum += v;
+        if (sum > 0.0f) for (float& v : visits) v = v / sum;
+        return visits;
+    }
+    // the same with the network in slot `network` of the model's engine (az_search_networks); network 0 is the overload above
+    Policy monte_carlo_tree_search(int num_simulations, int leaves_per_root, float virtual_loss, int network) {
+        Engine& e = model_->engine();
+        const int sims = num_simulations > 0 ? num_simulations : e.config().num_simulations;
+        const uint32_t offs[2] = {0, (uint32_t)state.pos_count.size()};
+        const uint8_t net = (uint8_t)network;
+        if (network < 0 || network >= AZ_MAX_NETWORKS) throw Error(AZ_ERR_INVALID_ARGUMENT, "network must be in [0, AZ_MAX_NETWORKS)");
+        Policy visits;
+        int32_t depth = 0;
+        e.check(az_search_networks(e.handle(), 1, &state.position, state.pos_count.data(), offs, sims, leaves_per_root, virtual_loss, &net,
+                                   noise_ ? &noise_game_ : nullptr, noise_ ? &noise_ply_ : nullptr, visits.data(), nullptr, &depth, nullptr),
+                "az_search_networks");
         depth_ = (std::size_t)depth;
         float sum = 0.0f;
         for (float v : visits) sum += v;
