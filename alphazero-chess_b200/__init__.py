@@ -362,12 +362,25 @@ class Engine:
         return visits, scores, depth, st
 
     # ---- training.rs ------------------------------------------------------------------------------------------
-    def selfplay_begin(self, n_games, first_game_id=0, total_games=0):
+    def selfplay_begin(self, n_games, first_game_id=0, total_games=0, leaves_per_game=None, virtual_loss=1.0):
         """run_all_episodes set-up.  total_games = 0: every finished game restarts with a fresh id (throughput runs);
         total_games = N: exactly the games first_game_id .. first_game_id + N - 1 are played to completion on n_games
-        concurrent slots (training.rs:352-361,376-377) and stats.active_games reaches 0 when the last one has ended."""
-        self._check(self._L.az_selfplay_begin_n(self._h, int(n_games), ctypes.c_uint64(first_game_id), ctypes.c_uint64(total_games)),
-                    "az_selfplay_begin_n")
+        concurrent slots (training.rs:352-361,376-377) and stats.active_games reaches 0 when the last one has ended.
+        leaves_per_game = K (any int, 1 included) searches every ply leaf-parallel with virtual loss (az_selfplay_begin_vl; not in
+        the reference, records identical to the default path at K = 1): up to K leaves per game share each network round."""
+        if leaves_per_game is None:
+            self._check(self._L.az_selfplay_begin_n(self._h, int(n_games), ctypes.c_uint64(first_game_id), ctypes.c_uint64(total_games)),
+                        "az_selfplay_begin_n")
+        else:
+            self._check(self._L.az_selfplay_begin_vl(self._h, int(n_games), ctypes.c_uint64(first_game_id), ctypes.c_uint64(total_games),
+                                                     int(leaves_per_game), ctypes.c_float(virtual_loss)), "az_selfplay_begin_vl")
+
+    def selfplay_vl_stats(self):
+        """SearchStats of the az_selfplay_begin_vl self-play since its begin call: waves, leaf evaluations, terminal leaves,
+        collisions."""
+        st = SearchStats()
+        self._check(self._L.az_selfplay_vl_stats(self._h, ctypes.byref(st)), "az_selfplay_vl_stats")
+        return st
 
     def selfplay_step(self, waves):
         st = SelfplayStats()

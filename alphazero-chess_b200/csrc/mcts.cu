@@ -1017,6 +1017,58 @@ __device__ __forceinline__ int vl_descend(Ctx& x, const VLPtrs& vl, uint2* path,
     }
 }
 
+// Backs up the root's previous batch (vl.count[g] leaves) in leaf order, so that the f32 additions on a shared edge happen in a
+// fixed order, and returns the number of leaves.  Without fused heads the evaluated leaves' priors are copied here first.
+__device__ __forceinline__ int vl_backup_batch(Ctx& x, const SearchParams& prm, const SearchPtrs& ptr, const VLPtrs& vl) {
+    const int nl = vl.count[x.g];
+    for (int k = 0; k < nl; k++) {
+        const int leaf = x.g * vl.K + k;
+        const int s = vl.slot[leaf];
+        float value;
+        if (s >= 0) {
+            if (!prm.priors_scattered) {
+                const size_t off = ptr.req_edge_off[s];
+                const int L = ptr.req_nedges[s];
+                const float* pol = ptr.res_policy + (size_t)s * AZ_ACTION_SPACE;
+                for (int e = x.lane; e < L; e += 32) ptr.edge_P[off + e] = pol[ptr.edge_mv[off + e] >> 16];
+            }
+            value = ptr.res_value[s];
+        } else {
+            value = vl.value[leaf];
+        }
+        const int len = vl.len[leaf];
+        const uint2* path = vl.path + (size_t)leaf * prm.node_cap;
+        for (int i = x.lane; i < len; i += 32) {
+            const size_t e = x.ebase + path[i].y;
+            const float v = ((len - 1 - i) & 1) ? value : -value;
+            ptr.edge_W[e] = __fadd_rn(ptr.edge_W[e], v);
+            ptr.edge_N[e] = __fadd_rn(ptr.edge_N[e], 1.0f);
+            vl.V[e] -= 1;
+        }
+        __syncwarp();
+    }
+    return nl;
+}
+
+// Gathers the root's next batch: up to min(K, S - sims_done) descents, ended early by a collision (collided = 1).  Returns the
+// number of leaves; depth_sum grows by the edges on their descents.
+__device__ __forceinline__ int vl_gather_batch(Ctx& x, const SearchParams& prm, const VLPtrs& vl, int& collided, unsigned int& depth_sum) {
+    int n_leaf = 0;
+    const int kb = min(vl.K, prm.S - (int)x.c.sims_done);
+    for (int k = 0; k < kb; k++) {
+        const int leaf = x.g * vl.K + k;
+        uint2* path = vl.path + (size_t)leaf * prm.node_cap;
+        const int depth = vl_descend(x, vl, path, __fadd_rn((float)(x.c.sims_done + k), 1.0f));
+        if (depth < 0) { collided = 1; break; }
+        for (int i = x.lane; i <= depth; i += 32) vl.V[x.ebase + path[i].y] += 1;
+        if (x.lane == 0) vl.len[leaf] = depth + 1;
+        __syncwarp();
+        depth_sum += depth + 1;
+        n_leaf++;
+    }
+    return n_leaf;
+}
+
 // one warp per root: consume the previous batch (the root's own evaluation on the first wave), then gather the next one
 __global__ void __launch_bounds__(WARPS * 32) k_vl_gather(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
                                                           const __grid_constant__ VLPtrs vl) {
@@ -1039,52 +1091,15 @@ __global__ void __launch_bounds__(WARPS * 32) k_vl_gather(const __grid_constant_
         if (x.c.flags & 1) apply_noise(x, 0, x.c.game_id, x.c.noise_ply);
         x.c.pending_node = -1;
     } else {
-        // backups in leaf order: the f32 additions on a shared edge happen in a fixed order
-        const int nl = vl.count[g];
-        for (int k = 0; k < nl; k++) {
-            const int leaf = g * vl.K + k;
-            const int s = vl.slot[leaf];
-            float value;
-            if (s >= 0) {
-                if (!prm.priors_scattered) {
-                    const size_t off = ptr.req_edge_off[s];
-                    const int L = ptr.req_nedges[s];
-                    const float* pol = ptr.res_policy + (size_t)s * AZ_ACTION_SPACE;
-                    for (int e = x.lane; e < L; e += 32) ptr.edge_P[off + e] = pol[ptr.edge_mv[off + e] >> 16];
-                }
-                value = ptr.res_value[s];
-            } else {
-                value = vl.value[leaf];
-            }
-            const int len = vl.len[leaf];
-            const uint2* path = vl.path + (size_t)leaf * prm.node_cap;
-            for (int i = x.lane; i < len; i += 32) {
-                const size_t e = x.ebase + path[i].y;
-                const float v = ((len - 1 - i) & 1) ? value : -value;
-                ptr.edge_W[e] = __fadd_rn(ptr.edge_W[e], v);
-                ptr.edge_N[e] = __fadd_rn(ptr.edge_N[e], 1.0f);
-                vl.V[e] -= 1;
-            }
-            __syncwarp();
-        }
-        x.c.sims_done += nl;
+        x.c.sims_done += vl_backup_batch(x, prm, ptr, vl);
     }
     // ---- 2. gather the next batch
     int n_leaf = 0, collided = 0;
     if ((int)x.c.sims_done >= prm.S) {
         x.c.status = 1;
     } else {
-        const int kb = min(vl.K, prm.S - (int)x.c.sims_done);
-        for (int k = 0; k < kb; k++) {
-            const int leaf = g * vl.K + k;
-            uint2* path = vl.path + (size_t)leaf * prm.node_cap;
-            const int depth = vl_descend(x, vl, path, __fadd_rn((float)(x.c.sims_done + k), 1.0f));
-            if (depth < 0) { collided = 1; break; }
-            for (int i = x.lane; i <= depth; i += 32) vl.V[x.ebase + path[i].y] += 1;
-            if (x.lane == 0) vl.len[leaf] = depth + 1;
-            __syncwarp();
-            n_leaf++;
-        }
+        unsigned int depth_sum = 0;
+        n_leaf = vl_gather_batch(x, prm, vl, collided, depth_sum);
     }
     if (x.lane == 0) {
         vl.count[g] = n_leaf;
@@ -1158,6 +1173,56 @@ __global__ void __launch_bounds__(WARPS * 32) k_vl_expand(const __grid_constant_
 __global__ void __launch_bounds__(WARPS * 32) k_vl_expand_nets(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
                                                                const __grid_constant__ VLPtrs vl, const __grid_constant__ NetRoute rt) {
     vl_expand_body<true>(prm, ptr, vl, rt);
+}
+
+// Self-play with leaf-parallel search (az_selfplay_begin_vl), one warp per game slot: publish a parked game, back up the previous
+// batch, play the move once the search has its S simulations (move_step: record, choose, traverse_new or finish / restart), then
+// gather the next batch -- of the next ply when a move was just played, so no wave is spent between plies.  k_vl_expand and the
+// network follow.  Root priors come from the start-position forward or from traverse_new, as in k_advance.
+__global__ void __launch_bounds__(WARPS * 32) k_vl_selfplay(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
+                                                            const __grid_constant__ VLPtrs vl) {
+    __shared__ WarpShared shared[WARPS];
+    const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (g == 0 && (threadIdx.x & 31) == 0) *ptr.batch_count = 0;   // requests of this wave are counted by k_vl_expand, which runs next
+    if (g >= prm.n_games) return;
+    Ctx x{prm, ptr, &shared[threadIdx.x >> 5], g, (int)(threadIdx.x & 31), (size_t)g * prm.node_cap, (size_t)g * prm.edge_cap,
+          ptr.ctl[g], 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    if (x.c.status != 0 && x.c.status != 4) return;   // idle slot or error: vl.count[g] is already 0
+    if (x.c.status == 4) {   // game over, samples staged: publish now if the host has drained the queue, else stay parked
+        const ColdOut o = finish_game_cold(&prm, &ptr, x.sh, g, x.c);
+        x.c = o.c; x.st_pos += o.st_pos; x.st_games += o.st_games; x.st_sdepth += o.st_sdepth;
+    }
+    int n_leaf = 0, collided = 0;
+    if (x.c.status == 0) {
+        const int nl = vl_backup_batch(x, prm, ptr, vl);   // 0 for a game that has just started
+        x.c.sims_done += nl;
+        if (x.lane == 0) x.st_sims += nl;
+        if ((int)x.c.sims_done >= prm.S) {
+            const ColdOut o = move_step_cold(&prm, &ptr, x.sh, g, x.c);
+            x.c = o.c; x.st_pos += o.st_pos; x.st_games += o.st_games; x.st_sdepth += o.st_sdepth;
+        }
+        if (x.c.status == 0) {
+            if (x.c.sims_done == 0) {   // a fresh root (game start or traverse_new): no descent is in flight through its edges
+                const int L = (int)((x.c.flags >> 8) & 0xFF);
+                for (int e = x.lane; e < L; e += 32) vl.V[x.ebase + e] = 0;
+                __syncwarp();
+            }
+            n_leaf = vl_gather_batch(x, prm, vl, collided, x.st_depth);
+        }
+    }
+    if (x.lane == 0) {
+        vl.count[g] = n_leaf;   // 0 when the slot parked, went idle or failed: the next wave backs up nothing
+        if (n_leaf) atomicAdd(&vl.stats[0], (unsigned long long)n_leaf);
+        if (collided) atomicAdd(&vl.stats[2], 1ULL);
+        ptr.ctl[g] = x.c;
+        // the statistics of az_selfplay_step, striped as in k_advance; evaluations and terminal leaves come from vl.stats
+        unsigned long long* ct = ptr.stats + (size_t)(blockIdx.x & (STAT_STRIPES - 1)) * STAT_WIDTH;
+        if (x.st_sims) atomicAdd(&ct[0], (unsigned long long)x.st_sims);
+        if (x.st_pos) atomicAdd(&ct[1], (unsigned long long)x.st_pos);
+        if (x.st_games) atomicAdd(&ct[5], (unsigned long long)x.st_games);
+        if (x.st_depth) atomicAdd(&ct[6], (unsigned long long)x.st_depth);
+        if (x.st_sdepth) atomicAdd(&ct[17], (unsigned long long)x.st_sdepth);
+    }
 }
 
 // ------------------------------------------------------------------------------------------- host side
@@ -1472,6 +1537,22 @@ int az_search(az_engine* e, int n, const az_position* roots, const az_position* 
 
 namespace azb {
 
+// the in-flight counts and the per-leaf records of az_search_vl and az_selfplay_begin_vl, allocated by the first such call
+static int vl_alloc(az_engine* e, SearchState* st) {
+    if (st->vl_V) return AZ_OK;
+    cudaSetDevice(e->cfg.device);
+    const size_t NE = (size_t)st->G * st->prm.edge_cap, B = (size_t)e->max_batch;
+    int a = salloc(e, st, &st->vl_V, NE);
+    a |= salloc(e, st, &st->vl_path, B * st->prm.node_cap);
+    a |= salloc(e, st, &st->vl_len, B); a |= salloc(e, st, &st->vl_slot, B); a |= salloc(e, st, &st->vl_value, B);
+    a |= salloc(e, st, &st->vl_count, (size_t)st->G); a |= salloc(e, st, &st->vl_stats, 4);
+    return a ? AZ_ERR_OUT_OF_MEMORY : AZ_OK;
+}
+
+static VLPtrs vl_ptrs(const SearchState* st, int K, float lambda) {
+    return VLPtrs{st->vl_V, st->vl_path, st->vl_len, st->vl_slot, st->vl_value, st->vl_count, st->vl_stats, K, lambda};
+}
+
 // az_search_vl, and az_search_networks when `network` (one id per root) is given: the requests of each root then go to the
 // range of its network (k_init_search_nets, k_vl_expand_nets) and every wave evaluates both ranges in one multi-network forward
 static int search_vl_run(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
@@ -1503,14 +1584,9 @@ static int search_vl_run(az_engine* e, int n, const az_position* roots, const az
         if (r0 + r1 > e->max_batch) return set_err(e, AZ_ERR_CAPACITY, "network ranges (roots x leaves_per_root each) exceed az_config.max_batch");
         base1 = (int)r0;
     }
-    if (n >= 0 && n <= st->G && !st->vl_V) {   // first call: the in-flight counts and the per-leaf records
-        cudaSetDevice(e->cfg.device);
-        const size_t NE = (size_t)st->G * st->prm.edge_cap, B = (size_t)e->max_batch;
-        int a = salloc(e, st, &st->vl_V, NE);
-        a |= salloc(e, st, &st->vl_path, B * st->prm.node_cap);
-        a |= salloc(e, st, &st->vl_len, B); a |= salloc(e, st, &st->vl_slot, B); a |= salloc(e, st, &st->vl_value, B);
-        a |= salloc(e, st, &st->vl_count, (size_t)st->G); a |= salloc(e, st, &st->vl_stats, 4);
-        if (a) return AZ_ERR_OUT_OF_MEMORY;
+    if (n >= 0 && n <= st->G) {
+        const int a = vl_alloc(e, st);
+        if (a) return a;
     }
     NetRoute route{nullptr, st->batch_base, base1};
     NetBatch nb{st->batch_base, base1, base1 + count[1] * leaves_per_root};
@@ -1528,7 +1604,7 @@ static int search_vl_run(az_engine* e, int n, const az_position* roots, const az
     int r = search_begin(e, n, roots, history, hist_offsets, num_simulations, noise_game_ids, noise_plies, visits_out, run, rt, nbp);
     if (r) return r == 1 ? AZ_OK : r;
     const int K = leaves_per_root;
-    VLPtrs vl{st->vl_V, st->vl_path, st->vl_len, st->vl_slot, st->vl_value, st->vl_count, st->vl_stats, K, virtual_loss};
+    const VLPtrs vl = vl_ptrs(st, K, virtual_loss);
     AZ_CUDA(e, cudaMemsetAsync(vl.count, 0, (size_t)n * sizeof(int), e->stream));
     AZ_CUDA(e, cudaMemsetAsync(vl.stats, 0, 4 * sizeof(unsigned long long), e->stream));
     run.prm.priors_scattered = (e->stub_kind == 0 && e->cfg.precision != 1) ? 1 : 0;
@@ -1602,13 +1678,25 @@ int az_search_networks(az_engine* e, int n, const az_position* roots, const az_p
 
 int az_selfplay_begin(az_engine* e, int n_games, uint64_t first_game_id) { return az_selfplay_begin_n(e, n_games, first_game_id, 0); }
 
-int az_selfplay_begin_n(az_engine* e, int n_games, uint64_t first_game_id, uint64_t total_games) {
-    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+}  // extern "C"
+
+namespace azb {
+
+// az_selfplay_begin_n (K = 0: k_advance waves) and az_selfplay_begin_vl (K >= 1: k_vl_selfplay waves with K leaves per game)
+static int selfplay_begin(az_engine* e, int n_games, uint64_t first_game_id, uint64_t total_games, int K, float virtual_loss) {
     SearchState* st = e->search;
     if (total_games != 0 && (uint64_t)n_games > total_games) n_games = (int)total_games;   // never more slots than games to play
     if (n_games <= 0 || n_games > st->G) return set_err(e, AZ_ERR_CAPACITY, "more games than az_config.max_games");
+    if (K > 0 && (long long)n_games * K > (long long)e->max_batch)
+        return set_err(e, AZ_ERR_CAPACITY, "games x leaves_per_game exceeds az_config.max_batch");
+    if (K > 0 && st->prm.cache_mask)
+        return set_err(e, AZ_ERR_STATE, "az_selfplay_begin_vl does not support the evaluation cache (cache_log2 > 0)");
     if (e->stub_kind == 0 && !e->net->loaded) return set_err(e, AZ_ERR_NO_WEIGHTS, "az_load_weights has not been called");
     cudaSetDevice(e->cfg.device);
+    if (K > 0) {
+        const int a = vl_alloc(e, st);
+        if (a) return a;
+    }
     SearchPtrs& q = st->ptr;
     if (!q.game_samples) {
         int r = salloc(e, st, &q.game_samples, (size_t)st->G * MAX_SAMPLE_PLIES);
@@ -1652,8 +1740,64 @@ int az_selfplay_begin_n(az_engine* e, int n_games, uint64_t first_game_id, uint6
     e->n_launches += 2;
     k_init_selfplay<<<blocks, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr, first_game_id);
     AZ_CUDA(e, cudaGetLastError());
+    if (K > 0) {   // no batch in flight, no statistics yet
+        AZ_CUDA(e, cudaMemsetAsync(st->vl_count, 0, (size_t)n_games * sizeof(int), e->stream));
+        AZ_CUDA(e, cudaMemsetAsync(st->vl_stats, 0, 4 * sizeof(unsigned long long), e->stream));
+    }
     AZ_CUDA(e, cudaStreamSynchronize(e->stream));
+    st->sp_vl_K = K;
+    st->sp_vl_lambda = virtual_loss;
+    st->sp_vl_waves = 0;
     st->selfplay_active = true;
+    return AZ_OK;
+}
+
+// one wave of az_selfplay_begin_vl's self-play: k_vl_selfplay, k_vl_expand, the network
+static int run_wave_vl(az_engine* e, SearchState* st) {
+    const int n = st->prm.n_games, K = st->sp_vl_K;
+    st->prm.priors_scattered = (e->stub_kind == 0 && e->cfg.precision != 1) ? 1 : 0;
+    const VLPtrs vl = vl_ptrs(st, K, st->sp_vl_lambda);
+    prof_mark_search(e);
+    e->n_launches += 2;
+    k_vl_selfplay<<<(n + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr, vl);
+    AZ_CUDA(e, cudaGetLastError());
+    k_vl_expand<<<(n * K + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr, vl);
+    AZ_CUDA(e, cudaGetLastError());
+    st->sp_vl_waves++;
+    return evaluate_batch(e, st);
+}
+
+}  // namespace azb
+
+extern "C" {
+
+int az_selfplay_begin_n(az_engine* e, int n_games, uint64_t first_game_id, uint64_t total_games) {
+    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+    return selfplay_begin(e, n_games, first_game_id, total_games, 0, 0.0f);
+}
+
+int az_selfplay_begin_vl(az_engine* e, int n_concurrent, uint64_t first_game_id, uint64_t total_games, int leaves_per_game,
+                         float virtual_loss) {
+    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+    if (leaves_per_game < 1) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "leaves_per_game must be >= 1");
+    if (!(virtual_loss >= 0.0f) || !std::isfinite(virtual_loss))
+        return set_err(e, AZ_ERR_INVALID_ARGUMENT, "virtual_loss must be finite and >= 0");
+    return selfplay_begin(e, n_concurrent, first_game_id, total_games, leaves_per_game, virtual_loss);
+}
+
+int az_selfplay_vl_stats(az_engine* e, az_search_stats* out) {
+    if (!e || !out) return AZ_ERR_INVALID_ARGUMENT;
+    std::memset(out, 0, sizeof *out);
+    SearchState* st = e->search;
+    if (!st->selfplay_active || !st->sp_vl_K) return set_err(e, AZ_ERR_STATE, "az_selfplay_begin_vl has not been called");
+    cudaSetDevice(e->cfg.device);
+    unsigned long long s[4];
+    AZ_CUDA(e, cudaMemcpyAsync(s, st->vl_stats, sizeof s, cudaMemcpyDeviceToHost, e->stream));
+    AZ_CUDA(e, cudaStreamSynchronize(e->stream));
+    out->waves = st->sp_vl_waves;
+    out->evaluations = s[0] - s[1];   // every gathered leaf that was not terminal
+    out->terminal_leaves = s[1];
+    out->collisions = s[2];
     return AZ_OK;
 }
 
@@ -1663,7 +1807,7 @@ int az_selfplay_step(az_engine* e, int waves, az_selfplay_stats* out) {
     if (!st->selfplay_active) return set_err(e, AZ_ERR_STATE, "az_selfplay_begin has not been called");
     cudaSetDevice(e->cfg.device);
     for (int w = 0; w < waves; w++) {
-        int r = run_wave(e, st);
+        int r = st->sp_vl_K ? run_wave_vl(e, st) : run_wave(e, st);
         if (r) return r;
     }
     Counters c;
@@ -1675,6 +1819,8 @@ int az_selfplay_step(az_engine* e, int waves, az_selfplay_stats* out) {
     AZ_CUDA(e, cudaMemcpyAsync(flags, d_flags, 16, cudaMemcpyDeviceToHost, e->stream));
     AZ_CUDA(e, cudaMemcpyAsync(&c, st->ptr.counters, sizeof c, cudaMemcpyDeviceToHost, e->stream));
     AZ_CUDA(e, cudaMemcpyAsync(stripes, st->ptr.stats, sizeof stripes, cudaMemcpyDeviceToHost, e->stream));
+    unsigned long long vls[4] = {0, 0, 0, 0};
+    if (st->sp_vl_K) AZ_CUDA(e, cudaMemcpyAsync(vls, st->vl_stats, sizeof vls, cudaMemcpyDeviceToHost, e->stream));
     AZ_CUDA(e, cudaStreamSynchronize(e->stream));
     {
         unsigned long long sum[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -1709,6 +1855,7 @@ int az_selfplay_step(az_engine* e, int waves, az_selfplay_stats* out) {
 #endif
         c.simulations = sum[0]; c.positions = sum[1]; c.evaluations = sum[2]; c.cache_hits = sum[3];
         c.terminal_leaves = sum[4]; c.games_finished = sum[5]; c.sum_leaf_depth = sum[6]; c.sum_edges = sum[7];
+        if (st->sp_vl_K) { c.evaluations = vls[0] - vls[1]; c.terminal_leaves = vls[1]; }   // k_vl_expand counts the terminal leaves
     }
     if (out) {
         out->simulations = c.simulations; out->positions = c.positions; out->evaluations = c.evaluations; out->cache_hits = c.cache_hits;

@@ -128,7 +128,12 @@ struct SearchState {
     unsigned long long wave_counter = 0;   // self-play waves since az_selfplay_begin (cache epoch = wave_counter / S)
     unsigned long long* d_noise_ids = nullptr;  // [max_games] az_search staging (no allocation per call)
     uint32_t* d_noise_plies = nullptr;
-    // az_search_vl, allocated on its first call (az_engine_create's footprint does not include them)
+    // az_selfplay_begin_vl: leaves per game of the self-play in progress (0: az_selfplay_begin_n's k_advance waves), its virtual
+    // loss and the waves run since the begin call
+    int sp_vl_K = 0;
+    float sp_vl_lambda = 0.0f;
+    unsigned long long sp_vl_waves = 0;
+    // az_search_vl and az_selfplay_begin_vl, allocated by the first such call (az_engine_create's footprint does not include them)
     uint32_t* vl_V = nullptr;              // [G * edge_cap] descents of the current batch through each edge
     uint2* vl_path = nullptr;              // [max_batch][node_cap] one descent per leaf
     int* vl_len = nullptr;                 // [max_batch]

@@ -181,14 +181,16 @@ def train_iteration(model, optimizer, replay, iteration, num_steps=NUM_TRAIN_STE
 
 
 def run_generation(engine, replay, model, optimizer, iteration, n_games, min_replay_size=MIN_REPLAY_SIZE, waves_per_call=64,
-                   num_steps=NUM_TRAIN_STEPS, batch_size=BATCH_SIZE, concurrent=None):
+                   num_steps=NUM_TRAIN_STEPS, batch_size=BATCH_SIZE, concurrent=None, leaves_per_game=None, virtual_loss=1.0):
     """One iteration of train() (training.rs:70-200) on the engine: EXACTLY n_games self-play games are played to completion
     (run_all_episodes, training.rs:352-361,376-377: a slot whose game ends takes the next unplayed game or goes idle; nothing
     is cut off), their steps go from device memory straight into the replay buffer, then the training steps, then the new
-    weights are loaded into the engine.  Returns a dict of the metrics the reference logs."""
+    weights are loaded into the engine.  Returns a dict of the metrics the reference logs.  leaves_per_game / virtual_loss:
+    leaf-parallel self-play (Engine.selfplay_begin; not in the reference), None = the reference's search."""
     engine.load_weights(export_weights(model))
     slots = min(n_games, concurrent or engine.config.max_games, engine.config.max_games)
-    engine.selfplay_begin(slots, first_game_id=iteration * (1 << 24), total_games=n_games)
+    engine.selfplay_begin(slots, first_game_id=iteration * (1 << 24), total_games=n_games, leaves_per_game=leaves_per_game,
+                          virtual_loss=virtual_loss)
     new_unique = steps = waves = 0
     while True:
         st = engine.selfplay_step(waves_per_call)
@@ -213,7 +215,8 @@ def run_generation(engine, replay, model, optimizer, iteration, n_games, min_rep
 
 
 def run_generation_sharded(engine, replay, model, optimizer, iteration, games_per_rank, dist, device, min_replay_size=MIN_REPLAY_SIZE,
-                           waves_per_call=64, num_steps=NUM_TRAIN_STEPS, batch_size=BATCH_SIZE, concurrent=None, exchange=None):
+                           waves_per_call=64, num_steps=NUM_TRAIN_STEPS, batch_size=BATCH_SIZE, concurrent=None, exchange=None,
+                           leaves_per_game=None, virtual_loss=1.0):
     """run_generation over several GPUs (BASELINE config 5; SURVEY 8(e)).  Every rank plays EXACTLY games_per_rank games to
     completion (disjoint game ids, no data-path collective) and holds its own replica of the replay buffer, model and
     optimizer.  On CUDA the finished games' steps go device -> NCCL all-gather -> device (sharding.DeviceSampleExchange) and
@@ -230,7 +233,8 @@ def run_generation_sharded(engine, replay, model, optimizer, iteration, games_pe
             dist.broadcast(t.data, src=0)
     engine.load_weights(export_weights(model))
     slots = min(games_per_rank, concurrent or engine.config.max_games, engine.config.max_games)
-    engine.selfplay_begin(slots, first_game_id=sharding.first_game_id(rank) + iteration * (1 << 24), total_games=games_per_rank)
+    engine.selfplay_begin(slots, first_game_id=sharding.first_game_id(rank) + iteration * (1 << 24), total_games=games_per_rank,
+                          leaves_per_game=leaves_per_game, virtual_loss=virtual_loss)
     if on_gpu and exchange is None:
         exchange = sharding.DeviceSampleExchange(engine, dist, device, max(engine.config.max_games * 128, 1 << 16))
     import time

@@ -58,6 +58,9 @@ extern "C" {
                               scores: *mut f32, depth: *mut i32, stats: *mut az_search_stats) -> c_int;
     pub fn az_selfplay_begin(eng: *mut az_engine, n_games: c_int, first_game_id: u64) -> c_int;
     pub fn az_selfplay_begin_n(eng: *mut az_engine, n_concurrent: c_int, first_game_id: u64, total_games: u64) -> c_int;
+    pub fn az_selfplay_begin_vl(eng: *mut az_engine, n_concurrent: c_int, first_game_id: u64, total_games: u64,
+                                leaves_per_game: c_int, virtual_loss: f32) -> c_int;                 // not in the reference
+    pub fn az_selfplay_vl_stats(eng: *mut az_engine, stats: *mut az_search_stats) -> c_int;
     pub fn az_selfplay_step(eng: *mut az_engine, waves: c_int, stats: *mut az_selfplay_stats) -> c_int;
     pub fn az_selfplay_drain(eng: *mut az_engine, out: *mut az_sample, max_samples: c_int, n_out: *mut c_int) -> c_int;
     pub fn az_selfplay_drain_dev(eng: *mut az_engine, out_dev: *mut az_sample, max_samples: c_int, n_out: *mut c_int) -> c_int;

@@ -128,8 +128,22 @@ impl Engine {
     /// run_all_episodes (training.rs:340-378): EXACTLY `n_games` self-play games (ids first_game_id ..), each played to
     /// completion; the callback receives the finished games' steps (values already back-filled) as they become available.
     /// Returns the average batch size (= evaluations per wave).
-    pub fn run_all_episodes<F: FnMut(&[sys::az_sample])>(&mut self, n_games: i32, first_game_id: u64, mut sink: F) -> Result<f32> {
+    pub fn run_all_episodes<F: FnMut(&[sys::az_sample])>(&mut self, n_games: i32, first_game_id: u64, sink: F) -> Result<f32> {
         self.check(unsafe { sys::az_selfplay_begin_n(self.raw, n_games, first_game_id, n_games as u64) })?;
+        self.collect_episodes(n_games, sink)
+    }
+
+    /// Not in the reference: `run_all_episodes` with every ply searched leaf-parallel, up to `leaves_per_game` leaves per game
+    /// and network round under `virtual_loss` (az_selfplay_begin_vl); `leaves_per_game = 1` plays the same games record for
+    /// record.  Needs `n_games * leaves_per_game <= max_batch`.
+    pub fn run_all_episodes_vl<F: FnMut(&[sys::az_sample])>(&mut self, n_games: i32, first_game_id: u64, leaves_per_game: i32,
+                                                            virtual_loss: f32, sink: F) -> Result<f32> {
+        self.check(unsafe { sys::az_selfplay_begin_vl(self.raw, n_games, first_game_id, n_games as u64, leaves_per_game, virtual_loss) })?;
+        self.collect_episodes(n_games, sink)
+    }
+
+    // steps the self-play just begun until every game has ended, handing the finished games' steps to `sink`
+    fn collect_episodes<F: FnMut(&[sys::az_sample])>(&mut self, n_games: i32, mut sink: F) -> Result<f32> {
         let mut buf: Vec<sys::az_sample> = Vec::with_capacity((n_games as usize * 128).max(1 << 16));
         let mut stats = sys::az_selfplay_stats::default();
         let mut waves = 0u64;

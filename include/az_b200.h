@@ -217,6 +217,22 @@ int az_selfplay_begin(az_engine* eng, int n_games, uint64_t first_game_id);
  * first_game_id .. first_game_id + total_games - 1; a slot whose game ends takes the next unplayed id or goes idle, and
  * stats.active_games reaches 0 when the generation is complete.  total_games = 0: games restart forever (az_selfplay_begin). */
 int az_selfplay_begin_n(az_engine* eng, int n_concurrent, uint64_t first_game_id, uint64_t total_games);
+/* NOT IN THE REFERENCE: az_selfplay_begin_n with the search of every ply run as in az_search_vl (a non-parity mode, except at
+ * leaves_per_game = 1, where every record is byte-identical to az_selfplay_begin_n's).  Each game puts up to leaves_per_game (K)
+ * leaves into every network round (virtual loss, collisions end a game's batch, expansion after the gather, backups in leaf
+ * order); a game whose search is complete plays its move and gathers the first batch of its next ply in the same wave.  Root
+ * priors, noise, move choice, exactly-N / endless generations, parking and draining are those of az_selfplay_begin_n, and a
+ * game's records depend only on (config, seed, game id, K, virtual_loss, network), not on the slots or the other games.
+ * az_selfplay_step then runs these waves, with stats as documented above except: evaluations = boards sent to the network,
+ * cache_hits = 0, sum_edges = 0.  Errors (the engine stays usable): AZ_ERR_INVALID_ARGUMENT for K < 1 or a negative or
+ * non-finite virtual_loss, AZ_ERR_CAPACITY when n_concurrent x K > az_config.max_batch, AZ_ERR_STATE with the evaluation cache
+ * (cache_log2 > 0), AZ_ERR_NO_WEIGHTS as az_selfplay_begin_n.  Uses the buffers of az_search_vl (allocated by the first call of
+ * either).  A later az_selfplay_begin_n or az_search* call returns the engine to the default path. */
+int az_selfplay_begin_vl(az_engine* eng, int n_concurrent, uint64_t first_game_id, uint64_t total_games, int leaves_per_game,
+                         float virtual_loss);
+/* since az_selfplay_begin_vl: waves (network rounds of az_selfplay_step), leaf evaluations (the start-position forward is not
+ * counted), terminal leaves and collisions.  AZ_ERR_STATE when no az_selfplay_begin_vl self-play is in progress. */
+int az_selfplay_vl_stats(az_engine* eng, az_search_stats* stats_out);
 int az_selfplay_step(az_engine* eng, int waves, az_selfplay_stats* stats_out);
 int az_selfplay_drain(az_engine* eng, az_sample* out, int max_samples, int* n_out);
 /* same, into DEVICE memory (e.g. the send buffer of an NCCL gather): no host hop between self-play and the replay buffer */

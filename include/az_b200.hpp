@@ -234,12 +234,10 @@ struct EpisodeStep {            // training.rs:15-20
     std::size_t search_depth;
 };
 
-// run_all_episodes(model): `n_games` self-play games on the device; returns (avg_batch_size, steps of the finished games)
-inline std::pair<float, std::vector<EpisodeStep>> run_all_episodes(AlphaZero& model, int n_games, uint64_t first_game_id = 0,
-                                                                   int waves_per_call = 64) {
-    Engine& e = model.engine();
-    // exactly the games first_game_id .. first_game_id + n_games - 1, each played to completion (training.rs:352-361,376-377)
-    e.check(az_selfplay_begin_n(e.handle(), n_games, first_game_id, (uint64_t)n_games), "az_selfplay_begin_n");
+namespace detail {
+// the games first_game_id .. first_game_id + n_games - 1 of the self-play just begun, each played to completion
+// (training.rs:352-361,376-377); returns (avg_batch_size, steps of the finished games)
+inline std::pair<float, std::vector<EpisodeStep>> collect_episodes(Engine& e, int n_games, uint64_t first_game_id, int waves_per_call) {
     std::vector<EpisodeStep> steps;
     std::vector<az_sample> buf((std::size_t)std::max(n_games * 128, 1 << 16));
     const float sims = (float)e.config().num_simulations;
@@ -269,6 +267,25 @@ inline std::pair<float, std::vector<EpisodeStep>> run_all_episodes(AlphaZero& mo
         if (st.active_games == 0 && st.pending_samples == 0) break;  // every slot is idle: all n_games episodes are complete
     }
     return {(float)(evals / batches), std::move(steps)};
+}
+}  // namespace detail
+
+// run_all_episodes(model): `n_games` self-play games on the device; returns (avg_batch_size, steps of the finished games)
+inline std::pair<float, std::vector<EpisodeStep>> run_all_episodes(AlphaZero& model, int n_games, uint64_t first_game_id = 0,
+                                                                   int waves_per_call = 64) {
+    Engine& e = model.engine();
+    e.check(az_selfplay_begin_n(e.handle(), n_games, first_game_id, (uint64_t)n_games), "az_selfplay_begin_n");
+    return detail::collect_episodes(e, n_games, first_game_id, waves_per_call);
+}
+
+// NOT IN THE REFERENCE: the same games with every ply searched leaf-parallel, up to leaves_per_game leaves per game and network
+// round under virtual loss (az_selfplay_begin_vl); leaves_per_game = 1 plays the overload above's games record for record
+inline std::pair<float, std::vector<EpisodeStep>> run_all_episodes(AlphaZero& model, int n_games, uint64_t first_game_id, int waves_per_call,
+                                                                   int leaves_per_game, float virtual_loss) {
+    Engine& e = model.engine();
+    e.check(az_selfplay_begin_vl(e.handle(), n_games, first_game_id, (uint64_t)n_games, leaves_per_game, virtual_loss),
+            "az_selfplay_begin_vl");
+    return detail::collect_episodes(e, n_games, first_game_id, waves_per_call);
 }
 
 // ---- memory.rs ----------------------------------------------------------------------------------------------------

@@ -32,6 +32,9 @@ def main():
     ap.add_argument("--iterations", type=int, default=3)
     ap.add_argument("--eval-games", type=int, default=32)
     ap.add_argument("--min-replay", type=int, default=5000)
+    ap.add_argument("--leaves-per-game", type=int, default=None,
+                    help="leaf-parallel self-play with virtual loss (not in the reference): up to K leaves per game and network round")
+    ap.add_argument("--virtual-loss", type=float, default=1.0, help="virtual loss of --leaves-per-game")
     ap.add_argument("--all-ranks", action="store_true", help="every rank prints its line (replica check)")
     args = ap.parse_args()
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -44,7 +47,9 @@ def main():
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=dev)
     torch.manual_seed(42)
-    eng = az.Engine(device=local, max_games=args.games, num_simulations=args.sims, seed=42)
+    vl = dict(leaves_per_game=args.leaves_per_game, virtual_loss=args.virtual_loss)
+    batch = {} if args.leaves_per_game is None else {"max_batch": args.games * args.leaves_per_game}   # one round: games x K boards
+    eng = az.Engine(device=local, max_games=args.games, num_simulations=args.sims, seed=42, **batch)
     # every rank holds a replica of the model, the optimizer and the replay buffer; they stay identical because every rank
     # adds the same steps in the same order and applies the same all-reduced gradients
     model = tr.import_weights(tr.AlphaZeroNet(), az.random_weights(seed=42)).to(dev)
@@ -60,9 +65,9 @@ def main():
             old.load_weights(tr.export_weights(model))
         t0 = time.perf_counter()
         if world == 1:
-            m = tr.run_generation(eng, replay, model, opt, it, args.games, min_replay_size=args.min_replay)
+            m = tr.run_generation(eng, replay, model, opt, it, args.games, min_replay_size=args.min_replay, **vl)
         else:
-            m = tr.run_generation_sharded(eng, replay, model, opt, it, args.games, dist, dev, min_replay_size=args.min_replay)
+            m = tr.run_generation_sharded(eng, replay, model, opt, it, args.games, dist, dev, min_replay_size=args.min_replay, **vl)
         torch.cuda.synchronize()
         m["generation_seconds"] = time.perf_counter() - t0
         m["positions_per_sec"] = m["positions"] / m["generation_seconds"]
