@@ -57,6 +57,24 @@ class SearchStats(ctypes.Structure):
     _fields_ = [(n, ctypes.c_uint64) for n in ("waves", "evaluations", "terminal_leaves", "collisions")]
 
 
+class MatchConfig(ctypes.Structure):
+    """az_match_config."""
+
+    _fields_ = [("player_kind", ctypes.c_int32), ("network", ctypes.c_uint8 * 2), ("num_simulations", ctypes.c_int32),
+                ("leaves_per_root", ctypes.c_int32), ("virtual_loss", ctypes.c_float), ("num_stochastic_moves", ctypes.c_uint32),
+                ("max_plies", ctypes.c_uint32), ("seed", ctypes.c_uint64)]
+
+
+class MatchStats(ctypes.Structure):
+    """az_match_stats: totals since az_match_begin."""
+
+    _fields_ = [("waves", ctypes.c_uint64), ("evaluations", ctypes.c_uint64 * 2)] + [
+        (n, ctypes.c_uint64) for n in ("leaves", "terminal_leaves", "collisions", "plies", "games_finished", "active_games")]
+
+
+MATCH_MCTS, MATCH_BASE_MODEL = 0, 1
+
+
 class EngineError(RuntimeError):
     pass
 
@@ -360,6 +378,39 @@ class Engine:
                                                ctypes.c_float(virtual_loss), _ptr(net), _ptr(ids), _ptr(pl), _ptr(visits), _ptr(scores),
                                                _ptr(depth), ctypes.byref(st)), "az_search_networks")
         return visits, scores, depth, st
+
+    # ---- validation.rs ----------------------------------------------------------------------------------------
+    def match_begin(self, n_concurrent, n_games, player_kind, networks=(0, 1), num_simulations=None, leaves_per_root=1,
+                    virtual_loss=1.0, num_stochastic_moves=15, max_plies=450, seed=0, first_game=0):
+        """evaluate (validation.rs:155-282) resident on the device (az_match_begin): games first_game .. first_game + n_games - 1
+        on n_concurrent slots, player 1 on network slot networks[0] and White in even games, player 2 on networks[1].
+        player_kind: MATCH_MCTS (both search, num_simulations None = the config's) or MATCH_BASE_MODEL (both play the policy)."""
+        c = MatchConfig()
+        c.player_kind = int(player_kind)
+        if any(int(s) < 0 for s in networks):
+            raise ValueError("network ids must be >= 0")
+        c.network[0], c.network[1] = (min(int(s), 255) for s in networks)
+        c.num_simulations = int(num_simulations or 0)
+        c.leaves_per_root, c.virtual_loss = int(leaves_per_root), float(virtual_loss)
+        c.num_stochastic_moves, c.max_plies, c.seed = int(num_stochastic_moves), int(max_plies), int(seed)
+        self._check(self._L.az_match_begin(self._h, int(n_concurrent), ctypes.c_uint32(first_game), ctypes.c_uint32(n_games),
+                                           ctypes.byref(c)), "az_match_begin")
+        self._match_shape = (int(n_games), int(max_plies))
+
+    def match_step(self, waves):
+        """Advances the match by `waves` network rounds; returns MatchStats (active_games == 0: complete)."""
+        st = MatchStats()
+        self._check(self._L.az_match_step(self._h, int(waves), ctypes.byref(st)), "az_match_step")
+        return st
+
+    def match_results(self):
+        """Per game of the last match begun: (result from White's side [n] int8, plies [n] uint16, finished by the rules [n]
+        bool, moves [n, max_plies] uint16 policy indices, MOVE_NONE after the last)."""
+        n, max_plies = getattr(self, "_match_shape", (0, 0))
+        result, plies = np.empty(n, np.int8), np.empty(n, np.uint16)
+        finished, moves = np.empty(n, np.uint8), np.empty((n, max_plies), np.uint16)
+        self._check(self._L.az_match_results(self._h, _ptr(result), _ptr(plies), _ptr(finished), _ptr(moves)), "az_match_results")
+        return result, plies, finished.astype(bool), moves
 
     # ---- training.rs ------------------------------------------------------------------------------------------
     def selfplay_begin(self, n_games, first_game_id=0, total_games=0, leaves_per_game=None, virtual_loss=1.0):

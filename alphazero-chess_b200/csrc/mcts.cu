@@ -1225,6 +1225,201 @@ __global__ void __launch_bounds__(WARPS * 32) k_vl_selfplay(const __grid_constan
     }
 }
 
+// ------------------------------------------------------------------------------------------- evaluation matches (az_match_*)
+// evaluate (validation.rs:155-282) as alphazero-chess_b200/evaluation.py plays it on one engine, resident: one warp per slot
+// searches a fresh root per ply with az_search_networks' semantics (or takes the priors, for BaseModel players), chooses the move
+// with evaluation.py's rules, plays it through the rules path of move_step and records it.  Semantics in DESIGN.md section 5.
+struct MatchParams {
+    az_position startpos;               // the initial position
+    unsigned long long seed;
+    unsigned long long first_game, end_game;   // the match's game indices [first_game, end_game)
+    unsigned long long* next_game;      // the next game index to start
+    unsigned long long* stats;          // [4] evaluations of network 0, of network 1, plies played, games ended
+    uint8_t* net;                       // [slots] the network of each slot's mover (what NetRoute::net reads)
+    int8_t* result;                     // [games] from White's side
+    uint16_t* plies;                    // [games]
+    uint8_t* finished;                  // [games] 1: ended by the rules
+    uint16_t* moves;                    // [games][row] policy indices played
+    uint32_t row, max_plies, n_stochastic;
+    int base_model;                     // 1: BaseModel players: the move comes from the root's priors, no search
+    int first_wave;                     // 1: every slot starts a game
+    uint8_t network[2];                 // network slot of player 1 and of player 2
+};
+
+// _uniform(seed, game, ply) of evaluation.py (its _mix, not rng_u64), rounded to f32 as _weighted_index does
+__device__ __forceinline__ float match_uniform(u64 seed, u64 game, u64 ply) {
+    u64 h = 0x9E3779B97F4A7C15ULL;
+    h = (h ^ seed) * 0xBF58476D1CE4E5B9ULL; h ^= h >> 29;
+    h = (h ^ game) * 0xBF58476D1CE4E5B9ULL; h ^= h >> 29;
+    h = (h ^ ply) * 0xBF58476D1CE4E5B9ULL; h ^= h >> 29;
+    return __double2float_rn(__dmul_rn((double)(h >> 11), 1.0 / 9007199254740992.0));
+}
+
+// the mover's network: player 1 is White in even games (validation.rs:196-200), so player 1 moves when game + ply is even
+__device__ __forceinline__ int match_network(const MatchParams& mp, u64 game, uint32_t ply) { return mp.network[(game + ply) & 1]; }
+
+// The root of the slot's next ply from sh->child / sh->moves, its evaluation queued in the range of the mover's network
+__device__ __forceinline__ void match_root(Ctx& x, const MatchParams& mp, const NetRoute& rt, unsigned int* evals) {
+    setup_root_from_shared(x);
+    const int s = match_network(mp, x.c.game_id, x.c.ply);
+    if (x.lane == 0) mp.net[x.g] = (uint8_t)s;
+    x.c.pending_node = 0;
+    x.c.pending_slot = submit_request<true>(x, 0, &rt);
+    evals[s]++;
+}
+
+// The next unplayed game starts in this slot (its root queued for evaluation), or the slot goes idle
+__device__ __forceinline__ void match_start_game(Ctx& x, const MatchParams& mp, const NetRoute& rt, unsigned int* evals) {
+    unsigned long long gid = 0;
+    if (x.lane == 0) gid = atomicAdd(mp.next_game, 1ULL);
+    gid = __shfl_sync(0xffffffffu, gid, 0);
+    if (gid >= mp.end_game) { x.c.status = 1; return; }
+    x.c.game_id = gid; x.c.ply = 0; x.c.hist_len = 1;
+    if (x.lane == 0) {
+        DPos s = dpos_from_wire(mp.startpos);
+        ListSink sink{x.sh->moves, 0};
+        const GenInfo gi = gen_legal(s, sink);
+        set_key_bits(s, gi.has_legal_ep);
+        x.sh->child = s; x.sh->n_moves = sink.n; x.sh->term = 0;
+        x.ptr.hist[(size_t)x.g * HIST_CAP] = s;
+    }
+    __syncwarp();
+    match_root(x, mp, rt, evals);
+}
+
+// evaluation.py's move choice at the root: the weights are the visit counts over their f32 sum (_choose_from_visits) or the priors
+// of the legal moves (_choose_from_policy), in policy-index order.  While fullmoves <= num_stochastic_moves: _weighted_index (f32
+// cumulative sums, the first one > f32(u) x total, else the last positive weight); after: _last_argmax.  Zero weights change no
+// cumulative sum and win no maximum, so only the positive ones are ranked.  Returns the chosen root edge.
+__device__ __forceinline__ int match_choose(Ctx& x, const MatchParams& mp, const DPos& root) {
+    const size_t off = x.ebase;   // the root's edges start at 0
+    const int L = (int)((x.c.flags >> 8) & 0xFF);
+    const float* w = mp.base_model ? x.ptr.edge_P + off : x.ptr.edge_N + off;
+    float sum = 0.0f;   // visit counts are integers below 2^24: the f32 sum is exact in any order
+    for (int e = x.lane; e < L; e += 32) sum = __fadd_rn(sum, w[e]);
+    for (int d = 16; d; d >>= 1) sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, d));
+    int nv = 0;
+    for (int e0 = 0; e0 < L; e0 += 32) {
+        const int e = e0 + x.lane;
+        int rank = -1;
+        if (e < L && w[e] > 0.0f) {
+            const uint32_t my = x.ptr.edge_mv[off + e] >> 16;
+            rank = 0;
+            for (int o = 0; o < L; o++)
+                if (w[o] > 0.0f && (x.ptr.edge_mv[off + o] >> 16) < my) rank++;
+            x.sh->sidx[rank] = (uint16_t)e;
+        }
+        nv += __popc(__ballot_sync(0xffffffffu, rank >= 0));
+    }
+    __syncwarp();
+    for (int i = x.lane; i < nv; i += 32) {
+        const float v = w[x.sh->sidx[i]];
+        x.sh->fval[i] = mp.base_model ? v : __fdiv_rn(v, sum);
+    }
+    __syncwarp();
+    int edge = 0;
+    if (x.lane == 0 && nv > 0) {
+        edge = x.sh->sidx[nv - 1];
+        if ((uint32_t)meta_fullmoves(root.meta) <= mp.n_stochastic) {
+            float total = 0.0f;
+            for (int i = 0; i < nv; i++) total = __fadd_rn(total, x.sh->fval[i]);
+            const float chosen = __fmul_rn(match_uniform(mp.seed, x.c.game_id, x.c.ply), total);
+            float cum = 0.0f;
+            for (int i = 0; i < nv; i++) {
+                cum = __fadd_rn(cum, x.sh->fval[i]);
+                if (cum > chosen) { edge = x.sh->sidx[i]; break; }
+            }
+        } else {
+            float best = -1.0f;
+            for (int i = 0; i < nv; i++)
+                if (x.sh->fval[i] >= best) { best = x.sh->fval[i]; edge = x.sh->sidx[i]; }
+        }
+    }
+    return __shfl_sync(0xffffffffu, edge, 0);
+}
+
+// One wave of a match, one warp per slot: consume the root's evaluation or back up the previous batch in leaf order; once the
+// root has S visits (BaseModel: at once) choose and play the move, then either queue the next ply's root in the new mover's
+// network range or record the game and start the next unplayed one; otherwise gather the next batch.  k_vl_expand_nets (leaves
+// routed by mp.net) and the multi-network forward follow.
+__global__ void __launch_bounds__(WARPS * 32) k_match(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
+                                                      const __grid_constant__ VLPtrs vl, const __grid_constant__ NetRoute rt,
+                                                      const __grid_constant__ MatchParams mp) {
+    __shared__ WarpShared shared[WARPS];
+    const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (g >= prm.n_games) return;
+    GameCtl c;
+    if (mp.first_wave) memset(&c, 0, sizeof c);
+    else c = ptr.ctl[g];
+    Ctx x{prm, ptr, &shared[threadIdx.x >> 5], g, (int)(threadIdx.x & 31), (size_t)g * prm.node_cap, (size_t)g * prm.edge_cap, c,
+          0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    if (!mp.first_wave && x.c.status != 0) return;   // idle slot or pool overflow: vl.count[g] is already 0
+    unsigned int evals[AZ_MAX_NETWORKS] = {0, 0}, plies = 0, games = 0;
+    int n_leaf = 0, collided = 0;
+    bool move = false;
+    if (mp.first_wave) {
+        match_start_game(x, mp, rt, evals);
+    } else if (x.c.pending_node == 0) {   // MCTree::init: the root's priors (no noise), no descent in flight
+        const int L = (int)((x.c.flags >> 8) & 0xFF);
+        if (!prm.priors_scattered) {
+            const float* pol = ptr.res_policy + (size_t)x.c.pending_slot * AZ_ACTION_SPACE;
+            for (int e = x.lane; e < L; e += 32) ptr.edge_P[x.ebase + e] = pol[ptr.edge_mv[x.ebase + e] >> 16];
+        }
+        for (int e = x.lane; e < L; e += 32) vl.V[x.ebase + e] = 0;
+        __syncwarp();
+        x.c.pending_node = -1;
+        move = mp.base_model != 0;
+    } else {
+        const int nl = vl.count[g];
+        int evaluated = 0;   // leaves that went to the network (the others were terminal)
+        for (int k0 = 0; k0 < nl; k0 += 32) {
+            const int k = k0 + x.lane;
+            evaluated += __popc(__ballot_sync(0xffffffffu, k < nl && vl.slot[g * vl.K + k] >= 0));
+        }
+        evals[match_network(mp, x.c.game_id, x.c.ply)] += evaluated;
+        x.c.sims_done += vl_backup_batch(x, prm, ptr, vl);
+        move = (int)x.c.sims_done >= prm.S;
+    }
+    if (move) {
+        const DPos root = ptr.node_pos[x.nbase];
+        const int e = match_choose(x, mp, root);
+        const uint32_t amv = ptr.edge_mv[x.ebase + e];
+        lane0_make_child(x, root, (uint16_t)(amv & 0xFFFF));
+        int term = x.sh->term;
+        if (term == 0 && draw_by_rules(x, ptr.path + (size_t)g * prm.node_cap, x.sh->child, 1)) term = 1;
+        const size_t gi = (size_t)(x.c.game_id - mp.first_game);
+        if (x.lane == 0 && x.c.ply < mp.row) mp.moves[gi * mp.row + x.c.ply] = (uint16_t)(amv >> 16);
+        plies++;
+        if (term != 0 || x.c.ply + 1 >= mp.max_plies) {
+            if (x.lane == 0) {   // term 2: the side to move in the child is mated, the mover won
+                mp.result[gi] = term == 2 ? (meta_turn(root.meta) == 0 ? 1 : -1) : 0;
+                mp.plies[gi] = (uint16_t)(x.c.ply + 1);
+                mp.finished[gi] = term != 0 ? 1 : 0;
+            }
+            games++;
+            match_start_game(x, mp, rt, evals);
+        } else {
+            if (x.lane == 0 && x.c.hist_len < HIST_CAP) ptr.hist[(size_t)g * HIST_CAP + x.c.hist_len] = x.sh->child;
+            x.c.hist_len = min(x.c.hist_len + 1, (uint32_t)HIST_CAP);
+            x.c.ply++;
+            match_root(x, mp, rt, evals);
+        }
+    } else if (x.c.status == 0 && x.c.pending_node < 0) {
+        unsigned int depth_sum = 0;
+        n_leaf = vl_gather_batch(x, prm, vl, collided, depth_sum);
+    }
+    if (x.lane == 0) {
+        vl.count[g] = n_leaf;   // 0 when the slot moved, went idle or waits for its root: the next wave backs up nothing
+        if (n_leaf) atomicAdd(&vl.stats[0], (unsigned long long)n_leaf);
+        if (collided) atomicAdd(&vl.stats[2], 1ULL);
+        if (evals[0]) atomicAdd(&mp.stats[0], (unsigned long long)evals[0]);
+        if (evals[1]) atomicAdd(&mp.stats[1], (unsigned long long)evals[1]);
+        if (plies) atomicAdd(&mp.stats[2], (unsigned long long)plies);
+        if (games) atomicAdd(&mp.stats[3], (unsigned long long)games);
+        ptr.ctl[g] = x.c;
+    }
+}
+
 // ------------------------------------------------------------------------------------------- host side
 template <class T>
 static int salloc(az_engine* e, SearchState* st, T** p, size_t n) {
@@ -1309,6 +1504,7 @@ void search_destroy(az_engine* e) {
     SearchState* st = e->search;
     if (!st) return;
     for (void* p : st->allocs) cudaFree(p);
+    for (void* p : {(void*)st->match_result, (void*)st->match_plies, (void*)st->match_finished, (void*)st->match_moves}) cudaFree(p);
     delete st;
     e->search = nullptr;
 }
@@ -1419,6 +1615,7 @@ static int search_begin(az_engine* e, int n, const az_position* roots, const az_
     if (e->stub_kind == 0 && !route && !e->net->loaded) return set_err(e, AZ_ERR_NO_WEIGHTS, "az_load_weights has not been called");
     cudaSetDevice(e->cfg.device);
     st->selfplay_active = false;
+    st->match_active = false;
     SearchParams prm = st->prm;
     prm.n_games = n; prm.S = num_simulations; prm.mode = 0;
     run = *st;
@@ -1749,6 +1946,7 @@ static int selfplay_begin(az_engine* e, int n_games, uint64_t first_game_id, uin
     st->sp_vl_lambda = virtual_loss;
     st->sp_vl_waves = 0;
     st->selfplay_active = true;
+    st->match_active = false;
     return AZ_OK;
 }
 
@@ -1914,6 +2112,186 @@ int az_dbg_selfplay_staged(az_engine* e, int slot, az_sample* out, int max_sampl
     const int n = std::min<int>((int)c.n_samples, max_samples);
     if (n) AZ_CUDA(e, cudaMemcpy(out, st->ptr.game_samples + (size_t)slot * MAX_SAMPLE_PLIES, (size_t)n * sizeof(az_sample), cudaMemcpyDeviceToHost));
     *n_out = n;
+    return AZ_OK;
+}
+
+}  // extern "C"
+
+namespace azb {
+
+// the match's per-game results, (re)allocated when a match needs more room than the last one (freed by search_destroy)
+static int match_alloc(az_engine* e, SearchState* st, size_t games, size_t row) {
+    if (!st->match_next && (salloc(e, st, &st->match_next, 1) || salloc(e, st, &st->match_stats, 4))) return AZ_ERR_OUT_OF_MEMORY;
+    if (games > st->match_cap) {
+        for (void* p : {(void*)st->match_result, (void*)st->match_plies, (void*)st->match_finished}) cudaFree(p);
+        st->match_result = nullptr; st->match_plies = nullptr; st->match_finished = nullptr; st->match_cap = 0;
+        AZ_CUDA(e, cudaMalloc(&st->match_result, games));
+        AZ_CUDA(e, cudaMalloc(&st->match_plies, games * sizeof(uint16_t)));
+        AZ_CUDA(e, cudaMalloc(&st->match_finished, games));
+        st->match_cap = games;
+    }
+    if (games * row > st->match_moves_cap) {
+        cudaFree(st->match_moves);
+        st->match_moves = nullptr; st->match_moves_cap = 0;
+        AZ_CUDA(e, cudaMalloc(&st->match_moves, games * row * sizeof(uint16_t)));
+        st->match_moves_cap = games * row;
+    }
+    return AZ_OK;
+}
+
+// network 0's range starts at board 0, network 1's at round4(slots x K): a slot queues at most K boards per wave (its batch or
+// its next root), all in its mover's range
+static int match_base1(const SearchState* st) { return (st->prm.n_games * st->match_K + 3) & ~3; }
+
+static MatchParams match_params(const SearchState* st) {
+    const az_match_config& c = st->match_cfg;
+    MatchParams mp;
+    mp.startpos = st->match_startpos;
+    mp.seed = c.seed;
+    mp.first_game = st->match_first;
+    mp.end_game = st->match_first + st->match_games;
+    mp.next_game = st->match_next;
+    mp.stats = st->match_stats;
+    mp.net = st->d_net;
+    mp.result = st->match_result; mp.plies = st->match_plies; mp.finished = st->match_finished; mp.moves = st->match_moves;
+    mp.row = st->match_row; mp.max_plies = c.max_plies; mp.n_stochastic = c.num_stochastic_moves;
+    mp.base_model = c.player_kind == 1 ? 1 : 0;
+    mp.first_wave = st->match_first_wave;
+    mp.network[0] = c.network[0]; mp.network[1] = c.network[1];
+    return mp;
+}
+
+}  // namespace azb
+
+extern "C" {
+
+int az_match_begin(az_engine* e, int n_concurrent, uint32_t first_game, uint32_t n_games, const az_match_config* cfg) {
+    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+    if (!cfg) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "null config");
+    SearchState* st = e->search;
+    const bool mcts = cfg->player_kind == 0;
+    if (cfg->player_kind != 0 && cfg->player_kind != 1) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "player_kind must be 0 (MCTS) or 1 (BaseModel)");
+    if (cfg->network[0] >= AZ_MAX_NETWORKS || cfg->network[1] >= AZ_MAX_NETWORKS)
+        return set_err(e, AZ_ERR_INVALID_ARGUMENT, "network id must be < AZ_MAX_NETWORKS");
+    const int S = cfg->num_simulations ? cfg->num_simulations : e->cfg.num_simulations;
+    if (mcts) {
+        if (cfg->leaves_per_root < 1) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "leaves_per_root must be >= 1");
+        if (!(cfg->virtual_loss >= 0.0f) || !std::isfinite(cfg->virtual_loss))
+            return set_err(e, AZ_ERR_INVALID_ARGUMENT, "virtual_loss must be finite and >= 0");
+        if (S < 1 || S > e->cfg.num_simulations)
+            return set_err(e, AZ_ERR_INVALID_ARGUMENT, "num_simulations must be in 1 .. az_config.num_simulations");
+    }
+    if (n_concurrent < 1 || n_games == 0 || cfg->max_plies == 0)
+        return set_err(e, AZ_ERR_INVALID_ARGUMENT, "n_concurrent, n_games and max_plies must be positive");
+    const int K = mcts ? cfg->leaves_per_root : 1;
+    if (n_concurrent > st->G) return set_err(e, AZ_ERR_CAPACITY, "more slots than az_config.max_games");
+    const int n = (int)std::min<uint64_t>((uint64_t)n_concurrent, n_games);
+    if (((long long)n * K + 3) / 4 * 4 * 2 > (long long)e->max_batch)
+        return set_err(e, AZ_ERR_CAPACITY, "network ranges (2 x round4(slots x leaves_per_root)) exceed az_config.max_batch");
+    if (e->stub_kind == 0) {
+        for (int p = 0; p < 2; p++) {
+            const NetWeights* w = net_slot(e, cfg->network[p]);
+            if (!w || !w->loaded) return set_err(e, AZ_ERR_NO_WEIGHTS, "a player names a network that has not been loaded");
+        }
+        const int r = net_networks_supported(e);
+        if (r) return r;
+    }
+    cudaSetDevice(e->cfg.device);
+    int r = vl_alloc(e, st);
+    if (r) return r;
+    if (!st->d_net && salloc(e, st, &st->d_net, (size_t)st->G)) return AZ_ERR_OUT_OF_MEMORY;
+    const uint32_t row = std::min<uint32_t>(cfg->max_plies, HIST_CAP);   // a game ends by the fullmove rule before HIST_CAP plies
+    r = match_alloc(e, st, n_games, row);
+    if (r) return r;
+    st->selfplay_active = false;
+    st->match_cfg = *cfg;
+    st->match_cfg.num_simulations = S;
+    st->match_first = first_game;
+    st->match_games = n_games;
+    st->match_K = K;
+    st->match_row = row;
+    st->match_first_wave = 1;
+    st->match_waves = 0;
+    az_position_start(&st->match_startpos);
+    st->prm.n_games = n; st->prm.S = S; st->prm.mode = 0;
+    st->prm.priors_scattered = (e->stub_kind == 0 && e->cfg.precision != 1) ? 1 : 0;
+    st->ptr.batch_count = st->batch_base;
+    st->ptr.batch_zero = nullptr;
+    const unsigned long long next = first_game;
+    AZ_CUDA(e, cudaMemcpyAsync(st->match_next, &next, sizeof next, cudaMemcpyHostToDevice, e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(st->match_stats, 0, 4 * sizeof(unsigned long long), e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(st->vl_stats, 0, 4 * sizeof(unsigned long long), e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(st->match_result, 0, n_games, e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(st->match_plies, 0, (size_t)n_games * sizeof(uint16_t), e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(st->match_finished, 0, n_games, e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(st->match_moves, 0xFF, (size_t)n_games * row * sizeof(uint16_t), e->stream));
+    AZ_CUDA(e, cudaStreamSynchronize(e->stream));
+    st->match_active = true;
+    return AZ_OK;
+}
+
+int az_match_step(az_engine* e, int waves, az_match_stats* out) {
+    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+    if (out) std::memset(out, 0, sizeof *out);
+    SearchState* st = e->search;
+    if (!st->match_active) return set_err(e, AZ_ERR_STATE, "no match in progress (az_match_begin)");
+    cudaSetDevice(e->cfg.device);
+    const int n = st->prm.n_games, K = st->match_K, base1 = match_base1(st);
+    const VLPtrs vl = vl_ptrs(st, K, st->match_cfg.virtual_loss);
+    const NetRoute route{st->d_net, st->batch_base, base1};
+    const NetBatch nb{st->batch_base, base1, base1 + n * K};
+    for (int w = 0; w < waves; w++) {
+        const MatchParams mp = match_params(st);
+        AZ_CUDA(e, cudaMemsetAsync(st->batch_base, 0, AZ_MAX_NETWORKS * sizeof(int), e->stream));   // both ranges start empty
+        prof_mark_search(e);
+        e->n_launches += 2;
+        k_match<<<(n + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr, vl, route, mp);
+        AZ_CUDA(e, cudaGetLastError());
+        k_vl_expand_nets<<<(n * K + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr, vl, route);
+        AZ_CUDA(e, cudaGetLastError());
+        const int r = evaluate_batch(e, st, &nb);
+        if (r) return r;
+        st->match_first_wave = 0;
+        st->match_waves++;
+    }
+    int flags[4] = {0, 0, 0, 0};
+    int* d_flags = st->batch_base + 4;
+    unsigned long long ms[4], vs[4];
+    AZ_CUDA(e, cudaMemsetAsync(d_flags, 0, 16, e->stream));
+    k_count_active<<<(n + 127) / 128, 128, 0, e->stream>>>(st->prm, st->ptr, d_flags);
+    AZ_CUDA(e, cudaGetLastError());
+    AZ_CUDA(e, cudaMemcpyAsync(flags, d_flags, sizeof flags, cudaMemcpyDeviceToHost, e->stream));
+    AZ_CUDA(e, cudaMemcpyAsync(ms, st->match_stats, sizeof ms, cudaMemcpyDeviceToHost, e->stream));
+    AZ_CUDA(e, cudaMemcpyAsync(vs, st->vl_stats, sizeof vs, cudaMemcpyDeviceToHost, e->stream));
+    AZ_CUDA(e, cudaStreamSynchronize(e->stream));
+    if (out) {
+        out->waves = st->match_waves;
+        out->evaluations[0] = ms[0]; out->evaluations[1] = ms[1];
+        out->leaves = vs[0]; out->terminal_leaves = vs[1]; out->collisions = vs[2];
+        out->plies = ms[2]; out->games_finished = ms[3];
+        out->active_games = st->match_first_wave ? std::min<uint64_t>((uint64_t)n, st->match_games) : (uint64_t)flags[0];
+    }
+    if (flags[1]) return set_err(e, AZ_ERR_CAPACITY, "a per-game node/edge pool overflowed during the match (raise edge_capacity_per_node)");
+    return AZ_OK;
+}
+
+int az_match_results(az_engine* e, int8_t* result_out, uint16_t* plies_out, uint8_t* finished_out, uint16_t* moves_out) {
+    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+    SearchState* st = e->search;
+    if (!st->match_games) return set_err(e, AZ_ERR_STATE, "az_match_begin has not been called");
+    if (!result_out || !plies_out || !finished_out) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "null buffer");
+    cudaSetDevice(e->cfg.device);
+    const size_t n = st->match_games;
+    AZ_CUDA(e, cudaMemcpyAsync(result_out, st->match_result, n, cudaMemcpyDeviceToHost, e->stream));
+    AZ_CUDA(e, cudaMemcpyAsync(plies_out, st->match_plies, n * sizeof(uint16_t), cudaMemcpyDeviceToHost, e->stream));
+    AZ_CUDA(e, cudaMemcpyAsync(finished_out, st->match_finished, n, cudaMemcpyDeviceToHost, e->stream));
+    if (moves_out) {   // [n][max_plies]: the device keeps row <= max_plies moves per game, the rest is AZ_MOVE_NONE
+        const size_t mp = st->match_cfg.max_plies, row = st->match_row;
+        if (row < mp) std::memset(moves_out, 0xFF, n * mp * sizeof(uint16_t));
+        AZ_CUDA(e, cudaMemcpy2DAsync(moves_out, mp * sizeof(uint16_t), st->match_moves, row * sizeof(uint16_t), row * sizeof(uint16_t), n,
+                                     cudaMemcpyDeviceToHost, e->stream));
+    }
+    AZ_CUDA(e, cudaStreamSynchronize(e->stream));
     return AZ_OK;
 }
 

@@ -142,6 +142,24 @@ struct SearchState {
     int* vl_count = nullptr;               // [G]
     unsigned long long* vl_stats = nullptr; // [4]
     uint8_t* d_net = nullptr;              // [G] az_search_networks: network of each root (allocated on its first call)
+    // az_match_*: the match in progress (match_active) and the results of the last one begun.  The result buffers belong to the
+    // match and are reallocated only when a larger match begins; the search buffers are shared with az_search_vl
+    bool match_active = false;
+    uint32_t match_games = 0;              // games of the last az_match_begin (0: none yet)
+    int match_K = 1;                       // leaves per root per wave (1 for BaseModel players)
+    uint32_t match_row = 0;                // moves stored per game on the device (<= HIST_CAP: a game ends by then)
+    unsigned long long match_first = 0;    // the first game index
+    int match_first_wave = 0;              // 1 until the first wave has run: every slot starts a game
+    unsigned long long match_waves = 0;
+    unsigned long long* match_next = nullptr;   // [1] next game index to start
+    unsigned long long* match_stats = nullptr;  // [4] evaluations of network 0, of network 1, plies, games ended
+    int8_t* match_result = nullptr;        // [match_cap]
+    uint16_t* match_plies = nullptr;
+    uint8_t* match_finished = nullptr;
+    uint16_t* match_moves = nullptr;       // [match_cap][match_row]
+    size_t match_cap = 0, match_moves_cap = 0;
+    az_match_config match_cfg{};
+    az_position match_startpos{};
     std::vector<void*> allocs;
 };
 

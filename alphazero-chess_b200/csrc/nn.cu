@@ -525,11 +525,17 @@ int net_forward_networks(az_engine* e, const NetBatch& nb, const float* planes_f
         }
         return 0;
     }
-    const az_engine::Knobs& k = e->knobs;
-    if (k.tower_fused != 1 || k.tower_wide != 2 || k.tower_inkernel != 1 || k.tower_split != 0 || k.input_k32 != 1 || k.input_epi2 != 0 ||
-        k.heads_tc != 1)
-        return set_err(e, AZ_ERR_STATE, "a multi-network forward needs the default AZ_TOWER_*, AZ_INPUT_* and AZ_HEADS_TC configuration");
+    const int r = net_networks_supported(e);
+    if (r) return r;
     return net_forward_bf16(e, nullptr, nb.cap, policy_out, value_out, scatter, &nb);
+}
+
+int net_networks_supported(az_engine* e) {
+    const az_engine::Knobs& k = e->knobs;
+    if (e->cfg.precision != 1 && (k.tower_fused != 1 || k.tower_wide != 2 || k.tower_inkernel != 1 || k.tower_split != 0 || k.input_k32 != 1 ||
+                                  k.input_epi2 != 0 || k.heads_tc != 1))
+        return set_err(e, AZ_ERR_STATE, "a multi-network forward needs the default AZ_TOWER_*, AZ_INPUT_* and AZ_HEADS_TC configuration");
+    return AZ_OK;
 }
 
 }  // namespace azb

@@ -82,6 +82,9 @@ int launch_heads_tc_nets(az_engine* e, const NetWeights* w0, const NetWeights* w
 // (net_forward_bf16 with nb), otherwise and on the fp32 path one network after the other over its range
 int net_forward_networks(az_engine* e, const NetBatch& nb, const float* planes_f32, float* policy_out, float* value_out,
                          const HeadScatter* scatter = nullptr);
+// AZ_ERR_STATE (with the engine's error message set) when the bf16 multi-network forward cannot run: it needs the default
+// AZ_TOWER_*, AZ_INPUT_* and AZ_HEADS_TC configuration; AZ_OK otherwise (the fp32 path runs under any configuration)
+int net_networks_supported(az_engine* e);
 // network slot s (0: e->net, 1: e->net1, null until its first load)
 NetWeights* net_slot(az_engine* e, int s);
 // f32 NCHW planes -> bf16 NHWC (`ch` = 64 or 32 channels per square) into net->a_in

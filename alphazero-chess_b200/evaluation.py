@@ -218,6 +218,52 @@ def evaluate(player_1, player_2, rules_engine, n_games=EVALUATION_GAMES, num_sto
             "p2_winrate": (n_games - wins - draws) / n_games, "results": p1, "unfinished": int(active.sum())}
 
 
+def evaluate_on_device(player_1, player_2, n_games=EVALUATION_GAMES, num_stochastic_moves=TEMPERATURE_ANNEALING, seed=0, max_plies=450,
+                       concurrent=None, waves_per_step=256):
+    """evaluate() played resident on the device (Engine.match_begin / match_step / match_results): the same games, bit for bit,
+    for the pairs whose plies evaluate() runs as one joint call -- two MctsPlayers with equal (num_simulations, leaves_per_root,
+    virtual_loss) or two BasePlayers, on one engine -- without a host round trip per ply.  `concurrent` games run at once (None:
+    as many as max_games and the two network ranges allow, 2 x round4(slots x leaves_per_root) <= max_batch).  All n_games run
+    at once, as evaluate() searches them, only when max_games >= n_games and max_batch >= 2 x round4(n_games x leaves_per_root);
+    with fewer slots the games are the same but the match takes more network rounds, so size the engine accordingly.  Returns
+    evaluate()'s dict plus `moves` [n_games, max_plies] (the policy indices played, MOVE_NONE after the last), `plies` [n_games]
+    and `stats` (MatchStats: waves, evaluations per network, ...).
+    Raises ValueError for other pairs."""
+    from . import MATCH_BASE_MODEL, MATCH_MCTS
+
+    kinds = (type(player_1), type(player_2))
+    if kinds[0] is not kinds[1] or kinds[0] not in (MctsPlayer, BasePlayer):
+        raise ValueError("evaluate_on_device plays two MctsPlayers or two BasePlayers; use evaluate() for other pairs")
+    if player_1.engine is not player_2.engine:
+        raise ValueError("evaluate_on_device needs both players on one engine (network slots 0 and 1)")
+    eng = player_1.engine
+    if max_plies < 1:
+        raise ValueError("max_plies must be >= 1")
+    kw = {}
+    if kinds[0] is MctsPlayer:
+        settings = [(p._num_simulations(), p.leaves_per_root, p.virtual_loss) for p in (player_1, player_2)]
+        if settings[0] != settings[1]:
+            raise ValueError("evaluate_on_device needs equal (num_simulations, leaves_per_root, virtual_loss) for both players")
+        kw = dict(num_simulations=settings[0][0], leaves_per_root=settings[0][1], virtual_loss=settings[0][2])
+    k = kw.get("leaves_per_root", 1)
+    if concurrent is None:   # all games at once, as far as max_games and the two network ranges (2 x round4(slots x K)) allow
+        max_batch = max(int(eng.config.max_batch), int(eng.config.max_games))
+        concurrent = min(n_games, int(eng.config.max_games), (max_batch // 2) // 4 * 4 // k)
+    slots = min(int(concurrent), n_games)
+    eng.match_begin(slots, n_games, MATCH_MCTS if kinds[0] is MctsPlayer else MATCH_BASE_MODEL, (player_1.network, player_2.network),
+                    num_stochastic_moves=num_stochastic_moves, max_plies=max_plies, seed=seed, **kw)
+    stats = eng.match_step(waves_per_step)
+    while stats.active_games:
+        stats = eng.match_step(waves_per_step)
+    white, plies, finished, moves = eng.match_results()
+    result = white.astype(np.float32)
+    p1 = np.where(np.arange(n_games) % 2 == 0, result, -result)   # validation.rs:196-200
+    wins, draws = float((p1 == 1).sum()), float((p1 == 0).sum())
+    return {"winrate": (wins + draws / 2.0) / n_games, "p1_winrate": wins / n_games, "drawrate": draws / n_games,
+            "p2_winrate": (n_games - wins - draws) / n_games, "results": p1, "unfinished": int((~finished).sum()),
+            "moves": moves, "plies": plies, "stats": stats}
+
+
 def compute_elos(winrate_matrix, base_elo):
     """ratings.rs:113-144 in f32: player 0 is the anchor, 1000 synchronous updates with step 8."""
     w = np.asarray(winrate_matrix, np.float32)

@@ -125,6 +125,37 @@ impl Engine {
         Ok((visits, depth, stats))
     }
 
+    /// evaluate (validation.rs:155-282) resident on the device (az_match_*): `n_games` games between network slot `network_1`
+    /// (player 1, White in even games) and `network_2`, both searching with `sims` simulations (0: the config's) at
+    /// `leaves_per_root` (1: az_search semantics; more is not in the reference), or both playing the raw policy when `base_model`.
+    /// Moves are sampled while fullmoves <= `num_stochastic_moves`, keyed by (seed, game, ply); games still on after `max_plies`
+    /// count as draws.  As many games run at once as max_games and the two network ranges (2 x round4(slots x K) <= max_batch)
+    /// allow.  Returns (winrate, drawrate, lossrate) from player 1's side.
+    pub fn evaluate(&mut self, network_1: u8, network_2: u8, n_games: u32, num_stochastic_moves: u32, seed: u64, max_plies: u32, sims: i32,
+                    leaves_per_root: i32, virtual_loss: f32, base_model: bool) -> Result<(f32, f32, f32)> {
+        let cfg = sys::az_match_config { player_kind: base_model as i32, network: [network_1, network_2], num_simulations: sims,
+                                         leaves_per_root, virtual_loss, num_stochastic_moves, max_plies, seed };
+        let k = if base_model { 1 } else { leaves_per_root.max(1) };
+        let max_batch = self.config().max_batch.max(self.config().max_games);
+        let slots = (n_games as i64).min(self.config().max_games as i64).min(((max_batch / 2) / 4 * 4 / k) as i64) as i32;
+        self.check(unsafe { sys::az_match_begin(self.raw, slots, 0, n_games, &cfg) })?;
+        let mut stats = sys::az_match_stats::default();
+        loop {
+            self.check(unsafe { sys::az_match_step(self.raw, 256, &mut stats) })?;
+            if stats.active_games == 0 { break; }
+        }
+        let n = n_games as usize;
+        let (mut white, mut plies, mut finished) = (vec![0i8; n], vec![0u16; n], vec![0u8; n]);
+        self.check(unsafe { sys::az_match_results(self.raw, white.as_mut_ptr(), plies.as_mut_ptr(), finished.as_mut_ptr(), ptr::null_mut()) })?;
+        let (mut wins, mut draws) = (0f32, 0f32);
+        for (g, w) in white.iter().enumerate() {
+            let p1 = if g % 2 == 0 { *w } else { -*w };   // validation.rs:196-200
+            if p1 == 1 { wins += 1.0 } else if p1 == 0 { draws += 1.0 }
+        }
+        let total = n_games as f32;
+        Ok(((wins + draws / 2.0) / total, draws / total, (total - wins - draws) / total))
+    }
+
     /// run_all_episodes (training.rs:340-378): EXACTLY `n_games` self-play games (ids first_game_id ..), each played to
     /// completion; the callback receives the finished games' steps (values already back-filled) as they become available.
     /// Returns the average batch size (= evaluations per wave).

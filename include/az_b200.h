@@ -238,6 +238,59 @@ int az_selfplay_drain(az_engine* eng, az_sample* out, int max_samples, int* n_ou
 /* same, into DEVICE memory (e.g. the send buffer of an NCCL gather): no host hop between self-play and the replay buffer */
 int az_selfplay_drain_dev(az_engine* eng, az_sample* out_dev, int max_samples, int* n_out);
 
+/* ---- validation.rs evaluate (validation.rs:155-282) ----------------------------------------------------------------
+ * A match is resident on the device: az_match_begin sets up n_games games (game indices first_game .. first_game + n_games - 1)
+ * on n_concurrent slots, az_match_step advances every slot by `waves` network rounds, az_match_results copies each game's result
+ * and moves to the host.  Both players live on this engine (network slots network[0] for player 1, network[1] for player 2,
+ * equal or not) and share every network round.  Player 1 is White in even games (validation.rs:196-200).  Each ply searches a
+ * fresh root (MCTree::init(model, state, false): no tree reuse, no noise) with the game's whole history, with az_search_vl
+ * semantics at leaves_per_root K (K = 1: az_search) -- or, for BaseModel players, takes the root's priors of the legal moves.
+ * The mover samples while the position's fullmove number <= num_stochastic_moves and otherwise takes the last maximum, over the
+ * weights visits / sum(visits) (MCTS, temperature ignored) or the priors (BaseModel) in policy-index order: f32 cumulative sums,
+ * the first one > f32(u) x total, u = (mix(seed, game, ply) >> 11) x 2^-53 with the splitmix-style mix of
+ * alphazero-chess_b200/evaluation.py (not the engine's generator).  Moves are played through the rules of az_play_move.  A game
+ * still on after max_plies plies is unfinished, with result 0.  A game's moves and result depend only on (config, seed, game
+ * index, the players' settings, the two networks), never on the slots or the other games, and equal those of evaluation.py's
+ * host loop `evaluate`.  NOT IN THE REFERENCE: the reference samples from an unseeded thread_rng, and leaves_per_root > 1 is a
+ * non-parity mode as in az_search_vl. */
+typedef struct az_match_config {
+    int32_t player_kind;           /* 0: Player::MctsModel for both sides, 1: Player::BaseModel for both sides */
+    uint8_t network[2];            /* network slot of player 1 and of player 2 */
+    int32_t num_simulations;       /* MCTS: 1 .. az_config.num_simulations (0: az_config.num_simulations) */
+    int32_t leaves_per_root;       /* MCTS: K >= 1 (1: az_search semantics) */
+    float virtual_loss;            /* MCTS: finite, >= 0 */
+    uint32_t num_stochastic_moves; /* TEMPERATURE_ANNEALING (parameters.rs:31: 15) */
+    uint32_t max_plies;            /* >= 1 (450 in evaluation.py) */
+    uint64_t seed;
+} az_match_config;
+typedef struct az_match_stats {   /* totals since az_match_begin */
+    uint64_t waves;                /* network rounds */
+    uint64_t evaluations[AZ_MAX_NETWORKS]; /* boards sent to each network: roots and non-terminal leaves */
+    uint64_t leaves;               /* leaves gathered by the searches */
+    uint64_t terminal_leaves;
+    uint64_t collisions;
+    uint64_t plies;                /* moves played */
+    uint64_t games_finished;       /* games with a recorded result: ended by the rules or cut at max_plies */
+    uint64_t active_games;         /* games in progress (0: the match is complete) */
+} az_match_stats;
+/* Errors (the engine stays usable): AZ_ERR_INVALID_ARGUMENT for an unknown player_kind, a network id >= AZ_MAX_NETWORKS, and for
+ * MCTS players K < 1, a negative or non-finite virtual_loss or num_simulations out of range; also for n_concurrent < 1, n_games
+ * = 0 or max_plies = 0.  AZ_ERR_NO_WEIGHTS for a network slot never loaded (not under the synthetic evaluator, where network s
+ * uses seed + s).  AZ_ERR_CAPACITY when n_concurrent > az_config.max_games or the two network ranges do not fit
+ * az_config.max_batch: network 0's range holds n_concurrent x K boards from board 0, network 1's as many from
+ * round4(n_concurrent x K), and round4(n_concurrent x K) x 2 must fit (K = 1 for BaseModel players).  AZ_ERR_STATE for a bf16
+ * engine with non-default AZ_TOWER_* / AZ_INPUT_* / AZ_HEADS_TC settings, as az_forward_networks.  Within max_games,
+ * n_concurrent > n_games plays on n_games slots.  The match uses the search buffers of az_search_vl (allocated by the first call of either), so a later
+ * az_selfplay_begin* or az_search* call ends it; az_engine_create's footprint is unchanged. */
+int az_match_begin(az_engine* eng, int n_concurrent, uint32_t first_game, uint32_t n_games, const az_match_config* config);
+/* AZ_ERR_STATE when no match is in progress; AZ_ERR_CAPACITY when a search pool overflowed (raise edge_capacity_per_node) */
+int az_match_step(az_engine* eng, int waves, az_match_stats* stats_out /* nullable */);
+/* per game of the last match begun, in game-index order: result from White's side (1, 0, -1), plies played, 1 if the game ended
+ * by the rules (0: cut at max_plies, or still in progress), and moves_out [n_games][max_plies] the policy indices played
+ * (AZ_MOVE_NONE after the last).  Readable until the next az_match_begin, also after a later search or self-play call ended the
+ * match; AZ_ERR_STATE before the first az_match_begin. */
+int az_match_results(az_engine* eng, int8_t* result_out, uint16_t* plies_out, uint8_t* finished_out, uint16_t* moves_out /* nullable */);
+
 /* ---- memory.rs: ReplayBuffer (SURVEY section 8(f) #1, the consumer of self-play output) ---------------------------
  * Device resident.  az_replay_add mirrors ReplayBuffer::add (memory.rs:41-76) for a batch of EpisodeSteps applied in
  * order: positions are de-duplicated by their FEN identity (pseudo-legal ep, counters), policy/value become running

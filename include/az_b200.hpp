@@ -288,6 +288,55 @@ inline std::pair<float, std::vector<EpisodeStep>> run_all_episodes(AlphaZero& mo
     return detail::collect_episodes(e, n_games, first_game_id, waves_per_call);
 }
 
+// ---- validation.rs ------------------------------------------------------------------------------------------------
+struct EvaluationResult {       // what evaluate (validation.rs:155-282) returns, from player 1's side
+    float winrate;              // (wins + draws / 2) / n_games
+    float drawrate;
+    float lossrate;             // player 2's wins
+};
+
+// evaluate(model, network_1, network_2): n_games games between the model's network slots network_1 (player 1, White in even games)
+// and network_2, both Player::MctsModel with num_simulations (0: the config's), or both Player::BaseModel when base_model is set;
+// played resident on the device (az_match_*), move sampling keyed by (seed, game, ply).  leaves_per_root > 1 (NOT IN THE
+// REFERENCE) searches with virtual loss as az_search_vl.  Games still on after max_plies plies count as draws.  n_concurrent = 0
+// plays as many games at once as max_games and the two network ranges (2 x round4(slots x K) <= max_batch) allow.
+inline EvaluationResult evaluate(AlphaZero& model, int network_1, int network_2, uint32_t n_games = 256, uint32_t num_stochastic_moves = 15,
+                                 uint64_t seed = 0, uint32_t max_plies = 450, int num_simulations = 0, int leaves_per_root = 1,
+                                 float virtual_loss = 1.0f, bool base_model = false, int n_concurrent = 0, int waves_per_call = 256) {
+    Engine& e = model.engine();
+    az_match_config c{};
+    c.player_kind = base_model ? 1 : 0;
+    c.network[0] = (uint8_t)network_1;
+    c.network[1] = (uint8_t)network_2;
+    c.num_simulations = num_simulations;
+    c.leaves_per_root = leaves_per_root;
+    c.virtual_loss = virtual_loss;
+    c.num_stochastic_moves = num_stochastic_moves;
+    c.max_plies = max_plies;
+    c.seed = seed;
+    if (n_concurrent <= 0) {
+        const int k = base_model ? 1 : std::max(leaves_per_root, 1);
+        const int max_batch = std::max(e.config().max_batch, e.config().max_games);
+        n_concurrent = std::min<int64_t>({(int64_t)n_games, (int64_t)e.config().max_games, (int64_t)((max_batch / 2) / 4 * 4 / k)});
+    }
+    e.check(az_match_begin(e.handle(), n_concurrent, 0, n_games, &c), "az_match_begin");
+    az_match_stats st{};
+    do e.check(az_match_step(e.handle(), waves_per_call, &st), "az_match_step");
+    while (st.active_games);
+    std::vector<int8_t> white(n_games);
+    std::vector<uint16_t> plies(n_games);
+    std::vector<uint8_t> finished(n_games);
+    e.check(az_match_results(e.handle(), white.data(), plies.data(), finished.data(), nullptr), "az_match_results");
+    float wins = 0.0f, draws = 0.0f;
+    for (uint32_t g = 0; g < n_games; g++) {
+        const int p1 = g % 2 == 0 ? white[g] : -white[g];   // validation.rs:196-200
+        wins += p1 == 1 ? 1.0f : 0.0f;
+        draws += p1 == 0 ? 1.0f : 0.0f;
+    }
+    const float n = (float)n_games;
+    return {(wins + draws / 2.0f) / n, draws / n, (n - wins - draws) / n};
+}
+
 // ---- memory.rs ----------------------------------------------------------------------------------------------------
 struct TrainingBatch {          // what ReplayBuffer::sample hands to train() (training.rs:150-172), already stacked
     std::size_t n = 0;
