@@ -322,12 +322,11 @@ class Engine:
     def set_evaluator_stub(self, kind, seed=0):
         self._check(self._L.az_set_evaluator_stub(self._h, int(kind), ctypes.c_uint64(seed)), "az_set_evaluator_stub")
 
-    def search(self, roots, num_simulations=None, history=None, hist_offsets=None, noise_game_ids=None, noise_plies=None,
-               want_scores=False):
-        """MCTree::init + monte_carlo_tree_search for a batch of roots: (visits [n,4096], scores or None, depth [n])."""
+    def _search_inputs(self, roots, history, hist_offsets, noise_game_ids, noise_plies, want_scores):
+        """The arguments and output arrays of the az_search* calls: (roots, n, visits, scores or None, depth, history,
+        hist_offsets, noise ids, noise plies), the optional inputs None when not given."""
         p = self._positions(roots)
         n = p.shape[0]
-        sims = int(num_simulations or self.config.num_simulations)
         visits = np.empty((n, ACTION_SPACE), np.float32)
         scores = np.empty((n, ACTION_SPACE), np.float32) if want_scores else None
         depth = np.empty(n, np.int32)
@@ -335,6 +334,14 @@ class Engine:
         ho = np.ascontiguousarray(hist_offsets, np.uint32) if hist_offsets is not None else None
         ids = np.ascontiguousarray(noise_game_ids, np.uint64) if noise_game_ids is not None else None
         pl = np.ascontiguousarray(noise_plies, np.uint32) if noise_plies is not None else None
+        return p, n, visits, scores, depth, h, ho, ids, pl
+
+    def search(self, roots, num_simulations=None, history=None, hist_offsets=None, noise_game_ids=None, noise_plies=None,
+               want_scores=False):
+        """MCTree::init + monte_carlo_tree_search for a batch of roots: (visits [n,4096], scores or None, depth [n])."""
+        p, n, visits, scores, depth, h, ho, ids, pl = self._search_inputs(roots, history, hist_offsets, noise_game_ids, noise_plies,
+                                                                          want_scores)
+        sims = int(num_simulations or self.config.num_simulations)
         self._check(self._L.az_search(self._h, n, _ptr(p), _ptr(h), _ptr(ho), sims, _ptr(ids), _ptr(pl), _ptr(visits), _ptr(scores),
                                       _ptr(depth)), "az_search")
         return visits, scores, depth
@@ -344,15 +351,8 @@ class Engine:
         """Leaf-parallel search with virtual loss (az_search_vl; not in the reference, identical to search() at
         leaves_per_root = 1): up to leaves_per_root leaves per root share one network round.
         Returns (visits [n,4096], scores or None, depth [n], SearchStats)."""
-        p = self._positions(roots)
-        n = p.shape[0]
-        visits = np.empty((n, ACTION_SPACE), np.float32)
-        scores = np.empty((n, ACTION_SPACE), np.float32) if want_scores else None
-        depth = np.empty(n, np.int32)
-        h = self._positions(history) if history is not None else None
-        ho = np.ascontiguousarray(hist_offsets, np.uint32) if hist_offsets is not None else None
-        ids = np.ascontiguousarray(noise_game_ids, np.uint64) if noise_game_ids is not None else None
-        pl = np.ascontiguousarray(noise_plies, np.uint32) if noise_plies is not None else None
+        p, n, visits, scores, depth, h, ho, ids, pl = self._search_inputs(roots, history, hist_offsets, noise_game_ids, noise_plies,
+                                                                          want_scores)
         st = SearchStats()
         self._check(self._L.az_search_vl(self._h, n, _ptr(p), _ptr(h), _ptr(ho), int(num_simulations), int(leaves_per_root),
                                          ctypes.c_float(virtual_loss), _ptr(ids), _ptr(pl), _ptr(visits), _ptr(scores), _ptr(depth),
@@ -363,16 +363,9 @@ class Engine:
                         noise_game_ids=None, noise_plies=None, want_scores=False):
         """search_vl() with a network slot per root (an int or [n] ids): the roots of both networks share every network round.
         Returns (visits [n,4096], scores or None, depth [n], SearchStats)."""
-        p = self._positions(roots)
-        n = p.shape[0]
+        p, n, visits, scores, depth, h, ho, ids, pl = self._search_inputs(roots, history, hist_offsets, noise_game_ids, noise_plies,
+                                                                          want_scores)
         net = self._networks(network, n)
-        visits = np.empty((n, ACTION_SPACE), np.float32)
-        scores = np.empty((n, ACTION_SPACE), np.float32) if want_scores else None
-        depth = np.empty(n, np.int32)
-        h = self._positions(history) if history is not None else None
-        ho = np.ascontiguousarray(hist_offsets, np.uint32) if hist_offsets is not None else None
-        ids = np.ascontiguousarray(noise_game_ids, np.uint64) if noise_game_ids is not None else None
-        pl = np.ascontiguousarray(noise_plies, np.uint32) if noise_plies is not None else None
         st = SearchStats()
         self._check(self._L.az_search_networks(self._h, n, _ptr(p), _ptr(h), _ptr(ho), int(num_simulations), int(leaves_per_root),
                                                ctypes.c_float(virtual_loss), _ptr(net), _ptr(ids), _ptr(pl), _ptr(visits), _ptr(scores),

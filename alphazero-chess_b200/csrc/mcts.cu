@@ -123,6 +123,26 @@ struct Ctx {
     unsigned int st_sdepth;        // sum of EpisodeStep::search_depth over the steps recorded (avg_search_depth, training.rs:91-97)
     unsigned long long new_link;   // edge_link value of the node create_node made last
 };
+// the initial position (az_position_start)
+__device__ __forceinline__ DPos start_dpos() {
+    az_position sp;
+    sp.roles[0] = 0x00FF00000000FF00ULL; sp.roles[1] = 0x4200000000000042ULL; sp.roles[2] = 0x2400000000000024ULL;
+    sp.roles[3] = 0x8100000000000081ULL; sp.roles[4] = 0x0800000000000008ULL; sp.roles[5] = 0x1000000000000010ULL;
+    sp.colors[0] = 0xFFFFULL; sp.colors[1] = 0xFFFF000000000000ULL;
+    sp.turn = 0; sp.castling = 15; sp.ep_square = -1; sp.reserved = 0; sp.halfmoves = 0; sp.fullmoves = 1;
+    return dpos_from_wire(sp);
+}
+
+// the legal-move priors of the L edges from `off`, out of the dense policy row of request `slot` (when the heads did not
+// scatter them into edge_P)
+__device__ __forceinline__ void copy_priors(const SearchPtrs& ptr, size_t off, int L, int slot, int lane) {
+    const float* pol = ptr.res_policy + (size_t)slot * AZ_ACTION_SPACE;
+    for (int e = lane; e < L; e += 32) ptr.edge_P[off + e] = pol[ptr.edge_mv[off + e] >> 16];
+}
+
+__device__ __forceinline__ Ctx make_ctx(const SearchParams& prm, const SearchPtrs& ptr, WarpShared* sh, int g, const GameCtl& c) {
+    return Ctx{prm, ptr, sh, g, (int)(threadIdx.x & 31), (size_t)g * prm.node_cap, (size_t)g * prm.edge_cap, c, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+}
 
 // Expands `mv` from `parent` on lane 0: child position, its legal moves (into shared memory), mate / stalemate /
 // insufficient material.  Repetition and move-count draws are decided afterwards by the whole warp.
@@ -472,12 +492,7 @@ __device__ void start_new_game(Ctx& x) {
     if (x.prm.last_game_id != 0 && gid >= x.prm.last_game_id) { x.c.status = 1; x.c.n_samples = 0; return; }
     x.c.game_id = gid; x.c.ply = 0; x.c.n_samples = 0; x.c.hist_len = 1;
     if (x.lane == 0) {
-        az_position sp;
-        sp.roles[0] = 0x00FF00000000FF00ULL; sp.roles[1] = 0x4200000000000042ULL; sp.roles[2] = 0x2400000000000024ULL;
-        sp.roles[3] = 0x8100000000000081ULL; sp.roles[4] = 0x0800000000000008ULL; sp.roles[5] = 0x1000000000000010ULL;
-        sp.colors[0] = 0xFFFFULL; sp.colors[1] = 0xFFFF000000000000ULL;
-        sp.turn = 0; sp.castling = 15; sp.ep_square = -1; sp.reserved = 0; sp.halfmoves = 0; sp.fullmoves = 1;
-        DPos s = dpos_from_wire(sp);
+        DPos s = start_dpos();
         ListSink sink{x.sh->moves, 0};
         GenInfo gi = gen_legal(s, sink);
         set_key_bits(s, gi.has_legal_ep);
@@ -653,21 +668,21 @@ struct ColdOut {
     GameCtl c;
     unsigned int st_pos, st_games, st_sdepth;
 };
-__device__ __forceinline__ Ctx cold_ctx(const SearchParams* prm, const SearchPtrs* ptr, WarpShared* sh, int g, const GameCtl& c) {
-    return Ctx{*prm, *ptr, sh, g, (int)(threadIdx.x & 31), (size_t)g * prm->node_cap, (size_t)g * prm->edge_cap, c, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+__device__ __forceinline__ void absorb(Ctx& x, const ColdOut& o) {
+    x.c = o.c; x.st_pos += o.st_pos; x.st_games += o.st_games; x.st_sdepth += o.st_sdepth;
 }
 __device__ __noinline__ ColdOut move_step_cold(const SearchParams* prm, const SearchPtrs* ptr, WarpShared* sh, int g, GameCtl c) {
-    Ctx x = cold_ctx(prm, ptr, sh, g, c);
+    Ctx x = make_ctx(*prm, *ptr, sh, g, c);
     move_step(x);
     return ColdOut{x.c, x.st_pos, x.st_games, x.st_sdepth};
 }
 __device__ __noinline__ ColdOut finish_game_cold(const SearchParams* prm, const SearchPtrs* ptr, WarpShared* sh, int g, GameCtl c) {
-    Ctx x = cold_ctx(prm, ptr, sh, g, c);
+    Ctx x = make_ctx(*prm, *ptr, sh, g, c);
     finish_game(x, __uint_as_float(c.park_scale));
     return ColdOut{x.c, x.st_pos, x.st_games, x.st_sdepth};
 }
 __device__ __noinline__ void root_noise_cold(const SearchParams* prm, const SearchPtrs* ptr, WarpShared* sh, int g, GameCtl c) {
-    Ctx x = cold_ctx(prm, ptr, sh, g, c);
+    Ctx x = make_ctx(*prm, *ptr, sh, g, c);
     apply_noise(x, 0, c.game_id, c.noise_ply);
 }
 
@@ -688,18 +703,14 @@ __global__ void __launch_bounds__(WARPS * 32, MINB * 4 / WARPS) k_advance(const 
     if (g >= prm.n_games) return;
     // the path of the pending simulation is requested together with the control block (its address needs only g)
     const uint2 path_spec = ptr.path[(size_t)g * prm.node_cap + min((int)(threadIdx.x & 31), prm.node_cap - 1)];
-    Ctx x{prm, ptr, &shared[threadIdx.x >> 5], g, (int)(threadIdx.x & 31), (size_t)g * prm.node_cap, (size_t)g * prm.edge_cap,
-          ptr.ctl[g], 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    Ctx x = make_ctx(prm, ptr, &shared[threadIdx.x >> 5], g, ptr.ctl[g]);
     if (g == 0 && x.lane == 0 && ptr.batch_zero) *ptr.batch_zero = 0;   // the other wave parity's request counter (see run_wave)
     if (x.c.status != 0 && x.c.status != 4) return;
     if (!prm.consume && x.c.pending_node >= 0) return;   // extra pass: this game already waits for the network
 
     ADV_T0();
     // ---- 0. game over, samples staged: publish now if the host has drained the queue, else stay parked
-    if (x.c.status == 4) {
-        const ColdOut o = finish_game_cold(&prm, &ptr, x.sh, g, x.c);
-        x.c = o.c; x.st_pos += o.st_pos; x.st_games += o.st_games; x.st_sdepth += o.st_sdepth;
-    }
+    if (x.c.status == 4) absorb(x, finish_game_cold(&prm, &ptr, x.sh, g, x.c));
     const bool runnable = x.c.status == 0;
     // ---- 1. the evaluation requested in the previous wave has arrived
     if (runnable && x.c.pending_node >= 0) {
@@ -731,8 +742,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB * 4 / WARPS) k_advance(const 
     for (int iter = 0; runnable && iter < prm.max_iters; iter++) {
         if ((int)x.c.sims_done >= prm.S) {
             if (prm.mode == 0) { x.c.status = 1; break; }
-            const ColdOut o = move_step_cold(&prm, &ptr, x.sh, g, x.c);
-            x.c = o.c; x.st_pos += o.st_pos; x.st_games += o.st_games; x.st_sdepth += o.st_sdepth;
+            absorb(x, move_step_cold(&prm, &ptr, x.sh, g, x.c));
             ADV_T(6);
             if (x.c.status != 0) break;   // idle (generation complete), parked (sample queue full) or an error
             continue;
@@ -820,8 +830,7 @@ __device__ __forceinline__ void init_search_body(const SearchParams& prm, const 
     if (g >= prm.n_games) return;
     GameCtl c;
     memset(&c, 0, sizeof c);
-    Ctx x{prm, ptr, &shared[threadIdx.x >> 5], g, (int)(threadIdx.x & 31), (size_t)g * prm.node_cap, (size_t)g * prm.edge_cap, c,
-          0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    Ctx x = make_ctx(prm, ptr, &shared[threadIdx.x >> 5], g, c);
     x.c.game_id = noise_ids ? noise_ids[g] : 0;
     x.c.noise_ply = noise_plies ? noise_plies[g] : 0;
     x.c.flags = noise_ids ? 1 : 0;
@@ -879,17 +888,11 @@ __global__ void __launch_bounds__(WARPS * 32) k_init_selfplay(SearchParams prm, 
     if (g >= prm.n_games) return;
     GameCtl c;
     memset(&c, 0, sizeof c);
-    Ctx x{prm, ptr, &shared[threadIdx.x >> 5], g, (int)(threadIdx.x & 31), (size_t)g * prm.node_cap, (size_t)g * prm.edge_cap, c,
-          0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    Ctx x = make_ctx(prm, ptr, &shared[threadIdx.x >> 5], g, c);
     x.c.game_id = first_game_id + g;
     x.c.hist_len = 1;
     if (x.lane == 0) {
-        az_position sp;
-        sp.roles[0] = 0x00FF00000000FF00ULL; sp.roles[1] = 0x4200000000000042ULL; sp.roles[2] = 0x2400000000000024ULL;
-        sp.roles[3] = 0x8100000000000081ULL; sp.roles[4] = 0x0800000000000008ULL; sp.roles[5] = 0x1000000000000010ULL;
-        sp.colors[0] = 0xFFFFULL; sp.colors[1] = 0xFFFF000000000000ULL;
-        sp.turn = 0; sp.castling = 15; sp.ep_square = -1; sp.reserved = 0; sp.halfmoves = 0; sp.fullmoves = 1;
-        DPos s = dpos_from_wire(sp);
+        DPos s = start_dpos();
         ListSink sink{x.sh->moves, 0};
         GenInfo gi = gen_legal(s, sink);
         set_key_bits(s, gi.has_legal_ep);
@@ -908,12 +911,7 @@ __global__ void __launch_bounds__(WARPS * 32) k_init_selfplay(SearchParams prm, 
 // start-position priors from a policy row (the single shared forward of training.rs:344-350)
 __global__ void k_start_prior(const float* __restrict__ policy_row, float* __restrict__ start_prior) {
     if (threadIdx.x == 0) {
-        az_position sp;
-        sp.roles[0] = 0x00FF00000000FF00ULL; sp.roles[1] = 0x4200000000000042ULL; sp.roles[2] = 0x2400000000000024ULL;
-        sp.roles[3] = 0x8100000000000081ULL; sp.roles[4] = 0x0800000000000008ULL; sp.roles[5] = 0x1000000000000010ULL;
-        sp.colors[0] = 0xFFFFULL; sp.colors[1] = 0xFFFF000000000000ULL;
-        sp.turn = 0; sp.castling = 15; sp.ep_square = -1; sp.reserved = 0; sp.halfmoves = 0; sp.fullmoves = 1;
-        DPos s = dpos_from_wire(sp);
+        DPos s = start_dpos();
         uint16_t mv[AZ_MAX_MOVES];
         ListSink sink{mv, 0};
         gen_legal(s, sink);
@@ -965,6 +963,13 @@ struct VLPtrs {
     int K;
     float lambda;
 };
+
+// lane 0 at the end of a leaf-parallel wave: the leaves of the slot's new batch (what the next wave backs up) and its statistics
+__device__ __forceinline__ void vl_publish(const VLPtrs& vl, int g, int n_leaf, int collided) {
+    vl.count[g] = n_leaf;
+    if (n_leaf) atomicAdd(&vl.stats[0], (unsigned long long)n_leaf);
+    if (collided) atomicAdd(&vl.stats[2], 1ULL);
+}
 
 // One descent of the gather: PUCT on N' = N + V and W' = W - lambda * V.  `total` is the root's N' (sims done + leaves
 // gathered so far + 1).  Writes path[0..depth] and returns the depth of the leaf edge, or -1 when the chosen edge has no child
@@ -1026,12 +1031,7 @@ __device__ __forceinline__ int vl_backup_batch(Ctx& x, const SearchParams& prm, 
         const int s = vl.slot[leaf];
         float value;
         if (s >= 0) {
-            if (!prm.priors_scattered) {
-                const size_t off = ptr.req_edge_off[s];
-                const int L = ptr.req_nedges[s];
-                const float* pol = ptr.res_policy + (size_t)s * AZ_ACTION_SPACE;
-                for (int e = x.lane; e < L; e += 32) ptr.edge_P[off + e] = pol[ptr.edge_mv[off + e] >> 16];
-            }
+            if (!prm.priors_scattered) copy_priors(ptr, ptr.req_edge_off[s], ptr.req_nedges[s], s, x.lane);
             value = ptr.res_value[s];
         } else {
             value = vl.value[leaf];
@@ -1076,16 +1076,12 @@ __global__ void __launch_bounds__(WARPS * 32) k_vl_gather(const __grid_constant_
     const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (g == 0 && (threadIdx.x & 31) == 0) *ptr.batch_count = 0;   // requests of this wave are counted by k_vl_expand, which runs next
     if (g >= prm.n_games) return;
-    Ctx x{prm, ptr, &shared[threadIdx.x >> 5], g, (int)(threadIdx.x & 31), (size_t)g * prm.node_cap, (size_t)g * prm.edge_cap,
-          ptr.ctl[g], 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    Ctx x = make_ctx(prm, ptr, &shared[threadIdx.x >> 5], g, ptr.ctl[g]);
     if (x.c.status != 0) return;
     // ---- 1. the evaluations of the previous wave have arrived
     if (x.c.pending_node == 0) {   // MCTree::init: root priors, optional noise
         const int L = ptr.node_nedges[x.nbase];
-        if (!prm.priors_scattered) {
-            const float* pol = ptr.res_policy + (size_t)x.c.pending_slot * AZ_ACTION_SPACE;
-            for (int e = x.lane; e < L; e += 32) ptr.edge_P[x.ebase + e] = pol[ptr.edge_mv[x.ebase + e] >> 16];
-        }
+        if (!prm.priors_scattered) copy_priors(ptr, x.ebase, L, x.c.pending_slot, x.lane);
         for (int e = x.lane; e < L; e += 32) vl.V[x.ebase + e] = 0;
         __syncwarp();
         if (x.c.flags & 1) apply_noise(x, 0, x.c.game_id, x.c.noise_ply);
@@ -1102,9 +1098,7 @@ __global__ void __launch_bounds__(WARPS * 32) k_vl_gather(const __grid_constant_
         n_leaf = vl_gather_batch(x, prm, vl, collided, depth_sum);
     }
     if (x.lane == 0) {
-        vl.count[g] = n_leaf;
-        if (n_leaf) atomicAdd(&vl.stats[0], (unsigned long long)n_leaf);
-        if (collided) atomicAdd(&vl.stats[2], 1ULL);
+        vl_publish(vl, g, n_leaf, collided);
         ptr.ctl[g] = x.c;
     }
 }
@@ -1119,8 +1113,7 @@ __device__ __forceinline__ void vl_expand_body(const SearchParams& prm, const Se
     GameCtl c;
     memset(&c, 0, sizeof c);
     c.hist_len = ptr.ctl[g].hist_len;
-    Ctx x{prm, ptr, &shared[threadIdx.x >> 5], g, (int)(threadIdx.x & 31), (size_t)g * prm.node_cap, (size_t)g * prm.edge_cap, c,
-          0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    Ctx x = make_ctx(prm, ptr, &shared[threadIdx.x >> 5], g, c);
     const uint2* path = vl.path + (size_t)leaf * prm.node_cap;
     const int len = vl.len[leaf];
     const uint2 last = path[len - 1];
@@ -1185,22 +1178,16 @@ __global__ void __launch_bounds__(WARPS * 32) k_vl_selfplay(const __grid_constan
     const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (g == 0 && (threadIdx.x & 31) == 0) *ptr.batch_count = 0;   // requests of this wave are counted by k_vl_expand, which runs next
     if (g >= prm.n_games) return;
-    Ctx x{prm, ptr, &shared[threadIdx.x >> 5], g, (int)(threadIdx.x & 31), (size_t)g * prm.node_cap, (size_t)g * prm.edge_cap,
-          ptr.ctl[g], 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    Ctx x = make_ctx(prm, ptr, &shared[threadIdx.x >> 5], g, ptr.ctl[g]);
     if (x.c.status != 0 && x.c.status != 4) return;   // idle slot or error: vl.count[g] is already 0
-    if (x.c.status == 4) {   // game over, samples staged: publish now if the host has drained the queue, else stay parked
-        const ColdOut o = finish_game_cold(&prm, &ptr, x.sh, g, x.c);
-        x.c = o.c; x.st_pos += o.st_pos; x.st_games += o.st_games; x.st_sdepth += o.st_sdepth;
-    }
+    if (x.c.status == 4)   // game over, samples staged: publish now if the host has drained the queue, else stay parked
+        absorb(x, finish_game_cold(&prm, &ptr, x.sh, g, x.c));
     int n_leaf = 0, collided = 0;
     if (x.c.status == 0) {
         const int nl = vl_backup_batch(x, prm, ptr, vl);   // 0 for a game that has just started
         x.c.sims_done += nl;
         if (x.lane == 0) x.st_sims += nl;
-        if ((int)x.c.sims_done >= prm.S) {
-            const ColdOut o = move_step_cold(&prm, &ptr, x.sh, g, x.c);
-            x.c = o.c; x.st_pos += o.st_pos; x.st_games += o.st_games; x.st_sdepth += o.st_sdepth;
-        }
+        if ((int)x.c.sims_done >= prm.S) absorb(x, move_step_cold(&prm, &ptr, x.sh, g, x.c));
         if (x.c.status == 0) {
             if (x.c.sims_done == 0) {   // a fresh root (game start or traverse_new): no descent is in flight through its edges
                 const int L = (int)((x.c.flags >> 8) & 0xFF);
@@ -1211,9 +1198,7 @@ __global__ void __launch_bounds__(WARPS * 32) k_vl_selfplay(const __grid_constan
         }
     }
     if (x.lane == 0) {
-        vl.count[g] = n_leaf;   // 0 when the slot parked, went idle or failed: the next wave backs up nothing
-        if (n_leaf) atomicAdd(&vl.stats[0], (unsigned long long)n_leaf);
-        if (collided) atomicAdd(&vl.stats[2], 1ULL);
+        vl_publish(vl, g, n_leaf, collided);   // 0 when the slot parked, went idle or failed: the next wave backs up nothing
         ptr.ctl[g] = x.c;
         // the statistics of az_selfplay_step, striped as in k_advance; evaluations and terminal leaves come from vl.stats
         unsigned long long* ct = ptr.stats + (size_t)(blockIdx.x & (STAT_STRIPES - 1)) * STAT_WIDTH;
@@ -1351,6 +1336,7 @@ __global__ void __launch_bounds__(WARPS * 32) k_match(const __grid_constant__ Se
     GameCtl c;
     if (mp.first_wave) memset(&c, 0, sizeof c);
     else c = ptr.ctl[g];
+    // not make_ctx: built from this conditionally initialised c, it orders the prologue's zero-initialisations differently
     Ctx x{prm, ptr, &shared[threadIdx.x >> 5], g, (int)(threadIdx.x & 31), (size_t)g * prm.node_cap, (size_t)g * prm.edge_cap, c,
           0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
     if (!mp.first_wave && x.c.status != 0) return;   // idle slot or pool overflow: vl.count[g] is already 0
@@ -1361,10 +1347,7 @@ __global__ void __launch_bounds__(WARPS * 32) k_match(const __grid_constant__ Se
         match_start_game(x, mp, rt, evals);
     } else if (x.c.pending_node == 0) {   // MCTree::init: the root's priors (no noise), no descent in flight
         const int L = (int)((x.c.flags >> 8) & 0xFF);
-        if (!prm.priors_scattered) {
-            const float* pol = ptr.res_policy + (size_t)x.c.pending_slot * AZ_ACTION_SPACE;
-            for (int e = x.lane; e < L; e += 32) ptr.edge_P[x.ebase + e] = pol[ptr.edge_mv[x.ebase + e] >> 16];
-        }
+        if (!prm.priors_scattered) copy_priors(ptr, x.ebase, L, x.c.pending_slot, x.lane);
         for (int e = x.lane; e < L; e += 32) vl.V[x.ebase + e] = 0;
         __syncwarp();
         x.c.pending_node = -1;
@@ -1409,9 +1392,7 @@ __global__ void __launch_bounds__(WARPS * 32) k_match(const __grid_constant__ Se
         n_leaf = vl_gather_batch(x, prm, vl, collided, depth_sum);
     }
     if (x.lane == 0) {
-        vl.count[g] = n_leaf;   // 0 when the slot moved, went idle or waits for its root: the next wave backs up nothing
-        if (n_leaf) atomicAdd(&vl.stats[0], (unsigned long long)n_leaf);
-        if (collided) atomicAdd(&vl.stats[2], 1ULL);
+        vl_publish(vl, g, n_leaf, collided);   // 0 when the slot moved, went idle or waits for its root: the next wave backs up nothing
         if (evals[0]) atomicAdd(&mp.stats[0], (unsigned long long)evals[0]);
         if (evals[1]) atomicAdd(&mp.stats[1], (unsigned long long)evals[1]);
         if (plies) atomicAdd(&mp.stats[2], (unsigned long long)plies);
@@ -1504,10 +1485,16 @@ void search_destroy(az_engine* e) {
     SearchState* st = e->search;
     if (!st) return;
     for (void* p : st->allocs) cudaFree(p);
-    for (void* p : {(void*)st->match_result, (void*)st->match_plies, (void*)st->match_finished, (void*)st->match_moves}) cudaFree(p);
+    const MatchState& m = st->match;
+    for (void* p : {(void*)m.result.p, (void*)m.plies.p, (void*)m.finished.p, (void*)m.moves.p}) cudaFree(p);
     delete st;
     e->search = nullptr;
 }
+
+// the bf16 network's heads write the legal-move priors straight into edge_P (HeadScatter)
+static bool fused_heads(const az_engine* e) { return e->stub_kind == 0 && e->cfg.precision != 1; }
+
+static bool selfplay_on(const SearchState* st) { return st->session == Session::selfplay || st->session == Session::selfplay_vl; }
 
 // evaluates the queued requests: the network (bf16 or fp32) or the synthetic evaluator.  nb: a multi-network batch (requests
 // routed by NetRoute); under the synthetic evaluator network s evaluates with seed stub_seed + s
@@ -1542,12 +1529,12 @@ static int evaluate_batch(az_engine* e, SearchState* st, const NetBatch* nb = nu
 
 int search_pending_samples(az_engine* e, const az_sample** d_samples, int* n) {
     SearchState* st = e->search;
-    if (!st->selfplay_active) return set_err(e, AZ_ERR_STATE, "az_selfplay_begin has not been called");
-    Counters c;
-    AZ_CUDA(e, cudaMemcpyAsync(&c, st->ptr.counters, sizeof c, cudaMemcpyDeviceToHost, e->stream));
+    if (!selfplay_on(st)) return set_err(e, AZ_ERR_STATE, "az_selfplay_begin has not been called");
+    unsigned long long out;
+    AZ_CUDA(e, cudaMemcpyAsync(&out, &st->ptr.counters->samples_out, sizeof out, cudaMemcpyDeviceToHost, e->stream));
     AZ_CUDA(e, cudaStreamSynchronize(e->stream));
     *d_samples = st->ptr.out_samples;
-    *n = (int)std::min<unsigned long long>(c.samples_out, st->prm.sample_cap);
+    *n = (int)std::min<unsigned long long>(out, st->prm.sample_cap);
     return 0;
 }
 int search_clear_pending(az_engine* e) {
@@ -1558,7 +1545,7 @@ int search_clear_pending(az_engine* e) {
 
 // az_profile: when the coming forward will be sampled, the search kernels launched from here on are timed up to its start
 static void prof_mark_search(az_engine* e) {
-    if (e->prof_every > 0 && e->stub_kind == 0 && e->cfg.precision != 1 && (e->prof_counter % (uint64_t)e->prof_every) == 0 &&
+    if (e->prof_every > 0 && fused_heads(e) && (e->prof_counter % (uint64_t)e->prof_every) == 0 &&
         !e->prof_adv_event) {
         cudaEventCreate(&e->prof_adv_event);
         cudaEventRecord(e->prof_adv_event, e->stream);
@@ -1567,7 +1554,7 @@ static void prof_mark_search(az_engine* e) {
 
 static int run_wave(az_engine* e, SearchState* st) {
     const int blocks = (st->prm.n_games + WARPS - 1) / WARPS;
-    st->prm.priors_scattered = (e->stub_kind == 0 && e->cfg.precision != 1) ? 1 : 0;
+    st->prm.priors_scattered = fused_heads(e) ? 1 : 0;
     if (st->prm.mode == 1) st->prm.cache_epoch = (uint32_t)((st->wave_counter++ / (unsigned long long)std::max(st->prm.S, 1)) & 63);
     // Two request counters alternate between waves: this wave's k_advance counts into one and clears the other, which the
     // previous wave's network kernels (complete by stream order) were the last to read -- no memset launch per wave.
@@ -1614,8 +1601,7 @@ static int search_begin(az_engine* e, int n, const az_position* roots, const az_
         return set_err(e, AZ_ERR_CAPACITY, "num_simulations exceeds az_config.num_simulations (pool size)");
     if (e->stub_kind == 0 && !route && !e->net->loaded) return set_err(e, AZ_ERR_NO_WEIGHTS, "az_load_weights has not been called");
     cudaSetDevice(e->cfg.device);
-    st->selfplay_active = false;
-    st->match_active = false;
+    st->session = Session::none;
     SearchParams prm = st->prm;
     prm.n_games = n; prm.S = num_simulations; prm.mode = 0;
     run = *st;
@@ -1682,57 +1668,23 @@ static int search_export(az_engine* e, const SearchState& run, int n, float* vis
     return AZ_OK;
 }
 
-// k_count_active over the call's roots: flags[0] active, flags[1] failed (pool overflow or illegal state)
-static int search_poll(az_engine* e, const SearchState& run, int n, int flags[4]) {
+// enqueues k_count_active over the first n slots and the copy of its flags to the host, where they are valid after the
+// caller's next stream synchronise: flags[0] active, flags[1] failed (pool overflow or illegal state), flags[2] parked
+static int enqueue_poll(az_engine* e, const SearchState& run, int n, int flags[4]) {
     int* d_flags = run.batch_base + 4;
     AZ_CUDA(e, cudaMemsetAsync(d_flags, 0, 16, e->stream));
     k_count_active<<<(n + 127) / 128, 128, 0, e->stream>>>(run.prm, run.ptr, d_flags);
+    AZ_CUDA(e, cudaGetLastError());
     AZ_CUDA(e, cudaMemcpyAsync(flags, d_flags, 16, cudaMemcpyDeviceToHost, e->stream));
+    return AZ_OK;
+}
+
+static int search_poll(az_engine* e, const SearchState& run, int n, int flags[4]) {
+    const int r = enqueue_poll(e, run, n, flags);
+    if (r) return r;
     AZ_CUDA(e, cudaStreamSynchronize(e->stream));
     return AZ_OK;
 }
-
-}  // namespace azb
-
-using namespace azb;
-
-extern "C" {
-
-int az_set_evaluator_stub(az_engine* e, int kind, uint64_t seed) {
-    if (!e || kind < 0 || kind > 1) return AZ_ERR_INVALID_ARGUMENT;
-    e->stub_kind = kind;
-    e->stub_seed = seed;
-    return AZ_OK;
-}
-
-int az_search(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
-              int num_simulations, const uint64_t* noise_game_ids, const uint32_t* noise_plies, float* visits_out, float* scores_out,
-              int32_t* depth_out) {
-    if (!e) return AZ_ERR_INVALID_ARGUMENT;
-    SearchState run;
-    int r = search_begin(e, n, roots, history, hist_offsets, num_simulations, noise_game_ids, noise_plies, visits_out, run);
-    if (r) return r == 1 ? AZ_OK : r;
-    // every wave completes at least one simulation per active game
-    int rc = AZ_OK;
-    for (int wave = 0;; wave++) {
-        r = run_wave(e, &run);
-        if (r) { rc = r; break; }
-        if (wave + 1 >= num_simulations && (wave + 1 - num_simulations) % 4 == 0) {
-            int flags[4] = {0, 0, 0, 0};
-            r = search_poll(e, run, n, flags);
-            if (r) return r;
-            if (flags[1]) { rc = set_err(e, AZ_ERR_CAPACITY, "a per-game node/edge pool overflowed (raise edge_capacity_per_node)"); break; }
-            if (flags[0] == 0) break;
-            if (wave > 4 * num_simulations + 16) { rc = set_err(e, AZ_ERR_STATE, "search did not converge"); break; }
-        }
-    }
-    if (rc == AZ_OK) rc = search_export(e, run, n, visits_out, scores_out, depth_out);
-    return rc;
-}
-
-}  // extern "C"
-
-namespace azb {
 
 // the in-flight counts and the per-leaf records of az_search_vl and az_selfplay_begin_vl, allocated by the first such call
 static int vl_alloc(az_engine* e, SearchState* st) {
@@ -1750,6 +1702,45 @@ static VLPtrs vl_ptrs(const SearchState* st, int K, float lambda) {
     return VLPtrs{st->vl_V, st->vl_path, st->vl_len, st->vl_slot, st->vl_value, st->vl_count, st->vl_stats, K, lambda};
 }
 
+// the leaves per root (`what`: leaves_per_root or leaves_per_game) and the virtual loss of a leaf-parallel call
+static int check_vl_args(az_engine* e, int K, float virtual_loss, const char* what) {
+    if (K < 1) return set_err(e, AZ_ERR_INVALID_ARGUMENT, (std::string(what) + " must be >= 1").c_str());
+    if (!(virtual_loss >= 0.0f) || !std::isfinite(virtual_loss))
+        return set_err(e, AZ_ERR_INVALID_ARGUMENT, "virtual_loss must be finite and >= 0");
+    return AZ_OK;
+}
+
+// the board ranges of a multi-network batch with n0 / n1 roots (or slots) of K leaves each: network 0 from board 0, network 1
+// from base1 = round4(n0 x K), so no tile of the network kernels mixes networks; `end` is the end of network 1's range rounded to 4
+struct NetLayout { long long base1, end; };
+static NetLayout net_layout(long long n0, long long n1, int K) {
+    const long long base1 = (n0 * K + 3) & ~3LL;
+    return NetLayout{base1, base1 + ((n1 * K + 3) & ~3LL)};
+}
+
+// no batch in flight for the first n roots or slots, no leaf-parallel statistics yet
+static int vl_clear(az_engine* e, const SearchState* st, int n) {
+    if (n) AZ_CUDA(e, cudaMemsetAsync(st->vl_count, 0, (size_t)n * sizeof(int), e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(st->vl_stats, 0, 4 * sizeof(unsigned long long), e->stream));
+    return AZ_OK;
+}
+
+// vl_stats (leaves gathered, terminal leaves, collisions) as az_search_stats: every gathered leaf that was not terminal was evaluated
+static az_search_stats vl_search_stats(const unsigned long long s[4], uint64_t waves) {
+    return az_search_stats{waves, s[0] - s[1], s[1], s[2]};
+}
+
+// the tail of a leaf-parallel wave after its gather kernel: k_vl_expand (k_vl_expand_nets into the networks' ranges when rt is
+// given) over n roots or slots, then the evaluation of the batch (a multi-network one when nb is given)
+static int vl_expand_evaluate(az_engine* e, SearchState* run, const VLPtrs& vl, int n, const NetRoute* rt = nullptr,
+                              const NetBatch* nb = nullptr) {
+    const int blocks = (n * vl.K + WARPS - 1) / WARPS;
+    if (rt) k_vl_expand_nets<<<blocks, WARPS * 32, 0, e->stream>>>(run->prm, run->ptr, vl, *rt);
+    else k_vl_expand<<<blocks, WARPS * 32, 0, e->stream>>>(run->prm, run->ptr, vl);
+    AZ_CUDA(e, cudaGetLastError());
+    return evaluate_batch(e, run, nb);
+}
+
 // az_search_vl, and az_search_networks when `network` (one id per root) is given: the requests of each root then go to the
 // range of its network (k_init_search_nets, k_vl_expand_nets) and every wave evaluates both ranges in one multi-network forward
 static int search_vl_run(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
@@ -1758,13 +1749,12 @@ static int search_vl_run(az_engine* e, int n, const az_position* roots, const az
                          int32_t* depth_out, az_search_stats* stats_out) {
     if (!e) return AZ_ERR_INVALID_ARGUMENT;
     if (stats_out) std::memset(stats_out, 0, sizeof *stats_out);
-    if (leaves_per_root < 1) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "leaves_per_root must be >= 1");
-    if (!(virtual_loss >= 0.0f) || !std::isfinite(virtual_loss))
-        return set_err(e, AZ_ERR_INVALID_ARGUMENT, "virtual_loss must be finite and >= 0");
-    if (n > 0 && (long long)n * leaves_per_root > (long long)e->max_batch)
+    const int K = leaves_per_root;
+    int r = check_vl_args(e, K, virtual_loss, "leaves_per_root");
+    if (r) return r;
+    if (n > 0 && (long long)n * K > (long long)e->max_batch)
         return set_err(e, AZ_ERR_CAPACITY, "roots x leaves_per_root exceeds az_config.max_batch");
     SearchState* st = e->search;
-    // network ranges: network 0 from slot 0, network 1 from the next multiple of 4 after network 0's n_0 * K slots
     int count[AZ_MAX_NETWORKS] = {0, 0};
     int base1 = 0;
     if (network && n > 0 && n <= st->G) {
@@ -1777,16 +1767,16 @@ static int search_vl_run(az_engine* e, int n, const az_position* roots, const az
             if (count[s] && e->stub_kind == 0 && (!w || !w->loaded))
                 return set_err(e, AZ_ERR_NO_WEIGHTS, "a root names a network that has not been loaded");
         }
-        const long long r0 = ((long long)count[0] * leaves_per_root + 3) & ~3LL, r1 = ((long long)count[1] * leaves_per_root + 3) & ~3LL;
-        if (r0 + r1 > e->max_batch) return set_err(e, AZ_ERR_CAPACITY, "network ranges (roots x leaves_per_root each) exceed az_config.max_batch");
-        base1 = (int)r0;
+        const NetLayout lay = net_layout(count[0], count[1], K);
+        if (lay.end > e->max_batch) return set_err(e, AZ_ERR_CAPACITY, "network ranges (roots x leaves_per_root each) exceed az_config.max_batch");
+        base1 = (int)lay.base1;
     }
     if (n >= 0 && n <= st->G) {
         const int a = vl_alloc(e, st);
         if (a) return a;
     }
     NetRoute route{nullptr, st->batch_base, base1};
-    NetBatch nb{st->batch_base, base1, base1 + count[1] * leaves_per_root};
+    NetBatch nb{st->batch_base, base1, base1 + count[1] * K};
     if (network && n > 0 && n <= st->G) {
         if (!st->d_net) {
             cudaSetDevice(e->cfg.device);
@@ -1798,13 +1788,12 @@ static int search_vl_run(az_engine* e, int n, const az_position* roots, const az
     const NetRoute* rt = route.net ? &route : nullptr;
     const NetBatch* nbp = route.net ? &nb : nullptr;
     SearchState run;
-    int r = search_begin(e, n, roots, history, hist_offsets, num_simulations, noise_game_ids, noise_plies, visits_out, run, rt, nbp);
+    r = search_begin(e, n, roots, history, hist_offsets, num_simulations, noise_game_ids, noise_plies, visits_out, run, rt, nbp);
     if (r) return r == 1 ? AZ_OK : r;
-    const int K = leaves_per_root;
     const VLPtrs vl = vl_ptrs(st, K, virtual_loss);
-    AZ_CUDA(e, cudaMemsetAsync(vl.count, 0, (size_t)n * sizeof(int), e->stream));
-    AZ_CUDA(e, cudaMemsetAsync(vl.stats, 0, 4 * sizeof(unsigned long long), e->stream));
-    run.prm.priors_scattered = (e->stub_kind == 0 && e->cfg.precision != 1) ? 1 : 0;
+    r = vl_clear(e, st, n);
+    if (r) return r;
+    run.prm.priors_scattered = fused_heads(e) ? 1 : 0;
     uint64_t waves = 1;   // the roots' evaluation
     // a batch adds at least one leaf per active root, so every root is done after at most S batches; the first poll comes
     // after the earliest wave at which the last batch can have been consumed
@@ -1823,14 +1812,9 @@ static int search_vl_run(az_engine* e, int n, const az_position* roots, const az
             if (flags[0] == 0) break;
             if (wave > num_simulations + 16) { rc = set_err(e, AZ_ERR_STATE, "search did not converge"); break; }
         }
-        if (rt) {   // both request counters start the wave at 0 (k_vl_gather clears only the first)
+        if (rt)   // both request counters start the wave at 0 (k_vl_gather clears only the first)
             AZ_CUDA(e, cudaMemsetAsync(run.batch_base, 0, AZ_MAX_NETWORKS * sizeof(int), e->stream));
-            k_vl_expand_nets<<<(n * K + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(run.prm, run.ptr, vl, *rt);
-        } else {
-            k_vl_expand<<<(n * K + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(run.prm, run.ptr, vl);
-        }
-        AZ_CUDA(e, cudaGetLastError());
-        r = evaluate_batch(e, &run, nbp);
+        r = vl_expand_evaluate(e, &run, vl, n, rt, nbp);
         if (r) return r;
         waves++;
     }
@@ -1841,43 +1825,13 @@ static int search_vl_run(az_engine* e, int n, const az_position* roots, const az
     if (rc == AZ_OK) rc = search_export(e, run, n, visits_out, scores_out, depth_out);
     if (rc == AZ_OK && stats_out) {
         unsigned long long s[4];
-        AZ_CUDA(e, cudaMemcpy(s, vl.stats, sizeof s, cudaMemcpyDeviceToHost));
-        stats_out->waves = waves;
-        stats_out->evaluations = (uint64_t)n + s[0] - s[1];   // the roots, then every leaf that was not terminal
-        stats_out->terminal_leaves = s[1];
-        stats_out->collisions = s[2];
+        AZ_CUDA(e, cudaMemcpyAsync(s, vl.stats, sizeof s, cudaMemcpyDeviceToHost, e->stream));
+        AZ_CUDA(e, cudaStreamSynchronize(e->stream));
+        *stats_out = vl_search_stats(s, waves);
+        stats_out->evaluations += (uint64_t)n;   // and the roots
     }
     return rc;
 }
-
-}  // namespace azb
-
-extern "C" {
-
-int az_search_vl(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
-                 int num_simulations, int leaves_per_root, float virtual_loss, const uint64_t* noise_game_ids, const uint32_t* noise_plies,
-                 float* visits_out, float* scores_out, int32_t* depth_out, az_search_stats* stats_out) {
-    return search_vl_run(e, n, roots, history, hist_offsets, num_simulations, leaves_per_root, virtual_loss, nullptr, noise_game_ids,
-                         noise_plies, visits_out, scores_out, depth_out, stats_out);
-}
-
-int az_search_networks(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
-                       int num_simulations, int leaves_per_root, float virtual_loss, const uint8_t* network, const uint64_t* noise_game_ids,
-                       const uint32_t* noise_plies, float* visits_out, float* scores_out, int32_t* depth_out, az_search_stats* stats_out) {
-    if (!e) return AZ_ERR_INVALID_ARGUMENT;
-    if (n > 0 && !network) {
-        if (stats_out) std::memset(stats_out, 0, sizeof *stats_out);
-        return set_err(e, AZ_ERR_INVALID_ARGUMENT, "null network buffer");
-    }
-    return search_vl_run(e, n, roots, history, hist_offsets, num_simulations, leaves_per_root, virtual_loss, network, noise_game_ids,
-                         noise_plies, visits_out, scores_out, depth_out, stats_out);
-}
-
-int az_selfplay_begin(az_engine* e, int n_games, uint64_t first_game_id) { return az_selfplay_begin_n(e, n_games, first_game_id, 0); }
-
-}  // extern "C"
-
-namespace azb {
 
 // az_selfplay_begin_n (K = 0: k_advance waves) and az_selfplay_begin_vl (K >= 1: k_vl_selfplay waves with K leaves per game)
 static int selfplay_begin(az_engine* e, int n_games, uint64_t first_game_id, uint64_t total_games, int K, float virtual_loss) {
@@ -1937,37 +1891,166 @@ static int selfplay_begin(az_engine* e, int n_games, uint64_t first_game_id, uin
     e->n_launches += 2;
     k_init_selfplay<<<blocks, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr, first_game_id);
     AZ_CUDA(e, cudaGetLastError());
-    if (K > 0) {   // no batch in flight, no statistics yet
-        AZ_CUDA(e, cudaMemsetAsync(st->vl_count, 0, (size_t)n_games * sizeof(int), e->stream));
-        AZ_CUDA(e, cudaMemsetAsync(st->vl_stats, 0, 4 * sizeof(unsigned long long), e->stream));
-    }
+    if (K > 0 && (r = vl_clear(e, st, n_games))) return r;
     AZ_CUDA(e, cudaStreamSynchronize(e->stream));
-    st->sp_vl_K = K;
-    st->sp_vl_lambda = virtual_loss;
-    st->sp_vl_waves = 0;
-    st->selfplay_active = true;
-    st->match_active = false;
+    st->sp_vl = SelfplayVL{K, virtual_loss, 0};
+    st->session = K > 0 ? Session::selfplay_vl : Session::selfplay;
     return AZ_OK;
 }
 
 // one wave of az_selfplay_begin_vl's self-play: k_vl_selfplay, k_vl_expand, the network
 static int run_wave_vl(az_engine* e, SearchState* st) {
-    const int n = st->prm.n_games, K = st->sp_vl_K;
-    st->prm.priors_scattered = (e->stub_kind == 0 && e->cfg.precision != 1) ? 1 : 0;
-    const VLPtrs vl = vl_ptrs(st, K, st->sp_vl_lambda);
+    const int n = st->prm.n_games;
+    st->prm.priors_scattered = fused_heads(e) ? 1 : 0;
+    const VLPtrs vl = vl_ptrs(st, st->sp_vl.K, st->sp_vl.lambda);
     prof_mark_search(e);
     e->n_launches += 2;
     k_vl_selfplay<<<(n + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr, vl);
     AZ_CUDA(e, cudaGetLastError());
-    k_vl_expand<<<(n * K + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr, vl);
-    AZ_CUDA(e, cudaGetLastError());
-    st->sp_vl_waves++;
-    return evaluate_batch(e, st);
+    st->sp_vl.waves++;
+    return vl_expand_evaluate(e, st, vl, n);
+}
+
+#ifdef AZ_ADV_TIMING
+// AZ_ADV_TIMING: k_advance's phase clocks and warp-time histogram (stripe fields 8..15 and 24..39) of the waves since the last
+// report, per game and wave
+static void adv_timing_report(const unsigned long long* stripes, int n_games, int waves) {
+    unsigned long long tc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    for (int i = 0; i < STAT_STRIPES * STAT_WIDTH; i++) if (i % STAT_WIDTH >= 8 && i % STAT_WIDTH < 16) tc[i % STAT_WIDTH - 8] += stripes[i];
+    unsigned long long hist[16] = {0};
+    for (int i = 0; i < STAT_STRIPES * STAT_WIDTH; i++) if (i % STAT_WIDTH >= 24) hist[i % STAT_WIDTH - 24] += stripes[i];
+    {   // the device counters are cumulative since az_selfplay_begin: report this call's share
+        static unsigned long long prev_tc[8], prev_hist[16];
+        for (int k = 0; k < 8; k++) { const unsigned long long c = tc[k]; tc[k] = c >= prev_tc[k] ? c - prev_tc[k] : c; prev_tc[k] = c; }
+        for (int k = 0; k < 16; k++) { const unsigned long long c = hist[k]; hist[k] = c >= prev_hist[k] ? c - prev_hist[k] : c; prev_hist[k] = c; }
+    }
+    if (waves <= 0) return;
+    fprintf(stderr, "azb: k_advance warp-time histogram (buckets of 4096 clocks):");
+    for (int k = 0; k < 16; k++) fprintf(stderr, " %llu", hist[k]);
+    fprintf(stderr, "\n");
+    const double per = (double)n_games * waves;
+    fprintf(stderr, "azb: k_advance phase clocks per warp-wave: consume %.0f select %.0f child %.0f rules %.0f create %.0f submit %.0f move %.0f total %.0f\n",
+            (double)tc[0] / per, (double)tc[1] / per, (double)tc[2] / per, (double)tc[3] / per, (double)tc[4] / per, (double)tc[5] / per,
+            (double)tc[6] / per, (double)tc[7] / per);
+}
+#endif
+
+// az_selfplay_drain (kind: device to host) and az_selfplay_drain_dev (device to device), ordered on the engine's stream after
+// the self-play waves and any az_replay_add_pending before it
+static int selfplay_drain(az_engine* e, az_sample* out, int max_samples, int* n_out, cudaMemcpyKind kind) {
+    if (!e || !n_out) return AZ_ERR_INVALID_ARGUMENT;
+    cudaSetDevice(e->cfg.device);
+    const az_sample* d_samples = nullptr;
+    int n = 0;
+    int r = search_pending_samples(e, &d_samples, &n);
+    if (r) return r;
+    if ((unsigned long long)n > (unsigned long long)max_samples) return set_err(e, AZ_ERR_CAPACITY, "drain buffer smaller than the pending sample count");
+    if (n && out) AZ_CUDA(e, cudaMemcpyAsync(out, d_samples, (size_t)n * sizeof(az_sample), kind, e->stream));
+    if ((r = search_clear_pending(e))) return r;
+    AZ_CUDA(e, cudaStreamSynchronize(e->stream));
+    *n_out = n;
+    return AZ_OK;
+}
+
+template <class T>
+static int grow(az_engine* e, GrowBuf<T>& b, size_t n) {
+    if (n <= b.cap) return AZ_OK;
+    cudaFree(b.p);
+    b.p = nullptr;
+    b.cap = 0;
+    AZ_CUDA(e, cudaMalloc(&b.p, n * sizeof(T)));
+    b.cap = n;
+    return AZ_OK;
+}
+
+// the match's per-game results, reallocated when a match needs more room than the last one (freed by search_destroy)
+static int match_alloc(az_engine* e, SearchState* st, size_t games, size_t row) {
+    MatchState& m = st->match;
+    if (!m.next && (salloc(e, st, &m.next, 1) || salloc(e, st, &m.stats, 4))) return AZ_ERR_OUT_OF_MEMORY;
+    int r = grow(e, m.result, games);
+    if (!r) r = grow(e, m.plies, games);
+    if (!r) r = grow(e, m.finished, games);
+    if (!r) r = grow(e, m.moves, games * row);
+    return r;
+}
+
+static MatchParams match_params(const SearchState* st) {
+    const MatchState& m = st->match;
+    const az_match_config& c = m.cfg;
+    MatchParams mp;
+    mp.startpos = m.startpos;
+    mp.seed = c.seed;
+    mp.first_game = m.first;
+    mp.end_game = m.first + m.games;
+    mp.next_game = m.next;
+    mp.stats = m.stats;
+    mp.net = st->d_net;
+    mp.result = m.result.p; mp.plies = m.plies.p; mp.finished = m.finished.p; mp.moves = m.moves.p;
+    mp.row = m.row; mp.max_plies = c.max_plies; mp.n_stochastic = c.num_stochastic_moves;
+    mp.base_model = c.player_kind == 1 ? 1 : 0;
+    mp.first_wave = m.first_wave;
+    mp.network[0] = c.network[0]; mp.network[1] = c.network[1];
+    return mp;
 }
 
 }  // namespace azb
 
+using namespace azb;
+
 extern "C" {
+
+int az_set_evaluator_stub(az_engine* e, int kind, uint64_t seed) {
+    if (!e || kind < 0 || kind > 1) return AZ_ERR_INVALID_ARGUMENT;
+    e->stub_kind = kind;
+    e->stub_seed = seed;
+    return AZ_OK;
+}
+
+int az_search(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
+              int num_simulations, const uint64_t* noise_game_ids, const uint32_t* noise_plies, float* visits_out, float* scores_out,
+              int32_t* depth_out) {
+    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+    SearchState run;
+    int r = search_begin(e, n, roots, history, hist_offsets, num_simulations, noise_game_ids, noise_plies, visits_out, run);
+    if (r) return r == 1 ? AZ_OK : r;
+    // every wave completes at least one simulation per active game
+    int rc = AZ_OK;
+    for (int wave = 0;; wave++) {
+        r = run_wave(e, &run);
+        if (r) { rc = r; break; }
+        if (wave + 1 >= num_simulations && (wave + 1 - num_simulations) % 4 == 0) {
+            int flags[4] = {0, 0, 0, 0};
+            r = search_poll(e, run, n, flags);
+            if (r) return r;
+            if (flags[1]) { rc = set_err(e, AZ_ERR_CAPACITY, "a per-game node/edge pool overflowed (raise edge_capacity_per_node)"); break; }
+            if (flags[0] == 0) break;
+            if (wave > 4 * num_simulations + 16) { rc = set_err(e, AZ_ERR_STATE, "search did not converge"); break; }
+        }
+    }
+    if (rc == AZ_OK) rc = search_export(e, run, n, visits_out, scores_out, depth_out);
+    return rc;
+}
+
+int az_search_vl(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
+                 int num_simulations, int leaves_per_root, float virtual_loss, const uint64_t* noise_game_ids, const uint32_t* noise_plies,
+                 float* visits_out, float* scores_out, int32_t* depth_out, az_search_stats* stats_out) {
+    return search_vl_run(e, n, roots, history, hist_offsets, num_simulations, leaves_per_root, virtual_loss, nullptr, noise_game_ids,
+                         noise_plies, visits_out, scores_out, depth_out, stats_out);
+}
+
+int az_search_networks(az_engine* e, int n, const az_position* roots, const az_position* history, const uint32_t* hist_offsets,
+                       int num_simulations, int leaves_per_root, float virtual_loss, const uint8_t* network, const uint64_t* noise_game_ids,
+                       const uint32_t* noise_plies, float* visits_out, float* scores_out, int32_t* depth_out, az_search_stats* stats_out) {
+    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+    if (n > 0 && !network) {
+        if (stats_out) std::memset(stats_out, 0, sizeof *stats_out);
+        return set_err(e, AZ_ERR_INVALID_ARGUMENT, "null network buffer");
+    }
+    return search_vl_run(e, n, roots, history, hist_offsets, num_simulations, leaves_per_root, virtual_loss, network, noise_game_ids,
+                         noise_plies, visits_out, scores_out, depth_out, stats_out);
+}
+
+int az_selfplay_begin(az_engine* e, int n_games, uint64_t first_game_id) { return az_selfplay_begin_n(e, n_games, first_game_id, 0); }
 
 int az_selfplay_begin_n(az_engine* e, int n_games, uint64_t first_game_id, uint64_t total_games) {
     if (!e) return AZ_ERR_INVALID_ARGUMENT;
@@ -1977,9 +2060,8 @@ int az_selfplay_begin_n(az_engine* e, int n_games, uint64_t first_game_id, uint6
 int az_selfplay_begin_vl(az_engine* e, int n_concurrent, uint64_t first_game_id, uint64_t total_games, int leaves_per_game,
                          float virtual_loss) {
     if (!e) return AZ_ERR_INVALID_ARGUMENT;
-    if (leaves_per_game < 1) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "leaves_per_game must be >= 1");
-    if (!(virtual_loss >= 0.0f) || !std::isfinite(virtual_loss))
-        return set_err(e, AZ_ERR_INVALID_ARGUMENT, "virtual_loss must be finite and >= 0");
+    const int r = check_vl_args(e, leaves_per_game, virtual_loss, "leaves_per_game");
+    if (r) return r;
     return selfplay_begin(e, n_concurrent, first_game_id, total_games, leaves_per_game, virtual_loss);
 }
 
@@ -1987,38 +2069,34 @@ int az_selfplay_vl_stats(az_engine* e, az_search_stats* out) {
     if (!e || !out) return AZ_ERR_INVALID_ARGUMENT;
     std::memset(out, 0, sizeof *out);
     SearchState* st = e->search;
-    if (!st->selfplay_active || !st->sp_vl_K) return set_err(e, AZ_ERR_STATE, "az_selfplay_begin_vl has not been called");
+    if (st->session != Session::selfplay_vl) return set_err(e, AZ_ERR_STATE, "az_selfplay_begin_vl has not been called");
     cudaSetDevice(e->cfg.device);
     unsigned long long s[4];
     AZ_CUDA(e, cudaMemcpyAsync(s, st->vl_stats, sizeof s, cudaMemcpyDeviceToHost, e->stream));
     AZ_CUDA(e, cudaStreamSynchronize(e->stream));
-    out->waves = st->sp_vl_waves;
-    out->evaluations = s[0] - s[1];   // every gathered leaf that was not terminal
-    out->terminal_leaves = s[1];
-    out->collisions = s[2];
+    *out = vl_search_stats(s, st->sp_vl.waves);
     return AZ_OK;
 }
 
 int az_selfplay_step(az_engine* e, int waves, az_selfplay_stats* out) {
     if (!e) return AZ_ERR_INVALID_ARGUMENT;
     SearchState* st = e->search;
-    if (!st->selfplay_active) return set_err(e, AZ_ERR_STATE, "az_selfplay_begin has not been called");
+    if (!selfplay_on(st)) return set_err(e, AZ_ERR_STATE, "az_selfplay_begin has not been called");
     cudaSetDevice(e->cfg.device);
+    const bool vl = st->session == Session::selfplay_vl;
     for (int w = 0; w < waves; w++) {
-        int r = st->sp_vl_K ? run_wave_vl(e, st) : run_wave(e, st);
+        int r = vl ? run_wave_vl(e, st) : run_wave(e, st);
         if (r) return r;
     }
     Counters c;
     unsigned long long stripes[STAT_STRIPES * STAT_WIDTH];
     int flags[4] = {0, 0, 0, 0};
-    int* d_flags = st->batch_base + 4;
-    AZ_CUDA(e, cudaMemsetAsync(d_flags, 0, 16, e->stream));
-    k_count_active<<<(st->prm.n_games + 127) / 128, 128, 0, e->stream>>>(st->prm, st->ptr, d_flags);
-    AZ_CUDA(e, cudaMemcpyAsync(flags, d_flags, 16, cudaMemcpyDeviceToHost, e->stream));
+    const int r = enqueue_poll(e, *st, st->prm.n_games, flags);
+    if (r) return r;
     AZ_CUDA(e, cudaMemcpyAsync(&c, st->ptr.counters, sizeof c, cudaMemcpyDeviceToHost, e->stream));
     AZ_CUDA(e, cudaMemcpyAsync(stripes, st->ptr.stats, sizeof stripes, cudaMemcpyDeviceToHost, e->stream));
     unsigned long long vls[4] = {0, 0, 0, 0};
-    if (st->sp_vl_K) AZ_CUDA(e, cudaMemcpyAsync(vls, st->vl_stats, sizeof vls, cudaMemcpyDeviceToHost, e->stream));
+    if (vl) AZ_CUDA(e, cudaMemcpyAsync(vls, st->vl_stats, sizeof vls, cudaMemcpyDeviceToHost, e->stream));
     AZ_CUDA(e, cudaStreamSynchronize(e->stream));
     {
         unsigned long long sum[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -2032,28 +2110,14 @@ int az_selfplay_step(az_engine* e, int waves, az_selfplay_stats* out) {
         st->cache_evictions = evictions;
         st->sum_search_depth = sdepth;
 #ifdef AZ_ADV_TIMING
-        unsigned long long tc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-        for (int i = 0; i < STAT_STRIPES * STAT_WIDTH; i++) if (i % STAT_WIDTH >= 8 && i % STAT_WIDTH < 16) tc[i % STAT_WIDTH - 8] += stripes[i];
-        unsigned long long hist[16] = {0};
-        for (int i = 0; i < STAT_STRIPES * STAT_WIDTH; i++) if (i % STAT_WIDTH >= 24) hist[i % STAT_WIDTH - 24] += stripes[i];
-        {   // the device counters are cumulative since az_selfplay_begin: report this call's share
-            static unsigned long long prev_tc[8], prev_hist[16];
-            for (int k = 0; k < 8; k++) { const unsigned long long c = tc[k]; tc[k] = c >= prev_tc[k] ? c - prev_tc[k] : c; prev_tc[k] = c; }
-            for (int k = 0; k < 16; k++) { const unsigned long long c = hist[k]; hist[k] = c >= prev_hist[k] ? c - prev_hist[k] : c; prev_hist[k] = c; }
-        }
-        if (waves > 0) {
-        fprintf(stderr, "azb: k_advance warp-time histogram (buckets of 4096 clocks):");
-        for (int k = 0; k < 16; k++) fprintf(stderr, " %llu", hist[k]);
-        fprintf(stderr, "\n");
-        fprintf(stderr, "azb: k_advance phase clocks per warp-wave: consume %.0f select %.0f child %.0f rules %.0f create %.0f submit %.0f move %.0f total %.0f\n",
-                (double)tc[0] / ((double)st->prm.n_games * waves), (double)tc[1] / ((double)st->prm.n_games * waves), (double)tc[2] / ((double)st->prm.n_games * waves),
-                (double)tc[3] / ((double)st->prm.n_games * waves), (double)tc[4] / ((double)st->prm.n_games * waves), (double)tc[5] / ((double)st->prm.n_games * waves),
-                (double)tc[6] / ((double)st->prm.n_games * waves), (double)tc[7] / ((double)st->prm.n_games * waves));
-        }
+        adv_timing_report(stripes, st->prm.n_games, waves);
 #endif
         c.simulations = sum[0]; c.positions = sum[1]; c.evaluations = sum[2]; c.cache_hits = sum[3];
         c.terminal_leaves = sum[4]; c.games_finished = sum[5]; c.sum_leaf_depth = sum[6]; c.sum_edges = sum[7];
-        if (st->sp_vl_K) { c.evaluations = vls[0] - vls[1]; c.terminal_leaves = vls[1]; }   // k_vl_expand counts the terminal leaves
+        if (vl) {   // k_vl_expand counts the terminal leaves
+            const az_search_stats v = vl_search_stats(vls, 0);
+            c.evaluations = v.evaluations; c.terminal_leaves = v.terminal_leaves;
+        }
     }
     if (out) {
         out->simulations = c.simulations; out->positions = c.positions; out->evaluations = c.evaluations; out->cache_hits = c.cache_hits;
@@ -2067,103 +2131,32 @@ int az_selfplay_step(az_engine* e, int waves, az_selfplay_stats* out) {
 }
 
 int az_selfplay_drain(az_engine* e, az_sample* out, int max_samples, int* n_out) {
-    if (!e || !n_out) return AZ_ERR_INVALID_ARGUMENT;
-    SearchState* st = e->search;
-    if (!st->selfplay_active) return set_err(e, AZ_ERR_STATE, "az_selfplay_begin has not been called");
-    cudaSetDevice(e->cfg.device);
-    Counters c;
-    AZ_CUDA(e, cudaMemcpy(&c, st->ptr.counters, sizeof c, cudaMemcpyDeviceToHost));
-    unsigned long long avail = std::min<unsigned long long>(c.samples_out, st->prm.sample_cap);
-    if (avail > (unsigned long long)max_samples) return set_err(e, AZ_ERR_CAPACITY, "drain buffer smaller than the pending sample count");
-    if (avail && out) AZ_CUDA(e, cudaMemcpy(out, st->ptr.out_samples, (size_t)avail * sizeof(az_sample), cudaMemcpyDeviceToHost));
-    unsigned long long zero = 0;
-    AZ_CUDA(e, cudaMemcpy(&st->ptr.counters->samples_out, &zero, sizeof zero, cudaMemcpyHostToDevice));
-    *n_out = (int)avail;
-    return AZ_OK;
+    return selfplay_drain(e, out, max_samples, n_out, cudaMemcpyDeviceToHost);
 }
 
 int az_selfplay_drain_dev(az_engine* e, az_sample* out_dev, int max_samples, int* n_out) {
-    if (!e || !n_out) return AZ_ERR_INVALID_ARGUMENT;
-    SearchState* st = e->search;
-    if (!st->selfplay_active) return set_err(e, AZ_ERR_STATE, "az_selfplay_begin has not been called");
-    cudaSetDevice(e->cfg.device);
-    Counters c;
-    AZ_CUDA(e, cudaMemcpyAsync(&c, st->ptr.counters, sizeof c, cudaMemcpyDeviceToHost, e->stream));
-    AZ_CUDA(e, cudaStreamSynchronize(e->stream));
-    const unsigned long long avail = std::min<unsigned long long>(c.samples_out, st->prm.sample_cap);
-    if (avail > (unsigned long long)max_samples) return set_err(e, AZ_ERR_CAPACITY, "drain buffer smaller than the pending sample count");
-    if (avail && out_dev)
-        AZ_CUDA(e, cudaMemcpyAsync(out_dev, st->ptr.out_samples, (size_t)avail * sizeof(az_sample), cudaMemcpyDeviceToDevice, e->stream));
-    AZ_CUDA(e, cudaMemsetAsync(&st->ptr.counters->samples_out, 0, sizeof(unsigned long long), e->stream));
-    AZ_CUDA(e, cudaStreamSynchronize(e->stream));
-    *n_out = (int)avail;
-    return AZ_OK;
+    return selfplay_drain(e, out_dev, max_samples, n_out, cudaMemcpyDeviceToDevice);
 }
 
 /* test hook: the EpisodeSteps the game in slot `slot` has staged so far (they are published when the game ends) */
 int az_dbg_selfplay_staged(az_engine* e, int slot, az_sample* out, int max_samples, int* n_out) {
     if (!e || !out || !n_out) return AZ_ERR_INVALID_ARGUMENT;
     SearchState* st = e->search;
-    if (!st->selfplay_active || !st->ptr.game_samples) return set_err(e, AZ_ERR_STATE, "az_selfplay_begin has not been called");
+    if (!selfplay_on(st)) return set_err(e, AZ_ERR_STATE, "az_selfplay_begin has not been called");
     if (slot < 0 || slot >= st->prm.n_games) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "slot out of range");
     cudaSetDevice(e->cfg.device);
     GameCtl c;
-    AZ_CUDA(e, cudaMemcpy(&c, st->ptr.ctl + slot, sizeof c, cudaMemcpyDeviceToHost));
+    AZ_CUDA(e, cudaMemcpyAsync(&c, st->ptr.ctl + slot, sizeof c, cudaMemcpyDeviceToHost, e->stream));
+    AZ_CUDA(e, cudaStreamSynchronize(e->stream));
     const int n = std::min<int>((int)c.n_samples, max_samples);
-    if (n) AZ_CUDA(e, cudaMemcpy(out, st->ptr.game_samples + (size_t)slot * MAX_SAMPLE_PLIES, (size_t)n * sizeof(az_sample), cudaMemcpyDeviceToHost));
+    if (n) {
+        AZ_CUDA(e, cudaMemcpyAsync(out, st->ptr.game_samples + (size_t)slot * MAX_SAMPLE_PLIES, (size_t)n * sizeof(az_sample),
+                                   cudaMemcpyDeviceToHost, e->stream));
+        AZ_CUDA(e, cudaStreamSynchronize(e->stream));
+    }
     *n_out = n;
     return AZ_OK;
 }
-
-}  // extern "C"
-
-namespace azb {
-
-// the match's per-game results, (re)allocated when a match needs more room than the last one (freed by search_destroy)
-static int match_alloc(az_engine* e, SearchState* st, size_t games, size_t row) {
-    if (!st->match_next && (salloc(e, st, &st->match_next, 1) || salloc(e, st, &st->match_stats, 4))) return AZ_ERR_OUT_OF_MEMORY;
-    if (games > st->match_cap) {
-        for (void* p : {(void*)st->match_result, (void*)st->match_plies, (void*)st->match_finished}) cudaFree(p);
-        st->match_result = nullptr; st->match_plies = nullptr; st->match_finished = nullptr; st->match_cap = 0;
-        AZ_CUDA(e, cudaMalloc(&st->match_result, games));
-        AZ_CUDA(e, cudaMalloc(&st->match_plies, games * sizeof(uint16_t)));
-        AZ_CUDA(e, cudaMalloc(&st->match_finished, games));
-        st->match_cap = games;
-    }
-    if (games * row > st->match_moves_cap) {
-        cudaFree(st->match_moves);
-        st->match_moves = nullptr; st->match_moves_cap = 0;
-        AZ_CUDA(e, cudaMalloc(&st->match_moves, games * row * sizeof(uint16_t)));
-        st->match_moves_cap = games * row;
-    }
-    return AZ_OK;
-}
-
-// network 0's range starts at board 0, network 1's at round4(slots x K): a slot queues at most K boards per wave (its batch or
-// its next root), all in its mover's range
-static int match_base1(const SearchState* st) { return (st->prm.n_games * st->match_K + 3) & ~3; }
-
-static MatchParams match_params(const SearchState* st) {
-    const az_match_config& c = st->match_cfg;
-    MatchParams mp;
-    mp.startpos = st->match_startpos;
-    mp.seed = c.seed;
-    mp.first_game = st->match_first;
-    mp.end_game = st->match_first + st->match_games;
-    mp.next_game = st->match_next;
-    mp.stats = st->match_stats;
-    mp.net = st->d_net;
-    mp.result = st->match_result; mp.plies = st->match_plies; mp.finished = st->match_finished; mp.moves = st->match_moves;
-    mp.row = st->match_row; mp.max_plies = c.max_plies; mp.n_stochastic = c.num_stochastic_moves;
-    mp.base_model = c.player_kind == 1 ? 1 : 0;
-    mp.first_wave = st->match_first_wave;
-    mp.network[0] = c.network[0]; mp.network[1] = c.network[1];
-    return mp;
-}
-
-}  // namespace azb
-
-extern "C" {
 
 int az_match_begin(az_engine* e, int n_concurrent, uint32_t first_game, uint32_t n_games, const az_match_config* cfg) {
     if (!e) return AZ_ERR_INVALID_ARGUMENT;
@@ -2175,9 +2168,8 @@ int az_match_begin(az_engine* e, int n_concurrent, uint32_t first_game, uint32_t
         return set_err(e, AZ_ERR_INVALID_ARGUMENT, "network id must be < AZ_MAX_NETWORKS");
     const int S = cfg->num_simulations ? cfg->num_simulations : e->cfg.num_simulations;
     if (mcts) {
-        if (cfg->leaves_per_root < 1) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "leaves_per_root must be >= 1");
-        if (!(cfg->virtual_loss >= 0.0f) || !std::isfinite(cfg->virtual_loss))
-            return set_err(e, AZ_ERR_INVALID_ARGUMENT, "virtual_loss must be finite and >= 0");
+        const int r = check_vl_args(e, cfg->leaves_per_root, cfg->virtual_loss, "leaves_per_root");
+        if (r) return r;
         if (S < 1 || S > e->cfg.num_simulations)
             return set_err(e, AZ_ERR_INVALID_ARGUMENT, "num_simulations must be in 1 .. az_config.num_simulations");
     }
@@ -2186,7 +2178,7 @@ int az_match_begin(az_engine* e, int n_concurrent, uint32_t first_game, uint32_t
     const int K = mcts ? cfg->leaves_per_root : 1;
     if (n_concurrent > st->G) return set_err(e, AZ_ERR_CAPACITY, "more slots than az_config.max_games");
     const int n = (int)std::min<uint64_t>((uint64_t)n_concurrent, n_games);
-    if (((long long)n * K + 3) / 4 * 4 * 2 > (long long)e->max_batch)
+    if (net_layout(n, n, K).end > (long long)e->max_batch)   // at worst every slot's mover is on the same network
         return set_err(e, AZ_ERR_CAPACITY, "network ranges (2 x round4(slots x leaves_per_root)) exceed az_config.max_batch");
     if (e->stub_kind == 0) {
         for (int p = 0; p < 2; p++) {
@@ -2203,30 +2195,31 @@ int az_match_begin(az_engine* e, int n_concurrent, uint32_t first_game, uint32_t
     const uint32_t row = std::min<uint32_t>(cfg->max_plies, HIST_CAP);   // a game ends by the fullmove rule before HIST_CAP plies
     r = match_alloc(e, st, n_games, row);
     if (r) return r;
-    st->selfplay_active = false;
-    st->match_cfg = *cfg;
-    st->match_cfg.num_simulations = S;
-    st->match_first = first_game;
-    st->match_games = n_games;
-    st->match_K = K;
-    st->match_row = row;
-    st->match_first_wave = 1;
-    st->match_waves = 0;
-    az_position_start(&st->match_startpos);
+    st->session = Session::none;
+    MatchState& m = st->match;
+    m.cfg = *cfg;
+    m.cfg.num_simulations = S;
+    m.first = first_game;
+    m.games = n_games;
+    m.K = K;
+    m.row = row;
+    m.first_wave = 1;
+    m.waves = 0;
+    az_position_start(&m.startpos);
     st->prm.n_games = n; st->prm.S = S; st->prm.mode = 0;
-    st->prm.priors_scattered = (e->stub_kind == 0 && e->cfg.precision != 1) ? 1 : 0;
+    st->prm.priors_scattered = fused_heads(e) ? 1 : 0;
     st->ptr.batch_count = st->batch_base;
     st->ptr.batch_zero = nullptr;
     const unsigned long long next = first_game;
-    AZ_CUDA(e, cudaMemcpyAsync(st->match_next, &next, sizeof next, cudaMemcpyHostToDevice, e->stream));
-    AZ_CUDA(e, cudaMemsetAsync(st->match_stats, 0, 4 * sizeof(unsigned long long), e->stream));
-    AZ_CUDA(e, cudaMemsetAsync(st->vl_stats, 0, 4 * sizeof(unsigned long long), e->stream));
-    AZ_CUDA(e, cudaMemsetAsync(st->match_result, 0, n_games, e->stream));
-    AZ_CUDA(e, cudaMemsetAsync(st->match_plies, 0, (size_t)n_games * sizeof(uint16_t), e->stream));
-    AZ_CUDA(e, cudaMemsetAsync(st->match_finished, 0, n_games, e->stream));
-    AZ_CUDA(e, cudaMemsetAsync(st->match_moves, 0xFF, (size_t)n_games * row * sizeof(uint16_t), e->stream));
+    AZ_CUDA(e, cudaMemcpyAsync(m.next, &next, sizeof next, cudaMemcpyHostToDevice, e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(m.stats, 0, 4 * sizeof(unsigned long long), e->stream));
+    if ((r = vl_clear(e, st, 0))) return r;   // k_match sets every slot's leaf count in the first wave
+    AZ_CUDA(e, cudaMemsetAsync(m.result.p, 0, n_games, e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(m.plies.p, 0, (size_t)n_games * sizeof(uint16_t), e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(m.finished.p, 0, n_games, e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(m.moves.p, 0xFF, (size_t)n_games * row * sizeof(uint16_t), e->stream));
     AZ_CUDA(e, cudaStreamSynchronize(e->stream));
-    st->match_active = true;
+    st->session = Session::match;
     return AZ_OK;
 }
 
@@ -2234,12 +2227,14 @@ int az_match_step(az_engine* e, int waves, az_match_stats* out) {
     if (!e) return AZ_ERR_INVALID_ARGUMENT;
     if (out) std::memset(out, 0, sizeof *out);
     SearchState* st = e->search;
-    if (!st->match_active) return set_err(e, AZ_ERR_STATE, "no match in progress (az_match_begin)");
+    if (st->session != Session::match) return set_err(e, AZ_ERR_STATE, "no match in progress (az_match_begin)");
     cudaSetDevice(e->cfg.device);
-    const int n = st->prm.n_games, K = st->match_K, base1 = match_base1(st);
-    const VLPtrs vl = vl_ptrs(st, K, st->match_cfg.virtual_loss);
+    MatchState& m = st->match;
+    // a slot queues at most K boards per wave (its batch or its next root), all in its mover's range
+    const int n = st->prm.n_games, base1 = (int)net_layout(n, n, m.K).base1;
+    const VLPtrs vl = vl_ptrs(st, m.K, m.cfg.virtual_loss);
     const NetRoute route{st->d_net, st->batch_base, base1};
-    const NetBatch nb{st->batch_base, base1, base1 + n * K};
+    const NetBatch nb{st->batch_base, base1, base1 + n * m.K};
     for (int w = 0; w < waves; w++) {
         const MatchParams mp = match_params(st);
         AZ_CUDA(e, cudaMemsetAsync(st->batch_base, 0, AZ_MAX_NETWORKS * sizeof(int), e->stream));   // both ranges start empty
@@ -2247,29 +2242,24 @@ int az_match_step(az_engine* e, int waves, az_match_stats* out) {
         e->n_launches += 2;
         k_match<<<(n + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr, vl, route, mp);
         AZ_CUDA(e, cudaGetLastError());
-        k_vl_expand_nets<<<(n * K + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr, vl, route);
-        AZ_CUDA(e, cudaGetLastError());
-        const int r = evaluate_batch(e, st, &nb);
+        const int r = vl_expand_evaluate(e, st, vl, n, &route, &nb);
         if (r) return r;
-        st->match_first_wave = 0;
-        st->match_waves++;
+        m.first_wave = 0;
+        m.waves++;
     }
     int flags[4] = {0, 0, 0, 0};
-    int* d_flags = st->batch_base + 4;
     unsigned long long ms[4], vs[4];
-    AZ_CUDA(e, cudaMemsetAsync(d_flags, 0, 16, e->stream));
-    k_count_active<<<(n + 127) / 128, 128, 0, e->stream>>>(st->prm, st->ptr, d_flags);
-    AZ_CUDA(e, cudaGetLastError());
-    AZ_CUDA(e, cudaMemcpyAsync(flags, d_flags, sizeof flags, cudaMemcpyDeviceToHost, e->stream));
-    AZ_CUDA(e, cudaMemcpyAsync(ms, st->match_stats, sizeof ms, cudaMemcpyDeviceToHost, e->stream));
+    const int r = enqueue_poll(e, *st, n, flags);
+    if (r) return r;
+    AZ_CUDA(e, cudaMemcpyAsync(ms, m.stats, sizeof ms, cudaMemcpyDeviceToHost, e->stream));
     AZ_CUDA(e, cudaMemcpyAsync(vs, st->vl_stats, sizeof vs, cudaMemcpyDeviceToHost, e->stream));
     AZ_CUDA(e, cudaStreamSynchronize(e->stream));
     if (out) {
-        out->waves = st->match_waves;
+        out->waves = m.waves;
         out->evaluations[0] = ms[0]; out->evaluations[1] = ms[1];
         out->leaves = vs[0]; out->terminal_leaves = vs[1]; out->collisions = vs[2];
         out->plies = ms[2]; out->games_finished = ms[3];
-        out->active_games = st->match_first_wave ? std::min<uint64_t>((uint64_t)n, st->match_games) : (uint64_t)flags[0];
+        out->active_games = m.first_wave ? std::min<uint64_t>((uint64_t)n, m.games) : (uint64_t)flags[0];
     }
     if (flags[1]) return set_err(e, AZ_ERR_CAPACITY, "a per-game node/edge pool overflowed during the match (raise edge_capacity_per_node)");
     return AZ_OK;
@@ -2277,18 +2267,18 @@ int az_match_step(az_engine* e, int waves, az_match_stats* out) {
 
 int az_match_results(az_engine* e, int8_t* result_out, uint16_t* plies_out, uint8_t* finished_out, uint16_t* moves_out) {
     if (!e) return AZ_ERR_INVALID_ARGUMENT;
-    SearchState* st = e->search;
-    if (!st->match_games) return set_err(e, AZ_ERR_STATE, "az_match_begin has not been called");
+    const MatchState& m = e->search->match;
+    if (!m.games) return set_err(e, AZ_ERR_STATE, "az_match_begin has not been called");
     if (!result_out || !plies_out || !finished_out) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "null buffer");
     cudaSetDevice(e->cfg.device);
-    const size_t n = st->match_games;
-    AZ_CUDA(e, cudaMemcpyAsync(result_out, st->match_result, n, cudaMemcpyDeviceToHost, e->stream));
-    AZ_CUDA(e, cudaMemcpyAsync(plies_out, st->match_plies, n * sizeof(uint16_t), cudaMemcpyDeviceToHost, e->stream));
-    AZ_CUDA(e, cudaMemcpyAsync(finished_out, st->match_finished, n, cudaMemcpyDeviceToHost, e->stream));
+    const size_t n = m.games;
+    AZ_CUDA(e, cudaMemcpyAsync(result_out, m.result.p, n, cudaMemcpyDeviceToHost, e->stream));
+    AZ_CUDA(e, cudaMemcpyAsync(plies_out, m.plies.p, n * sizeof(uint16_t), cudaMemcpyDeviceToHost, e->stream));
+    AZ_CUDA(e, cudaMemcpyAsync(finished_out, m.finished.p, n, cudaMemcpyDeviceToHost, e->stream));
     if (moves_out) {   // [n][max_plies]: the device keeps row <= max_plies moves per game, the rest is AZ_MOVE_NONE
-        const size_t mp = st->match_cfg.max_plies, row = st->match_row;
+        const size_t mp = m.cfg.max_plies, row = m.row;
         if (row < mp) std::memset(moves_out, 0xFF, n * mp * sizeof(uint16_t));
-        AZ_CUDA(e, cudaMemcpy2DAsync(moves_out, mp * sizeof(uint16_t), st->match_moves, row * sizeof(uint16_t), row * sizeof(uint16_t), n,
+        AZ_CUDA(e, cudaMemcpy2DAsync(moves_out, mp * sizeof(uint16_t), m.moves.p, row * sizeof(uint16_t), row * sizeof(uint16_t), n,
                                      cudaMemcpyDeviceToHost, e->stream));
     }
     AZ_CUDA(e, cudaStreamSynchronize(e->stream));

@@ -115,11 +115,48 @@ struct SearchPtrs {
     unsigned long long* stats;         // [STAT_STRIPES][STAT_WIDTH]: the statistics fields of Counters, striped by block to spread the atomics
 };
 
+// The session-bound calls an engine accepts.  az_selfplay_begin_n / az_selfplay_begin_vl / az_match_begin start a session once
+// their arguments are accepted; every az_search* call that gets past its argument checks ends it.
+enum class Session { none, selfplay, selfplay_vl, match };
+
+// az_selfplay_begin_vl: leaves per game of the self-play in progress, its virtual loss and the waves run since the begin call
+struct SelfplayVL {
+    int K = 0;
+    float lambda = 0.0f;
+    unsigned long long waves = 0;
+};
+
+// a device buffer that grows only when a larger one is needed (its owner frees `p`)
+template <class T>
+struct GrowBuf {
+    T* p = nullptr;
+    size_t cap = 0;   // elements
+};
+
+// az_match_*: the match in progress and the results of the last one begun (readable after a search has ended the match).
+// The result buffers belong to the match; the search buffers are shared with az_search_vl
+struct MatchState {
+    uint32_t games = 0;                    // games of the last az_match_begin (0: none yet)
+    int K = 1;                             // leaves per root per wave (1 for BaseModel players)
+    uint32_t row = 0;                      // moves stored per game on the device (<= HIST_CAP: a game ends by then)
+    unsigned long long first = 0;          // the first game index
+    int first_wave = 0;                    // 1 until the first wave has run: every slot starts a game
+    unsigned long long waves = 0;
+    unsigned long long* next = nullptr;    // [1] next game index to start
+    unsigned long long* stats = nullptr;   // [4] evaluations of network 0, of network 1, plies, games ended
+    GrowBuf<int8_t> result;                // [games]
+    GrowBuf<uint16_t> plies;
+    GrowBuf<uint8_t> finished;
+    GrowBuf<uint16_t> moves;               // [games][row]
+    az_match_config cfg{};
+    az_position startpos{};
+};
+
 struct SearchState {
     SearchParams prm;
     SearchPtrs ptr;
     int G = 0;
-    bool selfplay_active = false;
+    Session session = Session::none;
     unsigned long long cache_evictions = 0;
     unsigned long long sum_search_depth = 0;
     int adv_passes = 1;                    // k_advance launches per wave (AZ_ADV_PASSES, see run_wave)
@@ -128,11 +165,7 @@ struct SearchState {
     unsigned long long wave_counter = 0;   // self-play waves since az_selfplay_begin (cache epoch = wave_counter / S)
     unsigned long long* d_noise_ids = nullptr;  // [max_games] az_search staging (no allocation per call)
     uint32_t* d_noise_plies = nullptr;
-    // az_selfplay_begin_vl: leaves per game of the self-play in progress (0: az_selfplay_begin_n's k_advance waves), its virtual
-    // loss and the waves run since the begin call
-    int sp_vl_K = 0;
-    float sp_vl_lambda = 0.0f;
-    unsigned long long sp_vl_waves = 0;
+    SelfplayVL sp_vl;
     // az_search_vl and az_selfplay_begin_vl, allocated by the first such call (az_engine_create's footprint does not include them)
     uint32_t* vl_V = nullptr;              // [G * edge_cap] descents of the current batch through each edge
     uint2* vl_path = nullptr;              // [max_batch][node_cap] one descent per leaf
@@ -142,24 +175,7 @@ struct SearchState {
     int* vl_count = nullptr;               // [G]
     unsigned long long* vl_stats = nullptr; // [4]
     uint8_t* d_net = nullptr;              // [G] az_search_networks: network of each root (allocated on its first call)
-    // az_match_*: the match in progress (match_active) and the results of the last one begun.  The result buffers belong to the
-    // match and are reallocated only when a larger match begins; the search buffers are shared with az_search_vl
-    bool match_active = false;
-    uint32_t match_games = 0;              // games of the last az_match_begin (0: none yet)
-    int match_K = 1;                       // leaves per root per wave (1 for BaseModel players)
-    uint32_t match_row = 0;                // moves stored per game on the device (<= HIST_CAP: a game ends by then)
-    unsigned long long match_first = 0;    // the first game index
-    int match_first_wave = 0;              // 1 until the first wave has run: every slot starts a game
-    unsigned long long match_waves = 0;
-    unsigned long long* match_next = nullptr;   // [1] next game index to start
-    unsigned long long* match_stats = nullptr;  // [4] evaluations of network 0, of network 1, plies, games ended
-    int8_t* match_result = nullptr;        // [match_cap]
-    uint16_t* match_plies = nullptr;
-    uint8_t* match_finished = nullptr;
-    uint16_t* match_moves = nullptr;       // [match_cap][match_row]
-    size_t match_cap = 0, match_moves_cap = 0;
-    az_match_config match_cfg{};
-    az_position match_startpos{};
+    MatchState match;
     std::vector<void*> allocs;
 };
 
