@@ -73,6 +73,37 @@ class MatchStats(ctypes.Structure):
 
 
 MATCH_MCTS, MATCH_BASE_MODEL = 0, 1
+PLAYER_MCTS, PLAYER_BASE_MODEL, PLAYER_RANDOM = 0, 1, 2
+
+
+class MatchPlayer(ctypes.Structure):
+    """az_match_player."""
+
+    _fields_ = [("kind", ctypes.c_int32), ("network", ctypes.c_uint8), ("num_simulations", ctypes.c_int32),
+                ("leaves_per_root", ctypes.c_int32), ("virtual_loss", ctypes.c_float)]
+
+
+class MatchPlayersConfig(ctypes.Structure):
+    """az_match_players_config."""
+
+    _fields_ = [("player", MatchPlayer * 2), ("num_stochastic_moves", ctypes.c_uint32), ("max_plies", ctypes.c_uint32),
+                ("seed", ctypes.c_uint64)]
+
+
+def match_player(kind, network=0, num_simulations=None, leaves_per_root=1, virtual_loss=1.0):
+    """One player of Engine.match_begin_players: PLAYER_MCTS (num_simulations None = the config's), PLAYER_BASE_MODEL or
+    PLAYER_RANDOM (no network; its other fields are ignored)."""
+    kind = int(kind)
+    if kind not in (PLAYER_MCTS, PLAYER_BASE_MODEL, PLAYER_RANDOM):
+        raise ValueError("player kind must be PLAYER_MCTS, PLAYER_BASE_MODEL or PLAYER_RANDOM")
+    if kind == PLAYER_RANDOM:
+        return MatchPlayer(kind, 0, 0, 1, 0.0)
+    if int(network) < 0:
+        raise ValueError("network ids must be >= 0")
+    p = MatchPlayer(kind, min(int(network), 255), 0, 1, 0.0)
+    if kind == PLAYER_MCTS:
+        p.num_simulations, p.leaves_per_root, p.virtual_loss = int(num_simulations or 0), int(leaves_per_root), float(virtual_loss)
+    return p
 
 
 class EngineError(RuntimeError):
@@ -388,6 +419,23 @@ class Engine:
         c.num_stochastic_moves, c.max_plies, c.seed = int(num_stochastic_moves), int(max_plies), int(seed)
         self._check(self._L.az_match_begin(self._h, int(n_concurrent), ctypes.c_uint32(first_game), ctypes.c_uint32(n_games),
                                            ctypes.byref(c)), "az_match_begin")
+        self._match_shape = (int(n_games), int(max_plies))
+
+    def match_begin_players(self, n_concurrent, n_games, player_1, player_2, num_stochastic_moves=15, max_plies=450, seed=0,
+                            first_game=0):
+        """A match between two independent players (az_match_begin_players), each a MatchPlayer (see match_player) or a dict of
+        match_player's arguments: MCTS with its own network, num_simulations, leaves_per_root and virtual_loss, BaseModel with its
+        own network, or Random.  Otherwise as match_begin; match_step and match_results serve both."""
+        c = MatchPlayersConfig()
+        for i, p in enumerate((player_1, player_2)):
+            if isinstance(p, dict):
+                p = match_player(**p)
+            if not isinstance(p, MatchPlayer):
+                raise ValueError("a player is a MatchPlayer (match_player(...)) or a dict of match_player's arguments")
+            c.player[i] = p
+        c.num_stochastic_moves, c.max_plies, c.seed = int(num_stochastic_moves), int(max_plies), int(seed)
+        self._check(self._L.az_match_begin_players(self._h, int(n_concurrent), ctypes.c_uint32(first_game), ctypes.c_uint32(n_games),
+                                                   ctypes.byref(c)), "az_match_begin_players")
         self._match_shape = (int(n_games), int(max_plies))
 
     def match_step(self, waves):

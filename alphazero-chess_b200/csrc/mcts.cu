@@ -1050,11 +1050,11 @@ __device__ __forceinline__ int vl_backup_batch(Ctx& x, const SearchParams& prm, 
     return nl;
 }
 
-// Gathers the root's next batch: up to min(K, S - sims_done) descents, ended early by a collision (collided = 1).  Returns the
-// number of leaves; depth_sum grows by the edges on their descents.
-__device__ __forceinline__ int vl_gather_batch(Ctx& x, const SearchParams& prm, const VLPtrs& vl, int& collided, unsigned int& depth_sum) {
+// Gathers the root's next batch: up to kb descents into leaf records g * vl.K + k, ended early by a collision (collided = 1).
+// Returns the number of leaves; depth_sum grows by the edges on their descents.
+__device__ __forceinline__ int vl_gather_leaves(Ctx& x, const SearchParams& prm, const VLPtrs& vl, int kb, int& collided,
+                                                unsigned int& depth_sum) {
     int n_leaf = 0;
-    const int kb = min(vl.K, prm.S - (int)x.c.sims_done);
     for (int k = 0; k < kb; k++) {
         const int leaf = x.g * vl.K + k;
         uint2* path = vl.path + (size_t)leaf * prm.node_cap;
@@ -1067,6 +1067,10 @@ __device__ __forceinline__ int vl_gather_batch(Ctx& x, const SearchParams& prm, 
         n_leaf++;
     }
     return n_leaf;
+}
+// the batch of a search with S simulations and K leaves per root: up to min(K, S - sims_done) descents
+__device__ __forceinline__ int vl_gather_batch(Ctx& x, const SearchParams& prm, const VLPtrs& vl, int& collided, unsigned int& depth_sum) {
+    return vl_gather_leaves(x, prm, vl, min(vl.K, prm.S - (int)x.c.sims_done), collided, depth_sum);
 }
 
 // one warp per root: consume the previous batch (the root's own evaluation on the first wave), then gather the next one
@@ -1212,8 +1216,9 @@ __global__ void __launch_bounds__(WARPS * 32) k_vl_selfplay(const __grid_constan
 
 // ------------------------------------------------------------------------------------------- evaluation matches (az_match_*)
 // evaluate (validation.rs:155-282) as alphazero-chess_b200/evaluation.py plays it on one engine, resident: one warp per slot
-// searches a fresh root per ply with az_search_networks' semantics (or takes the priors, for BaseModel players), chooses the move
-// with evaluation.py's rules, plays it through the rules path of move_step and records it.  Semantics in DESIGN.md section 5.
+// plays each ply as its mover's kind does -- MCTS searches a fresh root with az_search_networks' semantics, BaseModel takes the
+// root's priors, Random draws a legal move -- chooses the move with evaluation.py's rules, plays it through the rules path of
+// move_step and records it.  Semantics in DESIGN.md section 5.
 struct MatchParams {
     az_position startpos;               // the initial position
     unsigned long long seed;
@@ -1226,39 +1231,67 @@ struct MatchParams {
     uint8_t* finished;                  // [games] 1: ended by the rules
     uint16_t* moves;                    // [games][row] policy indices played
     uint32_t row, max_plies, n_stochastic;
-    int base_model;                     // 1: BaseModel players: the move comes from the root's priors, no search
     int first_wave;                     // 1: every slot starts a game
-    uint8_t network[2];                 // network slot of player 1 and of player 2
+    // per player (player 1, player 2), indexed by the mover (match_mover)
+    int kind[2];                        // AZ_PLAYER_MCTS, AZ_PLAYER_BASE_MODEL or AZ_PLAYER_RANDOM
+    int S[2];                           // MCTS: simulations per ply
+    int K[2];                           // MCTS: leaves per root and wave (<= VLPtrs::K, the stride of the leaf records)
+    float lambda[2];                    // MCTS: virtual loss
+    uint8_t network[2];                 // MCTS and BaseModel: network slot
 };
 
-// _uniform(seed, game, ply) of evaluation.py (its _mix, not rng_u64), rounded to f32 as _weighted_index does
-__device__ __forceinline__ float match_uniform(u64 seed, u64 game, u64 ply) {
+// _uniform(seed, game, ply) of evaluation.py (its _mix, not rng_u64), in double
+__device__ __forceinline__ double match_uniform_d(u64 seed, u64 game, u64 ply) {
     u64 h = 0x9E3779B97F4A7C15ULL;
     h = (h ^ seed) * 0xBF58476D1CE4E5B9ULL; h ^= h >> 29;
     h = (h ^ game) * 0xBF58476D1CE4E5B9ULL; h ^= h >> 29;
     h = (h ^ ply) * 0xBF58476D1CE4E5B9ULL; h ^= h >> 29;
-    return __double2float_rn(__dmul_rn((double)(h >> 11), 1.0 / 9007199254740992.0));
+    return __dmul_rn((double)(h >> 11), 1.0 / 9007199254740992.0);
+}
+// the same rounded to f32, as _weighted_index does
+__device__ __forceinline__ float match_uniform(u64 seed, u64 game, u64 ply) { return __double2float_rn(match_uniform_d(seed, game, ply)); }
+
+// the mover (0: player 1, 1: player 2): player 1 is White in even games (validation.rs:196-200), so it moves when game + ply is even
+__device__ __forceinline__ int match_mover(u64 game, uint32_t ply) { return (int)((game + ply) & 1); }
+
+// evaluation.RandomPlayer: index[int(_uniform(seed ^ 0x5151, game, ply) x count)], the product in double, whatever the fullmove
+// number.  index and count are az_movegen's: the root's legal moves in sh->moves, in gen_legal order (warp_gen_legal lists the
+// same moves in the same order as gen_legal<ListSink>), under-promotions included.  The root's edges keep that order (create_node)
+// without the under-promotions, each of which follows the queen promotion of its squares and shares its policy index, so move i
+// is played as the edge of the last kept move among moves 0..i.  Returns that root edge.
+__device__ __forceinline__ int match_choose_random(Ctx& x, const MatchParams& mp) {
+    const int n = x.sh->n_moves;
+    const int i = (int)__dmul_rn(match_uniform_d(mp.seed ^ 0x5151ULL, x.c.game_id, x.c.ply), (double)n);
+    int kept = 0;
+    for (int j0 = 0; j0 <= i; j0 += 32) {
+        const int j = j0 + x.lane;
+        bool keep = false;
+        if (j <= i) { const int pr = (x.sh->moves[j] >> 12) & 7; keep = pr == 0 || pr == 4; }
+        kept += __popc(__ballot_sync(0xffffffffu, keep));
+    }
+    return kept - 1;
 }
 
-// the mover's network: player 1 is White in even games (validation.rs:196-200), so player 1 moves when game + ply is even
-__device__ __forceinline__ int match_network(const MatchParams& mp, u64 game, uint32_t ply) { return mp.network[(game + ply) & 1]; }
-
-// The root of the slot's next ply from sh->child / sh->moves, its evaluation queued in the range of the mover's network
-__device__ __forceinline__ void match_root(Ctx& x, const MatchParams& mp, const NetRoute& rt, unsigned int* evals) {
+// The root of the slot's next ply from sh->child / sh->moves.  An MCTS or BaseModel mover queues its evaluation in the range of
+// its network and -1 is returned; a Random mover needs no evaluation: its edge is returned, to be played in this wave.
+__device__ __forceinline__ int match_root(Ctx& x, const MatchParams& mp, const NetRoute& rt, unsigned int* evals) {
     setup_root_from_shared(x);
-    const int s = match_network(mp, x.c.game_id, x.c.ply);
+    const int p = match_mover(x.c.game_id, x.c.ply);
+    if (mp.kind[p] == AZ_PLAYER_RANDOM) return match_choose_random(x, mp);
+    const int s = mp.network[p];
     if (x.lane == 0) mp.net[x.g] = (uint8_t)s;
     x.c.pending_node = 0;
     x.c.pending_slot = submit_request<true>(x, 0, &rt);
     evals[s]++;
+    return -1;
 }
 
-// The next unplayed game starts in this slot (its root queued for evaluation), or the slot goes idle
-__device__ __forceinline__ void match_start_game(Ctx& x, const MatchParams& mp, const NetRoute& rt, unsigned int* evals) {
+// The next unplayed game starts in this slot (as match_root, which returns), or the slot goes idle (-1)
+__device__ __forceinline__ int match_start_game(Ctx& x, const MatchParams& mp, const NetRoute& rt, unsigned int* evals) {
     unsigned long long gid = 0;
     if (x.lane == 0) gid = atomicAdd(mp.next_game, 1ULL);
     gid = __shfl_sync(0xffffffffu, gid, 0);
-    if (gid >= mp.end_game) { x.c.status = 1; return; }
+    if (gid >= mp.end_game) { x.c.status = 1; return -1; }
     x.c.game_id = gid; x.c.ply = 0; x.c.hist_len = 1;
     if (x.lane == 0) {
         DPos s = dpos_from_wire(mp.startpos);
@@ -1269,7 +1302,7 @@ __device__ __forceinline__ void match_start_game(Ctx& x, const MatchParams& mp, 
         x.ptr.hist[(size_t)x.g * HIST_CAP] = s;
     }
     __syncwarp();
-    match_root(x, mp, rt, evals);
+    return match_root(x, mp, rt, evals);
 }
 
 // evaluation.py's move choice at the root: the weights are the visit counts over their f32 sum (_choose_from_visits) or the priors
@@ -1279,7 +1312,8 @@ __device__ __forceinline__ void match_start_game(Ctx& x, const MatchParams& mp, 
 __device__ __forceinline__ int match_choose(Ctx& x, const MatchParams& mp, const DPos& root) {
     const size_t off = x.ebase;   // the root's edges start at 0
     const int L = (int)((x.c.flags >> 8) & 0xFF);
-    const float* w = mp.base_model ? x.ptr.edge_P + off : x.ptr.edge_N + off;
+    const bool base_model = mp.kind[match_mover(x.c.game_id, x.c.ply)] == AZ_PLAYER_BASE_MODEL;
+    const float* w = base_model ? x.ptr.edge_P + off : x.ptr.edge_N + off;
     float sum = 0.0f;   // visit counts are integers below 2^24: the f32 sum is exact in any order
     for (int e = x.lane; e < L; e += 32) sum = __fadd_rn(sum, w[e]);
     for (int d = 16; d; d >>= 1) sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, d));
@@ -1299,7 +1333,7 @@ __device__ __forceinline__ int match_choose(Ctx& x, const MatchParams& mp, const
     __syncwarp();
     for (int i = x.lane; i < nv; i += 32) {
         const float v = w[x.sh->sidx[i]];
-        x.sh->fval[i] = mp.base_model ? v : __fdiv_rn(v, sum);
+        x.sh->fval[i] = base_model ? v : __fdiv_rn(v, sum);
     }
     __syncwarp();
     int edge = 0;
@@ -1324,9 +1358,10 @@ __device__ __forceinline__ int match_choose(Ctx& x, const MatchParams& mp, const
 }
 
 // One wave of a match, one warp per slot: consume the root's evaluation or back up the previous batch in leaf order; once the
-// root has S visits (BaseModel: at once) choose and play the move, then either queue the next ply's root in the new mover's
-// network range or record the game and start the next unplayed one; otherwise gather the next batch.  k_vl_expand_nets (leaves
-// routed by mp.net) and the multi-network forward follow.
+// root has the mover's S visits (BaseModel: at once) choose and play the move, then either queue the next ply's root in the new
+// mover's network range or record the game and start the next unplayed one.  A Random mover's ply is played as soon as its root is
+// set up, so a slot goes on playing until a root waits for a network.  Otherwise it gathers the next batch (up to the mover's K
+// leaves).  k_vl_expand_nets (leaves routed by mp.net) and the multi-network forward follow.
 __global__ void __launch_bounds__(WARPS * 32) k_match(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
                                                       const __grid_constant__ VLPtrs vl, const __grid_constant__ NetRoute rt,
                                                       const __grid_constant__ MatchParams mp) {
@@ -1342,31 +1377,31 @@ __global__ void __launch_bounds__(WARPS * 32) k_match(const __grid_constant__ Se
     if (!mp.first_wave && x.c.status != 0) return;   // idle slot or pool overflow: vl.count[g] is already 0
     unsigned int evals[AZ_MAX_NETWORKS] = {0, 0}, plies = 0, games = 0;
     int n_leaf = 0, collided = 0;
-    bool move = false;
+    int play = -1;   // the root edge the mover plays in this wave
     if (mp.first_wave) {
-        match_start_game(x, mp, rt, evals);
+        play = match_start_game(x, mp, rt, evals);
     } else if (x.c.pending_node == 0) {   // MCTree::init: the root's priors (no noise), no descent in flight
         const int L = (int)((x.c.flags >> 8) & 0xFF);
         if (!prm.priors_scattered) copy_priors(ptr, x.ebase, L, x.c.pending_slot, x.lane);
         for (int e = x.lane; e < L; e += 32) vl.V[x.ebase + e] = 0;
         __syncwarp();
         x.c.pending_node = -1;
-        move = mp.base_model != 0;
+        if (mp.kind[match_mover(x.c.game_id, x.c.ply)] == AZ_PLAYER_BASE_MODEL) play = match_choose(x, mp, ptr.node_pos[x.nbase]);
     } else {
+        const int p = match_mover(x.c.game_id, x.c.ply);
         const int nl = vl.count[g];
         int evaluated = 0;   // leaves that went to the network (the others were terminal)
         for (int k0 = 0; k0 < nl; k0 += 32) {
             const int k = k0 + x.lane;
             evaluated += __popc(__ballot_sync(0xffffffffu, k < nl && vl.slot[g * vl.K + k] >= 0));
         }
-        evals[match_network(mp, x.c.game_id, x.c.ply)] += evaluated;
+        evals[mp.network[p]] += evaluated;
         x.c.sims_done += vl_backup_batch(x, prm, ptr, vl);
-        move = (int)x.c.sims_done >= prm.S;
+        if ((int)x.c.sims_done >= mp.S[p]) play = match_choose(x, mp, ptr.node_pos[x.nbase]);
     }
-    if (move) {
+    while (play >= 0) {
         const DPos root = ptr.node_pos[x.nbase];
-        const int e = match_choose(x, mp, root);
-        const uint32_t amv = ptr.edge_mv[x.ebase + e];
+        const uint32_t amv = ptr.edge_mv[x.ebase + play];
         lane0_make_child(x, root, (uint16_t)(amv & 0xFFFF));
         int term = x.sh->term;
         if (term == 0 && draw_by_rules(x, ptr.path + (size_t)g * prm.node_cap, x.sh->child, 1)) term = 1;
@@ -1380,16 +1415,20 @@ __global__ void __launch_bounds__(WARPS * 32) k_match(const __grid_constant__ Se
                 mp.finished[gi] = term != 0 ? 1 : 0;
             }
             games++;
-            match_start_game(x, mp, rt, evals);
+            play = match_start_game(x, mp, rt, evals);
         } else {
             if (x.lane == 0 && x.c.hist_len < HIST_CAP) ptr.hist[(size_t)g * HIST_CAP + x.c.hist_len] = x.sh->child;
             x.c.hist_len = min(x.c.hist_len + 1, (uint32_t)HIST_CAP);
             x.c.ply++;
-            match_root(x, mp, rt, evals);
+            play = match_root(x, mp, rt, evals);
         }
-    } else if (x.c.status == 0 && x.c.pending_node < 0) {
+    }
+    if (x.c.status == 0 && x.c.pending_node < 0) {   // an MCTS root that still needs simulations
+        const int p = match_mover(x.c.game_id, x.c.ply);
+        VLPtrs v = vl;
+        v.lambda = mp.lambda[p];
         unsigned int depth_sum = 0;
-        n_leaf = vl_gather_batch(x, prm, vl, collided, depth_sum);
+        n_leaf = vl_gather_leaves(x, prm, v, min(mp.K[p], mp.S[p] - (int)x.c.sims_done), collided, depth_sum);
     }
     if (x.lane == 0) {
         vl_publish(vl, g, n_leaf, collided);   // 0 when the slot moved, went idle or waits for its root: the next wave backs up nothing
@@ -1976,7 +2015,7 @@ static int match_alloc(az_engine* e, SearchState* st, size_t games, size_t row) 
 
 static MatchParams match_params(const SearchState* st) {
     const MatchState& m = st->match;
-    const az_match_config& c = m.cfg;
+    const az_match_players_config& c = m.cfg;
     MatchParams mp;
     mp.startpos = m.startpos;
     mp.seed = c.seed;
@@ -1987,10 +2026,102 @@ static MatchParams match_params(const SearchState* st) {
     mp.net = st->d_net;
     mp.result = m.result.p; mp.plies = m.plies.p; mp.finished = m.finished.p; mp.moves = m.moves.p;
     mp.row = m.row; mp.max_plies = c.max_plies; mp.n_stochastic = c.num_stochastic_moves;
-    mp.base_model = c.player_kind == 1 ? 1 : 0;
     mp.first_wave = m.first_wave;
-    mp.network[0] = c.network[0]; mp.network[1] = c.network[1];
+    for (int p = 0; p < 2; p++) {
+        const az_match_player& q = c.player[p];
+        mp.kind[p] = q.kind;
+        mp.S[p] = q.num_simulations;
+        mp.K[p] = q.leaves_per_root;
+        mp.lambda[p] = q.virtual_loss;
+        mp.network[p] = q.network;
+    }
     return mp;
+}
+
+// the per-player checks of az_match_begin_players (az_match_begin checks its own config with its own texts); resolves
+// num_simulations 0 to the engine's and gives BaseModel and Random players S = K = 1, lambda = 0 and Random players network 0
+static int check_match_player(az_engine* e, az_match_player& q) {
+    if (q.kind != AZ_PLAYER_MCTS && q.kind != AZ_PLAYER_BASE_MODEL && q.kind != AZ_PLAYER_RANDOM)
+        return set_err(e, AZ_ERR_INVALID_ARGUMENT, "player kind must be AZ_PLAYER_MCTS, AZ_PLAYER_BASE_MODEL or AZ_PLAYER_RANDOM");
+    if (q.kind == AZ_PLAYER_RANDOM) q.network = 0;
+    if (q.network >= AZ_MAX_NETWORKS) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "network id must be < AZ_MAX_NETWORKS");
+    if (q.kind != AZ_PLAYER_MCTS) {
+        q.num_simulations = 1; q.leaves_per_root = 1; q.virtual_loss = 0.0f;
+        return AZ_OK;
+    }
+    const int r = check_vl_args(e, q.leaves_per_root, q.virtual_loss, "leaves_per_root");
+    if (r) return r;
+    if (!q.num_simulations) q.num_simulations = e->cfg.num_simulations;
+    if (q.num_simulations < 1 || q.num_simulations > e->cfg.num_simulations)
+        return set_err(e, AZ_ERR_INVALID_ARGUMENT, "num_simulations must be in 1 .. az_config.num_simulations");
+    return AZ_OK;
+}
+
+// The network ranges of a match on n slots: network s holds round4(n x k[s]) boards, k[s] the largest K of the players on it (1
+// for BaseModel, 0 when no player uses it), network 0's range from board 0 and network 1's from base1; k_max is the largest K of
+// all players (1 when there is none), the stride of the leaf records
+struct MatchLayout { long long base1, end; int k[AZ_MAX_NETWORKS]; int k_max; };
+static MatchLayout match_layout(const az_match_players_config& c, long long n) {
+    MatchLayout lay{0, 0, {0, 0}, 1};
+    for (const az_match_player& q : c.player) {
+        if (q.kind == AZ_PLAYER_RANDOM) continue;
+        lay.k[q.network] = std::max(lay.k[q.network], q.leaves_per_root);
+        lay.k_max = std::max(lay.k_max, q.leaves_per_root);
+    }
+    lay.base1 = (n * lay.k[0] + 3) & ~3LL;
+    lay.end = lay.base1 + ((n * lay.k[1] + 3) & ~3LL);
+    return lay;
+}
+
+// Starts a checked match (players resolved by check_match_player or az_match_begin): weights, knobs, buffers, session
+static int match_start(az_engine* e, int n_concurrent, uint32_t first_game, uint32_t n_games, const az_match_players_config& cfg) {
+    SearchState* st = e->search;
+    const int n = (int)std::min<uint64_t>((uint64_t)n_concurrent, n_games);
+    const MatchLayout lay = match_layout(cfg, n);
+    const bool evaluates = lay.k[0] || lay.k[1];
+    if (e->stub_kind == 0 && evaluates) {
+        for (int s = 0; s < AZ_MAX_NETWORKS; s++) {
+            const NetWeights* w = net_slot(e, s);
+            if (lay.k[s] && (!w || !w->loaded)) return set_err(e, AZ_ERR_NO_WEIGHTS, "a player names a network that has not been loaded");
+        }
+        const int r = net_networks_supported(e);
+        if (r) return r;
+    }
+    cudaSetDevice(e->cfg.device);
+    int r = vl_alloc(e, st);
+    if (r) return r;
+    if (!st->d_net && salloc(e, st, &st->d_net, (size_t)st->G)) return AZ_ERR_OUT_OF_MEMORY;
+    const uint32_t row = std::min<uint32_t>(cfg.max_plies, HIST_CAP);   // a game ends by the fullmove rule before HIST_CAP plies
+    r = match_alloc(e, st, n_games, row);
+    if (r) return r;
+    st->session = Session::none;
+    MatchState& m = st->match;
+    m.cfg = cfg;
+    m.first = first_game;
+    m.games = n_games;
+    m.K = lay.k_max;
+    m.base1 = (int)lay.base1;
+    m.cap = (int)lay.base1 + n * lay.k[1];
+    m.evaluates = evaluates;
+    m.row = row;
+    m.first_wave = 1;
+    m.waves = 0;
+    az_position_start(&m.startpos);
+    st->prm.n_games = n; st->prm.S = std::max(cfg.player[0].num_simulations, cfg.player[1].num_simulations); st->prm.mode = 0;
+    st->prm.priors_scattered = fused_heads(e) ? 1 : 0;
+    st->ptr.batch_count = st->batch_base;
+    st->ptr.batch_zero = nullptr;
+    const unsigned long long next = first_game;
+    AZ_CUDA(e, cudaMemcpyAsync(m.next, &next, sizeof next, cudaMemcpyHostToDevice, e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(m.stats, 0, 4 * sizeof(unsigned long long), e->stream));
+    if ((r = vl_clear(e, st, 0))) return r;   // k_match sets every slot's leaf count in the first wave
+    AZ_CUDA(e, cudaMemsetAsync(m.result.p, 0, n_games, e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(m.plies.p, 0, (size_t)n_games * sizeof(uint16_t), e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(m.finished.p, 0, n_games, e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(m.moves.p, 0xFF, (size_t)n_games * row * sizeof(uint16_t), e->stream));
+    AZ_CUDA(e, cudaStreamSynchronize(e->stream));
+    st->session = Session::match;
+    return AZ_OK;
 }
 
 }  // namespace azb
@@ -2180,47 +2311,32 @@ int az_match_begin(az_engine* e, int n_concurrent, uint32_t first_game, uint32_t
     const int n = (int)std::min<uint64_t>((uint64_t)n_concurrent, n_games);
     if (net_layout(n, n, K).end > (long long)e->max_batch)   // at worst every slot's mover is on the same network
         return set_err(e, AZ_ERR_CAPACITY, "network ranges (2 x round4(slots x leaves_per_root)) exceed az_config.max_batch");
-    if (e->stub_kind == 0) {
-        for (int p = 0; p < 2; p++) {
-            const NetWeights* w = net_slot(e, cfg->network[p]);
-            if (!w || !w->loaded) return set_err(e, AZ_ERR_NO_WEIGHTS, "a player names a network that has not been loaded");
-        }
-        const int r = net_networks_supported(e);
+    // two players of the same kind and settings
+    az_match_players_config pc{};
+    for (int p = 0; p < 2; p++)
+        pc.player[p] = mcts ? az_match_player{AZ_PLAYER_MCTS, cfg->network[p], S, cfg->leaves_per_root, cfg->virtual_loss}
+                            : az_match_player{AZ_PLAYER_BASE_MODEL, cfg->network[p], 1, 1, 0.0f};
+    pc.num_stochastic_moves = cfg->num_stochastic_moves;
+    pc.max_plies = cfg->max_plies;
+    pc.seed = cfg->seed;
+    return match_start(e, n_concurrent, first_game, n_games, pc);
+}
+
+int az_match_begin_players(az_engine* e, int n_concurrent, uint32_t first_game, uint32_t n_games, const az_match_players_config* cfg) {
+    if (!e) return AZ_ERR_INVALID_ARGUMENT;
+    if (!cfg) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "null config");
+    az_match_players_config pc = *cfg;
+    for (az_match_player& q : pc.player) {
+        const int r = check_match_player(e, q);
         if (r) return r;
     }
-    cudaSetDevice(e->cfg.device);
-    int r = vl_alloc(e, st);
-    if (r) return r;
-    if (!st->d_net && salloc(e, st, &st->d_net, (size_t)st->G)) return AZ_ERR_OUT_OF_MEMORY;
-    const uint32_t row = std::min<uint32_t>(cfg->max_plies, HIST_CAP);   // a game ends by the fullmove rule before HIST_CAP plies
-    r = match_alloc(e, st, n_games, row);
-    if (r) return r;
-    st->session = Session::none;
-    MatchState& m = st->match;
-    m.cfg = *cfg;
-    m.cfg.num_simulations = S;
-    m.first = first_game;
-    m.games = n_games;
-    m.K = K;
-    m.row = row;
-    m.first_wave = 1;
-    m.waves = 0;
-    az_position_start(&m.startpos);
-    st->prm.n_games = n; st->prm.S = S; st->prm.mode = 0;
-    st->prm.priors_scattered = fused_heads(e) ? 1 : 0;
-    st->ptr.batch_count = st->batch_base;
-    st->ptr.batch_zero = nullptr;
-    const unsigned long long next = first_game;
-    AZ_CUDA(e, cudaMemcpyAsync(m.next, &next, sizeof next, cudaMemcpyHostToDevice, e->stream));
-    AZ_CUDA(e, cudaMemsetAsync(m.stats, 0, 4 * sizeof(unsigned long long), e->stream));
-    if ((r = vl_clear(e, st, 0))) return r;   // k_match sets every slot's leaf count in the first wave
-    AZ_CUDA(e, cudaMemsetAsync(m.result.p, 0, n_games, e->stream));
-    AZ_CUDA(e, cudaMemsetAsync(m.plies.p, 0, (size_t)n_games * sizeof(uint16_t), e->stream));
-    AZ_CUDA(e, cudaMemsetAsync(m.finished.p, 0, n_games, e->stream));
-    AZ_CUDA(e, cudaMemsetAsync(m.moves.p, 0xFF, (size_t)n_games * row * sizeof(uint16_t), e->stream));
-    AZ_CUDA(e, cudaStreamSynchronize(e->stream));
-    st->session = Session::match;
-    return AZ_OK;
+    if (n_concurrent < 1 || n_games == 0 || pc.max_plies == 0)
+        return set_err(e, AZ_ERR_INVALID_ARGUMENT, "n_concurrent, n_games and max_plies must be positive");
+    if (n_concurrent > e->search->G) return set_err(e, AZ_ERR_CAPACITY, "more slots than az_config.max_games");
+    const int n = (int)std::min<uint64_t>((uint64_t)n_concurrent, n_games);
+    if (match_layout(pc, n).end > (long long)e->max_batch)
+        return set_err(e, AZ_ERR_CAPACITY, "network ranges (round4(slots x the largest leaves_per_root) per network used) exceed az_config.max_batch");
+    return match_start(e, n_concurrent, first_game, n_games, pc);
 }
 
 int az_match_step(az_engine* e, int waves, az_match_stats* out) {
@@ -2230,20 +2346,23 @@ int az_match_step(az_engine* e, int waves, az_match_stats* out) {
     if (st->session != Session::match) return set_err(e, AZ_ERR_STATE, "no match in progress (az_match_begin)");
     cudaSetDevice(e->cfg.device);
     MatchState& m = st->match;
-    // a slot queues at most K boards per wave (its batch or its next root), all in its mover's range
-    const int n = st->prm.n_games, base1 = (int)net_layout(n, n, m.K).base1;
-    const VLPtrs vl = vl_ptrs(st, m.K, m.cfg.virtual_loss);
-    const NetRoute route{st->d_net, st->batch_base, base1};
-    const NetBatch nb{st->batch_base, base1, base1 + n * m.K};
+    // a slot queues at most its mover's K boards per wave (its batch or its next root), all in its mover's range; k_match sets
+    // each mover's virtual loss
+    const int n = st->prm.n_games;
+    const VLPtrs vl = vl_ptrs(st, m.K, 0.0f);
+    const NetRoute route{st->d_net, st->batch_base, m.base1};
+    const NetBatch nb{st->batch_base, m.base1, m.cap};
     for (int w = 0; w < waves; w++) {
         const MatchParams mp = match_params(st);
         AZ_CUDA(e, cudaMemsetAsync(st->batch_base, 0, AZ_MAX_NETWORKS * sizeof(int), e->stream));   // both ranges start empty
         prof_mark_search(e);
-        e->n_launches += 2;
+        e->n_launches += m.evaluates ? 2 : 1;
         k_match<<<(n + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr, vl, route, mp);
         AZ_CUDA(e, cudaGetLastError());
-        const int r = vl_expand_evaluate(e, st, vl, n, &route, &nb);
-        if (r) return r;
+        if (m.evaluates) {   // Random vs Random: no slot ever waits for a network
+            const int r = vl_expand_evaluate(e, st, vl, n, &route, &nb);
+            if (r) return r;
+        }
         m.first_wave = 0;
         m.waves++;
     }

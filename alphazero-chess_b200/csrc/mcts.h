@@ -136,8 +136,10 @@ struct GrowBuf {
 // az_match_*: the match in progress and the results of the last one begun (readable after a search has ended the match).
 // The result buffers belong to the match; the search buffers are shared with az_search_vl
 struct MatchState {
-    uint32_t games = 0;                    // games of the last az_match_begin (0: none yet)
-    int K = 1;                             // leaves per root per wave (1 for BaseModel players)
+    uint32_t games = 0;                    // games of the last az_match_begin* (0: none yet)
+    int K = 1;                             // the stride of the leaf records: the players' largest leaves per root and wave
+    int base1 = 0, cap = 0;                // network 1's range starts at base1; the ranges end by cap (NetBatch)
+    bool evaluates = true;                 // a player uses a network (false: Random vs Random, no network round)
     uint32_t row = 0;                      // moves stored per game on the device (<= HIST_CAP: a game ends by then)
     unsigned long long first = 0;          // the first game index
     int first_wave = 0;                    // 1 until the first wave has run: every slot starts a game
@@ -148,7 +150,7 @@ struct MatchState {
     GrowBuf<uint16_t> plies;
     GrowBuf<uint8_t> finished;
     GrowBuf<uint16_t> moves;               // [games][row]
-    az_match_config cfg{};
+    az_match_players_config cfg{};         // num_simulations resolved (0: the engine's)
     az_position startpos{};
 };
 

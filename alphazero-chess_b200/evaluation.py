@@ -218,40 +218,54 @@ def evaluate(player_1, player_2, rules_engine, n_games=EVALUATION_GAMES, num_sto
             "p2_winrate": (n_games - wins - draws) / n_games, "results": p1, "unfinished": int(active.sum())}
 
 
+def _device_player(p):
+    """The az_match_player of an evaluate() player, or None for a player the device does not play."""
+    from . import PLAYER_BASE_MODEL, PLAYER_MCTS, PLAYER_RANDOM, match_player
+
+    if type(p) is MctsPlayer:
+        return match_player(PLAYER_MCTS, p.network, p._num_simulations(), p.leaves_per_root, p.virtual_loss)
+    if type(p) is BasePlayer:
+        return match_player(PLAYER_BASE_MODEL, p.network)
+    if type(p) is RandomPlayer:
+        return match_player(PLAYER_RANDOM)
+    return None
+
+
 def evaluate_on_device(player_1, player_2, n_games=EVALUATION_GAMES, num_stochastic_moves=TEMPERATURE_ANNEALING, seed=0, max_plies=450,
                        concurrent=None, waves_per_step=256):
-    """evaluate() played resident on the device (Engine.match_begin / match_step / match_results): the same games, bit for bit,
-    for the pairs whose plies evaluate() runs as one joint call -- two MctsPlayers with equal (num_simulations, leaves_per_root,
-    virtual_loss) or two BasePlayers, on one engine -- without a host round trip per ply.  `concurrent` games run at once (None:
-    as many as max_games and the two network ranges allow, 2 x round4(slots x leaves_per_root) <= max_batch).  All n_games run
-    at once, as evaluate() searches them, only when max_games >= n_games and max_batch >= 2 x round4(n_games x leaves_per_root);
-    with fewer slots the games are the same but the match takes more network rounds, so size the engine accordingly.  Returns
-    evaluate()'s dict plus `moves` [n_games, max_plies] (the policy indices played, MOVE_NONE after the last), `plies` [n_games]
-    and `stats` (MatchStats: waves, evaluations per network, ...).
-    Raises ValueError for other pairs."""
-    from . import MATCH_BASE_MODEL, MATCH_MCTS
+    """evaluate() played resident on the device (Engine.match_begin_players / match_step / match_results): the same games, bit for
+    bit, for any pairing of MctsPlayer, BasePlayer and RandomPlayer on one engine, without a host round trip per ply.  A
+    RandomPlayer's engine is not used (it needs no network): the match runs on the other player's engine, or on player 1's for two
+    RandomPlayers.  `concurrent` games run at once (None: as many as max_games and the network ranges allow: each network a player
+    uses holds round4(slots x K) boards, K the largest leaves_per_root of its players, 1 for a BasePlayer, and the ranges must fit
+    max_batch).  All n_games run at once, as evaluate() plays them, only when the engine allows n_games slots; with fewer slots
+    the games are the same but the match takes more network rounds, so size the engine accordingly.  Returns evaluate()'s dict
+    plus `moves` [n_games, max_plies] (the policy indices played, MOVE_NONE after the last), `plies` [n_games] and `stats`
+    (MatchStats: waves, evaluations per network, ...).
+    Raises ValueError for a MiniMaxPlayer (or any other player) and for two non-random players on different engines."""
+    from . import PLAYER_RANDOM
 
-    kinds = (type(player_1), type(player_2))
-    if kinds[0] is not kinds[1] or kinds[0] not in (MctsPlayer, BasePlayer):
-        raise ValueError("evaluate_on_device plays two MctsPlayers or two BasePlayers; use evaluate() for other pairs")
-    if player_1.engine is not player_2.engine:
+    players = (player_1, player_2)
+    desc = [_device_player(p) for p in players]
+    if any(d is None for d in desc):
+        raise ValueError("evaluate_on_device plays MctsPlayer, BasePlayer and RandomPlayer; use evaluate() for other players")
+    engines = [p.engine for p in players if type(p) is not RandomPlayer]
+    if len(engines) == 2 and engines[0] is not engines[1]:
         raise ValueError("evaluate_on_device needs both players on one engine (network slots 0 and 1)")
-    eng = player_1.engine
+    eng = engines[0] if engines else player_1.engine
     if max_plies < 1:
         raise ValueError("max_plies must be >= 1")
-    kw = {}
-    if kinds[0] is MctsPlayer:
-        settings = [(p._num_simulations(), p.leaves_per_root, p.virtual_loss) for p in (player_1, player_2)]
-        if settings[0] != settings[1]:
-            raise ValueError("evaluate_on_device needs equal (num_simulations, leaves_per_root, virtual_loss) for both players")
-        kw = dict(num_simulations=settings[0][0], leaves_per_root=settings[0][1], virtual_loss=settings[0][2])
-    k = kw.get("leaves_per_root", 1)
-    if concurrent is None:   # all games at once, as far as max_games and the two network ranges (2 x round4(slots x K)) allow
+    if concurrent is None:   # all games at once, as far as max_games and the network ranges allow
+        k = [0, 0]
+        for d in desc:
+            if d.kind != PLAYER_RANDOM:
+                k[d.network] = max(k[d.network], d.leaves_per_root)
         max_batch = max(int(eng.config.max_batch), int(eng.config.max_games))
-        concurrent = min(n_games, int(eng.config.max_games), (max_batch // 2) // 4 * 4 // k)
+        concurrent = min(n_games, int(eng.config.max_games))
+        while concurrent > 1 and sum((concurrent * kk + 3) // 4 * 4 for kk in k) > max_batch:
+            concurrent -= 1
     slots = min(int(concurrent), n_games)
-    eng.match_begin(slots, n_games, MATCH_MCTS if kinds[0] is MctsPlayer else MATCH_BASE_MODEL, (player_1.network, player_2.network),
-                    num_stochastic_moves=num_stochastic_moves, max_plies=max_plies, seed=seed, **kw)
+    eng.match_begin_players(slots, n_games, desc[0], desc[1], num_stochastic_moves=num_stochastic_moves, max_plies=max_plies, seed=seed)
     stats = eng.match_step(waves_per_step)
     while stats.active_games:
         stats = eng.match_step(waves_per_step)

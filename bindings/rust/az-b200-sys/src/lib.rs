@@ -27,6 +27,13 @@ pub struct az_config { pub device: i32, pub max_games: i32, pub max_batch: i32, 
 #[repr(C)] #[derive(Clone, Copy, Default)] pub struct az_match_config { pub player_kind: i32, pub network: [u8; 2],
     pub num_simulations: i32, pub leaves_per_root: i32, pub virtual_loss: f32, pub num_stochastic_moves: u32, pub max_plies: u32,
     pub seed: u64 }
+#[repr(C)] #[derive(Clone, Copy, Default)] pub struct az_match_player { pub kind: i32, pub network: u8, pub num_simulations: i32,
+    pub leaves_per_root: i32, pub virtual_loss: f32 }                                            // AZ_PLAYER_MCTS / _BASE_MODEL / _RANDOM
+#[repr(C)] #[derive(Clone, Copy, Default)] pub struct az_match_players_config { pub player: [az_match_player; 2],
+    pub num_stochastic_moves: u32, pub max_plies: u32, pub seed: u64 }
+pub const AZ_PLAYER_MCTS: i32 = 0;
+pub const AZ_PLAYER_BASE_MODEL: i32 = 1;
+pub const AZ_PLAYER_RANDOM: i32 = 2;
 #[repr(C)] #[derive(Default)] pub struct az_match_stats { pub waves: u64, pub evaluations: [u64; 2], pub leaves: u64,
     pub terminal_leaves: u64, pub collisions: u64, pub plies: u64, pub games_finished: u64, pub active_games: u64 }
 pub enum az_engine {}
@@ -68,6 +75,8 @@ extern "C" {
     pub fn az_selfplay_vl_stats(eng: *mut az_engine, stats: *mut az_search_stats) -> c_int;
     pub fn az_selfplay_step(eng: *mut az_engine, waves: c_int, stats: *mut az_selfplay_stats) -> c_int;
     pub fn az_match_begin(eng: *mut az_engine, n_concurrent: c_int, first_game: u32, n_games: u32, config: *const az_match_config) -> c_int;
+    pub fn az_match_begin_players(eng: *mut az_engine, n_concurrent: c_int, first_game: u32, n_games: u32,
+                                  config: *const az_match_players_config) -> c_int;
     pub fn az_match_step(eng: *mut az_engine, waves: c_int, stats: *mut az_match_stats) -> c_int;
     pub fn az_match_results(eng: *mut az_engine, result: *mut i8, plies: *mut u16, finished: *mut u8, moves: *mut u16) -> c_int;
     pub fn az_selfplay_drain(eng: *mut az_engine, out: *mut az_sample, max_samples: c_int, n_out: *mut c_int) -> c_int;

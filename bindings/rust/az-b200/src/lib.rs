@@ -139,6 +139,32 @@ impl Engine {
         let max_batch = self.config().max_batch.max(self.config().max_games);
         let slots = (n_games as i64).min(self.config().max_games as i64).min(((max_batch / 2) / 4 * 4 / k) as i64) as i32;
         self.check(unsafe { sys::az_match_begin(self.raw, slots, 0, n_games, &cfg) })?;
+        self.match_outcome(n_games)
+    }
+
+    /// evaluate (validation.rs:155-282) between two independent players, resident on the device (az_match_begin_players): each
+    /// player is MCTS (its own network slot, simulations (0: the config's), leaves_per_root and virtual_loss), BaseModel (its own
+    /// network slot) or Random (no network).  As many games run at once as max_games and the network ranges allow: each network a
+    /// player uses holds round4(slots x K) boards, K the largest leaves_per_root of its players (1 for BaseModel).  Returns
+    /// (winrate, drawrate, lossrate) from player 1's side.
+    pub fn evaluate_players(&mut self, player_1: sys::az_match_player, player_2: sys::az_match_player, n_games: u32,
+                            num_stochastic_moves: u32, seed: u64, max_plies: u32) -> Result<(f32, f32, f32)> {
+        let cfg = sys::az_match_players_config { player: [player_1, player_2], num_stochastic_moves, max_plies, seed };
+        let mut k = [0i64; 2];
+        for p in cfg.player.iter().filter(|p| p.kind != sys::AZ_PLAYER_RANDOM) {
+            let pk = if p.kind == sys::AZ_PLAYER_MCTS { p.leaves_per_root.max(1) as i64 } else { 1 };
+            let s = (p.network as usize).min(1);
+            k[s] = k[s].max(pk);
+        }
+        let max_batch = self.config().max_batch.max(self.config().max_games) as i64;
+        let mut slots = (n_games as i64).min(self.config().max_games as i64);
+        while slots > 1 && k.iter().map(|&kk| (slots * kk + 3) / 4 * 4).sum::<i64>() > max_batch { slots -= 1; }
+        self.check(unsafe { sys::az_match_begin_players(self.raw, slots as i32, 0, n_games, &cfg) })?;
+        self.match_outcome(n_games)
+    }
+
+    /// steps the match begun until every game is over and scores it from player 1's side
+    fn match_outcome(&mut self, n_games: u32) -> Result<(f32, f32, f32)> {
         let mut stats = sys::az_match_stats::default();
         loop {
             self.check(unsafe { sys::az_match_step(self.raw, 256, &mut stats) })?;

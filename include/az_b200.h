@@ -283,6 +283,41 @@ typedef struct az_match_stats {   /* totals since az_match_begin */
  * n_concurrent > n_games plays on n_games slots.  The match uses the search buffers of az_search_vl (allocated by the first call of either), so a later
  * az_selfplay_begin* or az_search* call ends it; az_engine_create's footprint is unchanged. */
 int az_match_begin(az_engine* eng, int n_concurrent, uint32_t first_game, uint32_t n_games, const az_match_config* config);
+
+/* Mixed pairings: each player has its own kind and settings (evaluation.py's MctsPlayer, BasePlayer and RandomPlayer).  The match
+ * plays the games evaluation.py's `evaluate` plays for those players on this engine, bit for bit, as az_match_begin does for two
+ * equal players (az_match_begin is this call with two players of its kind and settings).  An MCTS player searches each of its
+ * plies with its own num_simulations S, leaves_per_root K and virtual_loss on its network slot; a BaseModel player takes its
+ * network's priors of the legal moves; both choose as az_match_begin describes.  A Random player plays
+ * index[int(u x count)] of az_movegen's legal moves (az_movegen order, under-promotions included), u = (mix(seed ^ 0x5151, game,
+ * ply) >> 11) x 2^-53 and the product in double, whatever the fullmove number.  A Random ply needs no network round: the slot
+ * plays it in the wave in which its root is set up and goes on with the next ply, so Random vs Random needs no weights and makes
+ * no evaluation.  A Random ply counts in az_match_stats.plies and in no evaluations[]. */
+#define AZ_PLAYER_MCTS 0         /* Player::MctsModel */
+#define AZ_PLAYER_BASE_MODEL 1   /* Player::BaseModel */
+#define AZ_PLAYER_RANDOM 2       /* Player::Random */
+typedef struct az_match_player {
+    int32_t kind;                  /* AZ_PLAYER_* */
+    uint8_t network;               /* MCTS and BaseModel: network slot (ignored for Random) */
+    int32_t num_simulations;       /* MCTS: 1 .. az_config.num_simulations (0: az_config.num_simulations) */
+    int32_t leaves_per_root;       /* MCTS: K >= 1 (1: az_search semantics) */
+    float virtual_loss;            /* MCTS: finite, >= 0 */
+} az_match_player;
+typedef struct az_match_players_config {
+    az_match_player player[2];     /* player 1 (White in even games) and player 2 */
+    uint32_t num_stochastic_moves; /* TEMPERATURE_ANNEALING (parameters.rs:31: 15) */
+    uint32_t max_plies;            /* >= 1 (450 in evaluation.py) */
+    uint64_t seed;
+} az_match_players_config;
+/* Errors (the engine stays usable): AZ_ERR_INVALID_ARGUMENT for an unknown kind (MiniMax included), a network id >=
+ * AZ_MAX_NETWORKS of an MCTS or BaseModel player, for an MCTS player's K < 1, negative or non-finite virtual_loss or
+ * num_simulations out of range, and for n_concurrent < 1, n_games = 0 or max_plies = 0.  AZ_ERR_NO_WEIGHTS for a network slot
+ * never loaded that an MCTS or BaseModel player uses (not under the synthetic evaluator).  AZ_ERR_CAPACITY when n_concurrent >
+ * az_config.max_games or the network ranges do not fit az_config.max_batch: each network used by a player gets
+ * round4(slots x K) boards, K the largest leaves_per_root of its players (1 for BaseModel), network 0's range from board 0 and
+ * network 1's right after it; a network no player uses reserves nothing.  AZ_ERR_STATE as az_match_begin, when a network is
+ * used.  az_match_step, az_match_stats and az_match_results serve both begin calls. */
+int az_match_begin_players(az_engine* eng, int n_concurrent, uint32_t first_game, uint32_t n_games, const az_match_players_config* config);
 /* AZ_ERR_STATE when no match is in progress; AZ_ERR_CAPACITY when a search pool overflowed (raise edge_capacity_per_node) */
 int az_match_step(az_engine* eng, int waves, az_match_stats* stats_out /* nullable */);
 /* per game of the last match begun, in game-index order: result from White's side (1, 0, -1), plies played, 1 if the game ended

@@ -295,6 +295,27 @@ struct EvaluationResult {       // what evaluate (validation.rs:155-282) returns
     float lossrate;             // player 2's wins
 };
 
+namespace detail {
+// steps the match begun until every game is over and scores it from player 1's side
+inline EvaluationResult match_outcome(Engine& e, uint32_t n_games, int waves_per_call) {
+    az_match_stats st{};
+    do e.check(az_match_step(e.handle(), waves_per_call, &st), "az_match_step");
+    while (st.active_games);
+    std::vector<int8_t> white(n_games);
+    std::vector<uint16_t> plies(n_games);
+    std::vector<uint8_t> finished(n_games);
+    e.check(az_match_results(e.handle(), white.data(), plies.data(), finished.data(), nullptr), "az_match_results");
+    float wins = 0.0f, draws = 0.0f;
+    for (uint32_t g = 0; g < n_games; g++) {
+        const int p1 = g % 2 == 0 ? white[g] : -white[g];   // validation.rs:196-200
+        wins += p1 == 1 ? 1.0f : 0.0f;
+        draws += p1 == 0 ? 1.0f : 0.0f;
+    }
+    const float n = (float)n_games;
+    return {(wins + draws / 2.0f) / n, draws / n, (n - wins - draws) / n};
+}
+}  // namespace detail
+
 // evaluate(model, network_1, network_2): n_games games between the model's network slots network_1 (player 1, White in even games)
 // and network_2, both Player::MctsModel with num_simulations (0: the config's), or both Player::BaseModel when base_model is set;
 // played resident on the device (az_match_*), move sampling keyed by (seed, game, ply).  leaves_per_root > 1 (NOT IN THE
@@ -320,21 +341,38 @@ inline EvaluationResult evaluate(AlphaZero& model, int network_1, int network_2,
         n_concurrent = std::min<int64_t>({(int64_t)n_games, (int64_t)e.config().max_games, (int64_t)((max_batch / 2) / 4 * 4 / k)});
     }
     e.check(az_match_begin(e.handle(), n_concurrent, 0, n_games, &c), "az_match_begin");
-    az_match_stats st{};
-    do e.check(az_match_step(e.handle(), waves_per_call, &st), "az_match_step");
-    while (st.active_games);
-    std::vector<int8_t> white(n_games);
-    std::vector<uint16_t> plies(n_games);
-    std::vector<uint8_t> finished(n_games);
-    e.check(az_match_results(e.handle(), white.data(), plies.data(), finished.data(), nullptr), "az_match_results");
-    float wins = 0.0f, draws = 0.0f;
-    for (uint32_t g = 0; g < n_games; g++) {
-        const int p1 = g % 2 == 0 ? white[g] : -white[g];   // validation.rs:196-200
-        wins += p1 == 1 ? 1.0f : 0.0f;
-        draws += p1 == 0 ? 1.0f : 0.0f;
+    return detail::match_outcome(e, n_games, waves_per_call);
+}
+
+// evaluate(model, player_1, player_2): n_games games between two independent players (az_match_begin_players), each MCTS (its own
+// network slot, num_simulations (0: the config's), leaves_per_root and virtual_loss), BaseModel (its own network slot) or Random
+// (AZ_PLAYER_*; Random uses no network), played resident on the device.  n_concurrent = 0 plays as many games at once as
+// max_games and the network ranges allow: each network a player uses holds round4(slots x K) boards, K the largest
+// leaves_per_root of its players (1 for BaseModel).  Otherwise as the overload above.
+inline EvaluationResult evaluate(AlphaZero& model, const az_match_player& player_1, const az_match_player& player_2, uint32_t n_games = 256,
+                                 uint32_t num_stochastic_moves = 15, uint64_t seed = 0, uint32_t max_plies = 450, int n_concurrent = 0,
+                                 int waves_per_call = 256) {
+    Engine& e = model.engine();
+    az_match_players_config c{};
+    c.player[0] = player_1;
+    c.player[1] = player_2;
+    c.num_stochastic_moves = num_stochastic_moves;
+    c.max_plies = max_plies;
+    c.seed = seed;
+    if (n_concurrent <= 0) {
+        int64_t k[2] = {0, 0};
+        for (const az_match_player& p : c.player) {
+            if (p.kind == AZ_PLAYER_RANDOM) continue;
+            const int s = p.network ? 1 : 0;
+            k[s] = std::max<int64_t>(k[s], p.kind == AZ_PLAYER_MCTS ? std::max(p.leaves_per_root, 1) : 1);
+        }
+        const int64_t max_batch = std::max(e.config().max_batch, e.config().max_games);
+        int64_t slots = std::min<int64_t>((int64_t)n_games, (int64_t)e.config().max_games);
+        while (slots > 1 && (slots * k[0] + 3) / 4 * 4 + (slots * k[1] + 3) / 4 * 4 > max_batch) slots--;
+        n_concurrent = (int)slots;
     }
-    const float n = (float)n_games;
-    return {(wins + draws / 2.0f) / n, draws / n, (n - wins - draws) / n};
+    e.check(az_match_begin_players(e.handle(), n_concurrent, 0, n_games, &c), "az_match_begin_players");
+    return detail::match_outcome(e, n_games, waves_per_call);
 }
 
 // ---- memory.rs ----------------------------------------------------------------------------------------------------
