@@ -69,7 +69,8 @@ class MatchStats(ctypes.Structure):
     """az_match_stats: totals since az_match_begin."""
 
     _fields_ = [("waves", ctypes.c_uint64), ("evaluations", ctypes.c_uint64 * 2)] + [
-        (n, ctypes.c_uint64) for n in ("leaves", "terminal_leaves", "collisions", "plies", "games_finished", "active_games")]
+        (n, ctypes.c_uint64) for n in ("leaves", "terminal_leaves", "collisions", "plies", "games_finished", "active_games")] + [
+        ("cache_hits", ctypes.c_uint64 * 2)]
 
 
 MATCH_MCTS, MATCH_BASE_MODEL = 0, 1
@@ -87,7 +88,7 @@ class MatchPlayersConfig(ctypes.Structure):
     """az_match_players_config."""
 
     _fields_ = [("player", MatchPlayer * 2), ("num_stochastic_moves", ctypes.c_uint32), ("max_plies", ctypes.c_uint32),
-                ("seed", ctypes.c_uint64)]
+                ("seed", ctypes.c_uint64), ("cache_log2", ctypes.c_int32)]
 
 
 def match_player(kind, network=0, num_simulations=None, leaves_per_root=1, virtual_loss=1.0):
@@ -422,10 +423,12 @@ class Engine:
         self._match_shape = (int(n_games), int(max_plies))
 
     def match_begin_players(self, n_concurrent, n_games, player_1, player_2, num_stochastic_moves=15, max_plies=450, seed=0,
-                            first_game=0):
+                            first_game=0, cache_log2=0):
         """A match between two independent players (az_match_begin_players), each a MatchPlayer (see match_player) or a dict of
         match_player's arguments: MCTS with its own network, num_simulations, leaves_per_root and virtual_loss, BaseModel with its
-        own network, or Random.  Otherwise as match_begin; match_step and match_results serve both."""
+        own network, or Random.  Otherwise as match_begin; match_step and match_results serve both.  cache_log2 in 1..26 gives
+        the match its own evaluation cache of 2^cache_log2 slots of 1 KiB: the same games with fewer boards sent to the networks
+        (MatchStats.cache_hits); 0 plays without one."""
         c = MatchPlayersConfig()
         for i, p in enumerate((player_1, player_2)):
             if isinstance(p, dict):
@@ -434,6 +437,7 @@ class Engine:
                 raise ValueError("a player is a MatchPlayer (match_player(...)) or a dict of match_player's arguments")
             c.player[i] = p
         c.num_stochastic_moves, c.max_plies, c.seed = int(num_stochastic_moves), int(max_plies), int(seed)
+        c.cache_log2 = int(cache_log2)
         self._check(self._L.az_match_begin_players(self._h, int(n_concurrent), ctypes.c_uint32(first_game), ctypes.c_uint32(n_games),
                                                    ctypes.byref(c)), "az_match_begin_players")
         self._match_shape = (int(n_games), int(max_plies))

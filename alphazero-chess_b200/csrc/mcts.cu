@@ -475,6 +475,24 @@ __device__ __forceinline__ void cache_insert(Ctx& x, u64 h, int node, float valu
     __syncwarp();
     if (x.lane == 0) atomicExch(&x.ptr.cache_state[target], (tag << 14) | (target_seq << 8) | (x.prm.cache_epoch << 2) | 2u);
 }
+// whole warp: on a hit for the key in sh->key the entry's priors fill the L edges from `off` and its value goes to `value`.  False
+// on a miss or when the entry was replaced while it was read: the position is then evaluated, which overwrites those edges.
+__device__ __forceinline__ bool cache_fetch(Ctx& x, size_t off, int L, float& value) {
+    uint32_t seen = 0;
+    const int slot = cache_lookup(x, fen_key_hash(x.sh->key), seen);
+    if (slot < 0) return false;
+    const CacheEntry* ce = &x.ptr.cache_entry[slot];
+    for (int e = x.lane; e < L; e += 32) x.ptr.edge_P[off + e] = __ldcg(&ce->prior[e]);
+    value = __ldcg(&ce->value);
+    return cache_validate(x, slot, seen);
+}
+// the key of a match's evaluation cache: the position's FEN identity with the network slot in bit 5 of meta, which fen_key_of
+// leaves 0, so that the compare and the hash both see it and the two networks never share an entry
+__device__ __forceinline__ DPos match_cache_key(const DPos& p, int network) {
+    DPos k = fen_key_of(p);
+    k.meta |= (u64)network << 5;
+    return k;
+}
 
 __device__ __forceinline__ void setup_root_from_shared(Ctx& x) {
     // fresh tree whose root is sh->child / sh->moves (priors are written by the caller)
@@ -1024,7 +1042,9 @@ __device__ __forceinline__ int vl_descend(Ctx& x, const VLPtrs& vl, uint2* path,
 
 // Backs up the root's previous batch (vl.count[g] leaves) in leaf order, so that the f32 additions on a shared edge happen in a
 // fixed order, and returns the number of leaves.  Without fused heads the evaluated leaves' priors are copied here first.
-__device__ __forceinline__ int vl_backup_batch(Ctx& x, const SearchParams& prm, const SearchPtrs& ptr, const VLPtrs& vl) {
+// CACHE (a match with its evaluation cache): every evaluated leaf is inserted under its position and `network`.
+template <bool CACHE = false>
+__device__ __forceinline__ int vl_backup_batch(Ctx& x, const SearchParams& prm, const SearchPtrs& ptr, const VLPtrs& vl, int network = 0) {
     const int nl = vl.count[x.g];
     for (int k = 0; k < nl; k++) {
         const int leaf = x.g * vl.K + k;
@@ -1033,6 +1053,13 @@ __device__ __forceinline__ int vl_backup_batch(Ctx& x, const SearchParams& prm, 
         if (s >= 0) {
             if (!prm.priors_scattered) copy_priors(ptr, ptr.req_edge_off[s], ptr.req_nedges[s], s, x.lane);
             value = ptr.res_value[s];
+            if constexpr (CACHE) {   // the leaf's node is the child of the last edge of its descent
+                const uint2 last = vl.path[(size_t)leaf * prm.node_cap + vl.len[leaf] - 1];
+                const int node = (int)(ptr.edge_link[x.ebase + last.y] & 0xFFFF);
+                if (x.lane == 0) x.sh->key = match_cache_key(ptr.node_pos[x.nbase + node], network);
+                __syncwarp();
+                cache_insert(x, fen_key_hash(x.sh->key), node, value);
+            }
         } else {
             value = vl.value[leaf];
         }
@@ -1107,9 +1134,13 @@ __global__ void __launch_bounds__(WARPS * 32) k_vl_gather(const __grid_constant_
     }
 }
 
-// one warp per gathered leaf (g * K + k): tree.rs expand; the new node is linked to the leaf edge and queued for evaluation
-template <bool ROUTE>
-__device__ __forceinline__ void vl_expand_body(const SearchParams& prm, const SearchPtrs& ptr, const VLPtrs& vl, const NetRoute& rt) {
+// one warp per gathered leaf (g * K + k): tree.rs expand; the new node is linked to the leaf edge and queued for evaluation.
+// CACHE (a match with its evaluation cache, ROUTE too): a leaf whose position and network are in the cache takes the entry's priors
+// and is recorded like a terminal leaf (slot -1, its value in vl.value), so that the backup keeps the leaf order; hits[s] counts
+// the hits on network s.
+template <bool ROUTE, bool CACHE = false>
+__device__ __forceinline__ void vl_expand_body(const SearchParams& prm, const SearchPtrs& ptr, const VLPtrs& vl, const NetRoute& rt,
+                                               unsigned long long* hits = nullptr) {
     __shared__ WarpShared shared[WARPS];
     const int leaf = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int g = leaf / vl.K;
@@ -1159,6 +1190,20 @@ __device__ __forceinline__ void vl_expand_body(const SearchParams& prm, const Se
         ptr.edge_link[pe] = x.new_link;
         atomicMax(&ptr.ctl[g].max_depth, (uint32_t)len);
     }
+    if constexpr (CACHE) {
+        const int s = rt.net[g];
+        if (x.lane == 0) x.sh->key = match_cache_key(x.sh->child, s);
+        __syncwarp();
+        float value;
+        if (cache_fetch(x, x.ebase + eoff, L, value)) {
+            if (x.lane == 0) {
+                vl.slot[leaf] = -1;
+                vl.value[leaf] = value;
+                atomicAdd(hits + s, 1ULL);
+            }
+            return;
+        }
+    }
     const int slot = submit_request<ROUTE>(x, child, &rt);
     if (x.lane == 0) vl.slot[leaf] = slot;
 }
@@ -1170,6 +1215,12 @@ __global__ void __launch_bounds__(WARPS * 32) k_vl_expand(const __grid_constant_
 __global__ void __launch_bounds__(WARPS * 32) k_vl_expand_nets(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
                                                                const __grid_constant__ VLPtrs vl, const __grid_constant__ NetRoute rt) {
     vl_expand_body<true>(prm, ptr, vl, rt);
+}
+// the same with the match's evaluation cache (prm / ptr carry the match's table); hits [AZ_MAX_NETWORKS]
+__global__ void __launch_bounds__(WARPS * 32) k_vl_expand_nets_cache(const __grid_constant__ SearchParams prm,
+                                                                     const __grid_constant__ SearchPtrs ptr, const __grid_constant__ VLPtrs vl,
+                                                                     const __grid_constant__ NetRoute rt, unsigned long long* hits) {
+    vl_expand_body<true, true>(prm, ptr, vl, rt, hits);
 }
 
 // Self-play with leaf-parallel search (az_selfplay_begin_vl), one warp per game slot: publish a parked game, back up the previous
@@ -1224,7 +1275,8 @@ struct MatchParams {
     unsigned long long seed;
     unsigned long long first_game, end_game;   // the match's game indices [first_game, end_game)
     unsigned long long* next_game;      // the next game index to start
-    unsigned long long* stats;          // [4] evaluations of network 0, of network 1, plies played, games ended
+    unsigned long long* stats;          // [6] evaluations of network 0, of network 1, plies played, games ended, cache hits of
+                                        //     network 0, of network 1
     uint8_t* net;                       // [slots] the network of each slot's mover (what NetRoute::net reads)
     int8_t* result;                     // [games] from White's side
     uint16_t* plies;                    // [games]
@@ -1272,14 +1324,32 @@ __device__ __forceinline__ int match_choose_random(Ctx& x, const MatchParams& mp
     return kept - 1;
 }
 
+__device__ __forceinline__ int match_choose(Ctx& x, const MatchParams& mp, const DPos& root);
+
 // The root of the slot's next ply from sh->child / sh->moves.  An MCTS or BaseModel mover queues its evaluation in the range of
 // its network and -1 is returned; a Random mover needs no evaluation: its edge is returned, to be played in this wave.
-__device__ __forceinline__ int match_root(Ctx& x, const MatchParams& mp, const NetRoute& rt, unsigned int* evals) {
+// CACHE: a root found in the cache takes the entry's priors instead (hits[s] counts it) and needs no network round: a BaseModel
+// mover's chosen edge is returned, an MCTS mover returns -1 with no evaluation pending and gathers its first batch in this wave.
+template <bool CACHE = false>
+__device__ __forceinline__ int match_root(Ctx& x, const MatchParams& mp, const NetRoute& rt, unsigned int* evals, const VLPtrs* vl = nullptr,
+                                          unsigned int* hits = nullptr) {
     setup_root_from_shared(x);
     const int p = match_mover(x.c.game_id, x.c.ply);
     if (mp.kind[p] == AZ_PLAYER_RANDOM) return match_choose_random(x, mp);
     const int s = mp.network[p];
     if (x.lane == 0) mp.net[x.g] = (uint8_t)s;
+    if constexpr (CACHE) {
+        const int L = (int)((x.c.flags >> 8) & 0xFF);
+        if (x.lane == 0) x.sh->key = match_cache_key(x.sh->child, s);
+        __syncwarp();
+        float value;
+        if (cache_fetch(x, x.ebase, L, value)) {   // no descent is in flight through a fresh root's edges
+            for (int e = x.lane; e < L; e += 32) vl->V[x.ebase + e] = 0;
+            __syncwarp();
+            hits[s]++;
+            return mp.kind[p] == AZ_PLAYER_BASE_MODEL ? match_choose(x, mp, x.ptr.node_pos[x.nbase]) : -1;
+        }
+    }
     x.c.pending_node = 0;
     x.c.pending_slot = submit_request<true>(x, 0, &rt);
     evals[s]++;
@@ -1287,7 +1357,9 @@ __device__ __forceinline__ int match_root(Ctx& x, const MatchParams& mp, const N
 }
 
 // The next unplayed game starts in this slot (as match_root, which returns), or the slot goes idle (-1)
-__device__ __forceinline__ int match_start_game(Ctx& x, const MatchParams& mp, const NetRoute& rt, unsigned int* evals) {
+template <bool CACHE = false>
+__device__ __forceinline__ int match_start_game(Ctx& x, const MatchParams& mp, const NetRoute& rt, unsigned int* evals,
+                                                const VLPtrs* vl = nullptr, unsigned int* hits = nullptr) {
     unsigned long long gid = 0;
     if (x.lane == 0) gid = atomicAdd(mp.next_game, 1ULL);
     gid = __shfl_sync(0xffffffffu, gid, 0);
@@ -1302,7 +1374,7 @@ __device__ __forceinline__ int match_start_game(Ctx& x, const MatchParams& mp, c
         x.ptr.hist[(size_t)x.g * HIST_CAP] = s;
     }
     __syncwarp();
-    return match_root(x, mp, rt, evals);
+    return match_root<CACHE>(x, mp, rt, evals, vl, hits);
 }
 
 // evaluation.py's move choice at the root: the weights are the visit counts over their f32 sum (_choose_from_visits) or the priors
@@ -1440,6 +1512,92 @@ __global__ void __launch_bounds__(WARPS * 32) k_match(const __grid_constant__ Se
     }
 }
 
+// k_match with the match's evaluation cache (prm / ptr carry the match's table): a root is looked up in match_root and takes the
+// entry's priors on a hit, every evaluated root and leaf is inserted when it is consumed, and k_vl_expand_nets_cache follows.  It is
+// k_match's body with those additions, kept apart so that k_match compiles as before: a body shared through an inline function
+// changes k_match's instruction schedule.
+__global__ void __launch_bounds__(WARPS * 32) k_match_cache(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
+                                                            const __grid_constant__ VLPtrs vl, const __grid_constant__ NetRoute rt,
+                                                            const __grid_constant__ MatchParams mp) {
+    __shared__ WarpShared shared[WARPS];
+    const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (g >= prm.n_games) return;
+    GameCtl c;
+    if (mp.first_wave) memset(&c, 0, sizeof c);
+    else c = ptr.ctl[g];
+    Ctx x = make_ctx(prm, ptr, &shared[threadIdx.x >> 5], g, c);
+    if (!mp.first_wave && x.c.status != 0) return;   // idle slot or pool overflow: vl.count[g] is already 0
+    unsigned int evals[AZ_MAX_NETWORKS] = {0, 0}, plies = 0, games = 0;
+    int n_leaf = 0, collided = 0;
+    int play = -1;   // the root edge the mover plays in this wave
+    unsigned int hits[AZ_MAX_NETWORKS] = {0, 0};
+    if (mp.first_wave) {
+        play = match_start_game<true>(x, mp, rt, evals, &vl, hits);
+    } else if (x.c.pending_node == 0) {   // MCTree::init: the root's priors (no noise), no descent in flight
+        const int L = (int)((x.c.flags >> 8) & 0xFF);
+        if (!prm.priors_scattered) copy_priors(ptr, x.ebase, L, x.c.pending_slot, x.lane);
+        for (int e = x.lane; e < L; e += 32) vl.V[x.ebase + e] = 0;
+        __syncwarp();
+        if (x.lane == 0) x.sh->key = match_cache_key(ptr.node_pos[x.nbase], mp.network[match_mover(x.c.game_id, x.c.ply)]);
+        __syncwarp();
+        cache_insert(x, fen_key_hash(x.sh->key), 0, ptr.res_value[x.c.pending_slot]);
+        x.c.pending_node = -1;
+        if (mp.kind[match_mover(x.c.game_id, x.c.ply)] == AZ_PLAYER_BASE_MODEL) play = match_choose(x, mp, ptr.node_pos[x.nbase]);
+    } else {
+        const int p = match_mover(x.c.game_id, x.c.ply);
+        const int nl = vl.count[g];
+        int evaluated = 0;   // leaves that went to the network (the others were terminal or cache hits)
+        for (int k0 = 0; k0 < nl; k0 += 32) {
+            const int k = k0 + x.lane;
+            evaluated += __popc(__ballot_sync(0xffffffffu, k < nl && vl.slot[g * vl.K + k] >= 0));
+        }
+        evals[mp.network[p]] += evaluated;
+        x.c.sims_done += vl_backup_batch<true>(x, prm, ptr, vl, mp.network[p]);
+        if ((int)x.c.sims_done >= mp.S[p]) play = match_choose(x, mp, ptr.node_pos[x.nbase]);
+    }
+    while (play >= 0) {
+        const DPos root = ptr.node_pos[x.nbase];
+        const uint32_t amv = ptr.edge_mv[x.ebase + play];
+        lane0_make_child(x, root, (uint16_t)(amv & 0xFFFF));
+        int term = x.sh->term;
+        if (term == 0 && draw_by_rules(x, ptr.path + (size_t)g * prm.node_cap, x.sh->child, 1)) term = 1;
+        const size_t gi = (size_t)(x.c.game_id - mp.first_game);
+        if (x.lane == 0 && x.c.ply < mp.row) mp.moves[gi * mp.row + x.c.ply] = (uint16_t)(amv >> 16);
+        plies++;
+        if (term != 0 || x.c.ply + 1 >= mp.max_plies) {
+            if (x.lane == 0) {   // term 2: the side to move in the child is mated, the mover won
+                mp.result[gi] = term == 2 ? (meta_turn(root.meta) == 0 ? 1 : -1) : 0;
+                mp.plies[gi] = (uint16_t)(x.c.ply + 1);
+                mp.finished[gi] = term != 0 ? 1 : 0;
+            }
+            games++;
+            play = match_start_game<true>(x, mp, rt, evals, &vl, hits);
+        } else {
+            if (x.lane == 0 && x.c.hist_len < HIST_CAP) ptr.hist[(size_t)g * HIST_CAP + x.c.hist_len] = x.sh->child;
+            x.c.hist_len = min(x.c.hist_len + 1, (uint32_t)HIST_CAP);
+            x.c.ply++;
+            play = match_root<true>(x, mp, rt, evals, &vl, hits);
+        }
+    }
+    if (x.c.status == 0 && x.c.pending_node < 0) {   // an MCTS root that still needs simulations
+        const int p = match_mover(x.c.game_id, x.c.ply);
+        VLPtrs v = vl;
+        v.lambda = mp.lambda[p];
+        unsigned int depth_sum = 0;
+        n_leaf = vl_gather_leaves(x, prm, v, min(mp.K[p], mp.S[p] - (int)x.c.sims_done), collided, depth_sum);
+    }
+    if (x.lane == 0) {
+        vl_publish(vl, g, n_leaf, collided);   // 0 when the slot moved, went idle or waits for its root: the next wave backs up nothing
+        if (evals[0]) atomicAdd(&mp.stats[0], (unsigned long long)evals[0]);
+        if (evals[1]) atomicAdd(&mp.stats[1], (unsigned long long)evals[1]);
+        if (plies) atomicAdd(&mp.stats[2], (unsigned long long)plies);
+        if (games) atomicAdd(&mp.stats[3], (unsigned long long)games);
+        if (hits[0]) atomicAdd(&mp.stats[4], (unsigned long long)hits[0]);
+        if (hits[1]) atomicAdd(&mp.stats[5], (unsigned long long)hits[1]);
+        ptr.ctl[g] = x.c;
+    }
+}
+
 // ------------------------------------------------------------------------------------------- host side
 template <class T>
 static int salloc(az_engine* e, SearchState* st, T** p, size_t n) {
@@ -1525,7 +1683,8 @@ void search_destroy(az_engine* e) {
     if (!st) return;
     for (void* p : st->allocs) cudaFree(p);
     const MatchState& m = st->match;
-    for (void* p : {(void*)m.result.p, (void*)m.plies.p, (void*)m.finished.p, (void*)m.moves.p}) cudaFree(p);
+    for (void* p : {(void*)m.result.p, (void*)m.plies.p, (void*)m.finished.p, (void*)m.moves.p, (void*)m.cache_state.p, (void*)m.cache_entry.p})
+        cudaFree(p);
     delete st;
     e->search = nullptr;
 }
@@ -1770,11 +1929,13 @@ static az_search_stats vl_search_stats(const unsigned long long s[4], uint64_t w
 }
 
 // the tail of a leaf-parallel wave after its gather kernel: k_vl_expand (k_vl_expand_nets into the networks' ranges when rt is
-// given) over n roots or slots, then the evaluation of the batch (a multi-network one when nb is given)
+// given, k_vl_expand_nets_cache when cache_hits is given too) over n roots or slots, then the evaluation of the batch (a
+// multi-network one when nb is given)
 static int vl_expand_evaluate(az_engine* e, SearchState* run, const VLPtrs& vl, int n, const NetRoute* rt = nullptr,
-                              const NetBatch* nb = nullptr) {
+                              const NetBatch* nb = nullptr, unsigned long long* cache_hits = nullptr) {
     const int blocks = (n * vl.K + WARPS - 1) / WARPS;
-    if (rt) k_vl_expand_nets<<<blocks, WARPS * 32, 0, e->stream>>>(run->prm, run->ptr, vl, *rt);
+    if (rt && cache_hits) k_vl_expand_nets_cache<<<blocks, WARPS * 32, 0, e->stream>>>(run->prm, run->ptr, vl, *rt, cache_hits);
+    else if (rt) k_vl_expand_nets<<<blocks, WARPS * 32, 0, e->stream>>>(run->prm, run->ptr, vl, *rt);
     else k_vl_expand<<<blocks, WARPS * 32, 0, e->stream>>>(run->prm, run->ptr, vl);
     AZ_CUDA(e, cudaGetLastError());
     return evaluate_batch(e, run, nb);
@@ -2005,7 +2166,7 @@ static int grow(az_engine* e, GrowBuf<T>& b, size_t n) {
 // the match's per-game results, reallocated when a match needs more room than the last one (freed by search_destroy)
 static int match_alloc(az_engine* e, SearchState* st, size_t games, size_t row) {
     MatchState& m = st->match;
-    if (!m.next && (salloc(e, st, &m.next, 1) || salloc(e, st, &m.stats, 4))) return AZ_ERR_OUT_OF_MEMORY;
+    if (!m.next && (salloc(e, st, &m.next, 1) || salloc(e, st, &m.stats, 6))) return AZ_ERR_OUT_OF_MEMORY;
     int r = grow(e, m.result, games);
     if (!r) r = grow(e, m.plies, games);
     if (!r) r = grow(e, m.finished, games);
@@ -2092,10 +2253,22 @@ static int match_start(az_engine* e, int n_concurrent, uint32_t first_game, uint
     if (r) return r;
     if (!st->d_net && salloc(e, st, &st->d_net, (size_t)st->G)) return AZ_ERR_OUT_OF_MEMORY;
     const uint32_t row = std::min<uint32_t>(cfg.max_plies, HIST_CAP);   // a game ends by the fullmove rule before HIST_CAP plies
-    r = match_alloc(e, st, n_games, row);
-    if (r) return r;
+    // the buffers of the previous match may be replaced from here on: it ends, and its results are no longer readable, also when an
+    // allocation below fails (a later az_match_step or az_match_results then returns AZ_ERR_STATE)
     st->session = Session::none;
     MatchState& m = st->match;
+    m.games = 0;
+    r = match_alloc(e, st, n_games, row);
+    if (r) return r;
+    const size_t cache_slots = cfg.cache_log2 > 0 ? (size_t)1 << cfg.cache_log2 : 0;
+    if (cache_slots) {
+        r = grow(e, m.cache_state, cache_slots);
+        if (!r) r = grow(e, m.cache_entry, cache_slots);
+        if (r) {
+            cudaGetLastError();   // a failed allocation must not be reported again by the next launch check
+            return r;
+        }
+    }
     m.cfg = cfg;
     m.first = first_game;
     m.games = n_games;
@@ -2106,6 +2279,9 @@ static int match_start(az_engine* e, int n_concurrent, uint32_t first_game, uint
     m.row = row;
     m.first_wave = 1;
     m.waves = 0;
+    m.epoch_waves = 1;
+    for (const az_match_player& q : cfg.player)
+        if (q.kind != AZ_PLAYER_RANDOM) m.epoch_waves = std::max(m.epoch_waves, (q.num_simulations + q.leaves_per_root - 1) / q.leaves_per_root);
     az_position_start(&m.startpos);
     st->prm.n_games = n; st->prm.S = std::max(cfg.player[0].num_simulations, cfg.player[1].num_simulations); st->prm.mode = 0;
     st->prm.priors_scattered = fused_heads(e) ? 1 : 0;
@@ -2113,7 +2289,8 @@ static int match_start(az_engine* e, int n_concurrent, uint32_t first_game, uint
     st->ptr.batch_zero = nullptr;
     const unsigned long long next = first_game;
     AZ_CUDA(e, cudaMemcpyAsync(m.next, &next, sizeof next, cudaMemcpyHostToDevice, e->stream));
-    AZ_CUDA(e, cudaMemsetAsync(m.stats, 0, 4 * sizeof(unsigned long long), e->stream));
+    AZ_CUDA(e, cudaMemsetAsync(m.stats, 0, 6 * sizeof(unsigned long long), e->stream));
+    if (cache_slots) AZ_CUDA(e, cudaMemsetAsync(m.cache_state.p, 0, cache_slots * sizeof(uint32_t), e->stream));   // a new cache per match
     if ((r = vl_clear(e, st, 0))) return r;   // k_match sets every slot's leaf count in the first wave
     AZ_CUDA(e, cudaMemsetAsync(m.result.p, 0, n_games, e->stream));
     AZ_CUDA(e, cudaMemsetAsync(m.plies.p, 0, (size_t)n_games * sizeof(uint16_t), e->stream));
@@ -2330,6 +2507,7 @@ int az_match_begin_players(az_engine* e, int n_concurrent, uint32_t first_game, 
         const int r = check_match_player(e, q);
         if (r) return r;
     }
+    if (pc.cache_log2 < 0 || pc.cache_log2 > 26) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "cache_log2 must be in 0 .. 26");
     if (n_concurrent < 1 || n_games == 0 || pc.max_plies == 0)
         return set_err(e, AZ_ERR_INVALID_ARGUMENT, "n_concurrent, n_games and max_plies must be positive");
     if (n_concurrent > e->search->G) return set_err(e, AZ_ERR_CAPACITY, "more slots than az_config.max_games");
@@ -2352,22 +2530,37 @@ int az_match_step(az_engine* e, int waves, az_match_stats* out) {
     const VLPtrs vl = vl_ptrs(st, m.K, 0.0f);
     const NetRoute route{st->d_net, st->batch_base, m.base1};
     const NetBatch nb{st->batch_base, m.base1, m.cap};
+    // with the match's evaluation cache the kernels run on a copy of the search state that carries the match's table
+    const bool cached = m.cfg.cache_log2 > 0 && m.evaluates;
+    SearchState run;
+    if (cached) {
+        run.prm = st->prm;
+        run.ptr = st->ptr;
+        run.prm.cache_mask = (uint32_t)(((size_t)1 << m.cfg.cache_log2) - 1);
+        run.ptr.cache_state = m.cache_state.p;
+        run.ptr.cache_entry = m.cache_entry.p;
+    }
     for (int w = 0; w < waves; w++) {
         const MatchParams mp = match_params(st);
         AZ_CUDA(e, cudaMemsetAsync(st->batch_base, 0, AZ_MAX_NETWORKS * sizeof(int), e->stream));   // both ranges start empty
         prof_mark_search(e);
         e->n_launches += m.evaluates ? 2 : 1;
-        k_match<<<(n + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr, vl, route, mp);
+        if (cached) {   // entries age by one epoch per ply-length of waves, as self-play's do per S waves
+            run.prm.cache_epoch = (uint32_t)((m.waves / (unsigned long long)m.epoch_waves) & 63);
+            k_match_cache<<<(n + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(run.prm, run.ptr, vl, route, mp);
+        } else {
+            k_match<<<(n + WARPS - 1) / WARPS, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr, vl, route, mp);
+        }
         AZ_CUDA(e, cudaGetLastError());
         if (m.evaluates) {   // Random vs Random: no slot ever waits for a network
-            const int r = vl_expand_evaluate(e, st, vl, n, &route, &nb);
+            const int r = cached ? vl_expand_evaluate(e, &run, vl, n, &route, &nb, m.stats + 4) : vl_expand_evaluate(e, st, vl, n, &route, &nb);
             if (r) return r;
         }
         m.first_wave = 0;
         m.waves++;
     }
     int flags[4] = {0, 0, 0, 0};
-    unsigned long long ms[4], vs[4];
+    unsigned long long ms[6], vs[4];
     const int r = enqueue_poll(e, *st, n, flags);
     if (r) return r;
     AZ_CUDA(e, cudaMemcpyAsync(ms, m.stats, sizeof ms, cudaMemcpyDeviceToHost, e->stream));
@@ -2379,6 +2572,7 @@ int az_match_step(az_engine* e, int waves, az_match_stats* out) {
         out->leaves = vs[0]; out->terminal_leaves = vs[1]; out->collisions = vs[2];
         out->plies = ms[2]; out->games_finished = ms[3];
         out->active_games = m.first_wave ? std::min<uint64_t>((uint64_t)n, m.games) : (uint64_t)flags[0];
+        out->cache_hits[0] = ms[4]; out->cache_hits[1] = ms[5];
     }
     if (flags[1]) return set_err(e, AZ_ERR_CAPACITY, "a per-game node/edge pool overflowed during the match (raise edge_capacity_per_node)");
     return AZ_OK;

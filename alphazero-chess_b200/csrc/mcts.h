@@ -145,11 +145,17 @@ struct MatchState {
     int first_wave = 0;                    // 1 until the first wave has run: every slot starts a game
     unsigned long long waves = 0;
     unsigned long long* next = nullptr;    // [1] next game index to start
-    unsigned long long* stats = nullptr;   // [4] evaluations of network 0, of network 1, plies, games ended
+    unsigned long long* stats = nullptr;   // [6] evaluations of network 0, of network 1, plies, games ended, cache hits of network 0,
+                                           //     of network 1
     GrowBuf<int8_t> result;                // [games]
     GrowBuf<uint16_t> plies;
     GrowBuf<uint8_t> finished;
     GrowBuf<uint16_t> moves;               // [games][row]
+    // the match's evaluation cache (cfg.cache_log2 > 0): its own table, emptied by every begin; the engine's self-play cache
+    // (SearchPtrs::cache_state / cache_entry) is not touched
+    GrowBuf<uint32_t> cache_state;         // [2^cache_log2]
+    GrowBuf<CacheEntry> cache_entry;
+    int epoch_waves = 1;                   // waves per cache epoch: the largest ceil(S / K) of the players (1 for BaseModel)
     az_match_players_config cfg{};         // num_simulations resolved (0: the engine's)
     az_position startpos{};
 };

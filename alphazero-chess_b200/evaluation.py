@@ -232,7 +232,7 @@ def _device_player(p):
 
 
 def evaluate_on_device(player_1, player_2, n_games=EVALUATION_GAMES, num_stochastic_moves=TEMPERATURE_ANNEALING, seed=0, max_plies=450,
-                       concurrent=None, waves_per_step=256):
+                       concurrent=None, waves_per_step=256, cache_log2=0):
     """evaluate() played resident on the device (Engine.match_begin_players / match_step / match_results): the same games, bit for
     bit, for any pairing of MctsPlayer, BasePlayer and RandomPlayer on one engine, without a host round trip per ply.  A
     RandomPlayer's engine is not used (it needs no network): the match runs on the other player's engine, or on player 1's for two
@@ -241,7 +241,8 @@ def evaluate_on_device(player_1, player_2, n_games=EVALUATION_GAMES, num_stochas
     max_batch).  All n_games run at once, as evaluate() plays them, only when the engine allows n_games slots; with fewer slots
     the games are the same but the match takes more network rounds, so size the engine accordingly.  Returns evaluate()'s dict
     plus `moves` [n_games, max_plies] (the policy indices played, MOVE_NONE after the last), `plies` [n_games] and `stats`
-    (MatchStats: waves, evaluations per network, ...).
+    (MatchStats: waves, evaluations per network, ...).  cache_log2 > 0 gives the match an evaluation cache of 2^cache_log2 slots
+    (Engine.match_begin_players): the same games, with stats.cache_hits boards per network not sent to the network.
     Raises ValueError for a MiniMaxPlayer (or any other player) and for two non-random players on different engines."""
     from . import PLAYER_RANDOM
 
@@ -265,7 +266,8 @@ def evaluate_on_device(player_1, player_2, n_games=EVALUATION_GAMES, num_stochas
         while concurrent > 1 and sum((concurrent * kk + 3) // 4 * 4 for kk in k) > max_batch:
             concurrent -= 1
     slots = min(int(concurrent), n_games)
-    eng.match_begin_players(slots, n_games, desc[0], desc[1], num_stochastic_moves=num_stochastic_moves, max_plies=max_plies, seed=seed)
+    eng.match_begin_players(slots, n_games, desc[0], desc[1], num_stochastic_moves=num_stochastic_moves, max_plies=max_plies, seed=seed,
+                            cache_log2=cache_log2)
     stats = eng.match_step(waves_per_step)
     while stats.active_games:
         stats = eng.match_step(waves_per_step)

@@ -30,12 +30,13 @@ pub struct az_config { pub device: i32, pub max_games: i32, pub max_batch: i32, 
 #[repr(C)] #[derive(Clone, Copy, Default)] pub struct az_match_player { pub kind: i32, pub network: u8, pub num_simulations: i32,
     pub leaves_per_root: i32, pub virtual_loss: f32 }                                            // AZ_PLAYER_MCTS / _BASE_MODEL / _RANDOM
 #[repr(C)] #[derive(Clone, Copy, Default)] pub struct az_match_players_config { pub player: [az_match_player; 2],
-    pub num_stochastic_moves: u32, pub max_plies: u32, pub seed: u64 }
+    pub num_stochastic_moves: u32, pub max_plies: u32, pub seed: u64, pub cache_log2: i32 }   // cache_log2: 0 none, 1..26
 pub const AZ_PLAYER_MCTS: i32 = 0;
 pub const AZ_PLAYER_BASE_MODEL: i32 = 1;
 pub const AZ_PLAYER_RANDOM: i32 = 2;
 #[repr(C)] #[derive(Default)] pub struct az_match_stats { pub waves: u64, pub evaluations: [u64; 2], pub leaves: u64,
-    pub terminal_leaves: u64, pub collisions: u64, pub plies: u64, pub games_finished: u64, pub active_games: u64 }
+    pub terminal_leaves: u64, pub collisions: u64, pub plies: u64, pub games_finished: u64, pub active_games: u64,
+    pub cache_hits: [u64; 2] }
 pub enum az_engine {}
 
 extern "C" {

@@ -145,11 +145,12 @@ impl Engine {
     /// evaluate (validation.rs:155-282) between two independent players, resident on the device (az_match_begin_players): each
     /// player is MCTS (its own network slot, simulations (0: the config's), leaves_per_root and virtual_loss), BaseModel (its own
     /// network slot) or Random (no network).  As many games run at once as max_games and the network ranges allow: each network a
-    /// player uses holds round4(slots x K) boards, K the largest leaves_per_root of its players (1 for BaseModel).  Returns
-    /// (winrate, drawrate, lossrate) from player 1's side.
+    /// player uses holds round4(slots x K) boards, K the largest leaves_per_root of its players (1 for BaseModel).  cache_log2 in
+    /// 1..26 gives the match an evaluation cache of 2^cache_log2 slots of 1 KiB (the same games, fewer network evaluations); 0
+    /// plays without one.  Returns (winrate, drawrate, lossrate) from player 1's side.
     pub fn evaluate_players(&mut self, player_1: sys::az_match_player, player_2: sys::az_match_player, n_games: u32,
-                            num_stochastic_moves: u32, seed: u64, max_plies: u32) -> Result<(f32, f32, f32)> {
-        let cfg = sys::az_match_players_config { player: [player_1, player_2], num_stochastic_moves, max_plies, seed };
+                            num_stochastic_moves: u32, seed: u64, max_plies: u32, cache_log2: i32) -> Result<(f32, f32, f32)> {
+        let cfg = sys::az_match_players_config { player: [player_1, player_2], num_stochastic_moves, max_plies, seed, cache_log2 };
         let mut k = [0i64; 2];
         for p in cfg.player.iter().filter(|p| p.kind != sys::AZ_PLAYER_RANDOM) {
             let pk = if p.kind == sys::AZ_PLAYER_MCTS { p.leaves_per_root.max(1) as i64 } else { 1 };

@@ -272,6 +272,9 @@ typedef struct az_match_stats {   /* totals since az_match_begin */
     uint64_t plies;                /* moves played */
     uint64_t games_finished;       /* games with a recorded result: ended by the rules or cut at max_plies */
     uint64_t active_games;         /* games in progress (0: the match is complete) */
+    uint64_t cache_hits[AZ_MAX_NETWORKS]; /* az_match_players_config.cache_log2 > 0: roots and leaves of each network taken from the
+                                             match's evaluation cache instead of the network (evaluations + cache_hits = the
+                                             evaluations of the same match without the cache) */
 } az_match_stats;
 /* Errors (the engine stays usable): AZ_ERR_INVALID_ARGUMENT for an unknown player_kind, a network id >= AZ_MAX_NETWORKS, and for
  * MCTS players K < 1, a negative or non-finite virtual_loss or num_simulations out of range; also for n_concurrent < 1, n_games
@@ -308,10 +311,20 @@ typedef struct az_match_players_config {
     uint32_t num_stochastic_moves; /* TEMPERATURE_ANNEALING (parameters.rs:31: 15) */
     uint32_t max_plies;            /* >= 1 (450 in evaluation.py) */
     uint64_t seed;
+    int32_t cache_log2;            /* 0: no evaluation cache.  1 .. 26: the match gets its own cache of 2^cache_log2 slots of 1 KiB
+                                      each (cache_log2 = 20: 1 GiB of device memory), allocated by the first match that needs it,
+                                      kept for later ones and emptied by every begin call */
 } az_match_players_config;
-/* Errors (the engine stays usable): AZ_ERR_INVALID_ARGUMENT for an unknown kind (MiniMax included), a network id >=
+/* The evaluation cache (cache_log2 > 0) is the one self-play uses (az_config.cache_log2, training.rs:342) with the network slot in
+ * its key: a root or leaf whose position (FEN identity: board, turn, castling, pseudo-legal ep, both move counters) was evaluated
+ * earlier in the match by the same network takes that evaluation's priors and value instead of a network round.  Network rows
+ * are batch-invariant, so the games, the moves and every search are those of the match without the cache, bit for bit; only the
+ * boards sent to the network drop, by az_match_stats.cache_hits.  Hit counts may differ between runs (slots race to insert
+ * within a wave); the games do not.  The engine's self-play cache is neither used nor changed.
+ * Errors (the engine stays usable): AZ_ERR_INVALID_ARGUMENT for an unknown kind (MiniMax included), a network id >=
  * AZ_MAX_NETWORKS of an MCTS or BaseModel player, for an MCTS player's K < 1, negative or non-finite virtual_loss or
- * num_simulations out of range, and for n_concurrent < 1, n_games = 0 or max_plies = 0.  AZ_ERR_NO_WEIGHTS for a network slot
+ * num_simulations out of range, for cache_log2 < 0 or > 26, and for n_concurrent < 1, n_games = 0 or max_plies = 0.
+ * AZ_ERR_OUT_OF_MEMORY when the cache cannot be allocated.  AZ_ERR_NO_WEIGHTS for a network slot
  * never loaded that an MCTS or BaseModel player uses (not under the synthetic evaluator).  AZ_ERR_CAPACITY when n_concurrent >
  * az_config.max_games or the network ranges do not fit az_config.max_batch: each network used by a player gets
  * round4(slots x K) boards, K the largest leaves_per_root of its players (1 for BaseModel), network 0's range from board 0 and
@@ -322,8 +335,9 @@ int az_match_begin_players(az_engine* eng, int n_concurrent, uint32_t first_game
 int az_match_step(az_engine* eng, int waves, az_match_stats* stats_out /* nullable */);
 /* per game of the last match begun, in game-index order: result from White's side (1, 0, -1), plies played, 1 if the game ended
  * by the rules (0: cut at max_plies, or still in progress), and moves_out [n_games][max_plies] the policy indices played
- * (AZ_MOVE_NONE after the last).  Readable until the next az_match_begin, also after a later search or self-play call ended the
- * match; AZ_ERR_STATE before the first az_match_begin. */
+ * (AZ_MOVE_NONE after the last).  Readable until the next az_match_begin* call that passes its argument checks (one that then
+ * fails to allocate leaves no match and no results), also after a later search or self-play call ended the match; AZ_ERR_STATE
+ * before the first az_match_begin. */
 int az_match_results(az_engine* eng, int8_t* result_out, uint16_t* plies_out, uint8_t* finished_out, uint16_t* moves_out /* nullable */);
 
 /* ---- memory.rs: ReplayBuffer (SURVEY section 8(f) #1, the consumer of self-play output) ---------------------------

@@ -348,10 +348,11 @@ inline EvaluationResult evaluate(AlphaZero& model, int network_1, int network_2,
 // network slot, num_simulations (0: the config's), leaves_per_root and virtual_loss), BaseModel (its own network slot) or Random
 // (AZ_PLAYER_*; Random uses no network), played resident on the device.  n_concurrent = 0 plays as many games at once as
 // max_games and the network ranges allow: each network a player uses holds round4(slots x K) boards, K the largest
-// leaves_per_root of its players (1 for BaseModel).  Otherwise as the overload above.
+// leaves_per_root of its players (1 for BaseModel).  cache_log2 in 1..26 gives the match an evaluation cache of 2^cache_log2
+// slots of 1 KiB (the same games, fewer network evaluations); 0 plays without one.  Otherwise as the overload above.
 inline EvaluationResult evaluate(AlphaZero& model, const az_match_player& player_1, const az_match_player& player_2, uint32_t n_games = 256,
                                  uint32_t num_stochastic_moves = 15, uint64_t seed = 0, uint32_t max_plies = 450, int n_concurrent = 0,
-                                 int waves_per_call = 256) {
+                                 int waves_per_call = 256, int cache_log2 = 0) {
     Engine& e = model.engine();
     az_match_players_config c{};
     c.player[0] = player_1;
@@ -359,6 +360,7 @@ inline EvaluationResult evaluate(AlphaZero& model, const az_match_player& player
     c.num_stochastic_moves = num_stochastic_moves;
     c.max_plies = max_plies;
     c.seed = seed;
+    c.cache_log2 = cache_log2;
     if (n_concurrent <= 0) {
         int64_t k[2] = {0, 0};
         for (const az_match_player& p : c.player) {
