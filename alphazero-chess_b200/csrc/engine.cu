@@ -117,7 +117,6 @@ int az_engine_create(const az_config* cfg, az_engine** out) {
         e->knobs.tower_split = std::max(0, env_int("AZ_TOWER_SPLIT", 0));
         e->knobs.tower_inkernel = env_int("AZ_TOWER_INKERNEL", 1);
         e->knobs.tc_release_arrive = env_int("AZ_TC_RELEASE_ARRIVE", 0);
-        e->knobs.adv_minb = env_int("AZ_ADV_MINB", 7);
         e->knobs.tower_grid = std::max(0, env_int("AZ_TOWER_GRID", 0));
         e->knobs.tower_wide = std::min(2, std::max(0, env_int("AZ_TOWER_WIDE", 2)));
         e->knobs.tower_l2hint = env_int("AZ_TOWER_L2HINT", 1) & 15;

@@ -73,7 +73,6 @@ struct az_engine {
         int tower_split = 0;       // AZ_TOWER_SPLIT (0: automatic)
         int tower_inkernel = 1;    // AZ_TOWER_INKERNEL
         int tc_release_arrive = 0; // AZ_TC_RELEASE_ARRIVE
-        int adv_minb = 7;          // AZ_ADV_MINB
         int tower_grid = 0;        // AZ_TOWER_GRID (0: every SM; the SM-partition experiment of profiles/)
         int tower_wide = 2;        // AZ_TOWER_WIDE: ONE TMA box per channel half serves the three horizontal taps of the tower; 2 (default) = 10-file boxes, three stages; 1 = 16-file boxes, two stages; 0 = one 8-file box per tap (round 1)
         int tower_l2hint = 1;      // AZ_TOWER_L2HINT (default 1): L2::evict_last on the tower's activation stores (1), residual loads (2), TMA loads (4)

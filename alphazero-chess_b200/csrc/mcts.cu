@@ -712,10 +712,15 @@ __device__ __noinline__ void root_noise_cold(const SearchParams* prm, const Sear
 #define ADV_T0() do { } while (0)
 #define ADV_T(k) do { } while (0)
 #endif
-// MINB = resident groups of four warps per SM the register allocation is bounded for: the kernel is a chain of dependent global loads
-// per game, so resident warps (latency hiding) are worth more than registers (AZ_ADV_MINB selects, see launch below)
-template <int MINB>
-__global__ void __launch_bounds__(WARPS * 32, MINB * 4 / WARPS) k_advance(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr) {
+// Resident groups of four warps per SM that k_advance's register allocation is bounded for.  The kernel is a chain of dependent
+// global loads per game, so resident warps (latency hiding) are worth more than registers: 3 groups -> 162 registers, 4 -> 128,
+// 5 -> 96, 6 -> 80, 7 -> 72 with 216 bytes of spills.  With 7, all 4096 games of a wave are resident at once (148 SMs x 28 warps)
+// and the kernel is one round of latency chains instead of two: measured per wave 4 -> 67.6 us, 5 -> 68.5, 6 -> 69.6, 7 -> 54.7.
+// The bound is the template argument of the one instance, so the kernel keeps its name k_advance<7> in SASS dumps and profiles.
+constexpr int ADV_GROUPS_PER_SM = 7;
+template <int GROUPS_PER_SM>
+__global__ void __launch_bounds__(WARPS * 32, GROUPS_PER_SM * 4 / WARPS) k_advance(const __grid_constant__ SearchParams prm,
+                                                                                    const __grid_constant__ SearchPtrs ptr) {
     __shared__ WarpShared shared[WARPS];
     const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (g >= prm.n_games) return;
@@ -724,7 +729,6 @@ __global__ void __launch_bounds__(WARPS * 32, MINB * 4 / WARPS) k_advance(const 
     Ctx x = make_ctx(prm, ptr, &shared[threadIdx.x >> 5], g, ptr.ctl[g]);
     if (g == 0 && x.lane == 0 && ptr.batch_zero) *ptr.batch_zero = 0;   // the other wave parity's request counter (see run_wave)
     if (x.c.status != 0 && x.c.status != 4) return;
-    if (!prm.consume && x.c.pending_node >= 0) return;   // extra pass: this game already waits for the network
 
     ADV_T0();
     // ---- 0. game over, samples staged: publish now if the host has drained the queue, else stay parked
@@ -735,10 +739,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB * 4 / WARPS) k_advance(const 
         const int node = x.c.pending_node, slot = x.c.pending_slot;
         const size_t off = x.ebase + ptr.node_edge_off[x.nbase + node];
         const int L = ptr.node_nedges[x.nbase + node];
-        if (!prm.priors_scattered) {
-            const float* pol = ptr.res_policy + (size_t)slot * AZ_ACTION_SPACE;
-            for (int e = x.lane; e < L; e += 32) ptr.edge_P[off + e] = pol[ptr.edge_mv[off + e] >> 16];
-        }
+        if (!prm.priors_scattered) copy_priors(ptr, off, L, slot, x.lane);
         __syncwarp();
         if (prm.cache_mask && prm.mode == 1) {  // cache.insert (training.rs:413)
             if (x.lane == 0) x.sh->key = fen_key_of(ptr.node_pos[x.nbase + node]);
@@ -1330,9 +1331,9 @@ __device__ __forceinline__ int match_choose(Ctx& x, const MatchParams& mp, const
 // its network and -1 is returned; a Random mover needs no evaluation: its edge is returned, to be played in this wave.
 // CACHE: a root found in the cache takes the entry's priors instead (hits[s] counts it) and needs no network round: a BaseModel
 // mover's chosen edge is returned, an MCTS mover returns -1 with no evaluation pending and gathers its first batch in this wave.
-template <bool CACHE = false>
-__device__ __forceinline__ int match_root(Ctx& x, const MatchParams& mp, const NetRoute& rt, unsigned int* evals, const VLPtrs* vl = nullptr,
-                                          unsigned int* hits = nullptr) {
+template <bool CACHE>
+__device__ __forceinline__ int match_root(Ctx& x, const MatchParams& mp, const NetRoute& rt, unsigned int* evals, const VLPtrs* vl,
+                                          unsigned int* hits) {
     setup_root_from_shared(x);
     const int p = match_mover(x.c.game_id, x.c.ply);
     if (mp.kind[p] == AZ_PLAYER_RANDOM) return match_choose_random(x, mp);
@@ -1357,9 +1358,9 @@ __device__ __forceinline__ int match_root(Ctx& x, const MatchParams& mp, const N
 }
 
 // The next unplayed game starts in this slot (as match_root, which returns), or the slot goes idle (-1)
-template <bool CACHE = false>
+template <bool CACHE>
 __device__ __forceinline__ int match_start_game(Ctx& x, const MatchParams& mp, const NetRoute& rt, unsigned int* evals,
-                                                const VLPtrs* vl = nullptr, unsigned int* hits = nullptr) {
+                                                const VLPtrs* vl, unsigned int* hits) {
     unsigned long long gid = 0;
     if (x.lane == 0) gid = atomicAdd(mp.next_game, 1ULL);
     gid = __shfl_sync(0xffffffffu, gid, 0);
@@ -1434,91 +1435,11 @@ __device__ __forceinline__ int match_choose(Ctx& x, const MatchParams& mp, const
 // mover's network range or record the game and start the next unplayed one.  A Random mover's ply is played as soon as its root is
 // set up, so a slot goes on playing until a root waits for a network.  Otherwise it gathers the next batch (up to the mover's K
 // leaves).  k_vl_expand_nets (leaves routed by mp.net) and the multi-network forward follow.
-__global__ void __launch_bounds__(WARPS * 32) k_match(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
-                                                      const __grid_constant__ VLPtrs vl, const __grid_constant__ NetRoute rt,
-                                                      const __grid_constant__ MatchParams mp) {
-    __shared__ WarpShared shared[WARPS];
-    const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (g >= prm.n_games) return;
-    GameCtl c;
-    if (mp.first_wave) memset(&c, 0, sizeof c);
-    else c = ptr.ctl[g];
-    // not make_ctx: built from this conditionally initialised c, it orders the prologue's zero-initialisations differently
-    Ctx x{prm, ptr, &shared[threadIdx.x >> 5], g, (int)(threadIdx.x & 31), (size_t)g * prm.node_cap, (size_t)g * prm.edge_cap, c,
-          0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-    if (!mp.first_wave && x.c.status != 0) return;   // idle slot or pool overflow: vl.count[g] is already 0
-    unsigned int evals[AZ_MAX_NETWORKS] = {0, 0}, plies = 0, games = 0;
-    int n_leaf = 0, collided = 0;
-    int play = -1;   // the root edge the mover plays in this wave
-    if (mp.first_wave) {
-        play = match_start_game(x, mp, rt, evals);
-    } else if (x.c.pending_node == 0) {   // MCTree::init: the root's priors (no noise), no descent in flight
-        const int L = (int)((x.c.flags >> 8) & 0xFF);
-        if (!prm.priors_scattered) copy_priors(ptr, x.ebase, L, x.c.pending_slot, x.lane);
-        for (int e = x.lane; e < L; e += 32) vl.V[x.ebase + e] = 0;
-        __syncwarp();
-        x.c.pending_node = -1;
-        if (mp.kind[match_mover(x.c.game_id, x.c.ply)] == AZ_PLAYER_BASE_MODEL) play = match_choose(x, mp, ptr.node_pos[x.nbase]);
-    } else {
-        const int p = match_mover(x.c.game_id, x.c.ply);
-        const int nl = vl.count[g];
-        int evaluated = 0;   // leaves that went to the network (the others were terminal)
-        for (int k0 = 0; k0 < nl; k0 += 32) {
-            const int k = k0 + x.lane;
-            evaluated += __popc(__ballot_sync(0xffffffffu, k < nl && vl.slot[g * vl.K + k] >= 0));
-        }
-        evals[mp.network[p]] += evaluated;
-        x.c.sims_done += vl_backup_batch(x, prm, ptr, vl);
-        if ((int)x.c.sims_done >= mp.S[p]) play = match_choose(x, mp, ptr.node_pos[x.nbase]);
-    }
-    while (play >= 0) {
-        const DPos root = ptr.node_pos[x.nbase];
-        const uint32_t amv = ptr.edge_mv[x.ebase + play];
-        lane0_make_child(x, root, (uint16_t)(amv & 0xFFFF));
-        int term = x.sh->term;
-        if (term == 0 && draw_by_rules(x, ptr.path + (size_t)g * prm.node_cap, x.sh->child, 1)) term = 1;
-        const size_t gi = (size_t)(x.c.game_id - mp.first_game);
-        if (x.lane == 0 && x.c.ply < mp.row) mp.moves[gi * mp.row + x.c.ply] = (uint16_t)(amv >> 16);
-        plies++;
-        if (term != 0 || x.c.ply + 1 >= mp.max_plies) {
-            if (x.lane == 0) {   // term 2: the side to move in the child is mated, the mover won
-                mp.result[gi] = term == 2 ? (meta_turn(root.meta) == 0 ? 1 : -1) : 0;
-                mp.plies[gi] = (uint16_t)(x.c.ply + 1);
-                mp.finished[gi] = term != 0 ? 1 : 0;
-            }
-            games++;
-            play = match_start_game(x, mp, rt, evals);
-        } else {
-            if (x.lane == 0 && x.c.hist_len < HIST_CAP) ptr.hist[(size_t)g * HIST_CAP + x.c.hist_len] = x.sh->child;
-            x.c.hist_len = min(x.c.hist_len + 1, (uint32_t)HIST_CAP);
-            x.c.ply++;
-            play = match_root(x, mp, rt, evals);
-        }
-    }
-    if (x.c.status == 0 && x.c.pending_node < 0) {   // an MCTS root that still needs simulations
-        const int p = match_mover(x.c.game_id, x.c.ply);
-        VLPtrs v = vl;
-        v.lambda = mp.lambda[p];
-        unsigned int depth_sum = 0;
-        n_leaf = vl_gather_leaves(x, prm, v, min(mp.K[p], mp.S[p] - (int)x.c.sims_done), collided, depth_sum);
-    }
-    if (x.lane == 0) {
-        vl_publish(vl, g, n_leaf, collided);   // 0 when the slot moved, went idle or waits for its root: the next wave backs up nothing
-        if (evals[0]) atomicAdd(&mp.stats[0], (unsigned long long)evals[0]);
-        if (evals[1]) atomicAdd(&mp.stats[1], (unsigned long long)evals[1]);
-        if (plies) atomicAdd(&mp.stats[2], (unsigned long long)plies);
-        if (games) atomicAdd(&mp.stats[3], (unsigned long long)games);
-        ptr.ctl[g] = x.c;
-    }
-}
-
-// k_match with the match's evaluation cache (prm / ptr carry the match's table): a root is looked up in match_root and takes the
-// entry's priors on a hit, every evaluated root and leaf is inserted when it is consumed, and k_vl_expand_nets_cache follows.  It is
-// k_match's body with those additions, kept apart so that k_match compiles as before: a body shared through an inline function
-// changes k_match's instruction schedule.
-__global__ void __launch_bounds__(WARPS * 32) k_match_cache(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
-                                                            const __grid_constant__ VLPtrs vl, const __grid_constant__ NetRoute rt,
-                                                            const __grid_constant__ MatchParams mp) {
+// CACHE (the match's evaluation cache; prm / ptr carry the match's table): a root is looked up in match_root and takes the entry's
+// priors on a hit, every evaluated root and leaf is inserted when it is consumed, and k_vl_expand_nets_cache follows.
+template <bool CACHE>
+__device__ __forceinline__ void match_wave(const SearchParams& prm, const SearchPtrs& ptr, const VLPtrs& vl, const NetRoute& rt,
+                                           const MatchParams& mp) {
     __shared__ WarpShared shared[WARPS];
     const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (g >= prm.n_games) return;
@@ -1527,20 +1448,21 @@ __global__ void __launch_bounds__(WARPS * 32) k_match_cache(const __grid_constan
     else c = ptr.ctl[g];
     Ctx x = make_ctx(prm, ptr, &shared[threadIdx.x >> 5], g, c);
     if (!mp.first_wave && x.c.status != 0) return;   // idle slot or pool overflow: vl.count[g] is already 0
-    unsigned int evals[AZ_MAX_NETWORKS] = {0, 0}, plies = 0, games = 0;
+    unsigned int evals[AZ_MAX_NETWORKS] = {0, 0}, hits[AZ_MAX_NETWORKS] = {0, 0}, plies = 0, games = 0;
     int n_leaf = 0, collided = 0;
     int play = -1;   // the root edge the mover plays in this wave
-    unsigned int hits[AZ_MAX_NETWORKS] = {0, 0};
     if (mp.first_wave) {
-        play = match_start_game<true>(x, mp, rt, evals, &vl, hits);
+        play = match_start_game<CACHE>(x, mp, rt, evals, &vl, hits);
     } else if (x.c.pending_node == 0) {   // MCTree::init: the root's priors (no noise), no descent in flight
         const int L = (int)((x.c.flags >> 8) & 0xFF);
         if (!prm.priors_scattered) copy_priors(ptr, x.ebase, L, x.c.pending_slot, x.lane);
         for (int e = x.lane; e < L; e += 32) vl.V[x.ebase + e] = 0;
         __syncwarp();
-        if (x.lane == 0) x.sh->key = match_cache_key(ptr.node_pos[x.nbase], mp.network[match_mover(x.c.game_id, x.c.ply)]);
-        __syncwarp();
-        cache_insert(x, fen_key_hash(x.sh->key), 0, ptr.res_value[x.c.pending_slot]);
+        if constexpr (CACHE) {
+            if (x.lane == 0) x.sh->key = match_cache_key(ptr.node_pos[x.nbase], mp.network[match_mover(x.c.game_id, x.c.ply)]);
+            __syncwarp();
+            cache_insert(x, fen_key_hash(x.sh->key), 0, ptr.res_value[x.c.pending_slot]);
+        }
         x.c.pending_node = -1;
         if (mp.kind[match_mover(x.c.game_id, x.c.ply)] == AZ_PLAYER_BASE_MODEL) play = match_choose(x, mp, ptr.node_pos[x.nbase]);
     } else {
@@ -1552,7 +1474,7 @@ __global__ void __launch_bounds__(WARPS * 32) k_match_cache(const __grid_constan
             evaluated += __popc(__ballot_sync(0xffffffffu, k < nl && vl.slot[g * vl.K + k] >= 0));
         }
         evals[mp.network[p]] += evaluated;
-        x.c.sims_done += vl_backup_batch<true>(x, prm, ptr, vl, mp.network[p]);
+        x.c.sims_done += vl_backup_batch<CACHE>(x, prm, ptr, vl, mp.network[p]);
         if ((int)x.c.sims_done >= mp.S[p]) play = match_choose(x, mp, ptr.node_pos[x.nbase]);
     }
     while (play >= 0) {
@@ -1571,12 +1493,12 @@ __global__ void __launch_bounds__(WARPS * 32) k_match_cache(const __grid_constan
                 mp.finished[gi] = term != 0 ? 1 : 0;
             }
             games++;
-            play = match_start_game<true>(x, mp, rt, evals, &vl, hits);
+            play = match_start_game<CACHE>(x, mp, rt, evals, &vl, hits);
         } else {
             if (x.lane == 0 && x.c.hist_len < HIST_CAP) ptr.hist[(size_t)g * HIST_CAP + x.c.hist_len] = x.sh->child;
             x.c.hist_len = min(x.c.hist_len + 1, (uint32_t)HIST_CAP);
             x.c.ply++;
-            play = match_root<true>(x, mp, rt, evals, &vl, hits);
+            play = match_root<CACHE>(x, mp, rt, evals, &vl, hits);
         }
     }
     if (x.c.status == 0 && x.c.pending_node < 0) {   // an MCTS root that still needs simulations
@@ -1592,10 +1514,24 @@ __global__ void __launch_bounds__(WARPS * 32) k_match_cache(const __grid_constan
         if (evals[1]) atomicAdd(&mp.stats[1], (unsigned long long)evals[1]);
         if (plies) atomicAdd(&mp.stats[2], (unsigned long long)plies);
         if (games) atomicAdd(&mp.stats[3], (unsigned long long)games);
-        if (hits[0]) atomicAdd(&mp.stats[4], (unsigned long long)hits[0]);
-        if (hits[1]) atomicAdd(&mp.stats[5], (unsigned long long)hits[1]);
+        if constexpr (CACHE) {
+            if (hits[0]) atomicAdd(&mp.stats[4], (unsigned long long)hits[0]);
+            if (hits[1]) atomicAdd(&mp.stats[5], (unsigned long long)hits[1]);
+        }
         ptr.ctl[g] = x.c;
     }
+}
+
+__global__ void __launch_bounds__(WARPS * 32) k_match(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
+                                                      const __grid_constant__ VLPtrs vl, const __grid_constant__ NetRoute rt,
+                                                      const __grid_constant__ MatchParams mp) {
+    match_wave<false>(prm, ptr, vl, rt, mp);
+}
+
+__global__ void __launch_bounds__(WARPS * 32) k_match_cache(const __grid_constant__ SearchParams prm, const __grid_constant__ SearchPtrs ptr,
+                                                            const __grid_constant__ VLPtrs vl, const __grid_constant__ NetRoute rt,
+                                                            const __grid_constant__ MatchParams mp) {
+    match_wave<true>(prm, ptr, vl, rt, mp);
 }
 
 // ------------------------------------------------------------------------------------------- host side
@@ -1632,8 +1568,7 @@ int search_create(az_engine* e) {
     // With the evaluation cache a hit completes a simulation without the network, so games may go further per wave.
     p.mode = 0; p.max_iters = c.cache_log2 > 0 ? 4 : 2;
     if (const char* v = getenv("AZ_ADV_MAX_ITERS")) p.max_iters = std::max(1, atoi(v));
-    p.last_game_id = 0; p.cache_epoch = 0; p.consume = 1;
-    if (const char* v = getenv("AZ_ADV_PASSES")) st->adv_passes = std::max(1, std::min(4, atoi(v)));
+    p.last_game_id = 0; p.cache_epoch = 0;
     if (!(c.temperature > 0.0f)) return set_err(e, AZ_ERR_INVALID_ARGUMENT, "temperature must be positive");
     p.inv_temperature = 1.0f / c.temperature;
     p.fp32_planes = c.precision == 1 ? 1 : 0;
@@ -1760,27 +1695,8 @@ static int run_wave(az_engine* e, SearchState* st) {
     st->ptr.batch_count = st->batch_base + st->batch_parity;
     st->ptr.batch_zero = st->batch_base + (st->batch_parity ^ 1);
     prof_mark_search(e);
-    // AZ_ADV_PASSES > 1 (experiment, default 1): extra k_advance passes per wave in which only the games that completed their
-    // max_iters network-free simulations without needing the network go on.  Measured at 14 % / 45 % / 63 % cache hits
-    // (profiles/r2_passes_raw.jsonl): always slower -- the fuller batch costs tower time in proportion, and more simulations
-    // per wave mean more games evaluating the same position in the same wave before anybody's result reaches the cache.
-    const int passes = st->prm.mode == 1 && st->prm.cache_mask ? st->adv_passes : 1;
-    for (int pass = 0; pass < passes; pass++) {
-    st->prm.consume = pass == 0 ? 1 : 0;
     e->n_launches++;
-    const int minb = e->knobs.adv_minb;
-    // groups of four warps per SM (register bound): 3 -> 162 registers, 4 -> 128, 5 -> 96, 6 -> 80, 7 -> 72 with 216 bytes of
-    // spills.  With 7, all 4096 games of a wave are resident at once (148 SMs x 28 warps) and the kernel is one round of
-    // latency chains instead of two: measured per wave 4 -> 67.6 us, 5 -> 68.5, 6 -> 69.6, 7 -> 54.7.
-    switch (minb) {
-        case 4: k_advance<4><<<blocks, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr); break;
-        case 5: k_advance<5><<<blocks, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr); break;
-        case 6: k_advance<6><<<blocks, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr); break;
-        case 7: k_advance<7><<<blocks, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr); break;
-        default: k_advance<3><<<blocks, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr); break;
-    }
-    }
-    st->prm.consume = 1;
+    k_advance<ADV_GROUPS_PER_SM><<<blocks, WARPS * 32, 0, e->stream>>>(st->prm, st->ptr);
     AZ_CUDA(e, cudaGetLastError());
     return evaluate_batch(e, st);
 }

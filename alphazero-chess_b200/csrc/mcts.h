@@ -25,7 +25,9 @@ struct __align__(16) GameCtl {
     uint32_t park_scale;    // f32 bits
 };
 
-struct SearchParams {
+// 16-byte aligned: the SearchPtrs after it in a kernel's parameters then start on a 16-byte boundary, where the compiler loads
+// pointer pairs with one 128-bit constant load
+struct __align__(16) SearchParams {
     int n_games;
     int S;
     float c_puct, alpha, eps;
@@ -43,8 +45,6 @@ struct SearchParams {
     unsigned long long last_game_id;  // self-play: game ids >= this are not started (0: games restart forever)
     float inv_temperature;            // 1 / TEMPERATURE as f32 (tree.rs:174)
     uint32_t cache_epoch;             // coarse clock (one tick per ply of self-play) used to age cache entries, 6 bits
-    int consume;                      // 1: first k_advance pass of a wave (evaluations of the previous wave are consumed);
-                                      // 0: an extra pass -- only games that still have no request in flight run
 };
 
 // Position -> (legal-move priors, value) cache: the moka Cache<Fen, CacheEntry> of training.rs:342 / tree.rs:214-218.
@@ -167,7 +167,6 @@ struct SearchState {
     Session session = Session::none;
     unsigned long long cache_evictions = 0;
     unsigned long long sum_search_depth = 0;
-    int adv_passes = 1;                    // k_advance launches per wave (AZ_ADV_PASSES, see run_wave)
     int* batch_base = nullptr;             // [8] ints: two alternating request counters, then four flag words
     int batch_parity = 0;
     unsigned long long wave_counter = 0;   // self-play waves since az_selfplay_begin (cache epoch = wave_counter / S)
